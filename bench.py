@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- Gibbs window-scores/s and site-updates/s on B200 (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config C2]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config C2] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A "step" = one pass of the hot path over one batch: `chains` independent restarts of
@@ -244,6 +244,30 @@ def run_reference_arm(args, cfg_name, cfg) -> None:
 # ---------------------------------------------------------------------------------------------------
 # GPU arm
 # ---------------------------------------------------------------------------------------------------
+DUMP_CHAIN_BYTES = 56 << 20   # per-chain arrays of --dump-outputs; with the winner's rows the dump stays under 64 MB
+
+
+def last_step_outputs(eng, best) -> dict:
+    """--dump-outputs: the results of the engine's last run_device, as float64 arrays (sites are exact in float64).
+    best_*: the restart loop's winner as gibbs_fetch_best returns it (its scores and sites, their sum, which restart;
+    restart -1 = the loop's initial value). chain_*: every restart's sites, scores and sum (gibbs_fetch), row i being
+    restart chain_index[i]. When all restarts would exceed DUMP_CHAIN_BYTES, a fixed sample of them (seed SEED, rows in
+    ascending order) is written instead, so two builds run with the same arguments write the same rows."""
+    import numpy as np
+
+    out = {"best_sites": best.sites, "best_scores": best.scores, "best_total": [best.total], "best_restart": [best.restart]}
+    out = {name: np.array(v, dtype=np.float64) for name, v in out.items()}     # copies: `best` may be a reused pinned buffer
+    res = eng.fetch(want_counts=False)
+    chains, n = res.sites.shape
+    rows = np.arange(chains)
+    keep = DUMP_CHAIN_BYTES // (8 * (2 * n + 2))
+    if chains > keep:
+        rows = np.sort(np.random.default_rng(SEED).choice(chains, size=keep, replace=False))
+    out.update({"chain_index": rows, "chain_sites": res.sites[rows], "chain_scores": res.scores[rows],
+                "chain_sums": res.sums[rows]})
+    return {name: np.asarray(v, dtype=np.float64) for name, v in out.items()}
+
+
 def run_gpu_arm(args, cfg_name, cfg) -> None:
     import numpy as np
     import torch
@@ -312,7 +336,7 @@ def run_gpu_arm(args, cfg_name, cfg) -> None:
 
     def timed_steps(e, prm, n_steps, seed0):
         """n_steps device-resident steps, each inside its own CUDA-event window on the launch stream (L2 flushed
-        before the window opens). Returns (sum of windows in ms, per-step stats)."""
+        before the window opens). Returns (per-step windows in ms, per-step stats, the last step's winner)."""
         ev = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(n_steps)]
         stats = []
         for s_ in range(n_steps):
@@ -320,8 +344,9 @@ def run_gpu_arm(args, cfg_name, cfg) -> None:
             ev[s_][0].record(stream)
             e.run_device(prm, chains, chain_id_base=chain_base, seed=seed0 + s_)
             ev[s_][1].record(stream)
-            stats.append(finish_step(e).stats)  # sync + D2H of the winner (not inside the event window)
-        return [a_.elapsed_time(b_) for a_, b_ in ev], stats
+            best_ = finish_step(e)              # sync + D2H of the winner (not inside the event window)
+            stats.append(best_.stats)
+        return [a_.elapsed_time(b_) for a_, b_ in ev], stats, best_
 
     sampler = None
     if rank == 0:                            # ONE nvidia-smi for all GPUs of the job, started early (it needs a moment)
@@ -337,10 +362,11 @@ def run_gpu_arm(args, cfg_name, cfg) -> None:
     barrier()
     clk_first = sampler.mark() if sampler else 0
     t_wall0 = time.perf_counter()
-    win_ms, step_stats = timed_steps(eng, params, args.steps, SEED)
+    win_ms, step_stats, last_best = timed_steps(eng, params, args.steps, SEED)
     barrier()
     t_wall = time.perf_counter() - t_wall0
     clk_last = sampler.mark() if sampler else 0
+    outputs = last_step_outputs(eng, last_best) if (args.dump_outputs and rank == 0) else None
     dev_ms = sum(win_ms)
     tot_windows = sum(st["window_scores"] for st in step_stats)
     tot_updates = sum(st["site_updates"] for st in step_stats)
@@ -402,7 +428,7 @@ def run_gpu_arm(args, cfg_name, cfg) -> None:
             prm = params_of(fam)
             eng.run_device(prm, chains, chain_id_base=chain_base, seed=SEED - 7)     # warm-up (tables, allocations)
             finish_step(eng)
-            ms, sts = timed_steps(eng, prm, 2, SEED + 50)
+            ms, sts, _ = timed_steps(eng, prm, args.steps, SEED + 50)
             w_ = sum(st["window_scores"] for st in sts)
             kms = sum(st["kernel_ms"] for st in sts) / len(sts)
             rate = w_ / (sum(ms) * 1e-3)
@@ -481,6 +507,10 @@ def run_gpu_arm(args, cfg_name, cfg) -> None:
             "clocks": clocks,
         }
         print(json.dumps(line), flush=True)
+    if outputs is not None:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, arr in outputs.items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), arr)
     eng.close()
     if world > 1:
         dist.destroy_process_group()
@@ -500,6 +530,8 @@ def main() -> None:
     ap.add_argument("--opt", action="append", default=[], metavar="NAME=VALUE",
                     help="gibbs_set_option switch for A/B measurements, e.g. --opt coop=0 (include/gibbs_b200.h, GIBBS_OPT_*)")
     ap.add_argument("--no-families", action="store_true", help="skip the short runs of the other reference families")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last device-timed step computed to DIR/<name>.npy (float64), see last_step_outputs")
     args = ap.parse_args()
     cfg = CONFIGS[args.config]
     if args.impl == "reference":
