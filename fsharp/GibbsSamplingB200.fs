@@ -99,6 +99,18 @@ module Native =
                                 int& restartOut, int[] countsOut, GibbsRunStats& stats)
     [<DllImport(Lib, CallingConvention = CallingConvention.Cdecl)>]
     extern int gibbs_fetch_best_positions(IntPtr handle, int m, int[] positionsOut)
+    // many sequence sets in one batch (include/gibbs_b200.h, gibbs_batch_*)
+    [<DllImport(Lib, CallingConvention = CallingConvention.Cdecl)>]
+    extern int gibbs_batch_create(byte[] seqs, int64[] offsets, int[] setOffsets, int nSets, int device, IntPtr& batch)
+    [<DllImport(Lib, CallingConvention = CallingConvention.Cdecl)>]
+    extern int gibbs_batch_destroy(IntPtr batch)
+    [<DllImport(Lib, CallingConvention = CallingConvention.Cdecl)>]
+    extern int gibbs_batch_run_device(IntPtr batch, GibbsParams& p, float[] bgPerSetOrNull, int restartsPerSet, int64 chainIdBase, uint64 seed)
+    [<DllImport(Lib, CallingConvention = CallingConvention.Cdecl)>]
+    extern int gibbs_batch_fetch(IntPtr batch, int[] sitesOut, float[] scoresOut, float[] sumsOut, GibbsRunStats& stats)
+    [<DllImport(Lib, CallingConvention = CallingConvention.Cdecl)>]
+    extern int gibbs_batch_fetch_best(IntPtr batch, int repetitions, int[] sitesOut, float[] scoresOut, int[] nOut, float[] sumOut,
+                                      int[] restartOut, int[] countsOut, GibbsRunStats& stats)
 
     /// status code -> the exception the reference would have thrown (SURVEY.md section 8b)
     let check (rc:int) =
@@ -194,6 +206,31 @@ module Native =
         finally
             gibbs_multi_destroy m |> ignore
 
+    /// The restart loops of many sets in one batch on GPU 0: set s gets exactly what bestOfRestarts-style single-set calls
+    /// with the same seed give (restart r of every set draws from the stream (seed, r)); only the winners are copied back.
+    let bestOfRestartsOfSets (numberOfRepetitions:int) (seed:uint64) k pc alphabet (sets:BioArray.BioArray<#IBioItem>[][])
+                             (pcvs:CompositeVector.ProbabilityCompositeVector[] option) : (float*int)[][] =
+        let all = Array.concat sets
+        let buf, offsets = flatten all
+        let setOffsets = Array.zeroCreate<int> (sets.Length + 1)
+        sets |> Array.iteri (fun s src -> setOffsets.[s + 1] <- setOffsets.[s] + src.Length)
+        let mutable b = IntPtr.Zero
+        check (gibbs_batch_create(buf, offsets, setOffsets, sets.Length, 0, &b))
+        try
+            let mutable p = makeParams k pc alphabet (pcvs |> Option.map (fun v -> v.[0])) 0
+            let bg =
+                match pcvs with
+                | Some v -> v |> Array.collect (fun pcv -> [| for c in "ACGT" -> pcv.Array.[int c - 42] |])
+                | None -> null
+            check (gibbs_batch_run_device(b, &p, bg, numberOfRepetitions + 1, 0L, seed))
+            let sites, scores = Array.zeroCreate all.Length, Array.zeroCreate all.Length
+            let nOut = Array.zeroCreate sets.Length
+            let mutable stats = GibbsRunStats()
+            check (gibbs_batch_fetch_best(b, numberOfRepetitions, sites, scores, nOut, null, null, null, &stats))
+            Array.init sets.Length (fun s -> Array.init nOut.[s] (fun i -> scores.[setOffsets.[s] + i], sites.[setOffsets.[s] + i]))
+        finally
+            gibbs_batch_destroy b |> ignore
+
 open CompositeVector
 
 module SiteSampler =
@@ -221,6 +258,10 @@ module SiteSampler =
     let getMotifsWithBestInformationContentWithBPV (numberOfRepetitions:int) motifLength pseudoCount alphabet sources (pcv:ProbabilityCompositeVector) =
         Native.bestOfRestarts None numberOfRepetitions (seedOf None) motifLength pseudoCount alphabet sources (Some pcv)
 
+    /// getMotifsWithBestInformationContentWithBPV of every set (pcvs.[s] the background of sets.[s]) in one GPU batch
+    let getMotifsWithBestInformationContentWithBPVOfSets (numberOfRepetitions:int) motifLength pseudoCount alphabet sets (pcvs:ProbabilityCompositeVector[]) =
+        Native.bestOfRestartsOfSets numberOfRepetitions (seedOf None) motifLength pseudoCount alphabet sets (Some pcvs)
+
     // ---- data-derived background (fs:462-640, fs:697): background = 1, no pcv ---------------------------------
     /// fs:697-701
     let doSiteSampling motifLength pseudoCount alphabet sources =
@@ -234,6 +275,9 @@ module SiteSampler =
     /// fs:615-640 -- the script's live call (fsx:384)
     let getMotifsWithBestInformationContent (numberOfRepetitions:int) motifLength pseudoCount alphabet sources =
         Native.bestOfRestarts None numberOfRepetitions (seedOf None) motifLength pseudoCount alphabet sources None
+    /// getMotifsWithBestInformationContent of every set in one GPU batch
+    let getMotifsWithBestInformationContentOfSets (numberOfRepetitions:int) motifLength pseudoCount alphabet sets =
+        Native.bestOfRestartsOfSets numberOfRepetitions (seedOf None) motifLength pseudoCount alphabet sets None
     /// fs:664-689
     let getBestInformationContentOfPPM (numberOfRepetitions:int) motifLength pseudoCount alphabet sources (ppM:PositionMatrix.PositionProbabilityMatrix) =
         Native.bestOfRestarts (Some ppM) numberOfRepetitions (seedOf None) motifLength pseudoCount alphabet sources None

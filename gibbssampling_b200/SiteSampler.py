@@ -17,7 +17,7 @@ import numpy as np
 
 from . import _abi
 from .CompositeVector import ProbabilityCompositeVector
-from .engine import GibbsEngine, make_params, symbol_code
+from .engine import BatchEngine, GibbsEngine, make_params, symbol_code
 
 SiteArray = list  # (float*int)[]
 
@@ -278,3 +278,42 @@ def getBestInformationContentOfPPM(numberOfRepetitions, motifLength, pseudoCount
         raise _abi.GibbsArgumentError(_abi.GIBBS_ERR_ARG, "positionProbabilityMatrix is null (ArgumentNullException)")
     return _restart_loop(numberOfRepetitions, motifLength, pseudoCount, alphabet, sources, None,
                          ppM=positionProbabilityMatrix, **kw)
+
+
+# ---- many sets in one batch (gibbs_batch_*): one result per set, element s = the single-set function on sets[s] ------
+def _restart_loop_of_sets(numberOfRepetitions, motifLength, pseudoCount, alphabet, sets, pcvs, *, seed: int = 0,
+                          chain: int = 0, max_sweeps: int = 0, engine: Optional[BatchEngine] = None) -> list:
+    if sets is not None:
+        sets = list(sets)   # (a generator is read once)
+    if pcvs is None:
+        params = _params(0, motifLength, pseudoCount, alphabet, None, max_sweeps)
+        bg = None
+    else:
+        pcvs = list(pcvs)
+        if sets is not None and engine is None and len(pcvs) != len(sets):
+            raise _abi.GibbsArgumentError(_abi.GIBBS_ERR_ARG, f"{len(pcvs)} pcvs for {len(sets)} sets")
+        bg = [_bg_of(alphabet, pcv) for pcv in pcvs]
+        params = make_params(motifLength, pseudoCount, len(alphabet), bg[0] if bg else [0.25] * 4, max_sweeps=max_sweeps)
+    eng = engine if engine is not None else BatchEngine(sets)
+    try:
+        eng.run_device(params, max(int(numberOfRepetitions) + 1, 1), bg_per_set=bg, chain_id_base=chain, seed=seed)
+        return [_to_site_array(b.scores, b.sites) for b in eng.fetch_best(int(numberOfRepetitions))]
+    finally:
+        if engine is None:
+            eng.close()
+
+
+def getMotifsWithBestInformationContentWithBPVOfSets(numberOfRepetitions, motifLength, pseudoCount, alphabet, sets, pcvs,
+                                                     **kw) -> list:
+    """getMotifsWithBestInformationContentWithBPV (fs:434-459) of every set, pcvs[s] the background of sets[s]; the restarts
+    of all sets run in one batch. Element s equals getMotifsWithBestInformationContentWithBPV(..., sets[s], pcvs[s]) with
+    the same seed / chain."""
+    if pcvs is None:
+        raise _abi.GibbsArgumentError(_abi.GIBBS_ERR_ARG, "pcvs is null (ArgumentNullException)")
+    return _restart_loop_of_sets(numberOfRepetitions, motifLength, pseudoCount, alphabet, sets, pcvs, **kw)
+
+
+def getMotifsWithBestInformationContentOfSets(numberOfRepetitions, motifLength, pseudoCount, alphabet, sets, **kw) -> list:
+    """getMotifsWithBestInformationContent (fs:615-640) of every set, in one batch; element s equals
+    getMotifsWithBestInformationContent(..., sets[s]) with the same seed / chain."""
+    return _restart_loop_of_sets(numberOfRepetitions, motifLength, pseudoCount, alphabet, sets, None, **kw)

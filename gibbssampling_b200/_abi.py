@@ -40,6 +40,7 @@ EXPORTS = [
     "gibbs_set_start_motif_state",
     "gibbs_multi_create", "gibbs_multi_destroy", "gibbs_multi_num_devices", "gibbs_multi_handle",
     "gibbs_multi_run_device", "gibbs_multi_fetch_best",
+    "gibbs_batch_create", "gibbs_batch_destroy", "gibbs_batch_run_device", "gibbs_batch_fetch", "gibbs_batch_fetch_best",
 ]
 GIBBS_OPT_INIT_PATH, GIBBS_OPT_EXACT_SCANS, GIBBS_OPT_STAGE2_AT, GIBBS_OPT_STAGE3_AT, GIBBS_OPT_CLUSTER, GIBBS_OPT_MIN_WIDTH = 1, 2, 3, 4, 5, 6
 GIBBS_OPT_TILE_ROWS = 7
@@ -176,6 +177,11 @@ def load() -> C.CDLL:
     lib.gibbs_multi_handle.argtypes = [vp, i32]
     lib.gibbs_multi_run_device.argtypes = [vp, P(Params), i32, i64, u64, i32, P(f64), i64]
     lib.gibbs_multi_fetch_best.argtypes = [vp, i32, P(i32), P(f64), P(i32), P(f64), P(i32), P(i32), P(RunStats)]
+    lib.gibbs_batch_create.argtypes = [P(C.c_uint8), P(i64), P(i32), i32, i32, P(vp)]
+    lib.gibbs_batch_destroy.argtypes = [vp]
+    lib.gibbs_batch_run_device.argtypes = [vp, P(Params), P(f64), i32, i64, u64]
+    lib.gibbs_batch_fetch.argtypes = [vp, P(i32), P(f64), P(f64), P(RunStats)]
+    lib.gibbs_batch_fetch_best.argtypes = [vp, i32, P(i32), P(f64), P(i32), P(f64), P(i32), P(i32), P(RunStats)]
     for name in EXPORTS:
         fn = getattr(lib, name)
         if name not in ("gibbs_last_error", "gibbs_multi_handle"):

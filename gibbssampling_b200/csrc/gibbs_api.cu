@@ -9,6 +9,7 @@
 #include "gibbs_motif.cuh"
 #include "gibbs_motif2.cuh"
 #include "gibbs_drift.cuh"
+#include "gibbs_batch.cuh"
 
 #include <algorithm>
 #include <cmath>
@@ -58,6 +59,17 @@ cudaError_t launch_chain_cluster4(const ChainArgs &a, int n_clusters, cudaStream
 cudaError_t launch_chain_cluster8(const ChainArgs &a, int n_clusters, cudaStream_t stream, int *capacity_out);
 size_t launch_chain_cluster4_smem(int n, int row_words);
 size_t launch_chain_cluster8_smem(int n, int row_words);
+// gibbs_batch_tu.cu: chain_batch_kernel, one unit per (random starts only, masked symbols, drifting background, warps per chain)
+#define GIBBS_BATCH_TU(name) cudaError_t name(const ChainArgs &run, const BatchTable &bt, int grid, int smem, cudaStream_t stream)
+GIBBS_BATCH_TU(launch_batch_t4); GIBBS_BATCH_TU(launch_batch_t1);
+GIBBS_BATCH_TU(launch_batch_drift_t4); GIBBS_BATCH_TU(launch_batch_drift_t1);
+GIBBS_BATCH_TU(launch_batch_masked_t4); GIBBS_BATCH_TU(launch_batch_masked_t1);
+GIBBS_BATCH_TU(launch_batch_masked_drift_t4); GIBBS_BATCH_TU(launch_batch_masked_drift_t1);
+GIBBS_BATCH_TU(launch_batch_init_t4); GIBBS_BATCH_TU(launch_batch_init_t1);
+GIBBS_BATCH_TU(launch_batch_init_drift_t4); GIBBS_BATCH_TU(launch_batch_init_drift_t1);
+GIBBS_BATCH_TU(launch_batch_init_masked_t4); GIBBS_BATCH_TU(launch_batch_init_masked_t1);
+GIBBS_BATCH_TU(launch_batch_init_masked_drift_t4); GIBBS_BATCH_TU(launch_batch_init_masked_drift_t1);
+#undef GIBBS_BATCH_TU
 }
 
 using namespace gibbs;
@@ -255,12 +267,21 @@ int32_t ensure_wtab(gibbs_handle *h, const gibbs_params *p, int *launches, int s
 
 // The fixed-point ranking pass is valid when no partial product of k table entries can leave the
 // normal float64 range (and so the int32 key cannot overflow): |k * extreme log2| < 1000.
-int fast_path_ok(const gibbs_handle *h, int k) {
-    if (h->wt_abnormal) return 0;
+int fast_path_ok_range(int abnormal, int wt_min, int wt_max, int k) {
+    if (abnormal) return 0;
     const double unit = 1.0 / (double)(1 << LG_FRAC_BITS);
-    const double lo = (double)k * (h->wt_min < 0 ? h->wt_min : 0) * unit;
-    const double hi = (double)k * (h->wt_max > 0 ? h->wt_max : 0) * unit;
+    const double lo = (double)k * (wt_min < 0 ? wt_min : 0) * unit;
+    const double hi = (double)k * (wt_max > 0 ? wt_max : 0) * unit;
     return (lo > -1000.0 && hi < 1000.0) ? 1 : 0;
+}
+int fast_path_ok(const gibbs_handle *h, int k) { return fast_path_ok_range(h->wt_abnormal, h->wt_min, h->wt_max, k); }
+
+// the ranking pass of the drifting background (see gibbs_run_device): every odds ratio lies in [pc / den, den / pc]
+int drift_fast_path_ok(const int32_t gcnt[4], int32_t max_len, int32_t n, const gibbs_params *p) {
+    const double alpha_pc = (double)p->alphabet_size * p->pseudocount;
+    const double bases = (double)gcnt[0] + gcnt[1] + gcnt[2] + gcnt[3] + (double)max_len;
+    const double den = (bases > (double)n ? bases : (double)n) + alpha_pc;
+    return (p->pseudocount >= 1e-30 && (double)p->k * log2(den / p->pseudocount) < 1000.0) ? 1 : 0;
 }
 
 template <typename K>
@@ -609,14 +630,9 @@ int32_t ensure_bgtab(gibbs_handle *h, const gibbs_params *p, int *launches) {
     return GIBBS_OK;
 }
 
-int32_t ensure_drift(gibbs_handle *h, const gibbs_params *p, int *launches, int span_mult = 1) {
-    const int span = h->n * span_mult;
-    if (h->drift_valid && h->drift_pc == p->pseudocount && h->drift_alen == p->alphabet_size && h->drift_span >= span) return GIBBS_OK;
-    CUDA_TRY(h->pvals.reserve((size_t)span));
+// per sequence (any background parameters): A,C,G,T counts, symbols outside A,C,G,T, prefix tables of the ranking pass
+int32_t ensure_seq_counts(gibbs_handle *h, int *launches) {
     CUDA_TRY(h->basecnt.reserve((size_t)h->n * 4));
-    const double den = (double)(h->n - 1) + ((double)p->alphabet_size * p->pseudocount); // fs:257
-    pvals_kernel<<<(span + 255) / 256, 256, 0, h->stream>>>(span, p->pseudocount, den, h->pvals.p);
-    CUDA_TRY(cudaGetLastError());
     CUDA_TRY(h->maskcnt.reserve((size_t)h->n));
     basecount_kernel<<<(h->n + 127) / 128, 128, 0, h->stream>>>(dev_seqs(h), h->basecnt.p, h->maskcnt.p);
     CUDA_TRY(cudaGetLastError());
@@ -634,7 +650,20 @@ int32_t ensure_drift(gibbs_handle *h, const gibbs_params *p, int *launches, int 
         }
     }
     CUDA_TRY(cudaGetLastError());
-    if (launches) *launches += 2;
+    if (launches) *launches += 1;
+    return GIBBS_OK;
+}
+
+int32_t ensure_drift(gibbs_handle *h, const gibbs_params *p, int *launches, int span_mult = 1) {
+    const int span = h->n * span_mult;
+    if (h->drift_valid && h->drift_pc == p->pseudocount && h->drift_alen == p->alphabet_size && h->drift_span >= span) return GIBBS_OK;
+    CUDA_TRY(h->pvals.reserve((size_t)span));
+    const double den = (double)(h->n - 1) + ((double)p->alphabet_size * p->pseudocount); // fs:257
+    pvals_kernel<<<(span + 255) / 256, 256, 0, h->stream>>>(span, p->pseudocount, den, h->pvals.p);
+    CUDA_TRY(cudaGetLastError());
+    if (launches) *launches += 1;
+    int32_t rc = ensure_seq_counts(h, launches);
+    if (rc) return rc;
     std::vector<int32_t> bc((size_t)h->n * 4);
     CUDA_TRY(cudaMemcpyAsync(bc.data(), h->basecnt.p, bc.size() * sizeof(int32_t), cudaMemcpyDeviceToHost, h->stream));
     CUDA_TRY(cudaStreamSynchronize(h->stream));
@@ -1287,9 +1316,7 @@ int32_t gibbs_run_device(gibbs_handle *h, const gibbs_params *p, int32_t n_chain
         {   // Ranking pass allowed? Every odds ratio ppm / pcv lies in [pc / den, den / pc] with den <= all bases of the
             // set + one more sequence + |A| pc (or N - 1 + |A| pc): no float64 product of k of them may leave the
             // normal range (|log2| < 1000), and pc >= 1e-30 keeps every float32 logarithm argument normal and finite.
-            const double bases = (double)h->gcnt[0] + h->gcnt[1] + h->gcnt[2] + h->gcnt[3] + (double)h->max_len;
-            const double den = (bases > (double)h->n ? bases : (double)h->n) + a.alpha_pc;
-            a.drift_fast_ok = (p->pseudocount >= 1e-30 && (double)p->k * log2(den / p->pseudocount) < 1000.0) ? 1 : 0;
+            a.drift_fast_ok = drift_fast_path_ok(h->gcnt, h->max_len, h->n, p);
             if (h->opt_exact_scans) a.drift_fast_ok = 0; // gibbs_set_option(GIBBS_OPT_EXACT_SCANS): every window in float64
             a.fast_ok = a.drift_fast_ok;
         }
@@ -1845,6 +1872,453 @@ int32_t gibbs_measure_smem_bandwidth(int32_t device, int32_t iters, double *gbps
     cudaEventDestroy(e0);
     cudaEventDestroy(e1);
     cudaFree(sink);
+    return GIBBS_OK;
+}
+
+/* ---- many independent sequence sets in one launch ------------------------------------------------------------------ */
+// The sets are uploaded as one concatenation into an internal handle (rows with a common row_words, lengths, mask plane,
+// stream, events); every set then gets its own ChainArgs that point into it (gibbs_batch.cuh). Per-set W / drift tables
+// are built with the single-set setup kernels, one small launch per set, and kept while the parameters stay the same.
+struct gibbs_batch {
+    gibbs_handle *h = nullptr;
+    int32_t n_sets = 0, n_seqs = 0;
+    std::vector<int32_t> seq_off;               // [n_sets + 1] first sequence of each set
+    std::vector<int32_t> min_len, max_len;      // per set
+    std::vector<int64_t> n_masked;              // symbols outside A,C,G,T per set
+    std::vector<uint8_t> has_gap;               // per set: holds Gap '-'
+    std::vector<int64_t> gcnt;                  // [n_sets][4] A,C,G,T counts (the data-derived background)
+    DevBuf<int32_t> d_seq_off;
+    // per-set tables, keyed by the parameters they were built for
+    DevBuf<WEnt> wtab;
+    DevBuf<int> wt_range;                       // [n_sets][4]: min lg, max lg, non-normal W
+    DevBuf<double> pvals;
+    std::vector<int32_t> fast;                  // per set: the fixed-point ranking pass is usable
+    bool tab_valid = false;
+    int32_t tab_bgmode = -1, tab_alen = 0, tab_k = 0;
+    double tab_pc = 0;
+    std::vector<double> tab_bg;
+    // per-set arguments and launch groups (uploaded when they change)
+    std::vector<ChainArgs> args_host;
+    std::vector<int32_t> groups_host;           // per group: set ids, then chain offsets
+    DevBuf<ChainArgs> d_args;
+    DevBuf<int32_t> d_groups;
+    // results
+    DevBuf<int32_t> sites, win_sites;           // win_sites: [n_seqs] winners' sites + [n_sets] restart index
+    DevBuf<double> hv, scores, sums, win_scores; // win_scores: [n_seqs] winners' scores + [n_sets] sums
+    DevBuf<int32_t> counts;
+    DevBuf<unsigned long long> stats;
+    int32_t run_R = 0, run_k = 0, run_launches = 0, run_team = 0, run_fast = 0;
+    bool run_done = false;
+};
+
+namespace {
+
+constexpr int BATCH_GROUPS = 4; // (masked symbols) x (4 warps per chain, 1 warp)
+
+int batch_team(const gibbs_batch *b, int s) {
+    const int N = b->seq_off[s + 1] - b->seq_off[s];
+    return (N >= 4 && team_smem_bytes(b->h->row_words, 4) <= 200 * 1024) ? 4 : 1;
+}
+
+cudaError_t launch_batch_group(bool init, bool masked, bool drift, int team, const ChainArgs &run, const BatchTable &bt, int grid,
+                               int smem, cudaStream_t st) {
+#define PICK(sfx) (team == 4 ? launch_batch##sfx##_t4 : launch_batch##sfx##_t1)
+    decltype(&launch_batch_t4) f;
+    if (init) f = masked ? (drift ? PICK(_init_masked_drift) : PICK(_init_masked)) : (drift ? PICK(_init_drift) : PICK(_init));
+    else f = masked ? (drift ? PICK(_masked_drift) : PICK(_masked)) : (drift ? PICK(_drift) : PICK());
+#undef PICK
+    return f(run, bt, grid, smem, st);
+}
+
+int32_t batch_check(const gibbs_batch *b, const gibbs_params *p, const double *bg_per_set, int32_t R) {
+    if (!b) return fail(GIBBS_ERR_ARG, "null batch");
+    if (!p) return fail(GIBBS_ERR_ARG, "null params");
+    if (R < 1) return fail(GIBBS_ERR_ARG, "restarts_per_set must be >= 1");
+    if (p->sampler != GIBBS_SITE_SAMPLER)
+        return fail(p->sampler == GIBBS_MOTIF_SAMPLER ? GIBBS_ERR_UNSUPPORTED : GIBBS_ERR_ARG,
+                    "batches run the SiteSampler only (sampler = %d)", p->sampler);
+    if (p->motif_amount > 1) return fail(GIBBS_ERR_ARG, "motif_amount belongs to the MotifSampler");
+    if (p->phase_mask != 0) return fail(GIBBS_ERR_ARG, "batches run the whole pipeline: phase_mask must be 0");
+    if (p->k < 1 || p->k > GIBBS_MAX_K) return fail(GIBBS_ERR_ARG, "motif width k=%d outside 1..%d", p->k, GIBBS_MAX_K);
+    if (p->alphabet_size < 1) return fail(GIBBS_ERR_ARG, "alphabet_size must be >= 1");
+    if (!(p->pseudocount >= 0.0)) return fail(GIBBS_ERR_ARG, "pseudocount must be >= 0");
+    if (p->background != GIBBS_BG_FIXED && p->background != GIBBS_BG_DATA) return fail(GIBBS_ERR_ARG, "unknown background mode %d", p->background);
+    if ((int64_t)R * b->n_sets > INT32_MAX) return fail(GIBBS_ERR_ARG, "%d sets x %d restarts: too many chains", b->n_sets, R);
+    for (int32_t s = 0; s < b->n_sets; ++s) {
+        if (b->min_len[s] < p->k) {
+            int32_t i = b->seq_off[s];
+            while (b->h->len_host[i] >= p->k) ++i;
+            return fail(GIBBS_ERR_SHORT_SEQ, "set %d, sequence %d: length %d is shorter than k=%d (Array.take, fs:152)", s,
+                        i - b->seq_off[s], b->h->len_host[i], p->k);
+        }
+        if (b->has_gap[s] && p->alphabet_size >= 5)
+            return fail(GIBBS_ERR_UNSUPPORTED, "set %d holds Gap '-' and alphabet_size = %d includes it: a fifth PWM row is not built "
+                                               "(pass alphabet_size = 4 to score Gap like any other non-alphabet symbol)", s, p->alphabet_size);
+        const double *bg = p->background == GIBBS_BG_FIXED && bg_per_set ? bg_per_set + 4 * (size_t)s : p->bg;
+        if (p->background == GIBBS_BG_FIXED)
+            for (int x = 0; x < 4; ++x)
+                if (!(bg[x] > 0.0)) return fail(GIBBS_ERR_ARG, "set %d: background probability bg[%d] must be > 0", s, x);
+        if (p->background == GIBBS_BG_DATA)
+            for (int x = 0; x < 4; ++x)
+                if (b->gcnt[4 * (size_t)s + x] > INT32_MAX)
+                    return fail(GIBBS_ERR_ARG, "set %d: more than 2^31 bases of one kind: background counts overflow int32 (fs:34)", s);
+    }
+    return GIBBS_OK;
+}
+
+// W tables (fixed background) or PPM value tables (data-derived) of every set, with the kernels of ensure_wtab / ensure_drift
+int32_t batch_tables(gibbs_batch *b, const gibbs_params *p, const double *bg_per_set, int *launches) {
+    gibbs_handle *h = b->h;
+    std::vector<double> bg((size_t)b->n_sets * 4);
+    for (int32_t s = 0; s < b->n_sets; ++s)
+        for (int x = 0; x < 4; ++x) bg[4 * (size_t)s + x] = bg_per_set ? bg_per_set[4 * (size_t)s + x] : p->bg[x];
+    const bool fixed = p->background == GIBBS_BG_FIXED;
+    if (b->tab_valid && b->tab_bgmode == p->background && b->tab_pc == p->pseudocount && b->tab_alen == p->alphabet_size &&
+        b->tab_k == p->k && (!fixed || b->tab_bg == bg))
+        return GIBBS_OK;
+    b->tab_valid = false;
+    b->fast.assign((size_t)b->n_sets, 0);
+    if (fixed) {
+        CUDA_TRY(b->wtab.reserve((size_t)b->n_seqs * 4));
+        CUDA_TRY(b->wt_range.reserve((size_t)b->n_sets * 4));
+        std::vector<int> range((size_t)b->n_sets * 4);
+        for (int32_t s = 0; s < b->n_sets; ++s) {
+            range[4 * (size_t)s] = INT32_MAX;
+            range[4 * (size_t)s + 1] = INT32_MIN;
+            range[4 * (size_t)s + 2] = range[4 * (size_t)s + 3] = 0;
+        }
+        CUDA_TRY(cudaMemcpyAsync(b->wt_range.p, range.data(), range.size() * sizeof(int), cudaMemcpyHostToDevice, h->stream));
+        for (int32_t s = 0; s < b->n_sets; ++s) {
+            const int N = b->seq_off[s + 1] - b->seq_off[s];
+            const double den = (double)(N - 1) + ((double)p->alphabet_size * p->pseudocount); // fs:257, per set
+            const double *q = bg.data() + 4 * (size_t)s;
+            wtab_kernel<<<(N * 4 + 255) / 256, 256, 0, h->stream>>>(N, p->pseudocount, den, q[0], q[1], q[2], q[3],
+                                                                    b->wtab.p + 4 * (size_t)b->seq_off[s], b->wt_range.p + 4 * (size_t)s);
+            CUDA_TRY(cudaGetLastError());
+        }
+        *launches += b->n_sets;
+        CUDA_TRY(cudaMemcpyAsync(range.data(), b->wt_range.p, range.size() * sizeof(int), cudaMemcpyDeviceToHost, h->stream));
+        CUDA_TRY(cudaStreamSynchronize(h->stream));
+        for (int32_t s = 0; s < b->n_sets; ++s)
+            b->fast[s] = fast_path_ok_range(range[4 * (size_t)s + 2], range[4 * (size_t)s], range[4 * (size_t)s + 1], p->k);
+    } else {
+        // base counts, symbols outside A,C,G,T and prefix tables per sequence; the background counts of each set come from
+        // the host's per-set counts (checked against int32 per set in batch_check), not from the whole concatenation
+        int32_t rc = ensure_seq_counts(h, launches);
+        if (rc) return rc;
+        CUDA_TRY(b->pvals.reserve((size_t)b->n_seqs));
+        for (int32_t s = 0; s < b->n_sets; ++s) {
+            const int N = b->seq_off[s + 1] - b->seq_off[s];
+            const double den = (double)(N - 1) + ((double)p->alphabet_size * p->pseudocount);
+            pvals_kernel<<<(N + 255) / 256, 256, 0, h->stream>>>(N, p->pseudocount, den, b->pvals.p + b->seq_off[s]);
+            CUDA_TRY(cudaGetLastError());
+            int32_t g[4];
+            for (int x = 0; x < 4; ++x) g[x] = (int32_t)b->gcnt[4 * (size_t)s + x];
+            b->fast[s] = drift_fast_path_ok(g, b->max_len[s], N, p);
+        }
+        *launches += b->n_sets;
+    }
+    if (h->opt_exact_scans) b->fast.assign((size_t)b->n_sets, 0);
+    b->tab_bgmode = p->background;
+    b->tab_pc = p->pseudocount;
+    b->tab_alen = p->alphabet_size;
+    b->tab_k = p->k;
+    b->tab_bg = bg;
+    b->tab_valid = true;
+    return GIBBS_OK;
+}
+
+} // namespace
+
+int32_t gibbs_batch_create(const uint8_t *seqs, const int64_t *offsets, const int32_t *set_offsets, int32_t n_sets, int32_t device,
+                           gibbs_batch **out) {
+    if (!out) return fail(GIBBS_ERR_ARG, "null out pointer");
+    *out = nullptr;
+    if (!seqs || !offsets || !set_offsets) return fail(GIBBS_ERR_ARG, "null sequence buffer or set offsets (ArgumentNullException)");
+    if (n_sets < 1) return fail(GIBBS_ERR_ARG, "n_sets must be >= 1");
+    if (set_offsets[0] != 0) return fail(GIBBS_ERR_ARG, "set_offsets[0] must be 0 (it is %d)", set_offsets[0]);
+    for (int32_t s = 0; s < n_sets; ++s)
+        if (set_offsets[s + 1] <= set_offsets[s])
+            return fail(GIBBS_ERR_ARG, "set %d is empty or set_offsets decrease (%d .. %d)", s, set_offsets[s], set_offsets[s + 1]);
+    const int32_t n_seqs = set_offsets[n_sets];
+    gibbs_batch *b = new (std::nothrow) gibbs_batch();
+    if (!b) return fail(GIBBS_ERR_NOMEM, "host allocation failed");
+    try {
+        b->seq_off.assign(set_offsets, set_offsets + n_sets + 1);
+        b->min_len.assign((size_t)n_sets, INT32_MAX);
+        b->max_len.assign((size_t)n_sets, 0);
+        b->n_masked.assign((size_t)n_sets, 0);
+        b->has_gap.assign((size_t)n_sets, 0);
+        b->gcnt.assign((size_t)n_sets * 4, 0);
+    } catch (...) {
+        delete b;
+        return fail(GIBBS_ERR_NOMEM, "host allocation failed");
+    }
+    b->n_sets = n_sets;
+    b->n_seqs = n_seqs;
+    // per-set symbol classes; a failure names the set and the sequence (gibbs_create would only name the symbol)
+    for (int32_t s = 0; s < n_sets; ++s) {
+        for (int32_t i = set_offsets[s]; i < set_offsets[s + 1]; ++i) {
+            const int64_t l = offsets[i + 1] - offsets[i];
+            if (l < 0) {
+                delete b;
+                return fail(GIBBS_ERR_ARG, "set %d, sequence %d: offsets must be non-decreasing", s, i - set_offsets[s]);
+            }
+            if (l > GIBBS_MAX_LEN) {
+                delete b;
+                return fail(GIBBS_ERR_ARG, "set %d, sequence %d: longer than %d", s, i - set_offsets[s], GIBBS_MAX_LEN);
+            }
+            b->min_len[s] = std::min(b->min_len[s], (int32_t)l);
+            b->max_len[s] = std::max(b->max_len[s], (int32_t)l);
+            for (int64_t j = offsets[i]; j < offsets[i + 1]; ++j) {
+                const uint8_t c = seqs[j];
+                if (c == 'A') ++b->gcnt[4 * (size_t)s];
+                else if (c == 'C') ++b->gcnt[4 * (size_t)s + 1];
+                else if (c == 'G') ++b->gcnt[4 * (size_t)s + 2];
+                else if (c == 'T') ++b->gcnt[4 * (size_t)s + 3];
+                else if (c >= 42 && c <= 90) {
+                    ++b->n_masked[s];
+                    if (c == '-') b->has_gap[s] = 1;
+                } else {
+                    delete b;
+                    return fail(GIBBS_ERR_SYMBOL, "set %d, sequence %d: symbol '%c' (0x%02x) is outside '*'..'Z', the range of the "
+                                                  "49-slot tables (IndexOutOfRangeException, fs:17-20)",
+                                s, i - set_offsets[s], c >= 32 && c < 127 ? (char)c : '?', c);
+                }
+            }
+        }
+    }
+    int32_t rc = gibbs_create(seqs, offsets, n_seqs, device, &b->h);
+    if (!rc) {
+        gibbs_handle *h = b->h;
+        cudaError_t e = b->d_seq_off.reserve((size_t)n_sets + 1);
+        if (e == cudaSuccess)
+            e = cudaMemcpyAsync(b->d_seq_off.p, b->seq_off.data(), b->seq_off.size() * sizeof(int32_t), cudaMemcpyHostToDevice, h->stream);
+        if (e == cudaSuccess) e = cudaStreamSynchronize(h->stream);
+        if (e != cudaSuccess) rc = fail(GIBBS_ERR_CUDA, "batch upload: %s", cudaGetErrorString(e));
+    }
+    if (rc) {
+        gibbs_batch_destroy(b);
+        return rc;
+    }
+    *out = b;
+    return GIBBS_OK;
+}
+
+int32_t gibbs_batch_destroy(gibbs_batch *b) {
+    if (!b) return GIBBS_OK;
+    if (b->h) {
+        cudaSetDevice(b->h->device);
+        cudaStreamSynchronize(b->h->stream);
+    }
+    b->d_seq_off.release(); b->wtab.release(); b->wt_range.release(); b->pvals.release(); b->d_args.release(); b->d_groups.release();
+    b->sites.release(); b->win_sites.release(); b->hv.release(); b->scores.release(); b->sums.release(); b->win_scores.release();
+    b->counts.release(); b->stats.release();
+    gibbs_destroy(b->h);
+    delete b;
+    return GIBBS_OK;
+}
+
+int32_t gibbs_batch_run_device(gibbs_batch *b, const gibbs_params *p, const double *bg_per_set, int32_t restarts_per_set,
+                               int64_t chain_id_base, uint64_t seed) {
+    int32_t rc = batch_check(b, p, bg_per_set, restarts_per_set);
+    if (rc) return rc;
+    gibbs_handle *h = b->h;
+    rc = set_device(h);
+    if (rc) return rc;
+    b->run_done = false;
+    const int32_t R = restarts_per_set, S = b->n_sets;
+    const bool drift = p->background == GIBBS_BG_DATA;
+    int launches = 0;
+    rc = batch_tables(b, p, bg_per_set, &launches);
+    if (rc) return rc;
+    const size_t cells = (size_t)R * b->n_seqs;
+    CUDA_TRY(b->sites.reserve(cells));
+    CUDA_TRY(b->hv.reserve(cells));
+    CUDA_TRY(b->scores.reserve(cells));
+    CUDA_TRY(b->sums.reserve((size_t)S * R));
+    CUDA_TRY(b->stats.reserve(ST_NSLOTS));
+    CUDA_TRY(cudaMemsetAsync(b->stats.p, 0, ST_NSLOTS * sizeof(unsigned long long), h->stream));
+
+    // run-wide arguments (chain_batch_kernel copies them over the set's own)
+    ChainArgs run{};
+    run.k = p->k;
+    run.max_sweeps = p->max_sweeps > 0 ? p->max_sweeps : 1000000;
+    run.sampler = GIBBS_SITE_SAMPLER;
+    run.phase_mask = GIBBS_PHASE_GREEDY | (p->phase_shifts ? (GIBBS_PHASE_LEFT | GIBBS_PHASE_RIGHT) : 0);
+    run.rng_mode = GIBBS_RNG_PHILOX;
+    run.seed = seed;
+    run.chain_id_base = chain_id_base;
+    run.stats = b->stats.p;
+
+    // per-set arguments: the set's rows and tables, its slices of the results
+    std::vector<ChainArgs> args((size_t)S);
+    const int rw = h->row_words;
+    int fast_all = 1;
+    for (int32_t s = 0; s < S; ++s) {
+        const int32_t o = b->seq_off[s], N = b->seq_off[s + 1] - o;
+        ChainArgs &a = args[s];
+        memset(&a, 0, sizeof a);
+        a.s.packed = h->packed.p + (size_t)o * rw;
+        a.s.len = h->len.p + o;
+        a.s.n = N;
+        a.s.row_words = rw;
+        a.s.uniform_len = b->min_len[s] == b->max_len[s] ? b->max_len[s] : 0;
+        a.s.mask = b->n_masked[s] > 0 ? h->mask.p + (size_t)o * rw : nullptr;
+        a.s.rowflag = b->n_masked[s] > 0 ? h->rowflag.p + o : nullptr;
+        a.k = p->k;
+        a.sampler = GIBBS_SITE_SAMPLER;
+        a.n_chains = R;
+        a.sites = b->sites.p + (size_t)R * o;
+        a.hv = b->hv.p + (size_t)R * o;
+        a.scores = b->scores.p + (size_t)R * o;
+        a.sums = b->sums.p + (size_t)R * s;
+        a.fast_ok = b->fast[s];
+        fast_all &= b->fast[s];
+        if (drift) {
+            a.pvals = b->pvals.p + o;
+            a.basecnt = h->basecnt.p + 4 * (size_t)o;
+            a.maskcnt = b->n_masked[s] > 0 ? h->maskcnt.p + o : nullptr;
+            a.ss = h->ss_valid ? h->ss.p + (size_t)o * (size_t)(h->max_len + 2) * 4 : nullptr;
+            a.ss_stride = h->max_len + 2;
+            for (int x = 0; x < 4; ++x) a.gcnt[x] = (int32_t)b->gcnt[4 * (size_t)s + x];
+            a.alpha_pc = (double)p->alphabet_size * p->pseudocount; // fs:117
+            a.pc = p->pseudocount;
+            a.drift_fast_ok = b->fast[s];
+        } else {
+            a.wtab = b->wtab.p + 4 * (size_t)o;
+            memcpy(a.bg, b->tab_bg.data() + 4 * (size_t)s, sizeof a.bg);
+        }
+    }
+    // launch groups: (masked symbols) x (4 warps per chain for sets of >= 4 sequences, else 1)
+    std::vector<int32_t> ids[BATCH_GROUPS];
+    for (int32_t s = 0; s < S; ++s) ids[(b->n_masked[s] > 0 ? 2 : 0) + (batch_team(b, s) == 4 ? 0 : 1)].push_back(s);
+    std::vector<int32_t> groups;
+    size_t g_at[BATCH_GROUPS];
+    for (int g = 0; g < BATCH_GROUPS; ++g) {
+        g_at[g] = groups.size();
+        groups.insert(groups.end(), ids[g].begin(), ids[g].end());
+        for (size_t i = 0; i <= ids[g].size(); ++i) groups.push_back((int32_t)(i * (size_t)R));
+    }
+    if (args.size() * sizeof(ChainArgs) != b->args_host.size() * sizeof(ChainArgs) ||
+        memcmp(args.data(), b->args_host.data(), args.size() * sizeof(ChainArgs)) != 0) {
+        CUDA_TRY(b->d_args.reserve(args.size()));
+        CUDA_TRY(cudaMemcpyAsync(b->d_args.p, args.data(), args.size() * sizeof(ChainArgs), cudaMemcpyHostToDevice, h->stream));
+        b->args_host.swap(args);
+    }
+    if (groups != b->groups_host) {
+        CUDA_TRY(b->d_groups.reserve(groups.size()));
+        CUDA_TRY(cudaMemcpyAsync(b->d_groups.p, groups.data(), groups.size() * sizeof(int32_t), cudaMemcpyHostToDevice, h->stream));
+        b->groups_host.swap(groups);
+    }
+    const long long total_chains = (long long)S * R;
+    const long long per_sm = (total_chains + h->sm_count - 1) / h->sm_count;
+    b->run_team = 0;
+    CUDA_TRY(cudaEventRecord(h->ev0, h->stream));
+    for (int init = 1; init >= 0; --init) { // every group's random starts, then every group's sweeps
+        for (int g = 0; g < BATCH_GROUPS; ++g) {
+            const int n = (int)ids[g].size();
+            if (n == 0) continue;
+            const bool masked = g >= 2;
+            const int team = (g & 1) ? 1 : 4;
+            if (!b->run_team) b->run_team = team;
+            BatchTable bt;
+            bt.sets = b->d_args.p;
+            bt.set_ids = b->d_groups.p + g_at[g];
+            bt.chain_off = b->d_groups.p + g_at[g] + n;
+            bt.n = n;
+            ChainArgs r = run;
+            r.min_width = per_sm <= 1 ? team : 1; // (as launch_chain_kp: never narrow once a chain has an SM to itself)
+            CUDA_TRY(launch_batch_group(init != 0, masked, drift, team, r, bt, n * R, team_smem_bytes(h->row_words, team), h->stream));
+            ++launches;
+        }
+    }
+    CUDA_TRY(cudaEventRecord(h->ev1, h->stream));
+    b->run_R = R;
+    b->run_k = p->k;
+    b->run_fast = fast_all;
+    b->run_launches = launches;
+    b->run_done = true;
+    return GIBBS_OK;
+}
+
+static void batch_stats(const gibbs_batch *b, const unsigned long long *st, int extra_launches, gibbs_run_stats *out) {
+    float ms = 0.f;
+    if (cudaEventElapsedTime(&ms, b->h->ev0, b->h->ev1) != cudaSuccess) cudaGetLastError();
+    out->site_updates = (int64_t)st[ST_SITE_UPDATES];
+    out->window_scores = (int64_t)st[ST_WINDOW_SCORES];
+    out->sweeps = (int64_t)st[ST_SWEEPS];
+    out->exact_rescans = (int64_t)st[ST_EXACT_RESCANS];
+    out->capped_chains = (int64_t)st[ST_CAPPED];
+    out->speculative_discards = (int64_t)st[ST_SPECULATED];
+    out->kernel_launches = b->run_launches + extra_launches;
+    out->fast_path = b->run_fast;
+    out->team_warps = b->run_team;
+    out->init_path = GIBBS_INIT_CHAIN;
+    out->kernel_ms = (double)ms;
+}
+
+int32_t gibbs_batch_fetch(gibbs_batch *b, int32_t *sites_out, double *scores_out, double *sums_out, gibbs_run_stats *stats_out) {
+    if (!b) return fail(GIBBS_ERR_ARG, "null batch");
+    if (!b->run_done) return fail(GIBBS_ERR_ARG, "gibbs_batch_fetch without a preceding gibbs_batch_run_device");
+    gibbs_handle *h = b->h;
+    int32_t rc = set_device(h);
+    if (rc) return rc;
+    const size_t cells = (size_t)b->run_R * b->n_seqs;
+    if (sites_out) CUDA_TRY(cudaMemcpyAsync(sites_out, b->sites.p, cells * sizeof(int32_t), cudaMemcpyDeviceToHost, h->stream));
+    if (scores_out) CUDA_TRY(cudaMemcpyAsync(scores_out, b->scores.p, cells * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
+    if (sums_out)
+        CUDA_TRY(cudaMemcpyAsync(sums_out, b->sums.p, (size_t)b->run_R * b->n_sets * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
+    unsigned long long st[ST_NSLOTS];
+    CUDA_TRY(cudaMemcpyAsync(st, b->stats.p, sizeof st, cudaMemcpyDeviceToHost, h->stream));
+    CUDA_TRY(cudaStreamSynchronize(h->stream));
+    if (stats_out) batch_stats(b, st, 0, stats_out);
+    return GIBBS_OK;
+}
+
+int32_t gibbs_batch_fetch_best(gibbs_batch *b, int32_t repetitions, int32_t *sites_out, double *scores_out, int32_t *n_out,
+                               double *sum_out, int32_t *restart_out, int32_t *counts_out, gibbs_run_stats *stats_out) {
+    if (!b) return fail(GIBBS_ERR_ARG, "null batch");
+    if (!b->run_done) return fail(GIBBS_ERR_ARG, "gibbs_batch_fetch_best without a preceding gibbs_batch_run_device");
+    if (repetitions < 0) repetitions = 0;
+    gibbs_handle *h = b->h;
+    int32_t rc = set_device(h);
+    if (rc) return rc;
+    const int32_t S = b->n_sets, NT = b->n_seqs, k = b->run_k;
+    CUDA_TRY(b->win_sites.reserve((size_t)NT + S));
+    CUDA_TRY(b->win_scores.reserve((size_t)NT + S));
+    restart_select_batch_kernel<<<S, 32, 0, h->stream>>>(b->sums.p, b->sites.p, b->scores.p, b->d_seq_off.p, b->run_R, repetitions,
+                                                        b->win_sites.p + NT, b->win_sites.p, b->win_scores.p, b->win_scores.p + NT);
+    CUDA_TRY(cudaGetLastError());
+    int extra_launches = 1;
+    std::vector<int32_t> best((size_t)S);
+    CUDA_TRY(cudaMemcpyAsync(best.data(), b->win_sites.p + NT, (size_t)S * sizeof(int32_t), cudaMemcpyDeviceToHost, h->stream));
+    if (sum_out) CUDA_TRY(cudaMemcpyAsync(sum_out, b->win_scores.p + NT, (size_t)S * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
+    if (sites_out) CUDA_TRY(cudaMemcpyAsync(sites_out, b->win_sites.p, (size_t)NT * sizeof(int32_t), cudaMemcpyDeviceToHost, h->stream));
+    if (scores_out) CUDA_TRY(cudaMemcpyAsync(scores_out, b->win_scores.p, (size_t)NT * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
+    if (counts_out) { // PWM counts of every winner's sites (all zero where the initial value survived: its sites are -1)
+        CUDA_TRY(b->counts.reserve((size_t)S * k * 4));
+        switch ((k + 1) / 2) {
+#define X(KPV) case KPV: all_counts_batch_kernel<KPV><<<S, 32, 0, h->stream>>>(b->d_args.p, b->d_seq_off.p, b->win_sites.p, k, b->counts.p); break;
+            KP_CASES(X)
+#undef X
+        default: return fail(GIBBS_ERR_ARG, "unsupported k");
+        }
+        CUDA_TRY(cudaGetLastError());
+        ++extra_launches;
+        CUDA_TRY(cudaMemcpyAsync(counts_out, b->counts.p, (size_t)S * k * 4 * sizeof(int32_t), cudaMemcpyDeviceToHost, h->stream));
+    }
+    unsigned long long st[ST_NSLOTS];
+    CUDA_TRY(cudaMemcpyAsync(st, b->stats.p, sizeof st, cudaMemcpyDeviceToHost, h->stream));
+    CUDA_TRY(cudaStreamSynchronize(h->stream));
+    for (int32_t s = 0; s < S; ++s) {
+        const bool initial = best[s] < 0; // loop 0 [||] [|(0., 0)|] returned its initial value (quirk A.6-8)
+        if (initial && sites_out) sites_out[b->seq_off[s]] = 0;
+        if (initial && scores_out) scores_out[b->seq_off[s]] = 0.0;
+        if (n_out) n_out[s] = initial ? 1 : b->seq_off[s + 1] - b->seq_off[s];
+        if (restart_out) restart_out[s] = best[s];
+    }
+    if (stats_out) batch_stats(b, st, extra_launches, stats_out);
     return GIBBS_OK;
 }
 

@@ -653,236 +653,7 @@ static __global__ void __launch_bounds__(32 * T, (INIT_ONLY ? (T == 1 ? 8 : 4) :
         if ((int)blockIdx.x >= *a.pending_in_n) return;
         chain = a.pending_in[blockIdx.x];
     }
-    const TeamSmem S = carve_smem(smem_raw, T);
-    const WarpTables WT = warp_tables(S, warp);
-    require_aligned_tables(WT);
-
-    const int N = a.s.n, k = a.k;
-    int32_t *sites = a.sites + (size_t)chain * N;
-    double *hv = a.hv + (size_t)chain * N;
-    double *scores = a.scores + (size_t)chain * N;
-    const uint64_t chain_uid = (uint64_t)a.chain_id_base + (uint64_t)chain;
-
-    RowRing<R> ring;
-    ring.init(S, a.s, 0, tid);
-    if (tid < 16) S.lut[tid] = hist_lut_entry(tid);
-    team_sync<T>();
-    if (warp == 0) ring.fill_span(0u, 0, R, lane);
-
-    unsigned long long st_updates = 0, st_windows = 0, st_slow = 0, st_spec = 0;
-    int st_sweeps = 0, capped = 0;
-    uint32_t vbase = 0; // visit index of n = 0 in the current sweep (wraps harmlessly)
-
-    int phase = INIT_ONLY ? PH_INIT : next_phase(PH_GREEDY, a.phase_mask);
-    int sweeps_in_phase = 0;
-    bool resumed = false, paused = false;
-    if (a.from_list) {
-        const int r = a.resume[chain]; // phase | capped so far << 7 | sweeps in phase << 8
-        phase = r & 127;
-        capped = (r >> 7) & 1;
-        sweeps_in_phase = r >> 8;
-        resumed = true;
-    }
-    while (phase != PH_DONE) {
-        const int mode = phase == PH_LEFT ? SHIFT_LEFT : phase == PH_RIGHT ? SHIFT_RIGHT : SHIFT_NONE;
-        // all-sites counts: once when the greedy phase starts (then kept incrementally: -old site,
-        // +new site), once per sweep for the shift phases (they read the shifted snapshot, fs:357)
-        if (phase == PH_LEFT || phase == PH_RIGHT || (phase == PH_GREEDY && (sweeps_in_phase == 0 || resumed)))
-            site_counts<KP, T>(a.s, sites, -1, k, mode, S.total, S.lut, S.fix, tid);
-        else
-            team_sync<T>(); // the last round of the previous sweep wrote sites / hv after its only barrier: the block
-                            // loads below must see them (a stale hv_n could flip an accept of the sequential sweep)
-        resumed = false;
-        // state of two 32-sequence blocks (lengths, sites, raw scores): coalesced loads, kept one block ahead
-        auto load_block = [&](int b) {
-            const int i = b * 32 + tid;
-            if (tid < 32 && i < N) {
-                const int o = (b & 1) * 32 + tid;
-                S.blk_len[o] = __ldg(a.s.len + i);
-                if (!INIT_ONLY) {
-                    S.blk_site[o] = __ldcg(sites + i);
-                    S.blk_hv[o] = __ldcg(hv + i);
-                }
-            }
-        };
-        load_block(0);
-        load_block(1);
-        team_sync<T>();
-        bool changed = false;
-        int cur_blk = 0;
-        int n0 = 0;
-        // greedy sweeps: how many sequences a round attempts. Halved after a round that discarded work
-        // (a site moved), doubled after a quiet round: early sweeps, where almost every update moves a
-        // site, run nearly sequentially and waste no issue slots; late sweeps run T wide.
-        int width = (phase == PH_GREEDY) ? max(1, min(T, a.min_width)) : T;
-        unsigned round = 0;
-        while (n0 < N) {
-            if ((n0 >> 5) != cur_blk) { // entering a new block: fetch the one after it (not read this round)
-                cur_blk = n0 >> 5;
-                load_block(cur_blk + 1);
-            }
-            const int n = n0 + warp;
-            const bool active = n < N && warp < width;
-            int flag = 0, site_n = 0, w = 0, Wn = 0, masked_n = -1;
-            double p = 0.0;
-            uint64_t own = 0, neu = 0;
-            if (active) {
-                const uint32_t *row = ring.wait(vbase + (uint32_t)n);
-                const int o = ((n >> 5) & 1) * 32 + (n & 31);
-                const int len_n = S.blk_len[o];
-                Wn = len_n - k + 1;
-                double hv_n = 0.0;
-                if (MASKED) masked_n = __ldg(a.s.rowflag + n) != 0 ? n : -1; // the held-out sequence holds symbols outside A,C,G,T
-                bool slow;
-                if constexpr (DRIFT) {
-                    int f0[4], cn[4];
-                    const bool given = INIT_ONLY && a.ppm_given != nullptr;
-                    const bool fast = a.drift_fast_ok && !given; // (a supplied PPM may hold zeros or denormals: exact scan)
-                    if constexpr (INIT_ONLY) {
-                        random_loo_counts_impl<KP, GIBBS_P0_NB_CHAIN, MASKED>(a, chain_uid, chain, n, WT.counts, lane, WT.lgcol);
-                        drift_tables<KP>(WT, WT.counts, false, 0, k, a, given, fast, n, lane, f0, cn);
-                    } else {
-                        site_n = S.blk_site[o];
-                        hv_n = S.blk_hv[o];
-                        own = kmer_shared<KP>(row, shifted_site(site_n, len_n, k, mode));
-                        uint64_t own_mk = 0; // rare: the own site may cover symbols outside A,C,G,T
-                        if (MASKED && masked_n >= 0) own_mk = mask_kmer(a.s.mask, a.s.row_words, n, shifted_site(site_n, len_n, k, mode), k);
-                        drift_tables<KP>(WT, S.total, true, own, k, a, false, fast, n, lane, f0, cn, own_mk);
-                    }
-                    slow = drift_pick<KP>(WT, row, Wn, k, a, fast, f0, cn, lane, p, w, MASKED ? masked_n : -1, n);
-                } else {
-                    if constexpr (INIT_ONLY) {
-                        random_loo_counts_impl<KP, GIBBS_P0_NB_CHAIN, MASKED>(a, chain_uid, chain, n, WT.counts, lane, WT.lgcol);
-                        build_tables<KP>(WT, WT.counts, false, 0, k, a.wtab, lane);
-                    } else {
-                        site_n = S.blk_site[o];
-                        hv_n = S.blk_hv[o];
-                        own = kmer_shared<KP>(row, shifted_site(site_n, len_n, k, mode));
-                        if (MASKED && masked_n >= 0) // rare: the own site may cover symbols outside A,C,G,T
-                            build_tables_masked<KP>(WT, S.total, own, k, a.wtab, lane,
-                                                    mask_kmer(a.s.mask, a.s.row_words, n, shifted_site(site_n, len_n, k, mode), k));
-                        else
-                            build_tables<KP>(WT, S.total, true, own, k, a.wtab, lane);
-                    }
-                    slow = MASKED ? pick_argmax<KP>(WT, row, Wn, k, a.fast_ok, lane, p, w, &a.s, masked_n)
-                                  : pick_argmax<KP>(WT, row, Wn, k, a.fast_ok, lane, p, w);
-                }
-                bool accept = true, moved = false;
-                if (!INIT_ONLY) {
-                    accept = score_improves(p, hv_n, hv_n != hv_n ? __ldcg(scores + n) : 0.0); // fs:402
-                    moved = accept && (w != site_n);
-                    if (moved && phase == PH_GREEDY) neu = kmer_shared<KP>(row, w); // rows are not read after the sync
-                }
-                flag = (accept ? 1 : 0) | (moved ? 2 : 0) | (slow ? 4 : 0);
-            }
-            int32_t *flags = S.flags + (round & 1) * T; // double-buffered: one team sync per round suffices
-            ++round;
-            if (lane == 0) flags[warp] = flag;
-            team_sync<T>();
-            // greedy only: warps after the first mover of the round saw stale counts
-            const unsigned movers = __ballot_sync(FULL, lane < T && (flags[lane < T ? lane : 0] & 2) != 0);
-            const bool any_moved = movers != 0;
-            const int first_mover = (phase == PH_GREEDY && any_moved) ? __ffs(movers) - 1 : T;
-            const int last_commit = min(first_mover, width - 1);
-            changed |= any_moved; // (greedy: any mover of the round implies a committed mover)
-            if (active) {
-                if (warp <= last_commit) {
-                    st_updates += 1;
-                    st_windows += (unsigned long long)Wn;
-                    st_slow += (flag & 4) ? 1 : 0;
-                    if ((flag & 1) && lane == 0) {
-                        sites[n] = w;
-                        hv[n] = p;
-                    }
-                } else {
-                    st_spec += 1;
-                }
-            }
-            const int committed = min(last_commit + 1, N - n0);
-            if (warp == 0) ring.fill_span(vbase + (uint32_t)(n0 + R), n0 + R, committed, lane); // their rows are free
-            n0 += committed;
-            if (phase == PH_GREEDY) {
-                if (first_mover < T) { // in-place sweep: later n see the new site (fs:388): -old k-mer, +new k-mer
-                    if (MASKED && warp == first_mover && masked_n >= 0) { // rare: masked bases were never counted
-                        const int len_n = S.blk_len[((n >> 5) & 1) * 32 + (n & 31)];
-                        const uint64_t own_mk = mask_kmer(a.s.mask, a.s.row_words, n, shifted_site(site_n, len_n, k, mode), k);
-                        const uint64_t neu_mk = mask_kmer(a.s.mask, a.s.row_words, n, w, k);
-                        if (lane < k) {
-                            const int bo = (int)((own >> (2 * lane)) & 3u), bn = (int)((neu >> (2 * lane)) & 3u);
-                            if (!((own_mk >> (2 * lane)) & 1u)) S.total[lane * 4 + bo] -= 1;
-                            if (!((neu_mk >> (2 * lane)) & 1u)) S.total[lane * 4 + bn] += 1;
-                        }
-                    } else if (warp == first_mover && lane < k) {
-                        const int bo = (int)((own >> (2 * lane)) & 3u), bn = (int)((neu >> (2 * lane)) & 3u);
-                        if (bo != bn) {
-                            S.total[lane * 4 + bo] -= 1;
-                            S.total[lane * 4 + bn] += 1;
-                        }
-                    }
-                    team_sync<T>(); // counts updated before the next round builds its tables
-                    width = max(max(1, min(T, a.min_width)), width >> 1);
-                } else {
-                    width = min(T, width * 2);
-                }
-            }
-        }
-        vbase += (uint32_t)N;
-        st_sweeps += 1;
-        if (INIT_ONLY) break; // the sweep kernel continues from the state just written
-        ++sweeps_in_phase;
-        bool next = !changed; // positions(acc) = positions(bestMotif), fs:384
-        if (!next && sweeps_in_phase >= a.max_sweeps) {
-            next = true;
-            capped = 1;
-        }
-        if (next) {
-            sweeps_in_phase = 0;
-            phase = next_phase(phase + 1, a.phase_mask);
-        }
-        // sweep boundary: when few chains are still running, hand this one over to the wide-team launch
-        if (phase != PH_DONE && a.pause_below > 0) {
-            if (tid == 0) S.flags[2 * T] = (*(volatile int32_t *)a.active <= a.pause_below && st_sweeps >= a.pause_min_sweeps) ? 1 : 0;
-            team_sync<T>();
-            if (S.flags[2 * T]) {
-                paused = true;
-                break;
-            }
-        }
-    }
-    if (tid == 0) // the ring always has R rows in flight: let them land before the CTA exits
-        for (int i = 0; i < R; ++i) ring.wait(vbase + (uint32_t)i);
-    team_sync<T>();
-    if (lane == 0) {
-        atomicAdd(a.stats + ST_SITE_UPDATES, st_updates);
-        atomicAdd(a.stats + ST_WINDOW_SCORES, st_windows);
-        atomicAdd(a.stats + ST_EXACT_RESCANS, st_slow);
-        atomicAdd(a.stats + ST_SPECULATED, st_spec);
-    }
-    if (tid == 0) {
-        atomicAdd(a.stats + ST_SWEEPS, (unsigned long long)st_sweeps);
-        if (!paused) atomicAdd(a.stats + ST_CAPPED, (unsigned long long)capped); // (a chain counts once, where it ends)
-    }
-    if (INIT_ONLY) return;
-    if (paused) {
-        if (tid == 0) {
-            a.resume[chain] = phase | (capped << 7) | (sweeps_in_phase << 8);
-            a.pending_out[atomicAdd(a.pending_out_n, 1)] = chain;
-        }
-        return;
-    }
-
-    // (log2 highValue, highIndex), fs:303
-    for (int n = tid; n < N; n += THREADS) {
-        const double v = __ldcg(hv + n);
-        if (v == v) scores[n] = log2_ref(v); // NaN = untouched caller-supplied entry keeps its score
-    }
-    team_sync<T>();
-    if (tid == 0) {
-        double sum = 0.0; // Array.sum, left to right (fs:445)
-        for (int n = 0; n < N; ++n) sum = __dadd_rn(sum, __ldcg(scores + n));
-        a.sums[chain] = sum;
-        if (a.active) atomicSub(a.active, 1);
-    }
+#include "gibbs_chain_body.inc" // (shared with chain_batch_kernel, gibbs_batch.cuh)
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -1017,57 +788,7 @@ static __global__ void __launch_bounds__(32) restart_select_kernel(const double 
                                                                    int n_chains, int N, int NS, int reps, int motif, int32_t *out,
                                                                    int32_t *win_sites, double *win_scores, double *win_sum) {
     const int lane = threadIdx.x;
-    int best = -1;
-    double bsum = 0.0;
-    int r_next = 0;       // next restart to look at ...
-    long long n_next = 1; // ... and the iteration at which it sits in acc (restart 0 was run at iteration 0)
-    bool done = false;
-    while (!done && r_next < n_chains) {
-        const int r = r_next + lane;
-        const bool valid = r < n_chains;
-        const double s = valid ? sums[r] : 0.0;
-        const long long nj = n_next + lane;
-        const unsigned evs = __ballot_sync(FULL, valid && (nj > (long long)reps || s == bsum || s > bsum));
-        if (!evs) { // 32 restarts that are neither promoted nor equal to the best: one iteration each
-            const int cnt = min(32, n_chains - r_next);
-            r_next += cnt;
-            n_next += cnt;
-            continue;
-        }
-        const int j = __ffs(evs) - 1;
-        const int r_j = r_next + j;
-        const long long n_j = n_next + j;
-        const double s_j = __shfl_sync(FULL, s, j);
-        if (n_j > (long long)reps) break; // n > reps: the restart in acc is returned past, never compared
-        if (s_j == bsum) {                // acc = best? structural equality of the two arrays (F# (=): NaN <> NaN)
-            bool same;
-            if (best < 0) {
-                same = N == 1 && scores[(size_t)r_j * N] == 0.0 && sites[(size_t)r_j * NS] == (motif ? -1 : 0);
-            } else {
-                bool diff = false;
-                for (int i = lane; i < N; i += 32) diff |= !(scores[(size_t)r_j * N + i] == scores[(size_t)best * N + i]);
-                for (int i = lane; i < NS; i += 32) diff |= sites[(size_t)r_j * NS + i] != sites[(size_t)best * NS + i];
-                same = !__any_sync(FULL, diff);
-            }
-            if (same) break;
-            r_next = r_j + 1; // not promoted: the next restart is run at iteration n_j and sits in acc at n_j + 1
-            n_next = n_j + 1;
-            continue;
-        }
-        // promotion: best <- acc costs iteration n_j; the next restart is run at n_j + 1 and sits in acc at n_j + 2
-        best = r_j;
-        bsum = s_j;
-        if (bsum < 0.0) done = true; // `0. > sum best`: the loop promotes the empty acc until n > reps; nothing else runs
-        r_next = r_j + 1;
-        n_next = n_j + 2;
-    }
-    if (lane == 0) {
-        out[0] = best;
-        *win_sum = best < 0 ? 0.0 : sums[best];
-    }
-    // (no winner: -1 = no site, so that the PWM counts of the result are all zero)
-    for (int i = lane; i < NS; i += 32) win_sites[i] = best >= 0 ? sites[(size_t)best * NS + i] : -1;
-    for (int i = lane; i < N; i += 32) win_scores[i] = best >= 0 ? scores[(size_t)best * N + i] : 0.0;
+#include "gibbs_restart_select_body.inc" // (shared with restart_select_batch_kernel, gibbs_batch.cuh)
 }
 
 // element `which` of every Positions pair: the site arrays the one-site kernels take

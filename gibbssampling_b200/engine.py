@@ -412,6 +412,127 @@ class MultiEngine:
         return BestResult(sites[: n_out.value], scores[: n_out.value], total.value, int(restart.value), counts, stats)
 
 
+def flatten_sets(sets: Sequence[Sequence]) -> tuple[np.ndarray, np.ndarray, np.ndarray]:
+    """S sets of sequences -> (symbols, int64 offsets[n_seqs + 1], int32 set_offsets[S + 1]) of gibbs_batch_create.
+    Raises GibbsArgumentError for a null or empty list of sets and for an empty set."""
+    if sets is None:
+        raise _abi.GibbsArgumentError(_abi.GIBBS_ERR_ARG, "sets is null (ArgumentNullException)")
+    sets = list(sets)
+    if not sets:
+        raise _abi.GibbsArgumentError(_abi.GIBBS_ERR_ARG, "a batch needs at least one set")
+    set_off = np.zeros(len(sets) + 1, dtype=np.int32)
+    flat = []
+    for s, src in enumerate(sets):
+        if src is None:
+            raise _abi.GibbsArgumentError(_abi.GIBBS_ERR_ARG, f"set {s} is null (ArgumentNullException)")
+        src = list(src)
+        if not src:
+            raise _abi.GibbsArgumentError(_abi.GIBBS_ERR_ARG, f"set {s} is empty")
+        flat.extend(src)
+        set_off[s + 1] = set_off[s] + len(src)
+    buf, off = flatten_sources(flat)
+    return buf, off, set_off
+
+
+@dataclass
+class BatchRunResult:
+    """Every restart of every set: list entry s holds set s (sites / scores [R, N_s], sums [R])."""
+    sites: list
+    scores: list
+    sums: list
+    stats: dict
+
+
+class BatchEngine:
+    """Many independent sets of sequences (gibbs_batch_*): their restarts run together in a few launches; set s gives
+    exactly what a GibbsEngine over sets[s] alone gives for the same parameters, seed and chain_id_base."""
+
+    def __init__(self, sets: Sequence[Sequence], device: int = 0):
+        self._lib = _abi.load()
+        self._b = C.c_void_p()
+        buf, off, set_off = flatten_sets(sets)
+        self.n_sets = len(set_off) - 1
+        self.set_offsets = set_off.astype(np.int64)
+        self.sizes = np.diff(self.set_offsets)
+        _abi.check(self._lib.gibbs_batch_create(_ptr(buf, C.c_uint8), _ptr(off, C.c_int64), _ptr(set_off, C.c_int32),
+                                                C.c_int32(self.n_sets), C.c_int32(device), C.byref(self._b)))
+        self.device = device
+        self._last = None
+
+    def close(self) -> None:
+        if getattr(self, "_b", None) is not None and self._b.value:
+            self._lib.gibbs_batch_destroy(self._b)
+            self._b = C.c_void_p()
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *exc):
+        self.close()
+
+    def run_device(self, params: Params, restarts_per_set: int, *, bg_per_set=None, chain_id_base: int = 0, seed: int = 0) -> None:
+        """restarts_per_set restarts of every set; bg_per_set = [n_sets][4] backgrounds of the fixed-background family
+        (None = params.bg for every set). Results stay in HBM until fetch() / fetch_best()."""
+        bg = None
+        if bg_per_set is not None:
+            bg = np.ascontiguousarray(bg_per_set, dtype=np.float64)
+            if bg.shape != (self.n_sets, 4):
+                raise _abi.GibbsArgumentError(_abi.GIBBS_ERR_ARG, f"bg_per_set must be [{self.n_sets}][4]")
+        _abi.check(self._lib.gibbs_batch_run_device(self._b, C.byref(params), _ptr(bg, C.c_double), C.c_int32(restarts_per_set),
+                                                    C.c_int64(chain_id_base), C.c_uint64(seed)))
+        self._last = (int(restarts_per_set), int(params.k))
+
+    def _need_run(self) -> tuple[int, int]:
+        if self._last is None:
+            raise _abi.GibbsArgumentError(_abi.GIBBS_ERR_ARG, "no run_device on this batch yet")
+        return self._last
+
+    def fetch(self) -> BatchRunResult:
+        R, _ = self._need_run()
+        total = int(self.set_offsets[-1])
+        sites = np.zeros(R * total, dtype=np.int32)
+        scores = np.zeros(R * total, dtype=np.float64)
+        sums = np.zeros((self.n_sets, R), dtype=np.float64)
+        st = RunStats()
+        _abi.check(self._lib.gibbs_batch_fetch(self._b, _ptr(sites, C.c_int32), _ptr(scores, C.c_double), _ptr(sums, C.c_double),
+                                               C.byref(st)))
+        out_sites, out_scores = [], []
+        for s in range(self.n_sets):
+            a, n = R * int(self.set_offsets[s]), int(self.sizes[s])
+            out_sites.append(sites[a: a + R * n].reshape(R, n))
+            out_scores.append(scores[a: a + R * n].reshape(R, n))
+        stats = {f: getattr(st, f) for f, _ in RunStats._fields_}
+        return BatchRunResult(out_sites, out_scores, [sums[s] for s in range(self.n_sets)], stats)
+
+    def fetch_best(self, repetitions: int, *, want_counts: bool = False) -> list[BestResult]:
+        """The promote-or-restart loop of fs:435-459 of every set, decided on the GPU: one BestResult per set."""
+        _, k = self._need_run()
+        total = int(self.set_offsets[-1])
+        sites = np.zeros(total, dtype=np.int32)
+        scores = np.zeros(total, dtype=np.float64)
+        n_out = np.zeros(self.n_sets, dtype=np.int32)
+        sums = np.zeros(self.n_sets, dtype=np.float64)
+        restart = np.zeros(self.n_sets, dtype=np.int32)
+        counts = np.zeros((self.n_sets, k, 4), dtype=np.int32) if want_counts else None
+        st = RunStats()
+        _abi.check(self._lib.gibbs_batch_fetch_best(self._b, C.c_int32(repetitions), _ptr(sites, C.c_int32), _ptr(scores, C.c_double),
+                                                    _ptr(n_out, C.c_int32), _ptr(sums, C.c_double), _ptr(restart, C.c_int32),
+                                                    _ptr(counts, C.c_int32), C.byref(st)))
+        stats = {f: getattr(st, f) for f, _ in RunStats._fields_}
+        out = []
+        for s in range(self.n_sets):
+            a, n = int(self.set_offsets[s]), int(n_out[s])
+            out.append(BestResult(sites[a: a + n].copy(), scores[a: a + n].copy(), float(sums[s]), int(restart[s]),
+                                  counts[s] if counts is not None else None, stats))
+        return out
+
+
 def device_count() -> int:
     return int(_abi.load().gibbs_device_count())
 

@@ -297,6 +297,35 @@ int32_t gibbs_multi_fetch_best(gibbs_multi *m, int32_t repetitions, int32_t *sit
                                int32_t *n_out, double *sum_out, int32_t *restart_out, int32_t *counts_out,
                                gibbs_run_stats *stats_out);
 
+/* ---- many independent sequence sets in one launch ------------------------------------------------------------- */
+/*
+ * Replaces: a loop of getMotifsWithBestInformationContentWithBPV (fs:434-459) or getMotifsWithBestInformationContent
+ * (fs:615-640) calls over many small sets, e.g. one discovery run per gene group or promoter region (fsx:223-365).
+ * A batch holds S sets that share one gibbs_params; each set runs restarts_per_set restarts of the SiteSampler pipeline
+ * and restart r of EVERY set uses the uniform stream (seed, chain_id_base + r). Set s gives bit for bit what a handle
+ * created from set s alone gives for gibbs_run_device(h_s, p_s, restarts_per_set, chain_id_base, seed, GIBBS_RNG_PHILOX,
+ * NULL, 0), p_s being p with bg = bg_per_set[s]. The restarts of all sets run in a few launches on one stream.
+ * seqs / offsets as for gibbs_create over the concatenation of all sets; set s = sequences set_offsets[s] ..
+ * set_offsets[s+1]-1 (int32 set_offsets[n_sets + 1], set_offsets[0] = 0, no empty set).
+ * Errors follow the single-set rules per set and name the set (and sequence); a failed call leaves the batch usable.
+ * The MotifSampler, phase_mask, start states, start PPMs and injected uniforms are not part of this API.
+ */
+typedef struct gibbs_batch gibbs_batch;
+int32_t gibbs_batch_create(const uint8_t *seqs, const int64_t *offsets, const int32_t *set_offsets, int32_t n_sets,
+                           int32_t device, gibbs_batch **out);
+int32_t gibbs_batch_destroy(gibbs_batch *b);
+/* restarts_per_set restarts of every set; bg_per_set double [n_sets][4] for GIBBS_BG_FIXED (NULL = p->bg for every set) */
+int32_t gibbs_batch_run_device(gibbs_batch *b, const gibbs_params *p, const double *bg_per_set, int32_t restarts_per_set,
+                               int64_t chain_id_base, uint64_t seed);
+/* every restart of the last run (any may be NULL): sites_out int32 / scores_out double [sum_s R N_s], set-major then
+ * restart-major (set s starts at R * set_offsets[s]); sums_out double [n_sets][R]; stats summed over the sets */
+int32_t gibbs_batch_fetch(gibbs_batch *b, int32_t *sites_out, double *scores_out, double *sums_out, gibbs_run_stats *stats_out);
+/* the promote-or-restart loop (fs:435-459) of every set, decided on the device (see gibbs_fetch_best); any may be NULL:
+ * sites_out int32 / scores_out double [sum_s N_s] (set s at set_offsets[s], n_out[s] entries valid), n_out int32 [n_sets],
+ * sum_out double [n_sets], restart_out int32 [n_sets] (-1 = the initial value), counts_out int32 [n_sets][k][4] */
+int32_t gibbs_batch_fetch_best(gibbs_batch *b, int32_t repetitions, int32_t *sites_out, double *scores_out, int32_t *n_out,
+                               double *sum_out, int32_t *restart_out, int32_t *counts_out, gibbs_run_stats *stats_out);
+
 /* ---- host buffers ------------------------------------------------------------------------------- */
 /* Page-locked host memory for the *_out arrays above (results of 1024 chains x 1000 sequences are
  * 12 MB; into pageable memory the copy is staged by the driver and pays first-touch page faults).
