@@ -18,6 +18,7 @@
 #include <cstdlib>
 #include <cstring>
 #include <new>
+#include <type_traits>
 #include <vector>
 
 namespace gibbs { // gibbs_chain_tu.cu, one translation unit per group of chain_kernel instantiations (_build.py)
@@ -94,10 +95,18 @@ int32_t fail(int32_t code, const char *fmt, ...) {
                         cudaGetErrorString(e_));                                                           \
     } while (0)
 
+// Device buffer owned by a handle. The owner's destroy function makes the handle's device current before the
+// destructors run.
 template <typename T>
 struct DevBuf {
     T *p = nullptr;
     size_t cap = 0; // elements
+    DevBuf() = default;
+    DevBuf(const DevBuf &) = delete;
+    DevBuf &operator=(const DevBuf &) = delete;
+    ~DevBuf() {
+        if (p) cudaFree(p);
+    }
     cudaError_t reserve(size_t n) {
         if (n <= cap) return cudaSuccess;
         if (p) cudaFree(p);
@@ -106,11 +115,6 @@ struct DevBuf {
         cudaError_t e = cudaMalloc(&p, n * sizeof(T));
         if (e == cudaSuccess) cap = n;
         return e;
-    }
-    void release() {
-        if (p) cudaFree(p);
-        p = nullptr;
-        cap = 0;
     }
 };
 
@@ -192,7 +196,6 @@ struct gibbs_handle {
     int32_t opt_cluster = 8;           // largest cluster the last hand-over stages may use: 0 (none), 4 or 8 (GIBBS_OPT_CLUSTER)
     int32_t cluster_cap[2] = {-1, -1}; // clusters of 4 / 8 CTAs the device holds at once (queried once per shape)
     int32_t cluster_cap_n = 0, cluster_cap_rw = 0, cluster_cap_k = 0;
-    int32_t run_stages = 0;            // launches of the chain kernel family in the last run
     int32_t wt_span = 0, drift_span = 0; // counts the W / PPM value tables cover: n (one site per sequence) or 2 n
     DevBuf<int32_t> pos2;              // motifAmount = 2: Positions [chains][n][2], newest first
     DevBuf<double> sc2;                // motifAmount = 2: window products of the current held-out sequence, per chain
@@ -234,6 +237,10 @@ int32_t check_params(const gibbs_handle *h, const gibbs_params *p) {
     return GIBBS_OK;
 }
 
+// normalizePPM of a set of n sequences: sum = float sourceCount + float alphabet.Length * pseudoCount (fs:257), with
+// sourceCount = n - 1 sites
+double ppm_den(int n, const gibbs_params *p) { return (double)(n - 1) + ((double)p->alphabet_size * p->pseudocount); }
+
 // (re)build W(c, b) for c = 0..n-1 when the parameters it depends on changed
 // span = how many counts the table covers: n, or 2 n when a sequence may contribute two sites (motifAmount = 2)
 int32_t ensure_wtab(gibbs_handle *h, const gibbs_params *p, int *launches, int span_mult = 1) {
@@ -244,8 +251,7 @@ int32_t ensure_wtab(gibbs_handle *h, const gibbs_params *p, int *launches, int s
     CUDA_TRY(h->wtab.reserve((size_t)span * 4));
     const int init[3] = {INT32_MAX, INT32_MIN, 0};
     CUDA_TRY(cudaMemcpyAsync(h->flags.p + 1, init, sizeof init, cudaMemcpyHostToDevice, h->stream));
-    // normalizePPM: sum = float sourceCount + float alphabet.Length * pseudoCount (fs:257)
-    const double den = (double)(h->n - 1) + ((double)p->alphabet_size * p->pseudocount);
+    const double den = ppm_den(h->n, p);
     const int total = span * 4;
     wtab_kernel<<<(total + 255) / 256, 256, 0, h->stream>>>(span, p->pseudocount, den, p->bg[0], p->bg[1], p->bg[2],
                                                            p->bg[3], h->wtab.p, h->flags.p + 1);
@@ -276,7 +282,9 @@ int fast_path_ok_range(int abnormal, int wt_min, int wt_max, int k) {
 }
 int fast_path_ok(const gibbs_handle *h, int k) { return fast_path_ok_range(h->wt_abnormal, h->wt_min, h->wt_max, k); }
 
-// the ranking pass of the drifting background (see gibbs_run_device): every odds ratio lies in [pc / den, den / pc]
+// The ranking pass of the drifting background is valid when every odds ratio ppm / pcv, which lies in [pc / den, den / pc]
+// with den <= all bases of the set + one more sequence + |A| pc (or N - 1 + |A| pc), keeps every float64 product of k of
+// them in the normal range (|log2| < 1000), and pc >= 1e-30 keeps every float32 logarithm argument normal and finite.
 int drift_fast_path_ok(const int32_t gcnt[4], int32_t max_len, int32_t n, const gibbs_params *p) {
     const double alpha_pc = (double)p->alphabet_size * p->pseudocount;
     const double bases = (double)gcnt[0] + gcnt[1] + gcnt[2] + gcnt[3] + (double)max_len;
@@ -292,26 +300,85 @@ int32_t set_smem(K kernel, int bytes) {
 
 #define KP_CASES(X) X(1) X(2) X(3) X(4) X(5) X(6) X(7) X(8) X(9) X(10) X(11) X(12) X(13) X(14) X(15) X(16)
 
-// Warps per chain. Four warps work on four consecutive held-out sequences of the chain at once, which
-// shortens every chain's critical path (measured faster than one warp per chain both when all chains
-// are resident at once -- C2 -- and when they run in several waves); one warp is kept for sets with
-// fewer than 4 sequences or rows too long for four sets of staging buffers.
-// one stage of a run: the chain_kernel group for (warps per chain, masked symbols, drifting background)
-int32_t launch_team(gibbs_handle *h, int team, bool masked, bool drift, const ChainArgs &a, int grid) {
+// f(std::integral_constant<int, KP>()) with KP = (k + 1) / 2, the template argument of the kernels that hold a k-mer
+template <typename F>
+int32_t with_kp(int k, F &&f) {
+    switch ((k + 1) / 2) {
+#define X(KPV) case KPV: return f(std::integral_constant<int, KPV>());
+        KP_CASES(X)
+#undef X
+    default: return fail(GIBBS_ERR_ARG, "unsupported k");
+    }
+}
+
+// one CTA of one warp with the staging buffers of a one-warp team (the primitives)
+template <typename K, typename... A>
+int32_t launch_one_warp(gibbs_handle *h, K kernel, int row_words, const A &...args) {
+    const int smem = team_smem_bytes(row_words, 1);
+    const int32_t rc = set_smem(kernel, smem);
+    if (rc) return rc;
+    kernel<<<1, 32, smem, h->stream>>>(args...);
+    CUDA_TRY(cudaGetLastError());
+    return GIBBS_OK;
+}
+
+// The unit of a kernel family (_build.py) that holds the instantiation for (warps per chain, masked symbols, drifting
+// background, random starts only).
+template <typename F>
+struct Unit {
+    int team, masked, drift, init;
+    F launch;
+};
+
+template <typename F, size_t U>
+int32_t find_unit(const Unit<F> (&units)[U], const char *family, int team, bool masked, bool drift, bool init, F *out) {
+    for (const Unit<F> &u : units)
+        if (u.team == team && u.masked == masked && u.drift == drift && u.init == init) {
+            *out = u.launch;
+            return GIBBS_OK;
+        }
+    return fail(GIBBS_ERR_ARG, "no %s kernel is built for %d warps per chain (masked symbols %d, drifting background %d, "
+                               "random starts only %d)", family, team, masked, drift, init);
+}
+
+using ChainLaunch = cudaError_t (*)(const ChainArgs &, int, int, cudaStream_t);
+const Unit<ChainLaunch> CHAIN_UNITS[] = {
+    {1, 0, 0, 0, launch_chain_t1}, {4, 0, 0, 0, launch_chain_t4}, {8, 0, 0, 0, launch_chain_t8}, {16, 0, 0, 0, launch_chain_t16},
+    {1, 0, 1, 0, launch_chain_drift_t1}, {4, 0, 1, 0, launch_chain_drift_t4}, {8, 0, 1, 0, launch_chain_drift_t8},
+    {1, 1, 0, 0, launch_chain_masked_t1}, {4, 1, 0, 0, launch_chain_masked_t4},
+    {1, 1, 1, 0, launch_chain_masked_drift_t1}, {4, 1, 1, 0, launch_chain_masked_drift_t4},
+    {1, 0, 0, 1, launch_chain_init_t1}, {4, 0, 0, 1, launch_chain_init_t4},
+    {1, 0, 1, 1, launch_chain_init_drift_t1}, {4, 0, 1, 1, launch_chain_init_drift_t4},
+    {1, 1, 0, 1, launch_chain_init_masked_t1}, {4, 1, 0, 1, launch_chain_init_masked_t4},
+    {1, 1, 1, 1, launch_chain_init_masked_drift_t1}, {4, 1, 1, 1, launch_chain_init_masked_drift_t4},
+};
+
+// the MotifSampler units serve both backgrounds and continue from the random starts wherever those ran
+using MotifLaunch = cudaError_t (*)(const MotifArgs &, int, int, cudaStream_t);
+const Unit<MotifLaunch> MOTIF_UNITS[] = {
+    {1, 0, 0, 0, launch_motif_t1}, {4, 0, 0, 0, launch_motif_t4}, {8, 0, 0, 0, launch_motif_t8}, {16, 0, 0, 0, launch_motif_t16},
+    {1, 1, 0, 0, launch_motif_masked_t1}, {4, 1, 0, 0, launch_motif_masked_t4},
+};
+
+using BatchLaunch = cudaError_t (*)(const ChainArgs &, const BatchTable &, int, int, cudaStream_t);
+const Unit<BatchLaunch> BATCH_UNITS[] = {
+    {1, 0, 0, 0, launch_batch_t1}, {4, 0, 0, 0, launch_batch_t4}, {1, 0, 1, 0, launch_batch_drift_t1}, {4, 0, 1, 0, launch_batch_drift_t4},
+    {1, 1, 0, 0, launch_batch_masked_t1}, {4, 1, 0, 0, launch_batch_masked_t4},
+    {1, 1, 1, 0, launch_batch_masked_drift_t1}, {4, 1, 1, 0, launch_batch_masked_drift_t4},
+    {1, 0, 0, 1, launch_batch_init_t1}, {4, 0, 0, 1, launch_batch_init_t4},
+    {1, 0, 1, 1, launch_batch_init_drift_t1}, {4, 0, 1, 1, launch_batch_init_drift_t4},
+    {1, 1, 0, 1, launch_batch_init_masked_t1}, {4, 1, 0, 1, launch_batch_init_masked_t4},
+    {1, 1, 1, 1, launch_batch_init_masked_drift_t1}, {4, 1, 1, 1, launch_batch_init_masked_drift_t4},
+};
+
+// one launch of the chain_kernel unit for (warps per chain, masked symbols, drifting background, random starts only)
+int32_t launch_chain_unit(gibbs_handle *h, int team, bool masked, bool drift, bool init, const ChainArgs &a, int grid) {
     const int smem = team_smem_bytes(a.s.row_words, team);
     if (smem > 200 * 1024) return fail(GIBBS_ERR_ARG, "sequences too long for %d warps per chain", team);
-    cudaError_t e = cudaErrorInvalidValue;
-    if (masked && drift)
-        e = team == 4 ? launch_chain_masked_drift_t4(a, grid, smem, h->stream) : launch_chain_masked_drift_t1(a, grid, smem, h->stream);
-    else if (masked) e = team == 4 ? launch_chain_masked_t4(a, grid, smem, h->stream) : launch_chain_masked_t1(a, grid, smem, h->stream);
-    else if (drift)
-        e = team == 8 ? launch_chain_drift_t8(a, grid, smem, h->stream)
-            : team == 4 ? launch_chain_drift_t4(a, grid, smem, h->stream) : launch_chain_drift_t1(a, grid, smem, h->stream);
-    else
-        e = team == 16 ? launch_chain_t16(a, grid, smem, h->stream)
-            : team == 8 ? launch_chain_t8(a, grid, smem, h->stream)
-            : team == 4 ? launch_chain_t4(a, grid, smem, h->stream) : launch_chain_t1(a, grid, smem, h->stream);
-    CUDA_TRY(e);
+    ChainLaunch f;
+    const int32_t rc = find_unit(CHAIN_UNITS, "chain", team, masked, drift, init, &f);
+    if (rc) return rc;
+    CUDA_TRY(f(a, grid, smem, h->stream));
     return GIBBS_OK;
 }
 
@@ -322,19 +389,19 @@ int32_t launch_team(gibbs_handle *h, int team, bool masked, bool drift, const Ch
 //                     against the chain kernel's INIT sweep)
 //   GIBBS_INIT_CHAIN  inside the chain kernel: many chains of few sequences whose set does not fit
 // Launches the grid-wide kernel if one is chosen and clears GIBBS_PHASE_INIT from a.phase_mask.
-template <int KPV>
 int32_t launch_random_starts(gibbs_handle *h, ChainArgs &a, bool drift) {
     const bool masked = a.s.mask != nullptr; // symbols outside A,C,G,T: inside the MASKED chain kernel
+    const int kp = (a.k + 1) / 2;
     int init_path = GIBBS_INIT_CHAIN, tile_rows = 0;
     if ((a.phase_mask & GIBBS_PHASE_INIT) && !masked) {
-        const bool smem_ok = !drift && init_smem_total_bytes(a.s.n, a.s.row_words, KPV) <= h->smem_optin;
+        const bool smem_ok = !drift && init_smem_total_bytes(a.s.n, a.s.row_words, kp) <= h->smem_optin;
         const bool smem_fits = smem_ok && (long long)a.n_chains * a.s.n >= (long long)h->sm_count * ISM_WARPS;
         const bool wide_fits = init_smem_bytes(a.s.row_words) <= 200 * 1024;
         const bool wide_wins = a.n_chains < 4 * h->sm_count || a.s.n >= 4096 || a.sampler == GIBBS_MOTIF_SAMPLER;
         init_path = smem_fits ? GIBBS_INIT_SMEM : (wide_fits && wide_wins) ? GIBBS_INIT_WIDE : GIBBS_INIT_CHAIN;
         // the set streamed through shared memory in tiles: the Philox stream, fixed background, at least 256 sequences per
         // tile; chosen by itself where the global gathers of the wide kernel are the limit (many sequences, work for every SM)
-        tile_rows = (int)(((long long)h->smem_optin - 128 - 256 - (long long)TILED_WARPS * (ism_table_bytes(KPV) + a.s.row_words * 4)) / 2
+        tile_rows = (int)(((long long)h->smem_optin - 128 - 256 - (long long)TILED_WARPS * (ism_table_bytes(kp) + a.s.row_words * 4)) / 2
                           / ((long long)a.s.row_words * 4));
         const bool tile_auto = tile_rows >= 256;
         if (tile_rows > a.s.n) tile_rows = a.s.n;
@@ -349,7 +416,7 @@ int32_t launch_random_starts(gibbs_handle *h, ChainArgs &a, bool drift) {
     }
     h->run_init_path = init_path;
     if (init_path == GIBBS_INIT_TILED) {
-        const int smem = (int)init_tiled_total_bytes(tile_rows, a.s.row_words, KPV);
+        const int smem = (int)init_tiled_total_bytes(tile_rows, a.s.row_words, kp);
         const long long items = (long long)a.n_chains * a.s.n;
         long long grid = (items + TILED_WARPS - 1) / TILED_WARPS;
         if (grid > h->sm_count) grid = h->sm_count;
@@ -358,7 +425,7 @@ int32_t launch_random_starts(gibbs_handle *h, ChainArgs &a, bool drift) {
         h->run_extra_launches += 1;
     } else
     if (init_path == GIBBS_INIT_SMEM) {
-        const int smem = (int)init_smem_total_bytes(a.s.n, a.s.row_words, KPV);
+        const int smem = (int)init_smem_total_bytes(a.s.n, a.s.row_words, kp);
         const long long items = (long long)a.n_chains * a.s.n;
         long long grid = (items + ISM_WARPS - 1) / ISM_WARPS;
         if (grid > h->sm_count) grid = h->sm_count;
@@ -390,73 +457,76 @@ int32_t launch_random_starts(gibbs_handle *h, ChainArgs &a, bool drift) {
         h->run_extra_launches += 1;
     } else if (a.phase_mask & GIBBS_PHASE_INIT) { // on the chain's own team: one CTA of 4 warps (or 1) per chain
         const int team = (a.s.n >= 4 && team_smem_bytes(a.s.row_words, 4) <= 200 * 1024 && h->team_warps != 1) ? 4 : 1;
-        const int smem = team_smem_bytes(a.s.row_words, team);
-        if (smem > 200 * 1024) return fail(GIBBS_ERR_ARG, "sequences too long for shared-memory staging");
         ChainArgs b = a;
         b.from_list = 0;
         b.pause_below = 0;
-        cudaError_t e;
-        if (masked && drift) e = team == 4 ? launch_chain_init_masked_drift_t4(b, a.n_chains, smem, h->stream) : launch_chain_init_masked_drift_t1(b, a.n_chains, smem, h->stream);
-        else if (masked) e = team == 4 ? launch_chain_init_masked_t4(b, a.n_chains, smem, h->stream) : launch_chain_init_masked_t1(b, a.n_chains, smem, h->stream);
-        else if (drift) e = team == 4 ? launch_chain_init_drift_t4(b, a.n_chains, smem, h->stream) : launch_chain_init_drift_t1(b, a.n_chains, smem, h->stream);
-        else e = team == 4 ? launch_chain_init_t4(b, a.n_chains, smem, h->stream) : launch_chain_init_t1(b, a.n_chains, smem, h->stream);
-        CUDA_TRY(e);
+        const int32_t rc = launch_chain_unit(h, team, masked, drift, true, b, a.n_chains);
+        if (rc) return rc;
         a.phase_mask &= ~GIBBS_PHASE_INIT;
         h->run_extra_launches += 1;
     }
     return GIBBS_OK;
 }
 
-int32_t launch_random_starts_any(gibbs_handle *h, ChainArgs &a, bool drift) {
-    switch ((a.k + 1) / 2) {
-#define X(KPV) case KPV: return launch_random_starts<KPV>(h, a, drift);
-        KP_CASES(X)
-#undef X
-    default: return fail(GIBBS_ERR_ARG, "unsupported k");
-    }
-}
+// One launch of a run. Its chains pause at their next sweep boundary once fewer than pause_below are still running
+// (0 = run to the end) and the next stage continues them; cluster: CTAs per thread-block cluster (0 = one CTA per chain);
+// min_sweeps: sweeps a chain runs in the stage before it may pause; min_width: ChainArgs::min_width.
+struct Stage {
+    int team, pause_below, cluster, min_sweeps, min_width;
+};
+constexpr int MAX_STAGES = 8; // the control words hold one count per stage
 
-template <int KPV>
-int32_t launch_chain_kp(gibbs_handle *h, ChainArgs a, bool drift) {
-    h->run_extra_launches = 0;
-    const bool masked = a.s.mask != nullptr; // one launch of the MASKED instantiation (1 or 4 warps)
-    {
-        const int32_t rc = launch_random_starts<KPV>(h, a, drift);
-        if (rc) return rc;
-    }
-    // Warps per chain and the straggler hand-over. Chains need very different numbers of sweeps, so a
-    // one-wave launch ends with a few chains running on a mostly idle GPU. Stage 1 runs every chain with 4
-    // warps (7 chains per SM); once <= 2 chains per SM are still running they pause at their next sweep
-    // boundary and stage 2 continues them with 8 warps; once <= 1 chain per SM is left, stage 3 continues
-    // with 16 warps. Late sweeps move few sites, so the wider speculative rounds are rarely discarded.
-    const int N = a.s.n, sms = h->sm_count;
+// The stages of a run of either sampler (a: after the random starts).
+// Warps per chain. Four warps work on four consecutive held-out sequences of the chain at once, which
+// shortens every chain's critical path (measured faster than one warp per chain both when all chains
+// are resident at once -- C2 -- and when they run in several waves); one warp is kept for sets with
+// fewer than 4 sequences or rows too long for four sets of staging buffers.
+// Chains need very different numbers of sweeps, so a one-wave launch ends with a few chains running on a mostly idle GPU.
+// Stage 1 runs every chain with 4 warps (7 chains per SM); once <= opt_stage2_at chains per SM are still running they
+// pause at their next sweep boundary and stage 2 continues them with 8 warps; once <= opt_stage3_at chains per SM are
+// left, stage 3 continues with 16 warps. Runs with fewer chains start on the wider teams: those are used only while warp
+// slots are idle. Late sweeps move few sites, so the wider speculative rounds are rarely discarded.
+int plan_stages(gibbs_handle *h, const ChainArgs &a, bool drift, Stage *stages) {
+    const int N = a.s.n, sms = h->sm_count, chains = a.n_chains;
+    const bool masked = a.s.mask != nullptr;
     auto fits = [&](int t) { return N >= t && team_smem_bytes(a.s.row_words, t) <= 200 * 1024; };
-    struct Stage { int team, pause_below, cluster, min_sweeps; };
-    Stage stages[8] = {};
-    int n_stages = 0;
-    if (masked) {
-        stages[n_stages++] = {team_smem_bytes(a.s.row_words, 4) <= 200 * 1024 ? 4 : 1, 0, 0};
+    auto widest_fit = [&](int t) { // 16 -> 8 -> 4 -> 1 warps
+        while (t > 1 && !fits(t)) t = t > 4 ? t / 2 : 1;
+        return t;
+    };
+    int n = 0;
+    auto widen = [&](int at8, int at16) { // the last chains continue on 8, then on 16 warps (at16 = 0: no 16-warp stage)
+        if (stages[n - 1].team == 4 && fits(8)) {
+            stages[n - 1].pause_below = at8;
+            stages[n++] = {8};
+        }
+        if (at16 > 0 && stages[n - 1].team == 8 && fits(16)) {
+            stages[n - 1].pause_below = at16;
+            stages[n++] = {16};
+        }
+    };
+    const int at8 = h->opt_stage2_at * sms, at16 = h->opt_stage3_at * sms;
+    const int first = widest_fit(chains > at8 ? 4 : chains > at16 ? 8 : 16);
+    if (a.sampler == GIBBS_MOTIF_SAMPLER) {
+        // (One warp per restart for the first greedy sweeps, as the SiteSampler runs them, was measured here too: the sweeps
+        // themselves gain 1.4 ms on C2, the two hand-overs around them cost 2.5 ms -- tools/experiments/README.md.)
+        if (masked || h->team_warps != 0 || !fits(4)) { // one stage (a forced team of 8 or 16 warps runs on 4)
+            stages[n++] = {h->team_warps != 1 && fits(4) ? 4 : 1};
+        } else {
+            stages[n++] = {first};
+            widen(at8, at16);
+        }
+        return n; // (min_width stays 0)
+    }
+    if (masked) { // one launch of the MASKED instantiation (1 or 4 warps)
+        stages[n++] = {team_smem_bytes(a.s.row_words, 4) <= 200 * 1024 ? 4 : 1};
     } else if (drift) { // data-derived background: 4 warps per chain (4 chains per SM), the last 2 per SM continue with 8
         const int forced = h->team_warps == 16 ? 8 : h->team_warps;
-        if (forced != 0) {
-            stages[n_stages++] = {forced, 0, 0};
-        } else {
-            int first = a.n_chains > 2 * sms ? 4 : 8;
-            if (first == 8 && !fits(8)) first = 4;
-            if (first == 4 && !fits(4)) first = 1;
-            stages[n_stages++] = {first, 0, 0};
-            if (first == 4 && fits(8)) {
-                stages[n_stages - 1].pause_below = 2 * sms;
-                stages[n_stages++] = {8, 0, 0};
-            }
-        }
+        stages[n++] = {forced != 0 ? forced : widest_fit(chains > 2 * sms ? 4 : 8)};
+        if (forced == 0) widen(2 * sms, 0);
     } else if (h->team_warps != 0) {
-        stages[n_stages++] = {h->team_warps, 0, 0};
+        stages[n++] = {h->team_warps};
     } else {
-        int first = a.n_chains > h->opt_stage2_at * sms ? 4 : a.n_chains > h->opt_stage3_at * sms ? 8 : 16; // wider teams only while warp slots are idle
-        if (first == 16 && !fits(16)) first = 8;
-        if (first == 8 && !fits(8)) first = 4;
-        if (first == 4 && !fits(4)) first = 1;
         // The first greedy sweep moves a site in almost every update (C2: 99 %, then 28 % in sweep 1), so its rounds run at
         // width 1 and three warps of a four-warp team wait. One warp per chain with 128 registers and no team barrier runs
         // such a sweep faster (C2, sweeps 0 / 1 / 2 / 3 alone: 1.74 / 1.61 / 1.57 / 1.52 ms against 2.20 / 2.18 / 1.59 / 1.15 ms,
@@ -465,19 +535,12 @@ int32_t launch_chain_kp(gibbs_handle *h, ChainArgs a, bool drift) {
         // stage continues it. The hand-over itself costs ~0.3 ms (the slowest chain's sweep ends the launch), so whole C2
         // steps measure 23.76 / 23.18 / 23.48 / 24.2 ms for 0 / 1 / 2 / 3 such sweeps: the default is 1.
         if (first == 4 && N >= 64 && (a.phase_mask & GIBBS_PHASE_GREEDY) && h->opt_seq_sweeps > 0)
-            stages[n_stages++] = {1, a.n_chains, 0, h->opt_seq_sweeps};
-        stages[n_stages++] = {first, 0, 0};
-        if (first == 4 && fits(8)) {
-            stages[n_stages - 1].pause_below = h->opt_stage2_at * sms;
-            stages[n_stages++] = {8, 0, 0};
-        }
-        if (stages[n_stages - 1].team == 8 && fits(16)) {
-            stages[n_stages - 1].pause_below = h->opt_stage3_at * sms;
-            stages[n_stages++] = {16, 0, 0};
-        }
+            stages[n++] = {1, chains, 0, h->opt_seq_sweeps};
+        stages[n++] = {first};
+        widen(at8, at16);
         // With fewer chains than SMs left, one chain gets several SMs: a thread-block cluster of 4, then 8 CTAs of 16 warps
         // (chain_cluster_kernel). Needs the ranking pass, the W table in shared memory and rounds of 64 sequences to fill.
-        if (stages[n_stages - 1].team == 16 && h->opt_cluster >= 4 && a.fast_ok && N >= 128) {
+        if (stages[n - 1].team == 16 && h->opt_cluster >= 4 && a.fast_ok && N >= 128) {
             if (h->cluster_cap_n != N || h->cluster_cap_rw != a.s.row_words || h->cluster_cap_k != a.k) {
                 h->cluster_cap[0] = h->cluster_cap[1] = 0;
                 int cap = 0;
@@ -490,20 +553,36 @@ int32_t launch_chain_kp(gibbs_handle *h, ChainArgs a, bool drift) {
                 h->cluster_cap_n = N; h->cluster_cap_rw = a.s.row_words; h->cluster_cap_k = a.k;
             }
             if (h->cluster_cap[0] > 0) {
-                stages[n_stages - 1].pause_below = h->cluster_cap[0];
-                stages[n_stages++] = {16, 0, 4};
+                stages[n - 1].pause_below = h->cluster_cap[0];
+                stages[n++] = {16, 0, 4};
                 if (h->opt_cluster >= 8 && h->cluster_cap[1] > 0 && h->cluster_cap[1] < h->cluster_cap[0]) {
-                    stages[n_stages - 1].pause_below = h->cluster_cap[1];
-                    stages[n_stages++] = {16, 0, 8};
+                    stages[n - 1].pause_below = h->cluster_cap[1];
+                    stages[n++] = {16, 0, 8};
                 }
             }
         }
     }
-    h->run_team = stages[0].team == 1 && n_stages > 1 && stages[0].pause_below == a.n_chains ? 4 : stages[0].team; // (the team of the main stage)
-    h->run_stages = n_stages;
+    for (int st = 0; st < n; ++st) {
+        // chains that reach this stage per SM (at most): with an SM or more per chain, never narrow a speculative round
+        const int per_sm = ((st == 0 ? chains : stages[st - 1].pause_below) + sms - 1) / sms;
+        // Stages that share SMs (GIBBS_OPT_MIN_WIDTH): while the first sweep -- a mover in almost every update -- ran on the
+        // teams, narrowing after a discarded round saved the other chains' issue slots (width 1). With that sweep on
+        // stage 0 the remaining sweeps discard far less than they gain from never narrowing: C2 23.2 -> 22.6 ms.
+        const bool seq_stage = stages[0].team == 1 && stages[0].min_sweeps > 0;
+        stages[st].min_width = stages[st].cluster ? stages[st].cluster * 16 : per_sm <= 1 ? stages[st].team
+                               : h->opt_min_width >= 1 ? h->opt_min_width : seq_stage ? stages[st].team : 1;
+    }
+    return n;
+}
+
+// Runs the stages of a plan. Sets up the control words and the lists through which each stage hands its paused chains to
+// the next; launch(stage, args, grid) launches one stage on a grid of the chains the previous stage paused at most.
+template <typename Launch>
+int32_t run_stages(gibbs_handle *h, ChainArgs a, const Stage *stages, int n_stages, Launch &&launch) {
+    h->run_team = stages[0].min_sweeps > 0 ? stages[1].team : stages[0].team; // (the team of the main stage)
     // control words: [0] chains still running, [s] number of chains paused by stage s
-    CUDA_TRY(h->ctl.reserve(8));
-    const int32_t ctl0[8] = {a.n_chains, 0, 0, 0, 0, 0, 0, 0};
+    CUDA_TRY(h->ctl.reserve(MAX_STAGES));
+    const int32_t ctl0[MAX_STAGES] = {a.n_chains, 0, 0, 0, 0, 0, 0, 0};
     CUDA_TRY(cudaMemcpyAsync(h->ctl.p, ctl0, sizeof ctl0, cudaMemcpyHostToDevice, h->stream));
     a.active = h->ctl.p;
     if (n_stages > 1) {
@@ -515,97 +594,61 @@ int32_t launch_chain_kp(gibbs_handle *h, ChainArgs a, bool drift) {
         ChainArgs b = a;
         b.pause_below = stages[st].pause_below;
         b.pause_min_sweeps = stages[st].min_sweeps;
+        b.min_width = stages[st].min_width;
         b.from_list = st > 0;
-        {   // chains that reach this stage per SM (at most): with an SM or more per chain, never narrow a speculative round
-            const int per_sm = st == 0 ? (a.n_chains + sms - 1) / sms : (stages[st - 1].pause_below + sms - 1) / sms;
-            // Stages that share SMs (GIBBS_OPT_MIN_WIDTH): while the first sweep -- a mover in almost every update -- ran on the
-            // teams, narrowing after a discarded round saved the other chains' issue slots (width 1). With that sweep on
-            // stage 0 the remaining sweeps discard far less than they gain from never narrowing: C2 23.2 -> 22.6 ms.
-            const bool seq_stage = stages[0].team == 1 && stages[0].min_sweeps > 0;
-            b.min_width = stages[st].cluster ? stages[st].cluster * 16 : per_sm <= 1 ? stages[st].team
-                          : h->opt_min_width >= 1 ? h->opt_min_width : seq_stage ? stages[st].team : 1;
-        }
         b.pending_in = st > 0 ? h->pending.p + (size_t)(st - 1) * a.n_chains : nullptr;
         b.pending_in_n = st > 0 ? h->ctl.p + st : nullptr;
         b.pending_out = st + 1 < n_stages ? h->pending.p + (size_t)st * a.n_chains : nullptr;
         b.pending_out_n = st + 1 < n_stages ? h->ctl.p + st + 1 : nullptr;
-        const int grid = st == 0 ? a.n_chains : stages[st - 1].pause_below; // at most that many chains were paused
-        if (stages[st].cluster) {
-            CUDA_TRY(stages[st].cluster == 4 ? launch_chain_cluster4(b, grid, h->stream, nullptr) : launch_chain_cluster8(b, grid, h->stream, nullptr));
-        } else {
-            int32_t rc = launch_team(h, stages[st].team, masked, drift, b, grid);
-            if (rc) return rc;
-        }
+        const int32_t rc = launch(stages[st], b, st == 0 ? a.n_chains : stages[st - 1].pause_below);
+        if (rc) return rc;
         if (st > 0) h->run_extra_launches += 1;
     }
     return GIBBS_OK;
 }
 
-int32_t launch_chain(gibbs_handle *h, const ChainArgs &a, bool drift = false) {
-    const int kp = (a.k + 1) / 2;
-    switch (kp) {
-#define X(KPV) case KPV: return launch_chain_kp<KPV>(h, a, drift);
-        KP_CASES(X)
-#undef X
-    default: return fail(GIBBS_ERR_ARG, "unsupported k");
-    }
+int32_t launch_chain(gibbs_handle *h, ChainArgs a, bool drift) {
+    h->run_extra_launches = 0;
+    int32_t rc = launch_random_starts(h, a, drift);
+    if (rc) return rc;
+    Stage stages[MAX_STAGES] = {};
+    const int n_stages = plan_stages(h, a, drift, stages);
+    const bool masked = a.s.mask != nullptr;
+    return run_stages(h, a, stages, n_stages, [&](const Stage &s, const ChainArgs &b, int grid) -> int32_t {
+        if (s.cluster == 0) return launch_chain_unit(h, s.team, masked, drift, false, b, grid);
+        CUDA_TRY((s.cluster == 4 ? launch_chain_cluster4 : launch_chain_cluster8)(b, grid, h->stream, nullptr));
+        return GIBBS_OK;
+    });
+}
+
+// the stages of a MotifSampler run (m: after the random starts)
+int32_t launch_motif(gibbs_handle *h, const MotifArgs &m, const Stage *stages, int n_stages) {
+    const bool masked = m.c.s.mask != nullptr;
+    return run_stages(h, m.c, stages, n_stages, [&](const Stage &s, const ChainArgs &c, int grid) -> int32_t {
+        MotifLaunch f;
+        const int32_t rc = find_unit(MOTIF_UNITS, "MotifSampler", s.team, masked, false, false, &f);
+        if (rc) return rc;
+        MotifArgs b = m;
+        b.c = c;
+        CUDA_TRY(f(b, grid, team_smem_bytes(c.s.row_words, s.team), h->stream));
+        return GIBBS_OK;
+    });
 }
 
 int32_t launch_loo_counts(gibbs_handle *h, const PrimArgs &a) {
-    const int kp = (a.k + 1) / 2;
-    const int smem = team_smem_bytes(a.s.row_words, 1);
-    switch (kp) {
-#define X(KPV)                                                                          \
-    case KPV: {                                                                         \
-        int32_t rc = set_smem(loo_counts_kernel<KPV>, smem);                            \
-        if (rc) return rc;                                                              \
-        loo_counts_kernel<KPV><<<1, 32, smem, h->stream>>>(a);                          \
-        break;                                                                          \
-    }
-        KP_CASES(X)
-#undef X
-    default: return fail(GIBBS_ERR_ARG, "unsupported k");
-    }
-    CUDA_TRY(cudaGetLastError());
-    return GIBBS_OK;
+    return with_kp(a.k, [&](auto kp) { return launch_one_warp(h, loo_counts_kernel<kp()>, a.s.row_words, a); });
 }
 
 int32_t launch_scan(gibbs_handle *h, const PrimArgs &a, int mode) {
-    const int kp = (a.k + 1) / 2;
-    const int smem = team_smem_bytes(a.s.row_words, 1);
-    switch (kp) {
-#define X(KPV)                                                                          \
-    case KPV: {                                                                         \
-        int32_t rc = set_smem(scan_kernel<KPV>, smem);                                  \
-        if (rc) return rc;                                                              \
-        scan_kernel<KPV><<<1, 32, smem, h->stream>>>(a, mode);                          \
-        break;                                                                          \
-    }
-        KP_CASES(X)
-#undef X
-    default: return fail(GIBBS_ERR_ARG, "unsupported k");
-    }
-    CUDA_TRY(cudaGetLastError());
-    return GIBBS_OK;
+    return with_kp(a.k, [&](auto kp) { return launch_one_warp(h, scan_kernel<kp()>, a.s.row_words, a, mode); });
 }
 
 int32_t launch_all_counts(gibbs_handle *h, const DeviceSeqs &s, const int32_t *sites, int k, int32_t *out) {
-    const int kp = (k + 1) / 2;
-    const int smem = team_smem_bytes(s.row_words, 1);
-    switch (kp) {
-#define X(KPV)                                                                          \
-    case KPV: {                                                                         \
-        int32_t rc = set_smem(all_counts_kernel<KPV>, smem);                            \
-        if (rc) return rc;                                                              \
-        all_counts_kernel<KPV><<<1, 32, smem, h->stream>>>(s, sites, k, out);           \
-        break;                                                                          \
-    }
-        KP_CASES(X)
-#undef X
-    default: return fail(GIBBS_ERR_ARG, "unsupported k");
-    }
-    CUDA_TRY(cudaGetLastError());
-    return GIBBS_OK;
+    return with_kp(k, [&](auto kp) { return launch_one_warp(h, all_counts_kernel<kp()>, s.row_words, s, sites, k, out); });
+}
+
+int32_t launch_roulette(gibbs_handle *h, const RouletteArgs &r) {
+    return with_kp(r.p.k, [&](auto kp) { return launch_one_warp(h, roulette_kernel<kp()>, r.p.s.row_words, r); });
 }
 
 DeviceSeqs dev_seqs(const gibbs_handle *h);
@@ -658,8 +701,7 @@ int32_t ensure_drift(gibbs_handle *h, const gibbs_params *p, int *launches, int 
     const int span = h->n * span_mult;
     if (h->drift_valid && h->drift_pc == p->pseudocount && h->drift_alen == p->alphabet_size && h->drift_span >= span) return GIBBS_OK;
     CUDA_TRY(h->pvals.reserve((size_t)span));
-    const double den = (double)(h->n - 1) + ((double)p->alphabet_size * p->pseudocount); // fs:257
-    pvals_kernel<<<(span + 255) / 256, 256, 0, h->stream>>>(span, p->pseudocount, den, h->pvals.p);
+    pvals_kernel<<<(span + 255) / 256, 256, 0, h->stream>>>(span, p->pseudocount, ppm_den(h->n, p), h->pvals.p);
     CUDA_TRY(cudaGetLastError());
     if (launches) *launches += 1;
     int32_t rc = ensure_seq_counts(h, launches);
@@ -689,125 +731,6 @@ BgTables bg_tables(const gibbs_handle *h) {
     b.gmax_i = h->bg_max_i.p;
     b.wstride = h->bg_wstride;
     return b;
-}
-
-// warps per chain of the MotifSampler kernel (first stage)
-int motif_team(const gibbs_handle *h) {
-    if (h->team_warps == 1) return 1;
-    return (h->n >= 4 && team_smem_bytes(h->row_words, 4) <= 200 * 1024) ? 4 : 1;
-}
-
-// The stages of a MotifSampler run: teams of 4 warps for every restart, then -- A,C,G,T-only sets, automatic team size --
-// the restarts still running are handed over to teams of 8 and of 16 warps as in launch_chain_kp (same thresholds).
-struct MotifStage { int team, pause_below, min_sweeps; };
-int motif_stages(const gibbs_handle *h, int n_chains, MotifStage *stages) {
-    const int sms = h->sm_count, N = h->n;
-    auto fits = [&](int t) { return N >= t && team_smem_bytes(h->row_words, t) <= 200 * 1024; };
-    int n_stages = 0;
-    const int team = motif_team(h);
-    if (team != 4 || h->n_masked > 0 || h->team_warps != 0) {
-        stages[n_stages++] = {team, 0, 0};
-        return n_stages;
-    }
-    int first = n_chains > h->opt_stage2_at * sms ? 4 : n_chains > h->opt_stage3_at * sms ? 8 : 16;
-    if (first == 16 && !fits(16)) first = 8;
-    if (first == 8 && !fits(8)) first = 4;
-    // (One warp per restart for the first greedy sweeps, as launch_chain_kp does for the SiteSampler, was measured here too:
-    // the sweeps themselves gain 1.4 ms on C2, the two hand-overs around them cost 2.5 ms -- tools/experiments/README.md.)
-    stages[n_stages++] = {first, 0, 0};
-    if (first == 4 && fits(8)) {
-        stages[n_stages - 1].pause_below = h->opt_stage2_at * sms;
-        stages[n_stages++] = {8, 0, 0};
-    }
-    if (stages[n_stages - 1].team == 8 && fits(16)) {
-        stages[n_stages - 1].pause_below = h->opt_stage3_at * sms;
-        stages[n_stages++] = {16, 0, 0};
-    }
-    return n_stages;
-}
-// warps that hold a scratch list at once, over the stages of a run (the lists are indexed by CTA)
-size_t motif_scratch_warps(const gibbs_handle *h, int n_chains) {
-    MotifStage stages[8];
-    const int n_stages = motif_stages(h, n_chains, stages);
-    size_t most = 0;
-    for (int st = 0; st < n_stages; ++st) {
-        const size_t grid = st == 0 ? (size_t)n_chains : (size_t)stages[st - 1].pause_below;
-        most = std::max(most, grid * (size_t)stages[st].team);
-    }
-    return most;
-}
-
-template <int KPV>
-int32_t launch_motif_kp(gibbs_handle *h, MotifArgs m) {
-    h->run_extra_launches = 0;
-    {   // the random starts are the SiteSampler's (fs:876, fs:993): run them grid-wide whenever a kernel fits
-        const int before = m.c.phase_mask;
-        const int32_t rc = launch_random_starts<KPV>(h, m.c, m.data_bg != 0);
-        if (rc) return rc;
-        m.init_done = (before & GIBBS_PHASE_INIT) && !(m.c.phase_mask & GIBBS_PHASE_INIT);
-    }
-    MotifStage stages[8];
-    const int n_stages = motif_stages(h, m.c.n_chains, stages);
-    CUDA_TRY(h->ctl.reserve(8));
-    const int32_t ctl0[8] = {m.c.n_chains, 0, 0, 0, 0, 0, 0, 0};
-    CUDA_TRY(cudaMemcpyAsync(h->ctl.p, ctl0, sizeof ctl0, cudaMemcpyHostToDevice, h->stream));
-    m.c.active = h->ctl.p;
-    if (n_stages > 1) {
-        CUDA_TRY(h->resume.reserve((size_t)m.c.n_chains));
-        CUDA_TRY(h->pending.reserve((size_t)(n_stages - 1) * (size_t)m.c.n_chains));
-        m.c.resume = h->resume.p;
-    }
-    for (int st = 0; st < n_stages; ++st) {
-        MotifArgs b = m;
-        const int team = stages[st].team;
-        b.c.pause_below = stages[st].pause_below;
-        b.c.pause_min_sweeps = stages[st].min_sweeps;
-        b.c.from_list = st > 0;
-        b.c.pending_in = st > 0 ? h->pending.p + (size_t)(st - 1) * m.c.n_chains : nullptr;
-        b.c.pending_in_n = st > 0 ? h->ctl.p + st : nullptr;
-        b.c.pending_out = st + 1 < n_stages ? h->pending.p + (size_t)st * m.c.n_chains : nullptr;
-        b.c.pending_out_n = st + 1 < n_stages ? h->ctl.p + st + 1 : nullptr;
-        const int grid = st == 0 ? m.c.n_chains : stages[st - 1].pause_below; // at most that many restarts were paused
-        const int smem = team_smem_bytes(m.c.s.row_words, team);
-        if (m.c.s.mask != nullptr)
-            CUDA_TRY(team == 4 ? launch_motif_masked_t4(b, grid, smem, h->stream) : launch_motif_masked_t1(b, grid, smem, h->stream));
-        else
-            CUDA_TRY(team == 16 ? launch_motif_t16(b, grid, smem, h->stream)
-                     : team == 8 ? launch_motif_t8(b, grid, smem, h->stream)
-                     : team == 4 ? launch_motif_t4(b, grid, smem, h->stream) : launch_motif_t1(b, grid, smem, h->stream));
-        if (st > 0) h->run_extra_launches += 1;
-    }
-    h->run_team = stages[0].team;
-    h->run_stages = n_stages;
-    return GIBBS_OK;
-}
-
-int32_t launch_motif(gibbs_handle *h, const MotifArgs &m) {
-    switch ((m.c.k + 1) / 2) {
-#define X(KPV) case KPV: return launch_motif_kp<KPV>(h, m);
-        KP_CASES(X)
-#undef X
-    default: return fail(GIBBS_ERR_ARG, "unsupported k");
-    }
-}
-
-int32_t launch_roulette(gibbs_handle *h, const RouletteArgs &r) {
-    const int kp = (r.p.k + 1) / 2;
-    const int smem = team_smem_bytes(r.p.s.row_words, 1);
-    switch (kp) {
-#define X(KPV)                                                                          \
-    case KPV: {                                                                         \
-        int32_t rc = set_smem(roulette_kernel<KPV>, smem);                              \
-        if (rc) return rc;                                                              \
-        roulette_kernel<KPV><<<1, 32, smem, h->stream>>>(r);                            \
-        break;                                                                          \
-    }
-        KP_CASES(X)
-#undef X
-    default: return fail(GIBBS_ERR_ARG, "unsupported k");
-    }
-    CUDA_TRY(cudaGetLastError());
-    return GIBBS_OK;
 }
 
 DeviceSeqs dev_seqs(const gibbs_handle *h) {
@@ -900,6 +823,21 @@ int32_t stage_sites(gibbs_handle *h, const int32_t *sites, int32_t heldout, int3
     return GIBBS_OK;
 }
 
+// the statistics of a run: its device counters (ST_* slots) and what the host recorded when it launched the run
+void fill_stats(gibbs_run_stats *out, const unsigned long long *st, int launches, int fast, int team, int init_path, float ms) {
+    out->site_updates = (int64_t)st[ST_SITE_UPDATES];
+    out->window_scores = (int64_t)st[ST_WINDOW_SCORES];
+    out->sweeps = (int64_t)st[ST_SWEEPS];
+    out->exact_rescans = (int64_t)st[ST_EXACT_RESCANS];
+    out->capped_chains = (int64_t)st[ST_CAPPED];
+    out->speculative_discards = (int64_t)st[ST_SPECULATED];
+    out->kernel_launches = launches;
+    out->fast_path = fast;
+    out->team_warps = team;
+    out->init_path = init_path;
+    out->kernel_ms = (double)ms;
+}
+
 } // namespace
 
 extern "C" {
@@ -964,20 +902,10 @@ int32_t gibbs_destroy(gibbs_handle *h) {
     if (!h) return GIBBS_OK;
     cudaSetDevice(h->device);
     if (h->stream) cudaStreamSynchronize(h->stream);
-    h->ascii.release(); h->off.release(); h->packed.release(); h->len.release(); h->flags.release();
-    h->mask.release(); h->rowflag.release(); h->symflags.release(); h->wide.release();
-    h->wtab.release(); h->prim_sites.release(); h->prim_i32.release(); h->prim_f64.release();
-    h->sites.release(); h->hv.release(); h->scores.release(); h->sums.release(); h->uniforms.release();
-    h->stats.release(); h->best.release();
-    h->bg_g.release(); h->bg_sum.release(); h->bg_max.release(); h->bg_max_i.release();
-    h->cand_l.release(); h->cand_w.release(); h->err_flag.release();
-    h->pvals.release(); h->basecnt.release(); h->maskcnt.release(); h->ss.release(); h->gbuf.release(); h->start_ppm.release();
-    h->ctl.release(); h->resume.release(); h->pending.release();
-    h->win_sites.release(); h->win_scores.release(); h->pos2.release(); h->sc2.release();
     if (h->ev0) cudaEventDestroy(h->ev0);
     if (h->ev1) cudaEventDestroy(h->ev1);
     if (h->own_stream && h->stream) cudaStreamDestroy(h->stream);
-    delete h;
+    delete h; // the device buffers, on the handle's device
     return GIBBS_OK;
 }
 
@@ -1228,18 +1156,36 @@ int32_t gibbs_run_device(gibbs_handle *h, const gibbs_params *p, int32_t n_chain
         if (h->start_ppm_k != p->k) return fail(GIBBS_ERR_ARG, "the start PPM has %d columns, the run k = %d", h->start_ppm_k, p->k);
         a.ppm_given = h->start_ppm.p;
     }
+    const bool drift = p->background == GIBBS_BG_DATA;
+    if (drift) { // both samplers' random starts and the SiteSampler's scans (drift_tables / drift_pick)
+        a.pvals = h->pvals.p;
+        a.basecnt = h->basecnt.p;
+        a.maskcnt = h->n_masked > 0 ? h->maskcnt.p : nullptr; // symbols outside A,C,G,T per sequence (background denominators)
+        a.ss = h->ss_valid ? h->ss.p : nullptr;
+        a.ss_stride = h->max_len + 2;
+        memcpy(a.gcnt, h->gcnt, sizeof a.gcnt);
+        a.alpha_pc = (double)p->alphabet_size * p->pseudocount; // float alphabet.Length * pseudoCount, fs:117
+        a.pc = p->pseudocount;
+        // gibbs_set_option(GIBBS_OPT_EXACT_SCANS): every window in float64
+        a.drift_fast_ok = h->opt_exact_scans ? 0 : drift_fast_path_ok(h->gcnt, h->max_len, h->n, p);
+    }
     if (p->sampler == GIBBS_MOTIF_SAMPLER) {
-        if (p->background == GIBBS_BG_FIXED) {
+        Stage stages[MAX_STAGES] = {};
+        const int n_stages = plan_stages(h, a, drift, stages);
+        size_t warps = 0; // warps that hold a scratch list at once, over the stages of the run (the lists are indexed by CTA)
+        for (int st = 0; st < n_stages; ++st)
+            warps = std::max(warps, (size_t)(st == 0 ? n_chains : stages[st - 1].pause_below) * (size_t)stages[st].team);
+        if (!drift) {
             rc = ensure_bgtab(h, p, &launches);
             if (rc) return rc;
         } else {
             h->bg_valid = false; // the fixed-background tables are not used; only the window stride is
             h->bg_wstride = h->max_len - p->k + 1;
             if (h->n_masked > 0 && h->bg_wstride < 64) h->bg_wstride = 64; // the candidate scratch doubles as a 49-slot symbol-count table
-            CUDA_TRY(h->gbuf.reserve(motif_scratch_warps(h, n_chains) * h->bg_wstride));
+            CUDA_TRY(h->gbuf.reserve(warps * h->bg_wstride));
         }
-        CUDA_TRY(h->cand_l.reserve(motif_scratch_warps(h, n_chains) * h->bg_wstride)); // one scratch list per warp
-        CUDA_TRY(h->cand_w.reserve(motif_scratch_warps(h, n_chains) * h->bg_wstride));
+        CUDA_TRY(h->cand_l.reserve(warps * h->bg_wstride)); // one scratch list per warp
+        CUDA_TRY(h->cand_w.reserve(warps * h->bg_wstride));
         CUDA_TRY(h->err_flag.reserve(1));
         CUDA_TRY(cudaMemsetAsync(h->err_flag.p, 0, sizeof(int32_t), h->stream));
         MotifArgs m{};
@@ -1250,35 +1196,18 @@ int32_t gibbs_run_device(gibbs_handle *h, const gibbs_params *p, int32_t n_chain
         m.error = h->err_flag.p;
         m.ascii = h->ascii.p;
         m.off = h->off.p;
-        m.data_bg = p->background == GIBBS_BG_DATA ? 1 : 0;
-        m.greedy_fast_ok = a.fast_ok; // fixed background: the range check of the W table (ensure_wtab)
-        if (m.data_bg) {
-            m.pvals = h->pvals.p;
-            m.basecnt = h->basecnt.p;
-            memcpy(m.gcnt, h->gcnt, sizeof m.gcnt);
-            m.alpha_pc = (double)p->alphabet_size * p->pseudocount;
-            m.pc = p->pseudocount;
+        m.data_bg = drift ? 1 : 0;
+        // the range check of the W table (ensure_wtab) or of the PPM values (drift_fast_path_ok)
+        m.greedy_fast_ok = drift ? a.drift_fast_ok : a.fast_ok;
+        if (drift) {
+            m.pvals = a.pvals;
+            m.basecnt = a.basecnt;
+            memcpy(m.gcnt, a.gcnt, sizeof m.gcnt);
+            m.alpha_pc = a.alpha_pc;
+            m.pc = a.pc;
             m.gbuf = h->gbuf.p;
-            // every odds ratio lies in [pc / den, den / pc] (see the SiteSampler branch below): no product of k of them
-            // leaves the float64 normal range, the fixed-point keys stay far inside int32
-            const double bases = (double)h->gcnt[0] + h->gcnt[1] + h->gcnt[2] + h->gcnt[3] + (double)h->max_len;
-            const double den = (bases > (double)h->n ? bases : (double)h->n) + m.alpha_pc;
-            m.greedy_fast_ok = (p->pseudocount >= 1e-30 && (double)p->k * log2(den / p->pseudocount) < 1000.0) ? 1 : 0;
-            m.c.pvals = m.pvals; // the random starts use the SiteSampler's drifting-background routines (drift_tables / drift_pick)
-            m.c.basecnt = m.basecnt;
-            m.c.maskcnt = h->n_masked > 0 ? h->maskcnt.p : nullptr; // symbols outside A,C,G,T per sequence (background denominators)
-            m.c.ss = h->ss_valid ? h->ss.p : nullptr;
-            m.c.ss_stride = h->max_len + 2;
-            memcpy(m.c.gcnt, m.gcnt, sizeof m.gcnt);
-            m.c.alpha_pc = m.alpha_pc;
-            m.c.pc = m.pc;
         }
-        m.roulette_scan_ok = 1;
-        if (h->opt_exact_scans) { // gibbs_set_option(GIBBS_OPT_EXACT_SCANS): every window in float64, sequential roulette walk
-            m.greedy_fast_ok = 0;
-            m.roulette_scan_ok = 0;
-        }
-        m.c.drift_fast_ok = m.data_bg ? m.greedy_fast_ok : 0; // what the grid-wide random starts (init_kernel<.., DRIFT>) read
+        m.roulette_scan_ok = h->opt_exact_scans ? 0 : 1; // GIBBS_OPT_EXACT_SCANS: sequential roulette walk
         if (m_amount == 2) { // up to two sites per sequence: Positions lists beside the one-site state
             CUDA_TRY(h->pos2.reserve(cells * 2));
             CUDA_TRY(h->sc2.reserve((size_t)n_chains * h->bg_wstride));
@@ -1286,12 +1215,14 @@ int32_t gibbs_run_device(gibbs_handle *h, const gibbs_params *p, int32_t n_chain
                 CUDA_TRY(launch_motif2_seed(h->sites.p, (long long)cells, h->pos2.p, h->stream));
         }
         CUDA_TRY(cudaEventRecord(h->ev0, h->stream));
-        if (m_amount == 2) {
-            h->run_extra_launches = 0;
+        h->run_extra_launches = 0;
+        {   // the random starts are the SiteSampler's (fs:876, fs:993): run them grid-wide whenever a kernel fits
             const int before = m.c.phase_mask;
-            rc = launch_random_starts_any(h, m.c, m.data_bg != 0);
+            rc = launch_random_starts(h, m.c, drift);
             if (rc) return rc;
             m.init_done = (before & GIBBS_PHASE_INIT) && !(m.c.phase_mask & GIBBS_PHASE_INIT);
+        }
+        if (m_amount == 2) {
             Motif2Args q{};
             q.m = m;
             q.pos2 = h->pos2.p;
@@ -1299,37 +1230,17 @@ int32_t gibbs_run_device(gibbs_handle *h, const gibbs_params *p, int32_t n_chain
             CUDA_TRY(launch_motif2(q, n_chains, team_smem_bytes(h->row_words, 1), h->stream));
             h->run_team = 1;
         } else {
-            rc = launch_motif(h, m);
+            rc = launch_motif(h, m, stages, n_stages);
             if (rc) return rc;
         }
-        launches += h->run_extra_launches;
-    } else if (p->background == GIBBS_BG_DATA) {
-        // teams of warps, speculative rounds and the hand-over of chain_kernel, with the drifting-background scan
-        a.pvals = h->pvals.p;
-        a.basecnt = h->basecnt.p;
-        a.maskcnt = h->n_masked > 0 ? h->maskcnt.p : nullptr;
-        a.ss = h->ss_valid ? h->ss.p : nullptr;
-        a.ss_stride = h->max_len + 2;
-        memcpy(a.gcnt, h->gcnt, sizeof a.gcnt);
-        a.alpha_pc = (double)p->alphabet_size * p->pseudocount; // float alphabet.Length * pseudoCount, fs:117
-        a.pc = p->pseudocount;
-        {   // Ranking pass allowed? Every odds ratio ppm / pcv lies in [pc / den, den / pc] with den <= all bases of the
-            // set + one more sequence + |A| pc (or N - 1 + |A| pc): no float64 product of k of them may leave the
-            // normal range (|log2| < 1000), and pc >= 1e-30 keeps every float32 logarithm argument normal and finite.
-            a.drift_fast_ok = drift_fast_path_ok(h->gcnt, h->max_len, h->n, p);
-            if (h->opt_exact_scans) a.drift_fast_ok = 0; // gibbs_set_option(GIBBS_OPT_EXACT_SCANS): every window in float64
-            a.fast_ok = a.drift_fast_ok;
-        }
-        CUDA_TRY(cudaEventRecord(h->ev0, h->stream));
-        rc = launch_chain(h, a, true);
-        if (rc) return rc;
-        launches += h->run_extra_launches;
     } else {
+        // teams of warps, speculative rounds and the hand-over of chain_kernel
+        if (drift) a.fast_ok = a.drift_fast_ok;
         CUDA_TRY(cudaEventRecord(h->ev0, h->stream));
-        rc = launch_chain(h, a);
+        rc = launch_chain(h, a, drift);
         if (rc) return rc;
-        launches += h->run_extra_launches;
     }
+    launches += h->run_extra_launches;
     h->run_sampler = p->sampler;
     h->run_m = p->sampler == GIBBS_MOTIF_SAMPLER ? m_amount : 1;
     h->best_valid = false;
@@ -1476,17 +1387,7 @@ int32_t gibbs_fetch(gibbs_handle *h, int32_t *sites_out, double *scores_out, dou
     if (stats_out) {
         float ms = 0.f;
         CUDA_TRY(cudaEventElapsedTime(&ms, h->ev0, h->ev1));
-        stats_out->site_updates = (int64_t)st[ST_SITE_UPDATES];
-        stats_out->window_scores = (int64_t)st[ST_WINDOW_SCORES];
-        stats_out->sweeps = (int64_t)st[ST_SWEEPS];
-        stats_out->exact_rescans = (int64_t)st[ST_EXACT_RESCANS];
-        stats_out->capped_chains = (int64_t)st[ST_CAPPED];
-        stats_out->speculative_discards = (int64_t)st[ST_SPECULATED];
-        stats_out->kernel_launches = h->run_launches + extra_launches;
-        stats_out->fast_path = h->run_fast;
-        stats_out->team_warps = h->run_team;
-        stats_out->init_path = h->run_init_path;
-        stats_out->kernel_ms = (double)ms;
+        fill_stats(stats_out, st, h->run_launches + extra_launches, h->run_fast, h->run_team, h->run_init_path, ms);
     }
     return GIBBS_OK;
 }
@@ -1573,17 +1474,7 @@ int32_t gibbs_fetch_best(gibbs_handle *h, int32_t repetitions, int32_t *sites_ou
     if (stats_out) {
         float ms = 0.f;
         CUDA_TRY(cudaEventElapsedTime(&ms, h->ev0, h->ev1));
-        stats_out->site_updates = (int64_t)st[ST_SITE_UPDATES];
-        stats_out->window_scores = (int64_t)st[ST_WINDOW_SCORES];
-        stats_out->sweeps = (int64_t)st[ST_SWEEPS];
-        stats_out->exact_rescans = (int64_t)st[ST_EXACT_RESCANS];
-        stats_out->capped_chains = (int64_t)st[ST_CAPPED];
-        stats_out->speculative_discards = (int64_t)st[ST_SPECULATED];
-        stats_out->kernel_launches = h->run_launches + extra_launches;
-        stats_out->fast_path = h->run_fast;
-        stats_out->team_warps = h->run_team;
-        stats_out->init_path = h->run_init_path;
-        stats_out->kernel_ms = (double)ms;
+        fill_stats(stats_out, st, h->run_launches + extra_launches, h->run_fast, h->run_team, h->run_init_path, ms);
     }
     return GIBBS_OK;
 }
@@ -1920,16 +1811,6 @@ int batch_team(const gibbs_batch *b, int s) {
     return (N >= 4 && team_smem_bytes(b->h->row_words, 4) <= 200 * 1024) ? 4 : 1;
 }
 
-cudaError_t launch_batch_group(bool init, bool masked, bool drift, int team, const ChainArgs &run, const BatchTable &bt, int grid,
-                               int smem, cudaStream_t st) {
-#define PICK(sfx) (team == 4 ? launch_batch##sfx##_t4 : launch_batch##sfx##_t1)
-    decltype(&launch_batch_t4) f;
-    if (init) f = masked ? (drift ? PICK(_init_masked_drift) : PICK(_init_masked)) : (drift ? PICK(_init_drift) : PICK(_init));
-    else f = masked ? (drift ? PICK(_masked_drift) : PICK(_masked)) : (drift ? PICK(_drift) : PICK());
-#undef PICK
-    return f(run, bt, grid, smem, st);
-}
-
 int32_t batch_check(const gibbs_batch *b, const gibbs_params *p, const double *bg_per_set, int32_t R) {
     if (!b) return fail(GIBBS_ERR_ARG, "null batch");
     if (!p) return fail(GIBBS_ERR_ARG, "null params");
@@ -1990,9 +1871,8 @@ int32_t batch_tables(gibbs_batch *b, const gibbs_params *p, const double *bg_per
         CUDA_TRY(cudaMemcpyAsync(b->wt_range.p, range.data(), range.size() * sizeof(int), cudaMemcpyHostToDevice, h->stream));
         for (int32_t s = 0; s < b->n_sets; ++s) {
             const int N = b->seq_off[s + 1] - b->seq_off[s];
-            const double den = (double)(N - 1) + ((double)p->alphabet_size * p->pseudocount); // fs:257, per set
             const double *q = bg.data() + 4 * (size_t)s;
-            wtab_kernel<<<(N * 4 + 255) / 256, 256, 0, h->stream>>>(N, p->pseudocount, den, q[0], q[1], q[2], q[3],
+            wtab_kernel<<<(N * 4 + 255) / 256, 256, 0, h->stream>>>(N, p->pseudocount, ppm_den(N, p), q[0], q[1], q[2], q[3],
                                                                     b->wtab.p + 4 * (size_t)b->seq_off[s], b->wt_range.p + 4 * (size_t)s);
             CUDA_TRY(cudaGetLastError());
         }
@@ -2009,8 +1889,7 @@ int32_t batch_tables(gibbs_batch *b, const gibbs_params *p, const double *bg_per
         CUDA_TRY(b->pvals.reserve((size_t)b->n_seqs));
         for (int32_t s = 0; s < b->n_sets; ++s) {
             const int N = b->seq_off[s + 1] - b->seq_off[s];
-            const double den = (double)(N - 1) + ((double)p->alphabet_size * p->pseudocount);
-            pvals_kernel<<<(N + 255) / 256, 256, 0, h->stream>>>(N, p->pseudocount, den, b->pvals.p + b->seq_off[s]);
+            pvals_kernel<<<(N + 255) / 256, 256, 0, h->stream>>>(N, p->pseudocount, ppm_den(N, p), b->pvals.p + b->seq_off[s]);
             CUDA_TRY(cudaGetLastError());
             int32_t g[4];
             for (int x = 0; x < 4; ++x) g[x] = (int32_t)b->gcnt[4 * (size_t)s + x];
@@ -2107,15 +1986,13 @@ int32_t gibbs_batch_create(const uint8_t *seqs, const int64_t *offsets, const in
 
 int32_t gibbs_batch_destroy(gibbs_batch *b) {
     if (!b) return GIBBS_OK;
-    if (b->h) {
-        cudaSetDevice(b->h->device);
-        cudaStreamSynchronize(b->h->stream);
+    gibbs_handle *h = b->h;
+    if (h) {
+        cudaSetDevice(h->device);
+        cudaStreamSynchronize(h->stream);
     }
-    b->d_seq_off.release(); b->wtab.release(); b->wt_range.release(); b->pvals.release(); b->d_args.release(); b->d_groups.release();
-    b->sites.release(); b->win_sites.release(); b->hv.release(); b->scores.release(); b->sums.release(); b->win_scores.release();
-    b->counts.release(); b->stats.release();
-    gibbs_destroy(b->h);
-    delete b;
+    delete b; // the batch's device buffers, on the handle's device
+    gibbs_destroy(h);
     return GIBBS_OK;
 }
 
@@ -2228,8 +2105,11 @@ int32_t gibbs_batch_run_device(gibbs_batch *b, const gibbs_params *p, const doub
             bt.chain_off = b->d_groups.p + g_at[g] + n;
             bt.n = n;
             ChainArgs r = run;
-            r.min_width = per_sm <= 1 ? team : 1; // (as launch_chain_kp: never narrow once a chain has an SM to itself)
-            CUDA_TRY(launch_batch_group(init != 0, masked, drift, team, r, bt, n * R, team_smem_bytes(h->row_words, team), h->stream));
+            r.min_width = per_sm <= 1 ? team : 1; // (as plan_stages: never narrow once a chain has an SM to itself)
+            BatchLaunch f;
+            rc = find_unit(BATCH_UNITS, "batch", team, masked, drift, init != 0, &f);
+            if (rc) return rc;
+            CUDA_TRY(f(r, bt, n * R, team_smem_bytes(h->row_words, team), h->stream));
             ++launches;
         }
     }
@@ -2245,17 +2125,7 @@ int32_t gibbs_batch_run_device(gibbs_batch *b, const gibbs_params *p, const doub
 static void batch_stats(const gibbs_batch *b, const unsigned long long *st, int extra_launches, gibbs_run_stats *out) {
     float ms = 0.f;
     if (cudaEventElapsedTime(&ms, b->h->ev0, b->h->ev1) != cudaSuccess) cudaGetLastError();
-    out->site_updates = (int64_t)st[ST_SITE_UPDATES];
-    out->window_scores = (int64_t)st[ST_WINDOW_SCORES];
-    out->sweeps = (int64_t)st[ST_SWEEPS];
-    out->exact_rescans = (int64_t)st[ST_EXACT_RESCANS];
-    out->capped_chains = (int64_t)st[ST_CAPPED];
-    out->speculative_discards = (int64_t)st[ST_SPECULATED];
-    out->kernel_launches = b->run_launches + extra_launches;
-    out->fast_path = b->run_fast;
-    out->team_warps = b->run_team;
-    out->init_path = GIBBS_INIT_CHAIN;
-    out->kernel_ms = (double)ms;
+    fill_stats(out, st, b->run_launches + extra_launches, b->run_fast, b->run_team, GIBBS_INIT_CHAIN, ms);
 }
 
 int32_t gibbs_batch_fetch(gibbs_batch *b, int32_t *sites_out, double *scores_out, double *sums_out, gibbs_run_stats *stats_out) {
@@ -2298,13 +2168,12 @@ int32_t gibbs_batch_fetch_best(gibbs_batch *b, int32_t repetitions, int32_t *sit
     if (scores_out) CUDA_TRY(cudaMemcpyAsync(scores_out, b->win_scores.p, (size_t)NT * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
     if (counts_out) { // PWM counts of every winner's sites (all zero where the initial value survived: its sites are -1)
         CUDA_TRY(b->counts.reserve((size_t)S * k * 4));
-        switch ((k + 1) / 2) {
-#define X(KPV) case KPV: all_counts_batch_kernel<KPV><<<S, 32, 0, h->stream>>>(b->d_args.p, b->d_seq_off.p, b->win_sites.p, k, b->counts.p); break;
-            KP_CASES(X)
-#undef X
-        default: return fail(GIBBS_ERR_ARG, "unsupported k");
-        }
-        CUDA_TRY(cudaGetLastError());
+        rc = with_kp(k, [&](auto kp) -> int32_t {
+            all_counts_batch_kernel<kp()><<<S, 32, 0, h->stream>>>(b->d_args.p, b->d_seq_off.p, b->win_sites.p, k, b->counts.p);
+            CUDA_TRY(cudaGetLastError());
+            return GIBBS_OK;
+        });
+        if (rc) return rc;
         ++extra_launches;
         CUDA_TRY(cudaMemcpyAsync(counts_out, b->counts.p, (size_t)S * k * 4 * sizeof(int32_t), cudaMemcpyDeviceToHost, h->stream));
     }
