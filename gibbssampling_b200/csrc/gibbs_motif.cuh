@@ -167,17 +167,20 @@ __device__ __forceinline__ int motif_candidates(const WarpTables &T, const uint3
 }
 
 // The roulette pick of the stochastic sweep without a float64 logarithm per candidate. log2 of a gated product to 1e-6:
-// exponent + MUFU.LG2 of the float mantissa (|error| < 5e-7 for any normal product). With those weights the candidates
-// are decided (further than 1e-6 from the cut-off, else the exact path runs), their prefix sums locate the bucket of the
-// pick, and the error of any prefix -- (items + 64) * 1e-6 -- is far below a bucket width (a candidate weighs more than
-// the cut-off): when the pick clears both edges of its bucket by twice that bound the sequential float64 walk of
+// exponent + MUFU.LG2 of the float mantissa, added in double (exact: an integer below 2^11 plus a float in [0, 1]), so
+// |error| < 4.5e-7 for any normal product at any magnitude -- MUFU.LG2's 2^-21.4 on [1, 2] plus 2^-24 / ln 2 for rounding
+// the mantissa to float. (A float sum would round to half a float ulp of the result on top: 1.9e-6 above 32, 3.8e-6
+// above 64, enough to put a window on the wrong side of the cut-off.) With those weights the candidates are decided
+// (further than 1e-6 from the cut-off, else the exact path runs), their prefix sums locate the bucket of the pick, and
+// the error of any prefix -- (items + 64) * 1e-6 -- is far below a bucket width (a candidate weighs more than the
+// cut-off): when the pick clears both edges of its bucket by twice that bound the sequential float64 walk of
 // fs:746-754 must stop in the same bucket, and only that item's PWMS is computed with the reference's logarithm.
 // Needs cutOff >= 0 (no negative weights). false = undecided: the caller runs motif_logs + motif_roulette on the same list.
-__device__ __forceinline__ float log2_coarse(double s) {
+__device__ __forceinline__ double log2_coarse(double s) {
     const int hi = __double2hiint(s);
     const int e = ((hi >> 20) & 0x7ff) - 1023;
     const float m = (float)__hiloint2double((hi & 0x000fffff) | 0x3ff00000, __double2loint(s)); // mantissa in [1, 2]
-    return (float)e + __log2f(m);
+    return (double)e + (double)__log2f(m);
 }
 __device__ __forceinline__ bool motif_stoch_fast(double gsum, double cutoff, const double *cand_l, const int32_t *cand_w, int gated,
                                                  double pick, int lane, double &pwms_out, int &site_out) {
@@ -189,7 +192,7 @@ __device__ __forceinline__ bool motif_stoch_fast(double gsum, double cutoff, con
     bool unsure = false;
     for (int i = i0; i < i1; ++i) {
         const double s = cand_l[i];
-        const double l = (double)log2_coarse(s);
+        const double l = log2_coarse(s);
         unsure |= !(s >= 0x1p-1000 && s <= 0x1p1000) || fabs(l - cutoff) <= TOL;
         if (l > cutoff) part += l;
     }
@@ -211,7 +214,7 @@ __device__ __forceinline__ bool motif_stoch_fast(double gsum, double cutoff, con
     if (lane == src) {
         double acc = gsum + incl - part;
         for (int i = i0; i < i1; ++i) {
-            const double l = (double)log2_coarse(cand_l[i]);
+            const double l = log2_coarse(cand_l[i]);
             if (!(l > cutoff)) continue;
             const double nxt = acc + l;
             if (target <= nxt) {
@@ -329,8 +332,9 @@ __device__ __forceinline__ bool motif_roulette(const double *g, double gsum, int
             lo = __shfl_sync(FULL, lo, src);
             hi = __shfl_sync(FULL, hi, src);
             const double tol = eps * sum;
-            // clear of both edges: lo + tol < target < hi - tol (idx = 0 has no lower edge: the walk starts at 0 <= pick)
-            if (idx >= 0 && target < hi - tol && (idx == 0 || target > lo + tol)) {
+            // clear of both edges: lo + tol < target < hi - tol (idx = 0: the walk's lower edge is exactly 0, and a pick
+            // below it makes the reference throw, so the exact walk decides that)
+            if (idx >= 0 && target < hi - tol && (idx == 0 ? pick >= 0.0 : target > lo + tol)) {
                 if (idx < W) {
                     pwms_out = g[idx];
                     site_out = -1;
