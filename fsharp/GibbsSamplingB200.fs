@@ -111,6 +111,13 @@ module Native =
     [<DllImport(Lib, CallingConvention = CallingConvention.Cdecl)>]
     extern int gibbs_batch_fetch_best(IntPtr batch, int repetitions, int[] sitesOut, float[] scoresOut, int[] nOut, float[] sumOut,
                                       int[] restartOut, int[] countsOut, GibbsRunStats& stats)
+    [<DllImport(Lib, CallingConvention = CallingConvention.Cdecl)>]
+    extern int gibbs_batch_run_motif_device(IntPtr batch, GibbsParams& p, float[] bgPerSetOrNull, int restartsPerSet, int64 chainIdBase,
+                                            uint64 seed)
+    [<DllImport(Lib, CallingConvention = CallingConvention.Cdecl)>]
+    extern int gibbs_batch_fetch_positions(IntPtr batch, int m, int[] positionsOut)
+    [<DllImport(Lib, CallingConvention = CallingConvention.Cdecl)>]
+    extern int gibbs_batch_fetch_best_positions(IntPtr batch, int m, int[] positionsOut)
 
     /// status code -> the exception the reference would have thrown (SURVEY.md section 8b)
     let check (rc:int) =
@@ -367,3 +374,44 @@ module MotifSampler =
         (run 0 (numberOfRepetitions + 1) (seedOf None) motifAmount motifLength pseudoCount cutOff alphabet sources None None None (Some numberOfRepetitions)).[0]
     let getBestPWMSsOfPPM numberOfRepetitions motifAmount motifLength pseudoCount cutOff alphabet sources (ppM:PositionMatrix.PositionProbabilityMatrix) =
         (run 0 (numberOfRepetitions + 1) (seedOf None) motifAmount motifLength pseudoCount cutOff alphabet sources None (Some ppM) None (Some numberOfRepetitions)).[0]
+
+    /// The restart loops of many sets in one batch on GPU 0 (gibbs_batch_run_motif_device): set s gets exactly what the
+    /// single-set call with the same seed gives (restart r of every set draws from the stream (seed, r)); only the winners
+    /// are copied back.
+    let private bestOfSets (numberOfRepetitions:int) seed (motifAmount:int) k pc (cutOff:float) alphabet (sets:BioArray.BioArray<#IBioItem>[][])
+                           (pcvs:ProbabilityCompositeVector[] option) : MotifIndex[][] =
+        let m = max motifAmount 1
+        let all = Array.concat sets
+        let buf, offsets = Native.flatten all
+        let setOffsets = Array.zeroCreate<int> (sets.Length + 1)
+        sets |> Array.iteri (fun s src -> setOffsets.[s + 1] <- setOffsets.[s] + src.Length)
+        let mutable b = IntPtr.Zero
+        Native.check (Native.gibbs_batch_create(buf, offsets, setOffsets, sets.Length, 0, &b))
+        try
+            let mutable p = Native.makeParams k pc alphabet (pcvs |> Option.map (fun v -> v.[0])) 0
+            p.sampler <- 1; p.cutoff <- cutOff; p.motifAmount <- m
+            let bg =
+                match pcvs with
+                | Some v -> v |> Array.collect (fun pcv -> [| for c in "ACGT" -> pcv.Array.[int c - 42] |])
+                | None -> null
+            Native.check (Native.gibbs_batch_run_motif_device(b, &p, bg, numberOfRepetitions + 1, 0L, seed))
+            let sites, scores, pos = Array.zeroCreate all.Length, Array.zeroCreate all.Length, Array.zeroCreate (all.Length * m)
+            let nOut, restart = Array.zeroCreate sets.Length, Array.zeroCreate sets.Length
+            let mutable stats = Native.GibbsRunStats()
+            Native.check (Native.gibbs_batch_fetch_best(b, numberOfRepetitions, sites, scores, nOut, null, restart, null, &stats))
+            Native.check (Native.gibbs_batch_fetch_best_positions(b, m, pos))
+            Array.init sets.Length (fun s ->
+                let o = setOffsets.[s]
+                if restart.[s] < 0 then [| createMotifIndex 0. [] |]    // the loop's initial value survived
+                else Array.init nOut.[s] (fun i -> createMotifIndex scores.[o + i] ([ for j in 0 .. m - 1 do
+                                                                                         let q = pos.[(o + i) * m + j]
+                                                                                         if q >= 0 then yield q ])))
+        finally
+            Native.gibbs_batch_destroy b |> ignore
+
+    /// findBestInormationContentContainingMotifsWithPCV of every set (pcvs.[s] the background of sets.[s]) in one GPU batch
+    let findBestInormationContentContainingMotifsWithPCVOfSets numberOfRepetitions motifAmount motifLength pseudoCount cutOff alphabet sets (pcvs:ProbabilityCompositeVector[]) =
+        bestOfSets numberOfRepetitions (seedOf None) motifAmount motifLength pseudoCount cutOff alphabet sets (Some pcvs)
+    /// getMotifsWithBestInformationContents of every set in one GPU batch (e.g. the script's fsx:407 call per gene group)
+    let getMotifsWithBestInformationContentsOfSets numberOfRepetitions motifAmount motifLength pseudoCount cutOff alphabet sets =
+        bestOfSets numberOfRepetitions (seedOf None) motifAmount motifLength pseudoCount cutOff alphabet sets None

@@ -3,7 +3,8 @@
 `MotifIndex` = {PWMS: float; Positions: int list} (fs:712-716). motifAmount = 1 (one site per sequence or none) and
 motifAmount = 2 (up to two non-overlapping sites, fs:727-742 -- the reference script's second live call, fsx:407) are
 built; three and more sites per sequence raise GibbsUnsupportedError. Both the fixed-background (`...ByPCV` /
-`...WithPCV`) family and the data-derived-background family (fs:885-1038) run on the GPU.
+`...WithPCV`) family and the data-derived-background family (fs:885-1038) run on the GPU. The `...OfSets` functions run
+the restart loops of many sets in one batch (gibbs_batch_run_motif_device).
 """
 from __future__ import annotations
 
@@ -14,7 +15,7 @@ import numpy as np
 
 from . import _abi
 from .CompositeVector import ProbabilityCompositeVector
-from .engine import GibbsEngine, make_params
+from .engine import BatchEngine, GibbsEngine, make_params
 from .SiteSampler import _bg_of, _engine_for
 
 
@@ -224,3 +225,53 @@ def getBestPWMSsOfPPM(numberOfRepetitions, motifAmount, motifLength, pseudoCount
     return _run(0, motifAmount, motifLength, pseudoCount, cutOff, alphabet, sources, None, n_chains=n_restarts,
                seed=seed, chain=chain, uniforms=uniforms, engine=engine, max_sweeps=max_sweeps, ppM=ppM,
                best_of=int(numberOfRepetitions))
+
+
+# ---- many sets in one batch (gibbs_batch_run_motif_device): one result per set, element s = the single-set function on sets[s]
+def _motif_restart_loop_of_sets(numberOfRepetitions, motifAmount, motifLength, pseudoCount, cutOff, alphabet, sets, pcvs, *,
+                                seed: int = 0, chain: int = 0, max_sweeps: int = 0,
+                                engine: Optional[BatchEngine] = None) -> list:
+    m = _check_m(motifAmount)
+    if sets is not None:
+        sets = list(sets)   # (a generator is read once)
+    if pcvs is None:
+        _bg_of(alphabet, ProbabilityCompositeVector.ofACGT(1, 1, 1, 1))   # only checks A,C,G,T are in the alphabet
+        bg, bg0, background = None, [0.25] * 4, _abi.GIBBS_BG_DATA
+    else:
+        pcvs = list(pcvs)
+        if sets is not None and engine is None and len(pcvs) != len(sets):
+            raise _abi.GibbsArgumentError(_abi.GIBBS_ERR_ARG, f"{len(pcvs)} pcvs for {len(sets)} sets")
+        bg = [_bg_of(alphabet, pcv) for pcv in pcvs]
+        bg0, background = bg[0] if bg else [0.25] * 4, _abi.GIBBS_BG_FIXED
+    params = make_params(motifLength, pseudoCount, len(alphabet), bg0, cutoff=cutOff, background=background,
+                         sampler=_abi.GIBBS_MOTIF_SAMPLER, max_sweeps=max_sweeps, motif_amount=m)
+    eng = engine if engine is not None else BatchEngine(sets)
+    try:
+        eng.run_motif_device(params, max(int(numberOfRepetitions) + 1, 1), bg_per_set=bg, chain_id_base=chain, seed=seed)
+        best = eng.fetch_best(int(numberOfRepetitions))
+        if m == 1:
+            return [_to_motif_array(b.scores, b.sites) for b in best]
+        pos = eng.fetch_best_positions(m)
+        return [_to_motif_array(b.scores, b.sites if b.restart < 0 else pos[s]) for s, b in enumerate(best)]
+    finally:
+        if engine is None:
+            eng.close()
+
+
+def findBestInormationContentContainingMotifsWithPCVOfSets(numberOfRepetitions, motifAmount, motifLength, pseudoCount, cutOff,
+                                                           alphabet, sets, pcvs, **kw) -> list:
+    """findBestInormationContentContainingMotifsWithPCV (fs:856-881) of every set, pcvs[s] the background of sets[s]; the
+    restarts of all sets run in one batch. Element s equals findBestInormationContentContainingMotifsWithPCV(...,
+    sets[s], pcvs[s]) with the same seed / chain."""
+    if pcvs is None:
+        raise _abi.GibbsArgumentError(_abi.GIBBS_ERR_ARG, "pcvs is null (ArgumentNullException)")
+    return _motif_restart_loop_of_sets(numberOfRepetitions, motifAmount, motifLength, pseudoCount, cutOff, alphabet, sets, pcvs,
+                                       **kw)
+
+
+def getMotifsWithBestInformationContentsOfSets(numberOfRepetitions, motifAmount, motifLength, pseudoCount, cutOff, alphabet,
+                                               sets, **kw) -> list:
+    """getMotifsWithBestInformationContents (fs:973-998) of every set, in one batch -- e.g. the reference script's fsx:407
+    call per gene group. Element s equals getMotifsWithBestInformationContents(..., sets[s]) with the same seed / chain."""
+    return _motif_restart_loop_of_sets(numberOfRepetitions, motifAmount, motifLength, pseudoCount, cutOff, alphabet, sets, None,
+                                       **kw)

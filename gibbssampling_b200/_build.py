@@ -7,6 +7,7 @@ The library is several translation units compiled in parallel and linked by nvcc
   gibbs_cluster_tu.cu one chain on a thread-block cluster of 4 / 8 CTAs (the last hand-over stages), one size per unit
   gibbs_init_tu.cu    the grid-wide random-start kernels, one kind per unit (same reason as the chain units)
   gibbs_batch_tu.cu   chain_batch_kernel (many sequence sets per launch), one group per unit like the chain units
+  gibbs_motif_batch_tu.cu  the MotifSampler's batch kernels (motifAmount 1 and 2), one group per unit
   gibbs_chain_tu.cu   compiled once per GROUP of chain_kernel instantiations (warps per chain x masked symbols x
                       drifting background), without --split-compile: small modules give reproducible code for the
                       register-limited hot kernel (see the header of that file)
@@ -29,10 +30,13 @@ CLUSTER_SOURCE = os.path.join(CSRC, "gibbs_cluster_tu.cu")
 MOTIF_SOURCE = os.path.join(CSRC, "gibbs_motif_tu.cu")
 MOTIF2_SOURCE = os.path.join(CSRC, "gibbs_motif2_tu.cu")
 BATCH_SOURCE = os.path.join(CSRC, "gibbs_batch_tu.cu")
-DEPS = [API_SOURCE, CHAIN_SOURCE, INIT_SOURCE, CLUSTER_SOURCE, MOTIF_SOURCE, MOTIF2_SOURCE, BATCH_SOURCE] + [os.path.join(CSRC, f) for f in (
-    "gibbs_device.cuh", "gibbs_kernels.cuh", "gibbs_motif.cuh", "gibbs_drift.cuh", "gibbs_drift_dev.cuh", "gibbs_cluster.cuh", "gibbs_motif2.cuh",
-    "gibbs_batch.cuh", "gibbs_chain_body.inc", "gibbs_restart_select_body.inc",
-)] + [os.path.join(ROOT, "include", "gibbs_b200.h"), os.path.abspath(__file__)]
+MOTIF_BATCH_SOURCE = os.path.join(CSRC, "gibbs_motif_batch_tu.cu")
+DEPS = [API_SOURCE, CHAIN_SOURCE, INIT_SOURCE, CLUSTER_SOURCE, MOTIF_SOURCE, MOTIF2_SOURCE, BATCH_SOURCE, MOTIF_BATCH_SOURCE] + [
+    os.path.join(CSRC, f) for f in (
+        "gibbs_device.cuh", "gibbs_kernels.cuh", "gibbs_motif.cuh", "gibbs_drift.cuh", "gibbs_drift_dev.cuh", "gibbs_cluster.cuh",
+        "gibbs_motif2.cuh", "gibbs_batch.cuh", "gibbs_motif_batch.cuh", "gibbs_chain_body.inc", "gibbs_restart_select_body.inc",
+        "gibbs_motif_body.inc", "gibbs_motif2_body.inc",
+    )] + [os.path.join(ROOT, "include", "gibbs_b200.h"), os.path.abspath(__file__)]
 
 # (entry point declared in gibbs_api.cu, warps per chain, masked symbols, drifting background)
 CHAIN_GROUPS = [
@@ -63,6 +67,12 @@ BATCH_GROUPS = [
     (f"launch_batch{'_init' if init else ''}{'_masked' if masked else ''}{'_drift' if drift else ''}_t{team}", team, masked, drift, init)
     for init in (0, 1) for masked in (0, 1) for drift in (0, 1) for team in (4, 1)
 ]
+
+# motif_batch_kernel / motif2_batch_kernel (gibbs_motif_batch_tu.cu): (entry point, motifAmount, warps per restart, masked
+# symbols) -- motifAmount 1: 4 warps for sets of >= 4 sequences, 1 warp for the rest; motifAmount 2: one warp, A,C,G,T only
+MOTIF_BATCH_GROUPS = [
+    (f"launch_motif_batch{'_masked' if masked else ''}_t{team}", 1, team, masked) for masked in (0, 1) for team in (4, 1)
+] + [("launch_motif2_batch", 2, 1, 0)]
 
 COMMON_FLAGS = [
     "-O3", "-std=c++17",
@@ -103,6 +113,11 @@ def _jobs(nvcc: str, verbose: bool) -> list[tuple[str, list[str]]]:
         jobs.append((obj, [nvcc] + COMMON_FLAGS + extra + [
             f"-DGIBBS_TU_NAME={name}", f"-DGIBBS_TU_T={team}", f"-DGIBBS_TU_MASKED={masked}", f"-DGIBBS_TU_DRIFT={drift}",
             f"-DGIBBS_TU_INIT_ONLY={init}", "-c", "-o", obj, BATCH_SOURCE]))
+    for name, m, team, masked in MOTIF_BATCH_GROUPS:
+        obj = os.path.join(OBJ_DIR, name + ".o")
+        jobs.append((obj, [nvcc] + COMMON_FLAGS + extra + [
+            f"-DGIBBS_TU_NAME={name}", f"-DGIBBS_TU_M={m}", f"-DGIBBS_TU_T={team}", f"-DGIBBS_TU_MASKED={masked}",
+            "-c", "-o", obj, MOTIF_BATCH_SOURCE]))
     for kind, name in enumerate(("launch_init_wide", "launch_init_wide_drift", "launch_init_smem", "launch_init_tiled")):
         obj = os.path.join(OBJ_DIR, name + ".o")
         jobs.append((obj, [nvcc] + COMMON_FLAGS + extra + [f"-DGIBBS_INIT_TU_KIND={kind}", "-c", "-o", obj, INIT_SOURCE]))

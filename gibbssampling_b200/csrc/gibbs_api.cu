@@ -10,6 +10,7 @@
 #include "gibbs_motif2.cuh"
 #include "gibbs_drift.cuh"
 #include "gibbs_batch.cuh"
+#include "gibbs_motif_batch.cuh"
 
 #include <algorithm>
 #include <cmath>
@@ -71,6 +72,12 @@ GIBBS_BATCH_TU(launch_batch_init_drift_t4); GIBBS_BATCH_TU(launch_batch_init_dri
 GIBBS_BATCH_TU(launch_batch_init_masked_t4); GIBBS_BATCH_TU(launch_batch_init_masked_t1);
 GIBBS_BATCH_TU(launch_batch_init_masked_drift_t4); GIBBS_BATCH_TU(launch_batch_init_masked_drift_t1);
 #undef GIBBS_BATCH_TU
+// gibbs_motif_batch_tu.cu: motif_batch_kernel, one unit per (masked symbols, warps per restart); motif2_batch_kernel
+#define GIBBS_MOTIF_BATCH_TU(name) cudaError_t name(const MotifArgs &run, const MotifBatchTable &bt, int grid, int smem, cudaStream_t stream)
+GIBBS_MOTIF_BATCH_TU(launch_motif_batch_t4); GIBBS_MOTIF_BATCH_TU(launch_motif_batch_t1);
+GIBBS_MOTIF_BATCH_TU(launch_motif_batch_masked_t4); GIBBS_MOTIF_BATCH_TU(launch_motif_batch_masked_t1);
+GIBBS_MOTIF_BATCH_TU(launch_motif2_batch);
+#undef GIBBS_MOTIF_BATCH_TU
 }
 
 using namespace gibbs;
@@ -369,6 +376,13 @@ const Unit<BatchLaunch> BATCH_UNITS[] = {
     {1, 0, 1, 1, launch_batch_init_drift_t1}, {4, 0, 1, 1, launch_batch_init_drift_t4},
     {1, 1, 0, 1, launch_batch_init_masked_t1}, {4, 1, 0, 1, launch_batch_init_masked_t4},
     {1, 1, 1, 1, launch_batch_init_masked_drift_t1}, {4, 1, 1, 1, launch_batch_init_masked_drift_t4},
+};
+
+// motifAmount = 1; the units serve both backgrounds (motifAmount = 2: launch_motif2_batch)
+using MotifBatchLaunch = cudaError_t (*)(const MotifArgs &, const MotifBatchTable &, int, int, cudaStream_t);
+const Unit<MotifBatchLaunch> MOTIF_BATCH_UNITS[] = {
+    {1, 0, 0, 0, launch_motif_batch_t1}, {4, 0, 0, 0, launch_motif_batch_t4},
+    {1, 1, 0, 0, launch_motif_batch_masked_t1}, {4, 1, 0, 0, launch_motif_batch_masked_t4},
 };
 
 // one launch of the chain_kernel unit for (warps per chain, masked symbols, drifting background, random starts only)
@@ -836,6 +850,17 @@ void fill_stats(gibbs_run_stats *out, const unsigned long long *st, int launches
     out->team_warps = team;
     out->init_path = init_path;
     out->kernel_ms = (double)ms;
+}
+
+// copies host to the device array dev when it differs from what was uploaded last (cache)
+template <typename T>
+int32_t upload_if_changed(std::vector<T> &host, std::vector<T> &cache, DevBuf<T> &dev, cudaStream_t stream) {
+    if (host.size() * sizeof(T) != cache.size() * sizeof(T) || memcmp(host.data(), cache.data(), host.size() * sizeof(T)) != 0) {
+        CUDA_TRY(dev.reserve(host.size()));
+        CUDA_TRY(cudaMemcpyAsync(dev.p, host.data(), host.size() * sizeof(T), cudaMemcpyHostToDevice, stream));
+        cache.swap(host);
+    }
+    return GIBBS_OK;
 }
 
 } // namespace
@@ -1768,8 +1793,9 @@ int32_t gibbs_measure_smem_bandwidth(int32_t device, int32_t iters, double *gbps
 
 /* ---- many independent sequence sets in one launch ------------------------------------------------------------------ */
 // The sets are uploaded as one concatenation into an internal handle (rows with a common row_words, lengths, mask plane,
-// stream, events); every set then gets its own ChainArgs that point into it (gibbs_batch.cuh). Per-set W / drift tables
-// are built with the single-set setup kernels, one small launch per set, and kept while the parameters stay the same.
+// stream, events); every set then gets its own ChainArgs that point into it (gibbs_batch.cuh), and for the MotifSampler its
+// own Motif2Args (gibbs_motif_batch.cuh). Per-set W / drift / background window tables are built with the single-set setup
+// kernels, one small launch per set, and kept while the parameters stay the same.
 struct gibbs_batch {
     gibbs_handle *h = nullptr;
     int32_t n_sets = 0, n_seqs = 0;
@@ -1780,26 +1806,36 @@ struct gibbs_batch {
     std::vector<int64_t> gcnt;                  // [n_sets][4] A,C,G,T counts (the data-derived background)
     DevBuf<int32_t> d_seq_off;
     // per-set tables, keyed by the parameters they were built for
-    DevBuf<WEnt> wtab;
+    DevBuf<WEnt> wtab;                          // set s at 4 m seq_off[s]: counts 0 .. m N_s - 1 (m = motifAmount)
     DevBuf<int> wt_range;                       // [n_sets][4]: min lg, max lg, non-normal W
-    DevBuf<double> pvals;
+    DevBuf<double> pvals;                       // set s at m seq_off[s]
     std::vector<int32_t> fast;                  // per set: the fixed-point ranking pass is usable
+    // MotifSampler, fixed background: background-only window tables (bg_setup_kernel), set s at g_off[s] with its own stride
+    DevBuf<double> bg_g, bg_sum, bg_max;
+    DevBuf<int32_t> bg_max_i;
+    std::vector<size_t> g_off;
     bool tab_valid = false;
-    int32_t tab_bgmode = -1, tab_alen = 0, tab_k = 0;
+    int32_t tab_bgmode = -1, tab_alen = 0, tab_k = 0, tab_m = 0, tab_bgwin = 0;
     double tab_pc = 0;
     std::vector<double> tab_bg;
     // per-set arguments and launch groups (uploaded when they change)
     std::vector<ChainArgs> args_host;
+    std::vector<Motif2Args> margs_host;
     std::vector<int32_t> groups_host;           // per group: set ids, then chain offsets
     DevBuf<ChainArgs> d_args;
+    DevBuf<Motif2Args> d_margs;
     DevBuf<int32_t> d_groups;
+    // MotifSampler scratch (per-set slices), Positions lists of motifAmount = 2, roulette error flag per set
+    DevBuf<double> cand_l, gbuf, sc;
+    DevBuf<int32_t> cand_w, pos2, err;
     // results
-    DevBuf<int32_t> sites, win_sites;           // win_sites: [n_seqs] winners' sites + [n_sets] restart index
+    DevBuf<int32_t> sites, win_sites;           // win_sites: [m n_seqs] winners' sites + [n_sets] restart index (+ [2 n_seqs] pair elements)
     DevBuf<double> hv, scores, sums, win_scores; // win_scores: [n_seqs] winners' scores + [n_sets] sums
     DevBuf<int32_t> counts;
     DevBuf<unsigned long long> stats;
     int32_t run_R = 0, run_k = 0, run_launches = 0, run_team = 0, run_fast = 0;
-    bool run_done = false;
+    int32_t run_sampler = GIBBS_SITE_SAMPLER, run_m = 1; // sampler and motifAmount of the last run
+    bool run_done = false, best_valid = false;
 };
 
 namespace {
@@ -1811,14 +1847,24 @@ int batch_team(const gibbs_batch *b, int s) {
     return (N >= 4 && team_smem_bytes(b->h->row_words, 4) <= 200 * 1024) ? 4 : 1;
 }
 
-int32_t batch_check(const gibbs_batch *b, const gibbs_params *p, const double *bg_per_set, int32_t R) {
+// motif: gibbs_batch_run_motif_device (the MotifSampler), else gibbs_batch_run_device (the SiteSampler)
+int32_t batch_check(const gibbs_batch *b, const gibbs_params *p, const double *bg_per_set, int32_t R, bool motif) {
     if (!b) return fail(GIBBS_ERR_ARG, "null batch");
     if (!p) return fail(GIBBS_ERR_ARG, "null params");
     if (R < 1) return fail(GIBBS_ERR_ARG, "restarts_per_set must be >= 1");
-    if (p->sampler != GIBBS_SITE_SAMPLER)
-        return fail(p->sampler == GIBBS_MOTIF_SAMPLER ? GIBBS_ERR_UNSUPPORTED : GIBBS_ERR_ARG,
-                    "batches run the SiteSampler only (sampler = %d)", p->sampler);
-    if (p->motif_amount > 1) return fail(GIBBS_ERR_ARG, "motif_amount belongs to the MotifSampler");
+    if (!motif) {
+        if (p->sampler != GIBBS_SITE_SAMPLER)
+            return fail(p->sampler == GIBBS_MOTIF_SAMPLER ? GIBBS_ERR_UNSUPPORTED : GIBBS_ERR_ARG,
+                        "gibbs_batch_run_device runs the SiteSampler (sampler = %d); MotifSampler batches run in "
+                        "gibbs_batch_run_motif_device", p->sampler);
+        if (p->motif_amount > 1) return fail(GIBBS_ERR_ARG, "motif_amount belongs to the MotifSampler");
+    } else {
+        if (p->sampler != GIBBS_MOTIF_SAMPLER)
+            return fail(GIBBS_ERR_ARG, "gibbs_batch_run_motif_device runs the MotifSampler (sampler = %d)", p->sampler);
+        if (p->motif_amount > 2)
+            return fail(GIBBS_ERR_UNSUPPORTED, "motifAmount = %d: combinations of one and two windows are built (fs:727-742); three "
+                                               "and more sites per sequence are not", p->motif_amount);
+    }
     if (p->phase_mask != 0) return fail(GIBBS_ERR_ARG, "batches run the whole pipeline: phase_mask must be 0");
     if (p->k < 1 || p->k > GIBBS_MAX_K) return fail(GIBBS_ERR_ARG, "motif width k=%d outside 1..%d", p->k, GIBBS_MAX_K);
     if (p->alphabet_size < 1) return fail(GIBBS_ERR_ARG, "alphabet_size must be >= 1");
@@ -1835,6 +1881,9 @@ int32_t batch_check(const gibbs_batch *b, const gibbs_params *p, const double *b
         if (b->has_gap[s] && p->alphabet_size >= 5)
             return fail(GIBBS_ERR_UNSUPPORTED, "set %d holds Gap '-' and alphabet_size = %d includes it: a fifth PWM row is not built "
                                                "(pass alphabet_size = 4 to score Gap like any other non-alphabet symbol)", s, p->alphabet_size);
+        if (motif && p->motif_amount == 2 && b->n_masked[s] > 0)
+            return fail(GIBBS_ERR_UNSUPPORTED, "set %d holds symbols outside A,C,G,T: the MotifSampler builds them for motifAmount = 1 "
+                                               "(motifAmount = 2 needs ACGT-only sequences)", s);
         const double *bg = p->background == GIBBS_BG_FIXED && bg_per_set ? bg_per_set + 4 * (size_t)s : p->bg;
         if (p->background == GIBBS_BG_FIXED)
             for (int x = 0; x < 4; ++x)
@@ -1847,20 +1896,36 @@ int32_t batch_check(const gibbs_batch *b, const gibbs_params *p, const double *b
     return GIBBS_OK;
 }
 
-// W tables (fixed background) or PPM value tables (data-derived) of every set, with the kernels of ensure_wtab / ensure_drift
-int32_t batch_tables(gibbs_batch *b, const gibbs_params *p, const double *bg_per_set, int *launches) {
+DeviceSeqs batch_seqs(const gibbs_batch *b, int32_t s) {
+    const gibbs_handle *h = b->h;
+    const int32_t o = b->seq_off[s];
+    DeviceSeqs d{};
+    d.packed = h->packed.p + (size_t)o * h->row_words;
+    d.len = h->len.p + o;
+    d.n = b->seq_off[s + 1] - o;
+    d.row_words = h->row_words;
+    d.uniform_len = b->min_len[s] == b->max_len[s] ? b->max_len[s] : 0;
+    d.mask = b->n_masked[s] > 0 ? h->mask.p + (size_t)o * h->row_words : nullptr;
+    d.rowflag = b->n_masked[s] > 0 ? h->rowflag.p + o : nullptr;
+    return d;
+}
+
+// Tables of every set, with the kernels of ensure_wtab / ensure_drift / ensure_bgtab: W tables (fixed background) or PPM
+// value tables (data-derived) over m N_s counts (m = motifAmount; the denominator keeps N_s), and for the MotifSampler on
+// the fixed background (bg_win) the background-only window tables
+int32_t batch_tables(gibbs_batch *b, const gibbs_params *p, const double *bg_per_set, int m, bool bg_win, int *launches) {
     gibbs_handle *h = b->h;
     std::vector<double> bg((size_t)b->n_sets * 4);
     for (int32_t s = 0; s < b->n_sets; ++s)
         for (int x = 0; x < 4; ++x) bg[4 * (size_t)s + x] = bg_per_set ? bg_per_set[4 * (size_t)s + x] : p->bg[x];
     const bool fixed = p->background == GIBBS_BG_FIXED;
     if (b->tab_valid && b->tab_bgmode == p->background && b->tab_pc == p->pseudocount && b->tab_alen == p->alphabet_size &&
-        b->tab_k == p->k && (!fixed || b->tab_bg == bg))
+        b->tab_k == p->k && b->tab_m == m && b->tab_bgwin == (int)bg_win && (!fixed || b->tab_bg == bg))
         return GIBBS_OK;
     b->tab_valid = false;
     b->fast.assign((size_t)b->n_sets, 0);
     if (fixed) {
-        CUDA_TRY(b->wtab.reserve((size_t)b->n_seqs * 4));
+        CUDA_TRY(b->wtab.reserve((size_t)b->n_seqs * 4 * m));
         CUDA_TRY(b->wt_range.reserve((size_t)b->n_sets * 4));
         std::vector<int> range((size_t)b->n_sets * 4);
         for (int32_t s = 0; s < b->n_sets; ++s) {
@@ -1870,13 +1935,30 @@ int32_t batch_tables(gibbs_batch *b, const gibbs_params *p, const double *bg_per
         }
         CUDA_TRY(cudaMemcpyAsync(b->wt_range.p, range.data(), range.size() * sizeof(int), cudaMemcpyHostToDevice, h->stream));
         for (int32_t s = 0; s < b->n_sets; ++s) {
-            const int N = b->seq_off[s + 1] - b->seq_off[s];
+            const int N = b->seq_off[s + 1] - b->seq_off[s], span = N * m;
             const double *q = bg.data() + 4 * (size_t)s;
-            wtab_kernel<<<(N * 4 + 255) / 256, 256, 0, h->stream>>>(N, p->pseudocount, ppm_den(N, p), q[0], q[1], q[2], q[3],
-                                                                    b->wtab.p + 4 * (size_t)b->seq_off[s], b->wt_range.p + 4 * (size_t)s);
+            wtab_kernel<<<(span * 4 + 255) / 256, 256, 0, h->stream>>>(span, p->pseudocount, ppm_den(N, p), q[0], q[1], q[2], q[3],
+                                                                       b->wtab.p + 4 * (size_t)m * b->seq_off[s], b->wt_range.p + 4 * (size_t)s);
             CUDA_TRY(cudaGetLastError());
         }
         *launches += b->n_sets;
+        if (bg_win) {
+            b->g_off.assign((size_t)b->n_sets + 1, 0);
+            for (int32_t s = 0; s < b->n_sets; ++s)
+                b->g_off[s + 1] = b->g_off[s] + (size_t)(b->seq_off[s + 1] - b->seq_off[s]) * (size_t)(b->max_len[s] - p->k + 1);
+            CUDA_TRY(b->bg_g.reserve(b->g_off[b->n_sets]));
+            CUDA_TRY(b->bg_sum.reserve((size_t)b->n_seqs));
+            CUDA_TRY(b->bg_max.reserve((size_t)b->n_seqs));
+            CUDA_TRY(b->bg_max_i.reserve((size_t)b->n_seqs));
+            for (int32_t s = 0; s < b->n_sets; ++s) {
+                const int32_t o = b->seq_off[s], N = b->seq_off[s + 1] - o;
+                const double *q = bg.data() + 4 * (size_t)s;
+                bg_setup_kernel<<<(N + 127) / 128, 128, 0, h->stream>>>(batch_seqs(b, s), p->k, q[0], q[1], q[2], q[3], b->max_len[s] - p->k + 1,
+                                                                       b->bg_g.p + b->g_off[s], b->bg_sum.p + o, b->bg_max.p + o, b->bg_max_i.p + o);
+                CUDA_TRY(cudaGetLastError());
+            }
+            *launches += b->n_sets;
+        }
         CUDA_TRY(cudaMemcpyAsync(range.data(), b->wt_range.p, range.size() * sizeof(int), cudaMemcpyDeviceToHost, h->stream));
         CUDA_TRY(cudaStreamSynchronize(h->stream));
         for (int32_t s = 0; s < b->n_sets; ++s)
@@ -1886,10 +1968,10 @@ int32_t batch_tables(gibbs_batch *b, const gibbs_params *p, const double *bg_per
         // the host's per-set counts (checked against int32 per set in batch_check), not from the whole concatenation
         int32_t rc = ensure_seq_counts(h, launches);
         if (rc) return rc;
-        CUDA_TRY(b->pvals.reserve((size_t)b->n_seqs));
+        CUDA_TRY(b->pvals.reserve((size_t)b->n_seqs * m));
         for (int32_t s = 0; s < b->n_sets; ++s) {
-            const int N = b->seq_off[s + 1] - b->seq_off[s];
-            pvals_kernel<<<(N + 255) / 256, 256, 0, h->stream>>>(N, p->pseudocount, ppm_den(N, p), b->pvals.p + b->seq_off[s]);
+            const int N = b->seq_off[s + 1] - b->seq_off[s], span = N * m;
+            pvals_kernel<<<(span + 255) / 256, 256, 0, h->stream>>>(span, p->pseudocount, ppm_den(N, p), b->pvals.p + (size_t)m * b->seq_off[s]);
             CUDA_TRY(cudaGetLastError());
             int32_t g[4];
             for (int x = 0; x < 4; ++x) g[x] = (int32_t)b->gcnt[4 * (size_t)s + x];
@@ -1902,8 +1984,121 @@ int32_t batch_tables(gibbs_batch *b, const gibbs_params *p, const double *bg_per
     b->tab_pc = p->pseudocount;
     b->tab_alen = p->alphabet_size;
     b->tab_k = p->k;
+    b->tab_m = m;
+    b->tab_bgwin = bg_win ? 1 : 0;
     b->tab_bg = bg;
     b->tab_valid = true;
+    return GIBBS_OK;
+}
+
+// the result buffers of a run of R restarts per set, the statistics cleared
+int32_t batch_results(gibbs_batch *b, int32_t R) {
+    const size_t cells = (size_t)R * b->n_seqs;
+    CUDA_TRY(b->sites.reserve(cells));
+    CUDA_TRY(b->hv.reserve(cells));
+    CUDA_TRY(b->scores.reserve(cells));
+    CUDA_TRY(b->sums.reserve((size_t)b->n_sets * R));
+    CUDA_TRY(b->stats.reserve(ST_NSLOTS));
+    CUDA_TRY(cudaMemsetAsync(b->stats.p, 0, ST_NSLOTS * sizeof(unsigned long long), b->h->stream));
+    return GIBBS_OK;
+}
+
+// the ChainArgs of set s: its rows and tables (m = motifAmount of the tables), its slices of the results
+ChainArgs batch_set_args(const gibbs_batch *b, const gibbs_params *p, int32_t s, int32_t R, int m) {
+    const gibbs_handle *h = b->h;
+    const int32_t o = b->seq_off[s];
+    const bool drift = p->background == GIBBS_BG_DATA;
+    ChainArgs a;
+    memset(&a, 0, sizeof a);
+    a.s = batch_seqs(b, s);
+    a.k = p->k;
+    a.sampler = GIBBS_SITE_SAMPLER;
+    a.n_chains = R;
+    a.sites = b->sites.p + (size_t)R * o;
+    a.hv = b->hv.p + (size_t)R * o;
+    a.scores = b->scores.p + (size_t)R * o;
+    a.sums = b->sums.p + (size_t)R * s;
+    a.fast_ok = b->fast[s];
+    if (drift) {
+        a.pvals = b->pvals.p + (size_t)m * o;
+        a.basecnt = h->basecnt.p + 4 * (size_t)o;
+        a.maskcnt = b->n_masked[s] > 0 ? h->maskcnt.p + o : nullptr;
+        a.ss = h->ss_valid ? h->ss.p + (size_t)o * (size_t)(h->max_len + 2) * 4 : nullptr;
+        a.ss_stride = h->max_len + 2;
+        for (int x = 0; x < 4; ++x) a.gcnt[x] = (int32_t)b->gcnt[4 * (size_t)s + x];
+        a.alpha_pc = (double)p->alphabet_size * p->pseudocount; // fs:117
+        a.pc = p->pseudocount;
+        a.drift_fast_ok = b->fast[s];
+    } else {
+        a.wtab = b->wtab.p + 4 * (size_t)m * o;
+        memcpy(a.bg, b->tab_bg.data() + 4 * (size_t)s, sizeof a.bg);
+    }
+    return a;
+}
+
+// Launch groups: (masked symbols) x (4 warps per chain for sets of >= 4 sequences, else 1), then with all_sets one more
+// group of every set (motifAmount = 2: one warp per restart). ids[g] = the sets of group g, at[g] = its offset in groups.
+int32_t batch_groups(gibbs_batch *b, int32_t R, bool all_sets, std::vector<int32_t> *ids, size_t *at) {
+    for (int32_t s = 0; s < b->n_sets; ++s) ids[(b->n_masked[s] > 0 ? 2 : 0) + (batch_team(b, s) == 4 ? 0 : 1)].push_back(s);
+    if (all_sets)
+        for (int32_t s = 0; s < b->n_sets; ++s) ids[BATCH_GROUPS].push_back(s);
+    std::vector<int32_t> groups;
+    for (int g = 0; g < BATCH_GROUPS + (all_sets ? 1 : 0); ++g) {
+        at[g] = groups.size();
+        groups.insert(groups.end(), ids[g].begin(), ids[g].end());
+        for (size_t i = 0; i <= ids[g].size(); ++i) groups.push_back((int32_t)(i * (size_t)R));
+    }
+    if (groups != b->groups_host) {
+        CUDA_TRY(b->d_groups.reserve(groups.size()));
+        CUDA_TRY(cudaMemcpyAsync(b->d_groups.p, groups.data(), groups.size() * sizeof(int32_t), cudaMemcpyHostToDevice, b->h->stream));
+        b->groups_host.swap(groups);
+    }
+    return GIBBS_OK;
+}
+
+// every group's random starts (chain_batch_kernel<.., INIT_ONLY>) or sweeps of a SiteSampler run
+int32_t batch_launch_chains(gibbs_batch *b, const ChainArgs &run, bool drift, bool init, const std::vector<int32_t> *ids,
+                            const size_t *at, int R, int *launches) {
+    gibbs_handle *h = b->h;
+    const long long per_sm = ((long long)b->n_sets * R + h->sm_count - 1) / h->sm_count;
+    for (int g = 0; g < BATCH_GROUPS; ++g) {
+        const int n = (int)ids[g].size();
+        if (n == 0) continue;
+        const bool masked = g >= 2;
+        const int team = (g & 1) ? 1 : 4;
+        if (!b->run_team) b->run_team = team;
+        BatchTable bt;
+        bt.sets = b->d_args.p;
+        bt.set_ids = b->d_groups.p + at[g];
+        bt.chain_off = b->d_groups.p + at[g] + n;
+        bt.n = n;
+        ChainArgs r = run;
+        r.min_width = per_sm <= 1 ? team : 1; // (as plan_stages: never narrow once a chain has an SM to itself)
+        BatchLaunch f;
+        const int32_t rc = find_unit(BATCH_UNITS, "batch", team, masked, drift, init, &f);
+        if (rc) return rc;
+        CUDA_TRY(f(r, bt, n * R, team_smem_bytes(h->row_words, team), h->stream));
+        ++*launches;
+    }
+    return GIBBS_OK;
+}
+
+// copies the per-set roulette error flags of a MotifSampler run into err (queued; read after the stream synchronises)
+int32_t batch_queue_errors(const gibbs_batch *b, std::vector<int32_t> &err) {
+    if (b->run_sampler != GIBBS_MOTIF_SAMPLER) return GIBBS_OK;
+    try {
+        err.assign((size_t)b->n_sets, 0);
+    } catch (...) {
+        return fail(GIBBS_ERR_NOMEM, "host allocation failed");
+    }
+    CUDA_TRY(cudaMemcpyAsync(err.data(), b->err.p, (size_t)b->n_sets * sizeof(int32_t), cudaMemcpyDeviceToHost, b->h->stream));
+    return GIBBS_OK;
+}
+
+int32_t batch_check_errors(const std::vector<int32_t> &err) {
+    for (size_t s = 0; s < err.size(); ++s)
+        if (err[s])
+            return fail(GIBBS_ERR_ROULETTE, "set %d: a roulette pick lay beyond the accumulated mass (ArgumentException, fs:753)", (int)s);
     return GIBBS_OK;
 }
 
@@ -1998,7 +2193,7 @@ int32_t gibbs_batch_destroy(gibbs_batch *b) {
 
 int32_t gibbs_batch_run_device(gibbs_batch *b, const gibbs_params *p, const double *bg_per_set, int32_t restarts_per_set,
                                int64_t chain_id_base, uint64_t seed) {
-    int32_t rc = batch_check(b, p, bg_per_set, restarts_per_set);
+    int32_t rc = batch_check(b, p, bg_per_set, restarts_per_set, false);
     if (rc) return rc;
     gibbs_handle *h = b->h;
     rc = set_device(h);
@@ -2007,15 +2202,10 @@ int32_t gibbs_batch_run_device(gibbs_batch *b, const gibbs_params *p, const doub
     const int32_t R = restarts_per_set, S = b->n_sets;
     const bool drift = p->background == GIBBS_BG_DATA;
     int launches = 0;
-    rc = batch_tables(b, p, bg_per_set, &launches);
+    rc = batch_tables(b, p, bg_per_set, 1, false, &launches);
     if (rc) return rc;
-    const size_t cells = (size_t)R * b->n_seqs;
-    CUDA_TRY(b->sites.reserve(cells));
-    CUDA_TRY(b->hv.reserve(cells));
-    CUDA_TRY(b->scores.reserve(cells));
-    CUDA_TRY(b->sums.reserve((size_t)S * R));
-    CUDA_TRY(b->stats.reserve(ST_NSLOTS));
-    CUDA_TRY(cudaMemsetAsync(b->stats.p, 0, ST_NSLOTS * sizeof(unsigned long long), h->stream));
+    rc = batch_results(b, R);
+    if (rc) return rc;
 
     // run-wide arguments (chain_batch_kernel copies them over the set's own)
     ChainArgs run{};
@@ -2028,88 +2218,163 @@ int32_t gibbs_batch_run_device(gibbs_batch *b, const gibbs_params *p, const doub
     run.chain_id_base = chain_id_base;
     run.stats = b->stats.p;
 
-    // per-set arguments: the set's rows and tables, its slices of the results
     std::vector<ChainArgs> args((size_t)S);
-    const int rw = h->row_words;
     int fast_all = 1;
     for (int32_t s = 0; s < S; ++s) {
-        const int32_t o = b->seq_off[s], N = b->seq_off[s + 1] - o;
-        ChainArgs &a = args[s];
-        memset(&a, 0, sizeof a);
-        a.s.packed = h->packed.p + (size_t)o * rw;
-        a.s.len = h->len.p + o;
-        a.s.n = N;
-        a.s.row_words = rw;
-        a.s.uniform_len = b->min_len[s] == b->max_len[s] ? b->max_len[s] : 0;
-        a.s.mask = b->n_masked[s] > 0 ? h->mask.p + (size_t)o * rw : nullptr;
-        a.s.rowflag = b->n_masked[s] > 0 ? h->rowflag.p + o : nullptr;
-        a.k = p->k;
-        a.sampler = GIBBS_SITE_SAMPLER;
-        a.n_chains = R;
-        a.sites = b->sites.p + (size_t)R * o;
-        a.hv = b->hv.p + (size_t)R * o;
-        a.scores = b->scores.p + (size_t)R * o;
-        a.sums = b->sums.p + (size_t)R * s;
-        a.fast_ok = b->fast[s];
+        args[s] = batch_set_args(b, p, s, R, 1);
         fast_all &= b->fast[s];
-        if (drift) {
-            a.pvals = b->pvals.p + o;
-            a.basecnt = h->basecnt.p + 4 * (size_t)o;
-            a.maskcnt = b->n_masked[s] > 0 ? h->maskcnt.p + o : nullptr;
-            a.ss = h->ss_valid ? h->ss.p + (size_t)o * (size_t)(h->max_len + 2) * 4 : nullptr;
-            a.ss_stride = h->max_len + 2;
-            for (int x = 0; x < 4; ++x) a.gcnt[x] = (int32_t)b->gcnt[4 * (size_t)s + x];
-            a.alpha_pc = (double)p->alphabet_size * p->pseudocount; // fs:117
-            a.pc = p->pseudocount;
-            a.drift_fast_ok = b->fast[s];
-        } else {
-            a.wtab = b->wtab.p + 4 * (size_t)o;
-            memcpy(a.bg, b->tab_bg.data() + 4 * (size_t)s, sizeof a.bg);
-        }
     }
-    // launch groups: (masked symbols) x (4 warps per chain for sets of >= 4 sequences, else 1)
     std::vector<int32_t> ids[BATCH_GROUPS];
-    for (int32_t s = 0; s < S; ++s) ids[(b->n_masked[s] > 0 ? 2 : 0) + (batch_team(b, s) == 4 ? 0 : 1)].push_back(s);
-    std::vector<int32_t> groups;
     size_t g_at[BATCH_GROUPS];
-    for (int g = 0; g < BATCH_GROUPS; ++g) {
-        g_at[g] = groups.size();
-        groups.insert(groups.end(), ids[g].begin(), ids[g].end());
-        for (size_t i = 0; i <= ids[g].size(); ++i) groups.push_back((int32_t)(i * (size_t)R));
-    }
-    if (args.size() * sizeof(ChainArgs) != b->args_host.size() * sizeof(ChainArgs) ||
-        memcmp(args.data(), b->args_host.data(), args.size() * sizeof(ChainArgs)) != 0) {
-        CUDA_TRY(b->d_args.reserve(args.size()));
-        CUDA_TRY(cudaMemcpyAsync(b->d_args.p, args.data(), args.size() * sizeof(ChainArgs), cudaMemcpyHostToDevice, h->stream));
-        b->args_host.swap(args);
-    }
-    if (groups != b->groups_host) {
-        CUDA_TRY(b->d_groups.reserve(groups.size()));
-        CUDA_TRY(cudaMemcpyAsync(b->d_groups.p, groups.data(), groups.size() * sizeof(int32_t), cudaMemcpyHostToDevice, h->stream));
-        b->groups_host.swap(groups);
-    }
-    const long long total_chains = (long long)S * R;
-    const long long per_sm = (total_chains + h->sm_count - 1) / h->sm_count;
+    rc = batch_groups(b, R, false, ids, g_at);
+    if (rc) return rc;
+    rc = upload_if_changed(args, b->args_host, b->d_args, h->stream);
+    if (rc) return rc;
     b->run_team = 0;
     CUDA_TRY(cudaEventRecord(h->ev0, h->stream));
     for (int init = 1; init >= 0; --init) { // every group's random starts, then every group's sweeps
+        rc = batch_launch_chains(b, run, drift, init != 0, ids, g_at, R, &launches);
+        if (rc) return rc;
+    }
+    CUDA_TRY(cudaEventRecord(h->ev1, h->stream));
+    b->run_R = R;
+    b->run_k = p->k;
+    b->run_fast = fast_all;
+    b->run_launches = launches;
+    b->run_sampler = GIBBS_SITE_SAMPLER;
+    b->run_m = 1;
+    b->best_valid = false;
+    b->run_done = true;
+    return GIBBS_OK;
+}
+
+int32_t gibbs_batch_run_motif_device(gibbs_batch *b, const gibbs_params *p, const double *bg_per_set, int32_t restarts_per_set,
+                                     int64_t chain_id_base, uint64_t seed) {
+    int32_t rc = batch_check(b, p, bg_per_set, restarts_per_set, true);
+    if (rc) return rc;
+    gibbs_handle *h = b->h;
+    rc = set_device(h);
+    if (rc) return rc;
+    b->run_done = false;
+    const int32_t R = restarts_per_set, S = b->n_sets, M = p->motif_amount == 2 ? 2 : 1;
+    const bool drift = p->background == GIBBS_BG_DATA;
+    int launches = 0;
+    rc = batch_tables(b, p, bg_per_set, M, !drift, &launches);
+    if (rc) return rc;
+    rc = batch_results(b, R);
+    if (rc) return rc;
+
+    // scratch lists: set s holds R x T_s lists of its own window stride W_s (a 100 kb set does not widen the others')
+    std::vector<size_t> scr((size_t)S + 1, 0);
+    std::vector<int32_t> wstride((size_t)S);
+    for (int32_t s = 0; s < S; ++s) {
+        int W = b->max_len[s] - p->k + 1;
+        if (drift && b->n_masked[s] > 0 && W < 64) W = 64; // the candidate scratch doubles as a 49-slot symbol-count table
+        wstride[s] = W;
+        scr[s + 1] = scr[s] + (size_t)R * (M == 2 ? 1 : batch_team(b, s)) * W;
+    }
+    const size_t cells = (size_t)R * b->n_seqs;
+    CUDA_TRY(b->cand_l.reserve(scr[S]));
+    CUDA_TRY(b->cand_w.reserve(scr[S]));
+    if (drift) CUDA_TRY(b->gbuf.reserve(scr[S]));
+    if (M == 2) {
+        CUDA_TRY(b->sc.reserve(scr[S]));
+        CUDA_TRY(b->pos2.reserve(cells * 2));
+    }
+    CUDA_TRY(b->err.reserve((size_t)S));
+    CUDA_TRY(cudaMemsetAsync(b->err.p, 0, (size_t)S * sizeof(int32_t), h->stream));
+
+    // per-set arguments: the ChainArgs of the random starts and, around them, the MotifSampler's own
+    std::vector<ChainArgs> args((size_t)S);
+    std::vector<Motif2Args> margs((size_t)S);
+    int fast_all = 1;
+    for (int32_t s = 0; s < S; ++s) {
+        const int32_t o = b->seq_off[s];
+        ChainArgs &a = args[s];
+        a = batch_set_args(b, p, s, R, M);
+        a.sampler = GIBBS_MOTIF_SAMPLER;
+        a.cutoff = p->cutoff;
+        if (drift) a.fast_ok = 0; // (as gibbs_run_device: the data-derived background's range check is drift_fast_ok)
+        fast_all &= b->fast[s];
+        Motif2Args &q = margs[s];
+        memset(&q, 0, sizeof q);
+        MotifArgs &m = q.m;
+        m.c = a;
+        if (!drift) {
+            m.bg.g = b->bg_g.p + b->g_off[s];
+            m.bg.gsum = b->bg_sum.p + o;
+            m.bg.gmax = b->bg_max.p + o;
+            m.bg.gmax_i = b->bg_max_i.p + o;
+        }
+        m.bg.wstride = wstride[s];
+        m.cand_l = b->cand_l.p + scr[s];
+        m.cand_w = b->cand_w.p + scr[s];
+        m.error = b->err.p + s;
+        m.data_bg = drift ? 1 : 0;
+        m.greedy_fast_ok = b->fast[s];
+        if (drift) {
+            m.pvals = a.pvals;
+            m.basecnt = a.basecnt;
+            memcpy(m.gcnt, a.gcnt, sizeof m.gcnt);
+            m.alpha_pc = a.alpha_pc;
+            m.pc = a.pc;
+            m.gbuf = b->gbuf.p + scr[s];
+        }
+        m.roulette_scan_ok = h->opt_exact_scans ? 0 : 1;
+        m.ascii = h->ascii.p;
+        m.off = h->off.p + o;
+        if (M == 2) {
+            q.pos2 = b->pos2.p + 2 * (size_t)R * o;
+            q.sc = b->sc.p + scr[s];
+        }
+    }
+    std::vector<int32_t> ids[BATCH_GROUPS + 1];
+    size_t g_at[BATCH_GROUPS + 1];
+    rc = batch_groups(b, R, M == 2, ids, g_at);
+    if (rc) return rc;
+    rc = upload_if_changed(args, b->args_host, b->d_args, h->stream);
+    if (rc) return rc;
+    rc = upload_if_changed(margs, b->margs_host, b->d_margs, h->stream);
+    if (rc) return rc;
+
+    // run-wide arguments: the random starts are the SiteSampler's (fs:876, fs:993), then the stochastic and greedy sweeps
+    ChainArgs run{};
+    run.k = p->k;
+    run.max_sweeps = p->max_sweeps > 0 ? p->max_sweeps : 1000000;
+    run.sampler = GIBBS_MOTIF_SAMPLER;
+    run.phase_mask = GIBBS_PHASE_INIT | GIBBS_PHASE_STOCHASTIC | GIBBS_PHASE_MOTIF_GREEDY;
+    run.rng_mode = GIBBS_RNG_PHILOX;
+    run.seed = seed;
+    run.chain_id_base = chain_id_base;
+    run.stats = b->stats.p;
+    MotifArgs mrun{};
+    mrun.c = run;
+    mrun.c.phase_mask = GIBBS_PHASE_STOCHASTIC | GIBBS_PHASE_MOTIF_GREEDY;
+    mrun.c.cutoff = p->cutoff;
+    mrun.init_done = 1;
+    b->run_team = 0;
+    CUDA_TRY(cudaEventRecord(h->ev0, h->stream));
+    rc = batch_launch_chains(b, run, drift, true, ids, g_at, R, &launches);
+    if (rc) return rc;
+    if (M == 2) {
+        const int n = (int)ids[BATCH_GROUPS].size();
+        const MotifBatchTable bt{b->d_margs.p, b->d_groups.p + g_at[BATCH_GROUPS], b->d_groups.p + g_at[BATCH_GROUPS] + n, n};
+        CUDA_TRY(launch_motif2_batch(mrun, bt, n * R, team_smem_bytes(h->row_words, 1), h->stream));
+        ++launches;
+        b->run_team = 1;
+    } else {
+        b->run_team = 0;
         for (int g = 0; g < BATCH_GROUPS; ++g) {
             const int n = (int)ids[g].size();
             if (n == 0) continue;
             const bool masked = g >= 2;
             const int team = (g & 1) ? 1 : 4;
             if (!b->run_team) b->run_team = team;
-            BatchTable bt;
-            bt.sets = b->d_args.p;
-            bt.set_ids = b->d_groups.p + g_at[g];
-            bt.chain_off = b->d_groups.p + g_at[g] + n;
-            bt.n = n;
-            ChainArgs r = run;
-            r.min_width = per_sm <= 1 ? team : 1; // (as plan_stages: never narrow once a chain has an SM to itself)
-            BatchLaunch f;
-            rc = find_unit(BATCH_UNITS, "batch", team, masked, drift, init != 0, &f);
+            const MotifBatchTable bt{b->d_margs.p, b->d_groups.p + g_at[g], b->d_groups.p + g_at[g] + n, n};
+            MotifBatchLaunch f;
+            rc = find_unit(MOTIF_BATCH_UNITS, "MotifSampler batch", team, masked, false, false, &f);
             if (rc) return rc;
-            CUDA_TRY(f(r, bt, n * R, team_smem_bytes(h->row_words, team), h->stream));
+            CUDA_TRY(f(mrun, bt, n * R, team_smem_bytes(h->row_words, team), h->stream));
             ++launches;
         }
     }
@@ -2118,6 +2383,9 @@ int32_t gibbs_batch_run_device(gibbs_batch *b, const gibbs_params *p, const doub
     b->run_k = p->k;
     b->run_fast = fast_all;
     b->run_launches = launches;
+    b->run_sampler = GIBBS_MOTIF_SAMPLER;
+    b->run_m = M;
+    b->best_valid = false;
     b->run_done = true;
     return GIBBS_OK;
 }
@@ -2141,7 +2409,12 @@ int32_t gibbs_batch_fetch(gibbs_batch *b, int32_t *sites_out, double *scores_out
         CUDA_TRY(cudaMemcpyAsync(sums_out, b->sums.p, (size_t)b->run_R * b->n_sets * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
     unsigned long long st[ST_NSLOTS];
     CUDA_TRY(cudaMemcpyAsync(st, b->stats.p, sizeof st, cudaMemcpyDeviceToHost, h->stream));
+    std::vector<int32_t> err;
+    rc = batch_queue_errors(b, err);
+    if (rc) return rc;
     CUDA_TRY(cudaStreamSynchronize(h->stream));
+    rc = batch_check_errors(err);
+    if (rc) return rc;
     if (stats_out) batch_stats(b, st, 0, stats_out);
     return GIBBS_OK;
 }
@@ -2154,40 +2427,114 @@ int32_t gibbs_batch_fetch_best(gibbs_batch *b, int32_t repetitions, int32_t *sit
     gibbs_handle *h = b->h;
     int32_t rc = set_device(h);
     if (rc) return rc;
-    const int32_t S = b->n_sets, NT = b->n_seqs, k = b->run_k;
-    CUDA_TRY(b->win_sites.reserve((size_t)NT + S));
+    const int32_t S = b->n_sets, NT = b->n_seqs, k = b->run_k, M = b->run_m;
+    const bool motif = b->run_sampler == GIBBS_MOTIF_SAMPLER;
+    const size_t NS = (size_t)M * NT; // site entries of the winners (Positions lists for motifAmount = 2)
+    CUDA_TRY(b->win_sites.reserve(NS + S + (M == 2 ? 2 * (size_t)NT : 0)));
     CUDA_TRY(b->win_scores.reserve((size_t)NT + S));
-    restart_select_batch_kernel<<<S, 32, 0, h->stream>>>(b->sums.p, b->sites.p, b->scores.p, b->d_seq_off.p, b->run_R, repetitions,
-                                                        b->win_sites.p + NT, b->win_sites.p, b->win_scores.p, b->win_scores.p + NT);
+    if (motif)
+        restart_select_motif_batch_kernel<<<S, 32, 0, h->stream>>>(b->sums.p, M == 2 ? b->pos2.p : b->sites.p, b->scores.p, b->d_seq_off.p,
+                                                                   b->run_R, repetitions, M, b->win_sites.p + NS, b->win_sites.p,
+                                                                   b->win_scores.p, b->win_scores.p + NT);
+    else
+        restart_select_batch_kernel<<<S, 32, 0, h->stream>>>(b->sums.p, b->sites.p, b->scores.p, b->d_seq_off.p, b->run_R, repetitions,
+                                                            b->win_sites.p + NT, b->win_sites.p, b->win_scores.p, b->win_scores.p + NT);
     CUDA_TRY(cudaGetLastError());
     int extra_launches = 1;
-    std::vector<int32_t> best((size_t)S);
-    CUDA_TRY(cudaMemcpyAsync(best.data(), b->win_sites.p + NT, (size_t)S * sizeof(int32_t), cudaMemcpyDeviceToHost, h->stream));
+    std::vector<int32_t> best((size_t)S), pairs, counts2;
+    CUDA_TRY(cudaMemcpyAsync(best.data(), b->win_sites.p + NS, (size_t)S * sizeof(int32_t), cudaMemcpyDeviceToHost, h->stream));
     if (sum_out) CUDA_TRY(cudaMemcpyAsync(sum_out, b->win_scores.p + NT, (size_t)S * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
-    if (sites_out) CUDA_TRY(cudaMemcpyAsync(sites_out, b->win_sites.p, (size_t)NT * sizeof(int32_t), cudaMemcpyDeviceToHost, h->stream));
+    if (sites_out) {
+        if (M == 1) {
+            CUDA_TRY(cudaMemcpyAsync(sites_out, b->win_sites.p, (size_t)NT * sizeof(int32_t), cudaMemcpyDeviceToHost, h->stream));
+        } else { // sites_out gets the newest position of each Positions list
+            try {
+                pairs.resize(NS);
+            } catch (...) {
+                return fail(GIBBS_ERR_NOMEM, "host allocation failed");
+            }
+            CUDA_TRY(cudaMemcpyAsync(pairs.data(), b->win_sites.p, NS * sizeof(int32_t), cudaMemcpyDeviceToHost, h->stream));
+        }
+    }
     if (scores_out) CUDA_TRY(cudaMemcpyAsync(scores_out, b->win_scores.p, (size_t)NT * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
     if (counts_out) { // PWM counts of every winner's sites (all zero where the initial value survived: its sites are -1)
-        CUDA_TRY(b->counts.reserve((size_t)S * k * 4));
-        rc = with_kp(k, [&](auto kp) -> int32_t {
-            all_counts_batch_kernel<kp()><<<S, 32, 0, h->stream>>>(b->d_args.p, b->d_seq_off.p, b->win_sites.p, k, b->counts.p);
-            CUDA_TRY(cudaGetLastError());
-            return GIBBS_OK;
-        });
-        if (rc) return rc;
-        ++extra_launches;
-        CUDA_TRY(cudaMemcpyAsync(counts_out, b->counts.p, (size_t)S * k * 4 * sizeof(int32_t), cudaMemcpyDeviceToHost, h->stream));
+        const size_t per = (size_t)S * k * 4;
+        CUDA_TRY(b->counts.reserve(per * M));
+        for (int which = 0; which < M; ++which) { // motifAmount = 2: both elements of every Positions pair
+            const int32_t *src = b->win_sites.p;
+            if (M == 2) {
+                int32_t *tmp = b->win_sites.p + NS + S + (size_t)which * NT;
+                pair_element_kernel<<<(NT + 255) / 256, 256, 0, h->stream>>>(b->win_sites.p, NT, which, tmp);
+                CUDA_TRY(cudaGetLastError());
+                ++extra_launches;
+                src = tmp;
+            }
+            rc = with_kp(k, [&](auto kp) -> int32_t {
+                all_counts_batch_kernel<kp()><<<S, 32, 0, h->stream>>>(b->d_args.p, b->d_seq_off.p, src, k, b->counts.p + per * which);
+                CUDA_TRY(cudaGetLastError());
+                return GIBBS_OK;
+            });
+            if (rc) return rc;
+            ++extra_launches;
+        }
+        if (M == 1) {
+            CUDA_TRY(cudaMemcpyAsync(counts_out, b->counts.p, per * sizeof(int32_t), cudaMemcpyDeviceToHost, h->stream));
+        } else {
+            try {
+                counts2.resize(per * 2);
+            } catch (...) {
+                return fail(GIBBS_ERR_NOMEM, "host allocation failed");
+            }
+            CUDA_TRY(cudaMemcpyAsync(counts2.data(), b->counts.p, per * 2 * sizeof(int32_t), cudaMemcpyDeviceToHost, h->stream));
+        }
     }
     unsigned long long st[ST_NSLOTS];
     CUDA_TRY(cudaMemcpyAsync(st, b->stats.p, sizeof st, cudaMemcpyDeviceToHost, h->stream));
+    std::vector<int32_t> err;
+    rc = batch_queue_errors(b, err);
+    if (rc) return rc;
     CUDA_TRY(cudaStreamSynchronize(h->stream));
+    rc = batch_check_errors(err);
+    if (rc) return rc;
+    b->best_valid = true;
+    if (sites_out && M == 2)
+        for (int32_t i = 0; i < NT; ++i) sites_out[i] = pairs[(size_t)2 * i];
+    if (counts_out && M == 2)
+        for (size_t e = 0; e < (size_t)S * k * 4; ++e) counts_out[e] = counts2[e] + counts2[(size_t)S * k * 4 + e];
     for (int32_t s = 0; s < S; ++s) {
-        const bool initial = best[s] < 0; // loop 0 [||] [|(0., 0)|] returned its initial value (quirk A.6-8)
-        if (initial && sites_out) sites_out[b->seq_off[s]] = 0;
+        // loop 0 [||] [|(0., 0)|] returned its initial value (quirk A.6-8); the MotifSampler's is [|{PWMS 0; Positions []}|]
+        const bool initial = best[s] < 0;
+        if (initial && sites_out) sites_out[b->seq_off[s]] = motif ? -1 : 0;
         if (initial && scores_out) scores_out[b->seq_off[s]] = 0.0;
         if (n_out) n_out[s] = initial ? 1 : b->seq_off[s + 1] - b->seq_off[s];
         if (restart_out) restart_out[s] = best[s];
     }
     if (stats_out) batch_stats(b, st, extra_launches, stats_out);
+    return GIBBS_OK;
+}
+
+int32_t gibbs_batch_fetch_positions(gibbs_batch *b, int32_t m, int32_t *positions_out) {
+    if (!b || !positions_out) return fail(GIBBS_ERR_ARG, "null argument");
+    if (!b->run_done) return fail(GIBBS_ERR_ARG, "gibbs_batch_fetch_positions without a preceding run");
+    if (m != b->run_m) return fail(GIBBS_ERR_ARG, "the last run had motif_amount = %d", b->run_m);
+    gibbs_handle *h = b->h;
+    int32_t rc = set_device(h);
+    if (rc) return rc;
+    const size_t cells = (size_t)b->run_R * b->n_seqs;
+    CUDA_TRY(cudaMemcpyAsync(positions_out, m == 2 ? b->pos2.p : b->sites.p, cells * m * sizeof(int32_t), cudaMemcpyDeviceToHost, h->stream));
+    CUDA_TRY(cudaStreamSynchronize(h->stream));
+    return GIBBS_OK;
+}
+
+int32_t gibbs_batch_fetch_best_positions(gibbs_batch *b, int32_t m, int32_t *positions_out) {
+    if (!b || !positions_out) return fail(GIBBS_ERR_ARG, "null argument");
+    if (!b->run_done || !b->best_valid) return fail(GIBBS_ERR_ARG, "gibbs_batch_fetch_best_positions without a preceding gibbs_batch_fetch_best");
+    if (m != b->run_m) return fail(GIBBS_ERR_ARG, "the last run had motif_amount = %d", b->run_m);
+    gibbs_handle *h = b->h;
+    int32_t rc = set_device(h);
+    if (rc) return rc;
+    CUDA_TRY(cudaMemcpyAsync(positions_out, b->win_sites.p, (size_t)b->n_seqs * m * sizeof(int32_t), cudaMemcpyDeviceToHost, h->stream));
+    CUDA_TRY(cudaStreamSynchronize(h->stream));
     return GIBBS_OK;
 }
 

@@ -461,324 +461,7 @@ __global__ void __launch_bounds__(32 * T, (T == 1 ? 8 : T == 4 ? GIBBS_MOTIF_T4_
     double *cand_l = m.cand_l + ((size_t)blockIdx.x * T + warp) * m.bg.wstride;
     int32_t *cand_w = m.cand_w + ((size_t)blockIdx.x * T + warp) * m.bg.wstride;
     double *gbuf = m.data_bg ? m.gbuf + ((size_t)blockIdx.x * T + warp) * m.bg.wstride : nullptr;
-    const uint64_t chain_uid = (uint64_t)a.chain_id_base + (uint64_t)chain;
-    const double raw_gate = exp2(a.cutoff) * (1.0 - 0x1p-30);
-
-    RowRing<R> ring;
-    ring.init(S, a.s, 0, tid);
-    if (tid < 16) S.lut[tid] = hist_lut_entry(tid);
-    team_sync<T>();
-    if (warp == 0) ring.fill_span(0u, 0, R, lane);
-
-    unsigned long long st_updates = 0, st_windows = 0, st_slow = 0, st_spec = 0; // st_slow: updates that scored every window in float64
-    int st_sweeps = 0, capped = 0;
-    uint32_t vbase = 0;
-
-    if (m.init_done && !a.from_list) { // the random starts ran in their own kernel (gibbs_api.cu, launch_random_starts): the state is
-        // SiteSampler.getPWMOfRandomStarts[WithBPV] |> createMotifIndex prob [position] (fs:876-877, fs:993-994)
-        for (int n = tid; n < N; n += THREADS) pw[n] = log2_ref(__ldcg(hv + n));
-        team_sync<T>();
-    }
-    int phase = MPH_STOCH;
-    while (phase < MPH_DONE && !((a.phase_mask >> (phase == MPH_STOCH ? 4 : 5)) & 1)) ++phase;
-    int sweeps_in_phase = 0;
-    bool resumed = false, paused = false;
-    if (a.from_list) {
-        const int r = a.resume[chain]; // phase | capped so far << 7 | sweeps in phase << 8
-        phase = r & 127;
-        capped = (r >> 7) & 1;
-        sweeps_in_phase = r >> 8;
-        resumed = true;
-    }
-    while (phase != MPH_DONE) {
-        if (phase == MPH_STOCH || sweeps_in_phase == 0 || resumed) {
-            resumed = false;
-            site_counts<KP, T>(a.s, sites, -1, k, SHIFT_NONE, S.total, S.lut, S.fix, tid);
-            if (m.data_bg) {
-                if (tid < 4) bsum[tid] = 0;
-                team_sync<T>();
-                int part[4] = {0, 0, 0, 0};
-                for (int i = tid; i < N; i += THREADS)
-                    if (__ldcg(sites + i) >= 0) {
-#pragma unroll
-                        for (int b = 0; b < 4; ++b) part[b] += __ldg(m.basecnt + i * 4 + b);
-                    }
-#pragma unroll
-                for (int b = 0; b < 4; ++b) {
-                    const int s = __reduce_add_sync(FULL, part[b]);
-                    if (lane == 0 && s != 0) atomicAdd(&bsum[b], s);
-                }
-                team_sync<T>();
-            }
-        } else {
-            team_sync<T>(); // the previous sweep's last round wrote sites / pw after its only barrier
-        }
-        bool changed = false;
-        int n0 = 0;
-        // greedy: speculation width adapts as in chain_kernel. The first GIBBS_MOTIF_NARROW_SWEEPS greedy sweeps move a site in
-        // most updates: their rounds start at width 1 and narrow after a discard. Later sweeps never narrow: they discard
-        // little, and a round that stays wide costs the other restarts of the SM less than it gains.
-        const int min_w = (phase == MPH_GREEDY && sweeps_in_phase < GIBBS_MOTIF_NARROW_SWEEPS) ? 1 : T;
-        int width = (phase == MPH_GREEDY) ? min_w : T;
-        unsigned round = 0;
-        while (n0 < N) {
-            const int n = n0 + warp;
-            const bool active = n < N && warp < width;
-            int flag = 0, site_n = -1, new_site = -1, W = 0;
-            double new_pw = 0.0;
-            bool has_own = false;
-            uint64_t own = 0, neu = 0;
-            int cn[4] = {0, 0, 0, 0};
-            int masked_n = -1;
-            uint64_t own_mk = 0;
-            if (active) {
-                const uint32_t *row = ring.wait(vbase + (uint32_t)n);
-                W = __ldg(a.s.len + n) - k + 1;
-                {
-                    site_n = __ldcg(sites + n);
-                    const double pw_n = __ldcg(pw + n);
-                    has_own = site_n >= 0;
-                    own = has_own ? kmer_shared<KP>(row, site_n) : 0;
-                    if (MASKED && __ldg(a.s.rowflag + n) != 0) {
-                        masked_n = n;
-                        if (has_own) own_mk = mask_kmer(a.s.mask, a.s.row_words, n, site_n, k);
-                    }
-                    const double *g_n = m.bg.g + (size_t)n * m.bg.wstride;
-                    double gsum_n = 0.0, gmax_n = 0.0;
-                    if (!m.data_bg) {
-                        if (MASKED && own_mk != 0) build_tables_masked<KP>(WT, S.total, own, k, a.wtab, lane, own_mk);
-                        else build_tables<KP>(WT, S.total, has_own, own, k, a.wtab, lane);
-                        gsum_n = __ldg(m.bg.gsum + n);
-                        gmax_n = __ldg(m.bg.gmax + n);
-                    } else {
-                        // background of this held-out sequence (fs:896-905): the OTHER sequences that have a site, outside
-                        // those sites (fused over the alphabet), plus every base of the held-out sequence
-                        for (int e = lane; e < 4 * k; e += 32) {
-                            int c = S.total[e];
-                            if (has_own && (int)((own >> (2 * (e >> 2))) & 3u) == (e & 3) && !(MASKED && ((own_mk >> (2 * (e >> 2))) & 1u))) c -= 1;
-                            WT.lgcol[e] = c;
-                        }
-                        __syncwarp();
-                        int F[4], fs = 0;
-#pragma unroll
-                        for (int b = 0; b < 4; ++b) {
-                            int s = 0;
-                            for (int j = lane; j < k; j += 32) s += WT.lgcol[j * 4 + b];
-                            cn[b] = __ldg(m.basecnt + n * 4 + b);
-                            F[b] = bsum[b] - (has_own ? cn[b] : 0) - __reduce_add_sync(FULL, s) + cn[b];
-                            fs += F[b];
-                        }
-                        if (MASKED && masked_n >= 0) fs += __ldg(a.maskcnt + n); // its own symbols outside the alphabet (fs:953, fs:117)
-                        const double den = __dadd_rn((double)fs, m.alpha_pc);
-                        double q[4];
-#pragma unroll
-                        for (int b = 0; b < 4; ++b) q[b] = __ddiv_rn(__dadd_rn((double)F[b], m.pc), den); // fs:119
-                        for (int e = lane; e < 8 * KP; e += 32) { // PWM = PPM / pcv (fs:286); dummy column of an odd k = 1.0
-                            const int b = e & 3;
-                            const double qb = b == 0 ? q[0] : b == 1 ? q[1] : b == 2 ? q[2] : q[3];
-                            WT.wcol[e] = (e >> 2) < k ? __ddiv_rn(__ldg(m.pvals + WT.lgcol[e]), qb) : 1.0;
-                        }
-                        // background-only probability of every window (fs:776), first maximum, and their sum in list order:
-                        // the same left-to-right product as a window score, over a table whose every column is q
-                        // (kept in the pair-table space, which is rebuilt after this loop when the greedy ranking pass runs)
-                        double *qtab = reinterpret_cast<double *>(WT.ptab);
-                        for (int e = lane; e < 8 * KP; e += 32) {
-                            const int b = e & 3;
-                            qtab[e] = (e >> 2) < k ? (b == 0 ? q[0] : b == 1 ? q[1] : b == 2 ? q[2] : q[3]) : 1.0;
-                        }
-                        __syncwarp();
-                        const uint8_t *seq_n = nullptr;
-                        if (MASKED && masked_n >= 0) { // symbol counts of the held-out sequence (candidate scratch is free here)
-                            seq_n = m.ascii + __ldg(m.off + n);
-                            for (int e = lane; e < 64; e += 32) cand_w[e] = 0;
-                            __syncwarp();
-                            for (int i = lane; i < W + k - 1; i += 32) atomicAdd(&cand_w[seq_n[i] - 42], 1);
-                            __syncwarp();
-                        }
-                        double bestg = 0.0;
-                        for (int w0 = 0; w0 < W; w0 += 32) {
-                            const int w = w0 + lane;
-                            if (w < W) {
-                                double v = exact_window<KP>(row, w, k, qtab);
-                                if (MASKED && masked_n >= 0 && mask_kmer(a.s.mask, a.s.row_words, n, w, k) != 0)
-                                    v = masked_background_window(seq_n, w, k, q, cand_w);
-                                gbuf[w] = v;
-                                bestg = fmax(bestg, v);
-                            }
-                        }
-                        __syncwarp();
-                        {
-                            const uint32_t hi = (uint32_t)__double2hiint(bestg), mh = __reduce_max_sync(FULL, hi);
-                            const uint32_t lo = (hi == mh) ? (uint32_t)__double2loint(bestg) : 0u, ml = __reduce_max_sync(FULL, lo);
-                            gmax_n = __hiloint2double((int)mh, (int)ml);
-                        }
-                        if (phase == MPH_STOCH) { // List.sum visits the background entries first, in window order (fs:748)
-                            for (int w0 = 0; w0 < W; w0 += 32) {
-                                const double v = (w0 + lane < W) ? gbuf[w0 + lane] : 0.0;
-                                const int lim = min(32, W - w0);
-                                for (int j = 0; j < lim; ++j) gsum_n = __dadd_rn(gsum_n, __shfl_sync(FULL, v, j));
-                            }
-                        }
-                        g_n = gbuf;
-                    }
-                    double best_l;
-                    int best_w;
-                    int n_cand = -1;
-                    bool slow = false;
-                    if (phase == MPH_GREEDY && m.greedy_fast_ok && !(MASKED && masked_n >= 0)) { // only the best candidate matters: rank, re-score, compare
-                        if (m.data_bg) fixed_point_tables<KP>(WT, lane);
-                        double pbest;
-                        if (pick_unique_argmax<KP>(WT, row, W, k, lane, pbest, best_w)) {
-                            best_l = log2_ref(pbest);
-                            n_cand = best_l > a.cutoff ? 1 : 0; // fs:735
-                        }
-                    }
-                    int gated = -1;
-                    if (n_cand < 0) {
-                        gated = motif_gate<KP, MASKED>(WT, row, W, k, raw_gate, cand_l, cand_w, lane, &a.s, masked_n);
-                        if (phase != MPH_STOCH || !m.roulette_scan_ok) {
-                            n_cand = motif_logs(a.cutoff, cand_l, cand_w, gated, lane, best_l, best_w);
-                            gated = -1;
-                        }
-                        slow = true;
-                    }
-                    bool take;
-                    if (phase == MPH_STOCH) { // fs:828-853: one uniform per n, every n reads the input state
-                        const uint64_t d = (uint64_t)N * (uint64_t)(N - 1) + (uint64_t)n;
-                        double u;
-                        if (a.rng_mode == 0) {
-                            const uint64_t blk = d >> 2;
-                            const uint4 r = philox4x32_10(
-                                make_uint4((uint32_t)blk, (uint32_t)(blk >> 32), (uint32_t)chain_uid, (uint32_t)(chain_uid >> 32)),
-                                make_uint2((uint32_t)a.seed, (uint32_t)(a.seed >> 32)));
-                            const uint32_t word = (d & 3) == 0 ? r.x : (d & 3) == 1 ? r.y : (d & 3) == 2 ? r.z : r.w;
-                            u = (double)word * (1.0 / 4294967296.0);
-                        } else {
-                            u = ((int64_t)d < a.uniforms_per_chain) ? __ldg(a.uniforms + (size_t)chain * a.uniforms_per_chain + d) : 0.0;
-                        }
-                        bool ok = gated >= 0 && motif_stoch_fast(gsum_n, a.cutoff, cand_l, cand_w, gated, u, lane, new_pw, new_site);
-                        if (!ok) {
-                            if (gated >= 0) n_cand = motif_logs(a.cutoff, cand_l, cand_w, gated, lane, best_l, best_w);
-                            ok = motif_roulette(g_n, gsum_n, W, cand_l, cand_w, n_cand, u, lane, new_pw, new_site,
-                                                m.roulette_scan_ok != 0);
-                        }
-                        if (!ok) {
-                            if (lane == 0) atomicExch(m.error, 1);
-                            new_pw = pw_n;
-                            new_site = site_n;
-                        }
-                        take = true;
-                    } else { // fs:788-822: first maximum by PWMS over background entries ++ candidates
-                        if (n_cand > 0 && best_l > gmax_n) {
-                            new_pw = best_l;
-                            new_site = best_w;
-                        } else {
-                            new_pw = gmax_n;
-                            new_site = -1;
-                        }
-                        take = new_pw > pw_n; // fs:816
-                    }
-                    const bool moved = take && phase == MPH_GREEDY && new_site != site_n;
-                    if (moved && new_site >= 0) neu = kmer_shared<KP>(row, new_site); // rows are not read after the sync
-                    flag = (take ? 1 : 0) | (moved ? 2 : 0) | (slow ? 4 : 0);
-                }
-            }
-            int32_t *flags = S.flags + (round & 1) * T; // double-buffered: one team sync per round suffices
-            ++round;
-            if (lane == 0) flags[warp] = flag;
-            team_sync<T>();
-            // greedy only: warps after the first mover of the round saw stale counts
-            const unsigned movers = __ballot_sync(FULL, lane < T && (flags[lane < T ? lane : 0] & 2) != 0);
-            const int first_mover = movers ? __ffs(movers) - 1 : T; // (only greedy updates set the mover bit)
-            const int last_commit = min(first_mover, width - 1);
-            changed |= movers != 0;
-            if (active) {
-                if (warp <= last_commit) {
-                    st_updates += 1;
-                    st_windows += (unsigned long long)W;
-                    st_slow += (flag & 4) ? 1 : 0;
-                    if ((flag & 1) && lane == 0) {
-                        sites[n] = new_site;
-                        pw[n] = new_pw;
-                    }
-                } else {
-                    st_spec += 1;
-                }
-            }
-            const int committed = min(last_commit + 1, N - n0);
-            if (warp == 0) ring.fill_span(vbase + (uint32_t)(n0 + R), n0 + R, committed, lane); // their rows are free
-            n0 += committed;
-            if (phase == MPH_GREEDY) {
-                if (first_mover < T) { // in-place sweep: later n see the new state (fs:795 reads acc): -old k-mer, +new k-mer
-                    if (warp == first_mover) {
-                        uint64_t neu_mk = 0;
-                        if (MASKED && masked_n >= 0 && new_site >= 0) neu_mk = mask_kmer(a.s.mask, a.s.row_words, n, new_site, k);
-                        if (lane < k) { // (bases outside A,C,G,T were never counted)
-                            if (has_own && !(MASKED && ((own_mk >> (2 * lane)) & 1u))) S.total[lane * 4 + (int)((own >> (2 * lane)) & 3u)] -= 1;
-                            if (new_site >= 0 && !(MASKED && ((neu_mk >> (2 * lane)) & 1u))) S.total[lane * 4 + (int)((neu >> (2 * lane)) & 3u)] += 1;
-                        }
-                        if (m.data_bg && has_own != (new_site >= 0) && lane < 4) { // the sequence gained or lost its site
-                            const int d = lane == 0 ? cn[0] : lane == 1 ? cn[1] : lane == 2 ? cn[2] : cn[3];
-                            bsum[lane] += new_site >= 0 ? d : -d;
-                        }
-                    }
-                    team_sync<T>(); // counts updated before the next round builds its tables
-                    width = max(min_w, width >> 1);
-                } else {
-                    width = min(T, width * 2);
-                }
-            }
-        }
-        vbase += (uint32_t)N;
-        st_sweeps += 1;
-        bool next = true;
-        if (phase == MPH_GREEDY) {
-            ++sweeps_in_phase;
-            next = !changed; // Positions(acc) = Positions(bestMotif), fs:791
-            if (!next && sweeps_in_phase >= a.max_sweeps) {
-                next = true;
-                capped = 1;
-            }
-        }
-        if (next) {
-            sweeps_in_phase = 0;
-            ++phase;
-            while (phase < MPH_DONE && !((a.phase_mask >> (phase == MPH_STOCH ? 4 : 5)) & 1)) ++phase;
-        }
-        // sweep boundary: when few restarts are still running, hand this one over to the wide-team launch
-        if (phase != MPH_DONE && a.pause_below > 0) {
-            if (tid == 0) S.flags[2 * T] = (*(volatile int32_t *)a.active <= a.pause_below && st_sweeps >= a.pause_min_sweeps) ? 1 : 0;
-            team_sync<T>();
-            if (S.flags[2 * T]) {
-                paused = true;
-                break;
-            }
-        }
-    }
-    if (tid == 0) // the ring always has R rows in flight: let them land before the CTA exits
-        for (int i = 0; i < R; ++i) ring.wait(vbase + (uint32_t)i);
-    team_sync<T>();
-    if (!paused)
-        for (int n = tid; n < N; n += THREADS) hv[n] = __ldcg(pw + n);
-    if (lane == 0) {
-        atomicAdd(a.stats + ST_SITE_UPDATES, st_updates);
-        atomicAdd(a.stats + ST_EXACT_RESCANS, st_slow);
-        atomicAdd(a.stats + ST_WINDOW_SCORES, st_windows);
-        atomicAdd(a.stats + ST_SPECULATED, st_spec);
-    }
-    if (tid == 0) {
-        atomicAdd(a.stats + ST_SWEEPS, (unsigned long long)st_sweeps);
-        if (!paused) atomicAdd(a.stats + ST_CAPPED, (unsigned long long)capped); // (a restart counts once, where it ends)
-        if (paused) {
-            a.resume[chain] = phase | (capped << 7) | (sweeps_in_phase << 8);
-            a.pending_out[atomicAdd(a.pending_out_n, 1)] = chain;
-        } else {
-            double sum = 0.0;
-            for (int n = 0; n < N; ++n) sum = __dadd_rn(sum, __ldcg(pw + n));
-            a.sums[chain] = sum;
-            if (a.active) atomicSub(a.active, 1);
-        }
-    }
+#include "gibbs_motif_body.inc"
 }
 
 // primitive: candidate list + one roulette pick for a given state (gibbs_pick_roulette)

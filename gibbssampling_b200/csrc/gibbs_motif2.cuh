@@ -131,276 +131,7 @@ static __global__ void __launch_bounds__(32) motif2_kernel(const Motif2Args q) {
     int32_t *cand_w = m.cand_w + (size_t)chain * m.bg.wstride;
     double *gbuf = m.data_bg ? m.gbuf + (size_t)chain * m.bg.wstride : nullptr;
     double *sc = q.sc + (size_t)chain * m.bg.wstride;
-    int bsum[4] = {0, 0, 0, 0}; // data background: sum over sequences of (sites of the sequence) x (its base counts)
-    const uint64_t chain_uid = (uint64_t)a.chain_id_base + (uint64_t)chain;
-    const double raw_gate = exp2(a.cutoff) * (1.0 - 0x1p-30);
-
-    RowRing<4> ring;
-    ring.init(S, a.s, 0, lane);
-    if (lane < 16) S.lut[lane] = hist_lut_entry(lane);
-    __syncwarp();
-    if (lane == 0) ring.fill(4);
-
-    if (m.init_done) { // SiteSampler.getPWMOfRandomStarts[WithBPV] |> createMotifIndex prob [position] (fs:876-877, fs:993-994)
-        for (int n = lane; n < N; n += 32) {
-            pos2[2 * n] = __ldcg(sites + n);
-            pos2[2 * n + 1] = -1;
-            pw[n] = log2_ref(__ldcg(hv + n));
-        }
-        __syncwarp();
-    }
-    unsigned long long st_updates = 0, st_windows = 0;
-    int st_sweeps = 0, capped = 0;
-    uint32_t v = 0;
-    int phase = MPH_STOCH;
-    while (phase < MPH_DONE && !((a.phase_mask >> (phase == MPH_STOCH ? 4 : 5)) & 1)) ++phase;
-    int sweeps_in_phase = 0;
-    while (phase != MPH_DONE) {
-        if (phase == MPH_STOCH || sweeps_in_phase == 0) { // counts over every site of every sequence
-            for (int e = lane; e < MAX_COLS * 4; e += 32) S.total[e] = 0;
-            __syncwarp();
-            for (int i = 0; i < N; ++i) {
-                const uint32_t *rowi = a.s.packed + (size_t)i * a.s.row_words;
-#pragma unroll
-                for (int s = 0; s < 2; ++s) {
-                    const int p = __ldcg(pos2 + 2 * i + s);
-                    if (p >= 0 && lane < k) S.total[lane * 4 + (int)((kmer_global<KP>(rowi, p) >> (2 * lane)) & 3u)] += 1;
-                }
-            }
-            __syncwarp();
-            if (m.data_bg) {
-#pragma unroll
-                for (int b = 0; b < 4; ++b) {
-                    int s = 0;
-                    for (int i = lane; i < N; i += 32) {
-                        const int np = (__ldcg(pos2 + 2 * i) >= 0) + (__ldcg(pos2 + 2 * i + 1) >= 0);
-                        s += np * __ldg(m.basecnt + i * 4 + b);
-                    }
-                    bsum[b] = __reduce_add_sync(FULL, s);
-                }
-            }
-        }
-        bool changed = false;
-        for (int n = 0; n < N; ++n, ++v) {
-            const uint32_t *row = ring.wait(v);
-            const int W = __ldg(a.s.len + n) - k + 1;
-            const int o0 = __ldcg(pos2 + 2 * n), o1 = __ldcg(pos2 + 2 * n + 1);
-            const double pw_n = __ldcg(pw + n);
-            const int onp = (o0 >= 0) + (o1 >= 0);
-            const uint64_t own0 = o0 >= 0 ? kmer_shared<KP>(row, o0) : 0, own1 = o1 >= 0 ? kmer_shared<KP>(row, o1) : 0;
-            // leave-one-out counts: every site of every OTHER sequence (fs:794-806 / fs:891-913)
-            for (int e = lane; e < 8 * KP; e += 32) {
-                const int j = e >> 2, b = e & 3;
-                int c = 0;
-                if (j < k) {
-                    c = S.total[e];
-                    if (o0 >= 0 && (int)((own0 >> (2 * j)) & 3u) == b) c -= 1;
-                    if (o1 >= 0 && (int)((own1 >> (2 * j)) & 3u) == b) c -= 1;
-                }
-                WT.counts[e] = c;
-            }
-            __syncwarp();
-            const double *g_n = m.bg.g + (size_t)n * m.bg.wstride;
-            double gsum_n = 0.0, gmax_n = 0.0;
-            int gmax_i = 0;
-            int cn[4] = {0, 0, 0, 0};
-            if (!m.data_bg) {
-                build_tables<KP>(WT, WT.counts, false, 0, k, a.wtab, lane);
-                gsum_n = __ldg(m.bg.gsum + n);
-                gmax_n = __ldg(m.bg.gmax + n);
-                gmax_i = __ldg(m.bg.gmax_i + n);
-            } else {
-                // background of this held-out sequence (fs:896-905): for every site of every other sequence that
-                // sequence's bases outside the site (fused over the alphabet), plus every base of the held-out sequence
-                int F[4], fs = 0;
-#pragma unroll
-                for (int b = 0; b < 4; ++b) {
-                    int s = 0;
-                    for (int j = lane; j < k; j += 32) s += WT.counts[j * 4 + b];
-                    cn[b] = __ldg(m.basecnt + n * 4 + b);
-                    F[b] = bsum[b] - onp * cn[b] - __reduce_add_sync(FULL, s) + cn[b];
-                    fs += F[b];
-                }
-                const double den = __dadd_rn((double)fs, m.alpha_pc);
-                double qb[4];
-#pragma unroll
-                for (int b = 0; b < 4; ++b) qb[b] = __ddiv_rn(__dadd_rn((double)F[b], m.pc), den); // fs:119
-                for (int e = lane; e < 8 * KP; e += 32) { // PWM = PPM / pcv (fs:286); dummy column of an odd k = 1.0
-                    const int b = e & 3;
-                    const double qq = b == 0 ? qb[0] : b == 1 ? qb[1] : b == 2 ? qb[2] : qb[3];
-                    WT.wcol[e] = (e >> 2) < k ? __ddiv_rn(__ldg(m.pvals + WT.counts[e]), qq) : 1.0;
-                }
-                double *qtab = reinterpret_cast<double *>(WT.ptab);
-                for (int e = lane; e < 8 * KP; e += 32) {
-                    const int b = e & 3;
-                    qtab[e] = (e >> 2) < k ? (b == 0 ? qb[0] : b == 1 ? qb[1] : b == 2 ? qb[2] : qb[3]) : 1.0;
-                }
-                __syncwarp();
-                double bestg = -1.0;
-                int besti = INT32_MAX;
-                for (int w0 = 0; w0 < W; w0 += 32) {
-                    const int w = w0 + lane;
-                    if (w < W) {
-                        const double gv = exact_window<KP>(row, w, k, qtab);
-                        gbuf[w] = gv;
-                        if (gv > bestg) { // ascending windows per lane: strict > keeps the first maximum
-                            bestg = gv;
-                            besti = w;
-                        }
-                    }
-                }
-                __syncwarp();
-                warp_argmax(bestg, besti);
-                gmax_n = bestg;
-                gmax_i = besti;
-                for (int w0 = 0; w0 < W; w0 += 32) { // List.sum visits the background entries first, in window order (fs:748)
-                    const double gv = (w0 + lane < W) ? gbuf[w0 + lane] : 0.0;
-                    const int lim = min(32, W - w0);
-                    for (int j = 0; j < lim; ++j) gsum_n = __dadd_rn(gsum_n, __shfl_sync(FULL, gv, j));
-                }
-                g_n = gbuf;
-            }
-            // every window's product (fs:773), then the single candidates (ascending position, log2 > cutOff, fs:735)
-            for (int w0 = 0; w0 < W; w0 += 32)
-                if (w0 + lane < W) sc[w0 + lane] = exact_window<KP>(row, w0 + lane, k, WT.wcol);
-            __syncwarp();
-            double best_l;
-            int best_w;
-            const int n_single = motif_candidates<KP>(WT, row, W, k, a.cutoff, raw_gate, cand_l, cand_w, lane, best_l, best_w);
-            double new_pw;
-            int na, nb; // new Positions [na; nb] (newest first), -1 = absent
-            bool take;
-            if (phase == MPH_STOCH) { // fs:935-970 / fs:828-853: one uniform per n, every n reads the input state
-                const uint64_t d = (uint64_t)N * (uint64_t)(N - 1) + (uint64_t)n;
-                double u;
-                if (a.rng_mode == 0) {
-                    const uint64_t blk = d >> 2;
-                    const uint4 r = philox4x32_10(make_uint4((uint32_t)blk, (uint32_t)(blk >> 32), (uint32_t)chain_uid, (uint32_t)(chain_uid >> 32)),
-                                                  make_uint2((uint32_t)a.seed, (uint32_t)(a.seed >> 32)));
-                    const uint32_t word = (d & 3) == 0 ? r.x : (d & 3) == 1 ? r.y : (d & 3) == 2 ? r.z : r.w;
-                    u = (double)word * (1.0 / 4294967296.0);
-                } else {
-                    u = ((int64_t)d < a.uniforms_per_chain) ? __ldg(a.uniforms + (size_t)chain * a.uniforms_per_chain + d) : 0.0;
-                }
-                ListWalk L;
-                L.sum = gsum_n; // the background entries come first; gsum was accumulated in that order
-                L.acc = 0.0;
-                L.pick = u;
-                L.found = 0;
-                L.sel_v = 0.0;
-                L.sel_a = L.sel_b = -1;
-                for (int i0 = 0; i0 < n_single; i0 += 32)
-                    list_sum_block(L, (i0 + lane < n_single) ? cand_l[i0 + lane] : 0.0, i0 + lane < n_single);
-                for_each_pair_block(sc, cand_w, n_single, W, k, a.cutoff, lane,
-                                    [&](double l, bool valid, int, int, long long) { list_sum_block(L, l, valid); });
-                for (int w0 = 0; w0 < W && !L.found; w0 += 32)
-                    list_walk_block(L, (w0 + lane < W) ? g_n[w0 + lane] : 0.0, w0 + lane < W, -1, -1);
-                for (int i0 = 0; i0 < n_single && !L.found; i0 += 32)
-                    list_walk_block(L, (i0 + lane < n_single) ? cand_l[i0 + lane] : 0.0, i0 + lane < n_single,
-                                    (i0 + lane < n_single) ? cand_w[i0 + lane] : -1, -1);
-                if (!L.found)
-                    for_each_pair_block(sc, cand_w, n_single, W, k, a.cutoff, lane,
-                                        [&](double l, bool valid, int j, int i, long long) { list_walk_block(L, l, valid, j, i); });
-                if (!L.found) { // the pick ran past the list: the reference throws (fs:753)
-                    if (lane == 0) atomicExch(m.error, 1);
-                    new_pw = pw_n;
-                    na = o0;
-                    nb = o1;
-                } else {
-                    new_pw = L.sel_v;
-                    na = L.sel_a;
-                    nb = L.sel_b;
-                }
-                take = true;
-            } else { // fs:885-929 / fs:788-822: head of the list sorted by PWMS (stable)
-                ListHead H;
-                H.v = gmax_n;               // category order: background, singles, pairs; a later one needs a larger PWMS
-                H.key = -2;
-                H.a = H.b = -1;
-                if (n_single > 0 && best_l > H.v) {
-                    H.v = best_l;
-                    H.a = best_w;
-                }
-                ListHead P;
-                P.v = -INFINITY;
-                P.key = INT64_MAX;
-                P.a = P.b = -1;
-                for_each_pair_block(sc, cand_w, n_single, W, k, a.cutoff, lane, [&](double l, bool valid, int j, int i, long long key) {
-                    if (valid) head_offer(P, l, key, j, i);
-                });
-                head_reduce(P);
-                if (P.a >= 0 && P.v > H.v) {
-                    H.v = P.v;
-                    H.a = P.a;
-                    H.b = P.b;
-                }
-                new_pw = H.v;
-                na = H.a;
-                nb = H.b;
-                take = new_pw > pw_n; // fs:816 / fs:923
-                (void)gmax_i;
-            }
-            if (take) {
-                if (phase == MPH_GREEDY && (na != o0 || nb != o1)) {
-                    changed = true;
-                    const uint64_t n0k = na >= 0 ? kmer_shared<KP>(row, na) : 0, n1k = nb >= 0 ? kmer_shared<KP>(row, nb) : 0;
-                    if (lane < k) { // in-place sweep: later n see the new state
-                        if (o0 >= 0) S.total[lane * 4 + (int)((own0 >> (2 * lane)) & 3u)] -= 1;
-                        if (o1 >= 0) S.total[lane * 4 + (int)((own1 >> (2 * lane)) & 3u)] -= 1;
-                        if (na >= 0) S.total[lane * 4 + (int)((n0k >> (2 * lane)) & 3u)] += 1;
-                        if (nb >= 0) S.total[lane * 4 + (int)((n1k >> (2 * lane)) & 3u)] += 1;
-                    }
-                    if (m.data_bg) {
-                        const int dn = (na >= 0) + (nb >= 0) - onp;
-#pragma unroll
-                        for (int b = 0; b < 4; ++b) bsum[b] += dn * cn[b];
-                    }
-                }
-                if (lane == 0) {
-                    pos2[2 * n] = na;
-                    pos2[2 * n + 1] = nb;
-                    sites[n] = na;
-                    pw[n] = new_pw;
-                }
-            }
-            st_updates += 1;
-            st_windows += (unsigned long long)W;
-            __syncwarp();
-            if (lane == 0) ring.fill(v + 1 + 4);
-        }
-        st_sweeps += 1;
-        bool next = true;
-        if (phase == MPH_GREEDY) {
-            ++sweeps_in_phase;
-            next = !changed; // Positions(acc) = Positions(bestMotif)
-            if (!next && sweeps_in_phase >= a.max_sweeps) {
-                next = true;
-                capped = 1;
-            }
-        }
-        if (next) {
-            sweeps_in_phase = 0;
-            ++phase;
-            while (phase < MPH_DONE && !((a.phase_mask >> (phase == MPH_STOCH ? 4 : 5)) & 1)) ++phase;
-        }
-    }
-    if (lane == 0)
-        for (int i = 0; i < 4; ++i) ring.wait(v + (uint32_t)i);
-    __syncwarp();
-    for (int n = lane; n < N; n += 32) {
-        hv[n] = __ldcg(pw + n);
-        sites[n] = __ldcg(pos2 + 2 * n);
-    }
-    if (lane == 0) {
-        double sum = 0.0;
-        for (int n = 0; n < N; ++n) sum = __dadd_rn(sum, __ldcg(pw + n));
-        a.sums[chain] = sum;
-        atomicAdd(a.stats + ST_SITE_UPDATES, st_updates);
-        atomicAdd(a.stats + ST_EXACT_RESCANS, st_updates);
-        atomicAdd(a.stats + ST_WINDOW_SCORES, st_windows);
-        atomicAdd(a.stats + ST_SWEEPS, (unsigned long long)st_sweeps);
-        atomicAdd(a.stats + ST_CAPPED, (unsigned long long)capped);
-    }
+#include "gibbs_motif2_body.inc"
 }
 
 // start state of a run without the random starts: Positions lists from the one-site state of gibbs_set_start_state

@@ -445,7 +445,8 @@ class BatchRunResult:
 
 class BatchEngine:
     """Many independent sets of sequences (gibbs_batch_*): their restarts run together in a few launches; set s gives
-    exactly what a GibbsEngine over sets[s] alone gives for the same parameters, seed and chain_id_base."""
+    exactly what a GibbsEngine over sets[s] alone gives for the same parameters, seed and chain_id_base. run_device runs
+    the SiteSampler, run_motif_device the MotifSampler; fetch / fetch_best serve the last run of either."""
 
     def __init__(self, sets: Sequence[Sequence], device: int = 0):
         self._lib = _abi.load()
@@ -476,25 +477,39 @@ class BatchEngine:
     def __exit__(self, *exc):
         self.close()
 
+    def _bg_per_set(self, bg_per_set):
+        if bg_per_set is None:
+            return None
+        bg = np.ascontiguousarray(bg_per_set, dtype=np.float64)
+        if bg.shape != (self.n_sets, 4):
+            raise _abi.GibbsArgumentError(_abi.GIBBS_ERR_ARG, f"bg_per_set must be [{self.n_sets}][4]")
+        return bg
+
     def run_device(self, params: Params, restarts_per_set: int, *, bg_per_set=None, chain_id_base: int = 0, seed: int = 0) -> None:
         """restarts_per_set restarts of every set; bg_per_set = [n_sets][4] backgrounds of the fixed-background family
         (None = params.bg for every set). Results stay in HBM until fetch() / fetch_best()."""
-        bg = None
-        if bg_per_set is not None:
-            bg = np.ascontiguousarray(bg_per_set, dtype=np.float64)
-            if bg.shape != (self.n_sets, 4):
-                raise _abi.GibbsArgumentError(_abi.GIBBS_ERR_ARG, f"bg_per_set must be [{self.n_sets}][4]")
+        bg = self._bg_per_set(bg_per_set)
         _abi.check(self._lib.gibbs_batch_run_device(self._b, C.byref(params), _ptr(bg, C.c_double), C.c_int32(restarts_per_set),
                                                     C.c_int64(chain_id_base), C.c_uint64(seed)))
-        self._last = (int(restarts_per_set), int(params.k))
+        self._last = (int(restarts_per_set), int(params.k), 1)
 
-    def _need_run(self) -> tuple[int, int]:
+    def run_motif_device(self, params: Params, restarts_per_set: int, *, bg_per_set=None, chain_id_base: int = 0,
+                         seed: int = 0) -> None:
+        """The MotifSampler (params.sampler = GIBBS_MOTIF_SAMPLER, motif_amount 1 or 2) on every set, arguments as
+        run_device. fetch() then returns the newest position of every sequence (-1 = no site), fetch_positions(m) the
+        Positions lists."""
+        bg = self._bg_per_set(bg_per_set)
+        _abi.check(self._lib.gibbs_batch_run_motif_device(self._b, C.byref(params), _ptr(bg, C.c_double),
+                                                          C.c_int32(restarts_per_set), C.c_int64(chain_id_base), C.c_uint64(seed)))
+        self._last = (int(restarts_per_set), int(params.k), max(int(params.motif_amount), 1))
+
+    def _need_run(self) -> tuple[int, int, int]:
         if self._last is None:
             raise _abi.GibbsArgumentError(_abi.GIBBS_ERR_ARG, "no run_device on this batch yet")
         return self._last
 
     def fetch(self) -> BatchRunResult:
-        R, _ = self._need_run()
+        R, _, _ = self._need_run()
         total = int(self.set_offsets[-1])
         sites = np.zeros(R * total, dtype=np.int32)
         scores = np.zeros(R * total, dtype=np.float64)
@@ -511,8 +526,8 @@ class BatchEngine:
         return BatchRunResult(out_sites, out_scores, [sums[s] for s in range(self.n_sets)], stats)
 
     def fetch_best(self, repetitions: int, *, want_counts: bool = False) -> list[BestResult]:
-        """The promote-or-restart loop of fs:435-459 of every set, decided on the GPU: one BestResult per set."""
-        _, k = self._need_run()
+        """The promote-or-restart loop of fs:435-459 (fs:857-881) of every set, decided on the GPU: one BestResult per set."""
+        _, k, _ = self._need_run()
         total = int(self.set_offsets[-1])
         sites = np.zeros(total, dtype=np.int32)
         scores = np.zeros(total, dtype=np.float64)
@@ -531,6 +546,26 @@ class BatchEngine:
             out.append(BestResult(sites[a: a + n].copy(), scores[a: a + n].copy(), float(sums[s]), int(restart[s]),
                                   counts[s] if counts is not None else None, stats))
         return out
+
+    def fetch_positions(self, m: int) -> list:
+        """Positions lists of every restart of the last run (m = its motif_amount): entry s is int32 [R, N_s, m], newest
+        first, -1 = absent."""
+        R, _, _ = self._need_run()
+        total = int(self.set_offsets[-1])
+        pos = np.zeros(R * total * int(m), dtype=np.int32)
+        _abi.check(self._lib.gibbs_batch_fetch_positions(self._b, C.c_int32(m), _ptr(pos, C.c_int32)))
+        return [pos[R * int(m) * int(self.set_offsets[s]): R * int(m) * int(self.set_offsets[s + 1])].reshape(R, int(self.sizes[s]), int(m))
+                for s in range(self.n_sets)]
+
+    def fetch_best_positions(self, m: int) -> list:
+        """The winners' Positions lists of the last fetch_best: entry s is int32 [N_s, m] (all -1 where the loop's initial
+        value survived)."""
+        self._need_run()
+        total = int(self.set_offsets[-1])
+        pos = np.zeros(total * int(m), dtype=np.int32)
+        _abi.check(self._lib.gibbs_batch_fetch_best_positions(self._b, C.c_int32(m), _ptr(pos, C.c_int32)))
+        return [pos[int(m) * int(self.set_offsets[s]): int(m) * int(self.set_offsets[s + 1])].reshape(int(self.sizes[s]), int(m))
+                for s in range(self.n_sets)]
 
 
 def device_count() -> int:

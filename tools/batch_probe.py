@@ -6,7 +6,12 @@ and both compute the same per-set winners (checked before timing). Workloads:
   a  1024 sets of 20 x 100 bp, k = 8, R = 2, fixed background (the script's reps = 1 on C1-shaped sets)
   b  62 sets of 9-31 sequences of 45-1300 bp, k = 6, R = 2, data-derived background, alphabet size 5 without Gap
   c  64 sets of 100 x 500 bp, k = 12, R = 64, fixed background
-Usage: python tools/batch_probe.py [--reps 5] [--only a,b,c]   (needs a GPU; prints the device name and power limit)
+MotifSampler (run_motif_device; pc = 1e-4, cutOff = 1.0; motifAmount 2 also fetches the winners' Positions lists):
+  d  the sets of a, k = 8, R = 2, fixed background, motifAmount 1
+  e  the sets of b, k = 6, R = 2, data-derived background, alphabet size 5, motifAmount 2 (fsx:407 per gene group)
+  f  the same with motifAmount 1
+  g  the sets of c, k = 12, R = 64, fixed background, motifAmount 1
+Usage: python tools/batch_probe.py [--reps 5] [--only a,b,c,d,e,f,g]   (needs a GPU; prints the device name and power limit)
 """
 from __future__ import annotations
 
@@ -26,15 +31,16 @@ from gibbssampling_b200.synthetic import background_of, planted_motif_set  # noq
 
 
 def workload(name):
-    if name == "a":
+    """(sets, k, R, background, alphabet size, motifAmount: 0 = the SiteSampler)"""
+    if name in "ad":
         seqs = planted_motif_set(1024 * 20, 100, 8, seed=11).sequences()
-        return [seqs[20 * s: 20 * s + 20] for s in range(1024)], 8, 2, _abi.GIBBS_BG_FIXED, 4
-    if name == "b":
+        return [seqs[20 * s: 20 * s + 20] for s in range(1024)], 8, 2, _abi.GIBBS_BG_FIXED, 4, 1 if name == "d" else 0
+    if name in "bef":
         rng = np.random.default_rng(62)
         sets = [planted_motif_set(int(rng.integers(9, 32)), 1300, 6, seed=500 + s, min_length=45).sequences() for s in range(62)]
-        return sets, 6, 2, _abi.GIBBS_BG_DATA, 5
+        return sets, 6, 2, _abi.GIBBS_BG_DATA, 5, {"b": 0, "e": 2, "f": 1}[name]
     seqs = planted_motif_set(64 * 100, 500, 12, seed=13).sequences()
-    return [seqs[100 * s: 100 * s + 100] for s in range(64)], 12, 64, _abi.GIBBS_BG_FIXED, 4
+    return [seqs[100 * s: 100 * s + 100] for s in range(64)], 12, 64, _abi.GIBBS_BG_FIXED, 4, 1 if name == "g" else 0
 
 
 def device_info():
@@ -51,33 +57,37 @@ def device_info():
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--reps", type=int, default=5)
-    ap.add_argument("--only", default="a,b,c")
+    ap.add_argument("--only", default="a,b,c,d,e,f,g")
     args = ap.parse_args()
     import torch
     dev_name, power = device_info()
     for name in args.only.split(","):
-        sets, k, R, bgmode, alen = workload(name)
+        sets, k, R, bgmode, alen, m = workload(name)
         bgs = [background_of(np.frombuffer(b"".join(s), dtype=np.uint8), 1e-4, alen) for s in sets]
         fixed = bgmode == _abi.GIBBS_BG_FIXED
-        params = [make_params(k, 1e-4, alen, bgs[s], background=bgmode) for s in range(len(sets))]
+        motif = {"cutoff": 1.0, "sampler": _abi.GIBBS_MOTIF_SAMPLER, "motif_amount": m} if m else {}
+        params = [make_params(k, 1e-4, alen, bgs[s], background=bgmode, **motif) for s in range(len(sets))]
         batch = BatchEngine(sets)
         singles = [GibbsEngine(s) for s in sets]
         ev = [torch.cuda.Event(enable_timing=True) for _ in range(2)]
 
         def run_batch():
-            batch.run_device(params[0], R, bg_per_set=bgs if fixed else None, chain_id_base=0, seed=1)
-            return batch.fetch_best(R - 1)
+            (batch.run_motif_device if m else batch.run_device)(params[0], R, bg_per_set=bgs if fixed else None, chain_id_base=0, seed=1)
+            best = batch.fetch_best(R - 1)
+            return best, batch.fetch_best_positions(2) if m == 2 else [None] * len(sets)
 
         def run_loop():
-            out = []
+            best, pos = [], []
             for s, eng in enumerate(singles):
                 eng.run_device(params[s], R, chain_id_base=0, seed=1)
-                out.append(eng.fetch_best(R - 1))
+                best.append(eng.fetch_best(R - 1))
+                pos.append(eng.fetch_best_positions(2) if m == 2 else None)
             torch.cuda.synchronize()
-            return out
+            return best, pos
 
-        got, want = run_batch(), run_loop()   # warm-up of every shape, and the results must agree
+        (got, got_pos), (want, want_pos) = run_batch(), run_loop()   # warm-up of every shape, and the results must agree
         same = all(g.sites.tolist() == w.sites.tolist() and g.scores.tobytes() == w.scores.tobytes() for g, w in zip(got, want))
+        same = same and all(gp is None or np.array_equal(gp, wp) for gp, wp in zip(got_pos, want_pos))
         windows = sum(b.stats["window_scores"] for b in got[:1])   # (stats of a batch fetch are batch-wide)
 
         def timed(fn):
@@ -94,7 +104,8 @@ def main():
         tb, tl = timed(run_batch), timed(run_loop)
         print(json.dumps({
             "workload": name, "sets": len(sets), "seqs": int(sum(len(s) for s in sets)), "k": k, "restarts_per_set": R,
-            "background": "fixed" if fixed else "data", "identical_to_single_handles": bool(same),
+            "background": "fixed" if fixed else "data", "sampler": f"MotifSampler m={m}" if m else "SiteSampler",
+            "identical_to_single_handles": bool(same),
             "window_scores": int(windows),
             "batch_ms": round(tb[0], 3), "batch_ms_min_max": [round(tb[1], 3), round(tb[2], 3)],
             "loop_ms": round(tl[0], 3), "loop_ms_min_max": [round(tl[1], 3), round(tl[2], 3)],
