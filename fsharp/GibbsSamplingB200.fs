@@ -118,6 +118,31 @@ module Native =
     extern int gibbs_batch_fetch_positions(IntPtr batch, int m, int[] positionsOut)
     [<DllImport(Lib, CallingConvention = CallingConvention.Cdecl)>]
     extern int gibbs_batch_fetch_best_positions(IntPtr batch, int m, int[] positionsOut)
+    // the same batch with its sets split over every GPU of the box (gibbs_multi_batch_*): outputs in the caller's set order
+    [<DllImport(Lib, CallingConvention = CallingConvention.Cdecl)>]
+    extern int gibbs_multi_batch_create(byte[] seqs, int64[] offsets, int[] setOffsets, int nSets, int[] devicesOrNull, int nDevices,
+                                        IntPtr& multiBatch)
+    [<DllImport(Lib, CallingConvention = CallingConvention.Cdecl)>]
+    extern int gibbs_multi_batch_destroy(IntPtr multiBatch)
+    [<DllImport(Lib, CallingConvention = CallingConvention.Cdecl)>]
+    extern int gibbs_multi_batch_num_devices(IntPtr multiBatch)
+    [<DllImport(Lib, CallingConvention = CallingConvention.Cdecl)>]
+    extern int gibbs_multi_batch_slot_sets(IntPtr multiBatch, int slot, int& firstSet, int& nSets)
+    [<DllImport(Lib, CallingConvention = CallingConvention.Cdecl)>]
+    extern int gibbs_multi_batch_run_device(IntPtr multiBatch, GibbsParams& p, float[] bgPerSetOrNull, int restartsPerSet,
+                                            int64 chainIdBase, uint64 seed)
+    [<DllImport(Lib, CallingConvention = CallingConvention.Cdecl)>]
+    extern int gibbs_multi_batch_run_motif_device(IntPtr multiBatch, GibbsParams& p, float[] bgPerSetOrNull, int restartsPerSet,
+                                                  int64 chainIdBase, uint64 seed)
+    [<DllImport(Lib, CallingConvention = CallingConvention.Cdecl)>]
+    extern int gibbs_multi_batch_fetch(IntPtr multiBatch, int[] sitesOut, float[] scoresOut, float[] sumsOut, GibbsRunStats& stats)
+    [<DllImport(Lib, CallingConvention = CallingConvention.Cdecl)>]
+    extern int gibbs_multi_batch_fetch_best(IntPtr multiBatch, int repetitions, int[] sitesOut, float[] scoresOut, int[] nOut,
+                                            float[] sumOut, int[] restartOut, int[] countsOut, GibbsRunStats& stats)
+    [<DllImport(Lib, CallingConvention = CallingConvention.Cdecl)>]
+    extern int gibbs_multi_batch_fetch_positions(IntPtr multiBatch, int m, int[] positionsOut)
+    [<DllImport(Lib, CallingConvention = CallingConvention.Cdecl)>]
+    extern int gibbs_multi_batch_fetch_best_positions(IntPtr multiBatch, int m, int[] positionsOut)
 
     /// status code -> the exception the reference would have thrown (SURVEY.md section 8b)
     let check (rc:int) =
@@ -213,8 +238,9 @@ module Native =
         finally
             gibbs_multi_destroy m |> ignore
 
-    /// The restart loops of many sets in one batch on GPU 0: set s gets exactly what bestOfRestarts-style single-set calls
-    /// with the same seed give (restart r of every set draws from the stream (seed, r)); only the winners are copied back.
+    /// The restart loops of many sets in one batch over EVERY GPU of the box (contiguous blocks of sets, one per device): set s
+    /// gets exactly what bestOfRestarts-style single-set calls with the same seed give (restart r of every set draws from the
+    /// stream (seed, r)), whatever the number of devices; only the winners are copied back.
     let bestOfRestartsOfSets (numberOfRepetitions:int) (seed:uint64) k pc alphabet (sets:BioArray.BioArray<#IBioItem>[][])
                              (pcvs:CompositeVector.ProbabilityCompositeVector[] option) : (float*int)[][] =
         let all = Array.concat sets
@@ -222,21 +248,21 @@ module Native =
         let setOffsets = Array.zeroCreate<int> (sets.Length + 1)
         sets |> Array.iteri (fun s src -> setOffsets.[s + 1] <- setOffsets.[s] + src.Length)
         let mutable b = IntPtr.Zero
-        check (gibbs_batch_create(buf, offsets, setOffsets, sets.Length, 0, &b))
+        check (gibbs_multi_batch_create(buf, offsets, setOffsets, sets.Length, null, 0, &b))   // 0 = every visible device
         try
             let mutable p = makeParams k pc alphabet (pcvs |> Option.map (fun v -> v.[0])) 0
             let bg =
                 match pcvs with
                 | Some v -> v |> Array.collect (fun pcv -> [| for c in "ACGT" -> pcv.Array.[int c - 42] |])
                 | None -> null
-            check (gibbs_batch_run_device(b, &p, bg, numberOfRepetitions + 1, 0L, seed))
+            check (gibbs_multi_batch_run_device(b, &p, bg, numberOfRepetitions + 1, 0L, seed))
             let sites, scores = Array.zeroCreate all.Length, Array.zeroCreate all.Length
             let nOut = Array.zeroCreate sets.Length
             let mutable stats = GibbsRunStats()
-            check (gibbs_batch_fetch_best(b, numberOfRepetitions, sites, scores, nOut, null, null, null, &stats))
+            check (gibbs_multi_batch_fetch_best(b, numberOfRepetitions, sites, scores, nOut, null, null, null, &stats))
             Array.init sets.Length (fun s -> Array.init nOut.[s] (fun i -> scores.[setOffsets.[s] + i], sites.[setOffsets.[s] + i]))
         finally
-            gibbs_batch_destroy b |> ignore
+            gibbs_multi_batch_destroy b |> ignore
 
 open CompositeVector
 
@@ -265,7 +291,7 @@ module SiteSampler =
     let getMotifsWithBestInformationContentWithBPV (numberOfRepetitions:int) motifLength pseudoCount alphabet sources (pcv:ProbabilityCompositeVector) =
         Native.bestOfRestarts None numberOfRepetitions (seedOf None) motifLength pseudoCount alphabet sources (Some pcv)
 
-    /// getMotifsWithBestInformationContentWithBPV of every set (pcvs.[s] the background of sets.[s]) in one GPU batch
+    /// getMotifsWithBestInformationContentWithBPV of every set (pcvs.[s] the background of sets.[s]) in one batch over every GPU
     let getMotifsWithBestInformationContentWithBPVOfSets (numberOfRepetitions:int) motifLength pseudoCount alphabet sets (pcvs:ProbabilityCompositeVector[]) =
         Native.bestOfRestartsOfSets numberOfRepetitions (seedOf None) motifLength pseudoCount alphabet sets (Some pcvs)
 
@@ -282,7 +308,7 @@ module SiteSampler =
     /// fs:615-640 -- the script's live call (fsx:384)
     let getMotifsWithBestInformationContent (numberOfRepetitions:int) motifLength pseudoCount alphabet sources =
         Native.bestOfRestarts None numberOfRepetitions (seedOf None) motifLength pseudoCount alphabet sources None
-    /// getMotifsWithBestInformationContent of every set in one GPU batch
+    /// getMotifsWithBestInformationContent of every set in one batch over every GPU
     let getMotifsWithBestInformationContentOfSets (numberOfRepetitions:int) motifLength pseudoCount alphabet sets =
         Native.bestOfRestartsOfSets numberOfRepetitions (seedOf None) motifLength pseudoCount alphabet sets None
     /// fs:664-689
@@ -375,9 +401,9 @@ module MotifSampler =
     let getBestPWMSsOfPPM numberOfRepetitions motifAmount motifLength pseudoCount cutOff alphabet sources (ppM:PositionMatrix.PositionProbabilityMatrix) =
         (run 0 (numberOfRepetitions + 1) (seedOf None) motifAmount motifLength pseudoCount cutOff alphabet sources None (Some ppM) None (Some numberOfRepetitions)).[0]
 
-    /// The restart loops of many sets in one batch on GPU 0 (gibbs_batch_run_motif_device): set s gets exactly what the
-    /// single-set call with the same seed gives (restart r of every set draws from the stream (seed, r)); only the winners
-    /// are copied back.
+    /// The restart loops of many sets in one batch over EVERY GPU of the box (gibbs_multi_batch_run_motif_device): set s gets
+    /// exactly what the single-set call with the same seed gives (restart r of every set draws from the stream (seed, r)),
+    /// whatever the number of devices; only the winners are copied back.
     let private bestOfSets (numberOfRepetitions:int) seed (motifAmount:int) k pc (cutOff:float) alphabet (sets:BioArray.BioArray<#IBioItem>[][])
                            (pcvs:ProbabilityCompositeVector[] option) : MotifIndex[][] =
         let m = max motifAmount 1
@@ -386,7 +412,7 @@ module MotifSampler =
         let setOffsets = Array.zeroCreate<int> (sets.Length + 1)
         sets |> Array.iteri (fun s src -> setOffsets.[s + 1] <- setOffsets.[s] + src.Length)
         let mutable b = IntPtr.Zero
-        Native.check (Native.gibbs_batch_create(buf, offsets, setOffsets, sets.Length, 0, &b))
+        Native.check (Native.gibbs_multi_batch_create(buf, offsets, setOffsets, sets.Length, null, 0, &b))   // 0 = every visible device
         try
             let mutable p = Native.makeParams k pc alphabet (pcvs |> Option.map (fun v -> v.[0])) 0
             p.sampler <- 1; p.cutoff <- cutOff; p.motifAmount <- m
@@ -394,12 +420,12 @@ module MotifSampler =
                 match pcvs with
                 | Some v -> v |> Array.collect (fun pcv -> [| for c in "ACGT" -> pcv.Array.[int c - 42] |])
                 | None -> null
-            Native.check (Native.gibbs_batch_run_motif_device(b, &p, bg, numberOfRepetitions + 1, 0L, seed))
+            Native.check (Native.gibbs_multi_batch_run_motif_device(b, &p, bg, numberOfRepetitions + 1, 0L, seed))
             let sites, scores, pos = Array.zeroCreate all.Length, Array.zeroCreate all.Length, Array.zeroCreate (all.Length * m)
             let nOut, restart = Array.zeroCreate sets.Length, Array.zeroCreate sets.Length
             let mutable stats = Native.GibbsRunStats()
-            Native.check (Native.gibbs_batch_fetch_best(b, numberOfRepetitions, sites, scores, nOut, null, restart, null, &stats))
-            Native.check (Native.gibbs_batch_fetch_best_positions(b, m, pos))
+            Native.check (Native.gibbs_multi_batch_fetch_best(b, numberOfRepetitions, sites, scores, nOut, null, restart, null, &stats))
+            Native.check (Native.gibbs_multi_batch_fetch_best_positions(b, m, pos))
             Array.init sets.Length (fun s ->
                 let o = setOffsets.[s]
                 if restart.[s] < 0 then [| createMotifIndex 0. [] |]    // the loop's initial value survived
@@ -407,11 +433,11 @@ module MotifSampler =
                                                                                          let q = pos.[(o + i) * m + j]
                                                                                          if q >= 0 then yield q ])))
         finally
-            Native.gibbs_batch_destroy b |> ignore
+            Native.gibbs_multi_batch_destroy b |> ignore
 
-    /// findBestInormationContentContainingMotifsWithPCV of every set (pcvs.[s] the background of sets.[s]) in one GPU batch
+    /// findBestInormationContentContainingMotifsWithPCV of every set (pcvs.[s] the background of sets.[s]) in one batch over every GPU
     let findBestInormationContentContainingMotifsWithPCVOfSets numberOfRepetitions motifAmount motifLength pseudoCount cutOff alphabet sets (pcvs:ProbabilityCompositeVector[]) =
         bestOfSets numberOfRepetitions (seedOf None) motifAmount motifLength pseudoCount cutOff alphabet sets (Some pcvs)
-    /// getMotifsWithBestInformationContents of every set in one GPU batch (e.g. the script's fsx:407 call per gene group)
+    /// getMotifsWithBestInformationContents of every set in one batch over every GPU (e.g. the script's fsx:407 call per gene group)
     let getMotifsWithBestInformationContentsOfSets numberOfRepetitions motifAmount motifLength pseudoCount cutOff alphabet sets =
         bestOfSets numberOfRepetitions (seedOf None) motifAmount motifLength pseudoCount cutOff alphabet sets None

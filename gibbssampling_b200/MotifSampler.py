@@ -4,7 +4,8 @@
 motifAmount = 2 (up to two non-overlapping sites, fs:727-742 -- the reference script's second live call, fsx:407) are
 built; three and more sites per sequence raise GibbsUnsupportedError. Both the fixed-background (`...ByPCV` /
 `...WithPCV`) family and the data-derived-background family (fs:885-1038) run on the GPU. The `...OfSets` functions run
-the restart loops of many sets in one batch (gibbs_batch_run_motif_device).
+the restart loops of many sets in one batch (gibbs_batch_run_motif_device); by default on one GPU, on several with
+engine=MultiBatchEngine(sets, ...).
 """
 from __future__ import annotations
 

@@ -281,6 +281,7 @@ def getBestInformationContentOfPPM(numberOfRepetitions, motifLength, pseudoCount
 
 
 # ---- many sets in one batch (gibbs_batch_*): one result per set, element s = the single-set function on sets[s] ------
+# (engine=None: a BatchEngine on GPU 0; engine=MultiBatchEngine(sets, ...) spreads the sets over several GPUs)
 def _restart_loop_of_sets(numberOfRepetitions, motifLength, pseudoCount, alphabet, sets, pcvs, *, seed: int = 0,
                           chain: int = 0, max_sweeps: int = 0, engine: Optional[BatchEngine] = None) -> list:
     if sets is not None:

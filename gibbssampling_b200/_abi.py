@@ -42,6 +42,9 @@ EXPORTS = [
     "gibbs_multi_run_device", "gibbs_multi_fetch_best",
     "gibbs_batch_create", "gibbs_batch_destroy", "gibbs_batch_run_device", "gibbs_batch_fetch", "gibbs_batch_fetch_best",
     "gibbs_batch_run_motif_device", "gibbs_batch_fetch_positions", "gibbs_batch_fetch_best_positions",
+    "gibbs_multi_batch_create", "gibbs_multi_batch_destroy", "gibbs_multi_batch_num_devices", "gibbs_multi_batch_slot_sets",
+    "gibbs_multi_batch_run_device", "gibbs_multi_batch_run_motif_device", "gibbs_multi_batch_fetch", "gibbs_multi_batch_fetch_best",
+    "gibbs_multi_batch_fetch_positions", "gibbs_multi_batch_fetch_best_positions",
 ]
 GIBBS_OPT_INIT_PATH, GIBBS_OPT_EXACT_SCANS, GIBBS_OPT_STAGE2_AT, GIBBS_OPT_STAGE3_AT, GIBBS_OPT_CLUSTER, GIBBS_OPT_MIN_WIDTH = 1, 2, 3, 4, 5, 6
 GIBBS_OPT_TILE_ROWS = 7
@@ -186,6 +189,16 @@ def load() -> C.CDLL:
     lib.gibbs_batch_run_motif_device.argtypes = [vp, P(Params), P(f64), i32, i64, u64]
     lib.gibbs_batch_fetch_positions.argtypes = [vp, i32, P(i32)]
     lib.gibbs_batch_fetch_best_positions.argtypes = [vp, i32, P(i32)]
+    lib.gibbs_multi_batch_create.argtypes = [P(C.c_uint8), P(i64), P(i32), i32, P(i32), i32, P(vp)]
+    lib.gibbs_multi_batch_destroy.argtypes = [vp]
+    lib.gibbs_multi_batch_num_devices.argtypes = [vp]
+    lib.gibbs_multi_batch_slot_sets.argtypes = [vp, i32, P(i32), P(i32)]
+    lib.gibbs_multi_batch_run_device.argtypes = [vp, P(Params), P(f64), i32, i64, u64]
+    lib.gibbs_multi_batch_run_motif_device.argtypes = [vp, P(Params), P(f64), i32, i64, u64]
+    lib.gibbs_multi_batch_fetch.argtypes = [vp, P(i32), P(f64), P(f64), P(RunStats)]
+    lib.gibbs_multi_batch_fetch_best.argtypes = [vp, i32, P(i32), P(f64), P(i32), P(f64), P(i32), P(i32), P(RunStats)]
+    lib.gibbs_multi_batch_fetch_positions.argtypes = [vp, i32, P(i32)]
+    lib.gibbs_multi_batch_fetch_best_positions.argtypes = [vp, i32, P(i32)]
     for name in EXPORTS:
         fn = getattr(lib, name)
         if name not in ("gibbs_last_error", "gibbs_multi_handle"):

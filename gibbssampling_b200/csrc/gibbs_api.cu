@@ -1799,6 +1799,9 @@ int32_t gibbs_measure_smem_bandwidth(int32_t device, int32_t iters, double *gbps
 struct gibbs_batch {
     gibbs_handle *h = nullptr;
     int32_t n_sets = 0, n_seqs = 0;
+    // a block of a gibbs_multi_batch holds sets set_base .. set_base + n_sets - 1 of set_total: messages name sets by that
+    // number and the chain-count limit applies to set_total (a batch of its own: 0 and n_sets)
+    int32_t set_base = 0, set_total = 0;
     std::vector<int32_t> seq_off;               // [n_sets + 1] first sequence of each set
     std::vector<int32_t> min_len, max_len;      // per set
     std::vector<int64_t> n_masked;              // symbols outside A,C,G,T per set
@@ -1870,28 +1873,29 @@ int32_t batch_check(const gibbs_batch *b, const gibbs_params *p, const double *b
     if (p->alphabet_size < 1) return fail(GIBBS_ERR_ARG, "alphabet_size must be >= 1");
     if (!(p->pseudocount >= 0.0)) return fail(GIBBS_ERR_ARG, "pseudocount must be >= 0");
     if (p->background != GIBBS_BG_FIXED && p->background != GIBBS_BG_DATA) return fail(GIBBS_ERR_ARG, "unknown background mode %d", p->background);
-    if ((int64_t)R * b->n_sets > INT32_MAX) return fail(GIBBS_ERR_ARG, "%d sets x %d restarts: too many chains", b->n_sets, R);
+    if ((int64_t)R * b->set_total > INT32_MAX) return fail(GIBBS_ERR_ARG, "%d sets x %d restarts: too many chains", b->set_total, R);
     for (int32_t s = 0; s < b->n_sets; ++s) {
+        const int32_t gs = b->set_base + s; // the set's number in the caller's list
         if (b->min_len[s] < p->k) {
             int32_t i = b->seq_off[s];
             while (b->h->len_host[i] >= p->k) ++i;
-            return fail(GIBBS_ERR_SHORT_SEQ, "set %d, sequence %d: length %d is shorter than k=%d (Array.take, fs:152)", s,
+            return fail(GIBBS_ERR_SHORT_SEQ, "set %d, sequence %d: length %d is shorter than k=%d (Array.take, fs:152)", gs,
                         i - b->seq_off[s], b->h->len_host[i], p->k);
         }
         if (b->has_gap[s] && p->alphabet_size >= 5)
             return fail(GIBBS_ERR_UNSUPPORTED, "set %d holds Gap '-' and alphabet_size = %d includes it: a fifth PWM row is not built "
-                                               "(pass alphabet_size = 4 to score Gap like any other non-alphabet symbol)", s, p->alphabet_size);
+                                               "(pass alphabet_size = 4 to score Gap like any other non-alphabet symbol)", gs, p->alphabet_size);
         if (motif && p->motif_amount == 2 && b->n_masked[s] > 0)
             return fail(GIBBS_ERR_UNSUPPORTED, "set %d holds symbols outside A,C,G,T: the MotifSampler builds them for motifAmount = 1 "
-                                               "(motifAmount = 2 needs ACGT-only sequences)", s);
+                                               "(motifAmount = 2 needs ACGT-only sequences)", gs);
         const double *bg = p->background == GIBBS_BG_FIXED && bg_per_set ? bg_per_set + 4 * (size_t)s : p->bg;
         if (p->background == GIBBS_BG_FIXED)
             for (int x = 0; x < 4; ++x)
-                if (!(bg[x] > 0.0)) return fail(GIBBS_ERR_ARG, "set %d: background probability bg[%d] must be > 0", s, x);
+                if (!(bg[x] > 0.0)) return fail(GIBBS_ERR_ARG, "set %d: background probability bg[%d] must be > 0", gs, x);
         if (p->background == GIBBS_BG_DATA)
             for (int x = 0; x < 4; ++x)
                 if (b->gcnt[4 * (size_t)s + x] > INT32_MAX)
-                    return fail(GIBBS_ERR_ARG, "set %d: more than 2^31 bases of one kind: background counts overflow int32 (fs:34)", s);
+                    return fail(GIBBS_ERR_ARG, "set %d: more than 2^31 bases of one kind: background counts overflow int32 (fs:34)", gs);
     }
     return GIBBS_OK;
 }
@@ -2095,25 +2099,28 @@ int32_t batch_queue_errors(const gibbs_batch *b, std::vector<int32_t> &err) {
     return GIBBS_OK;
 }
 
-int32_t batch_check_errors(const std::vector<int32_t> &err) {
+int32_t batch_check_errors(const gibbs_batch *b, const std::vector<int32_t> &err) {
     for (size_t s = 0; s < err.size(); ++s)
         if (err[s])
-            return fail(GIBBS_ERR_ROULETTE, "set %d: a roulette pick lay beyond the accumulated mass (ArgumentException, fs:753)", (int)s);
+            return fail(GIBBS_ERR_ROULETTE, "set %d: a roulette pick lay beyond the accumulated mass (ArgumentException, fs:753)",
+                        b->set_base + (int)s);
     return GIBBS_OK;
 }
 
-} // namespace
-
-int32_t gibbs_batch_create(const uint8_t *seqs, const int64_t *offsets, const int32_t *set_offsets, int32_t n_sets, int32_t device,
-                           gibbs_batch **out) {
-    if (!out) return fail(GIBBS_ERR_ARG, "null out pointer");
-    *out = nullptr;
+// the argument checks of gibbs_batch_create that need no device (pointers and set_offsets)
+int32_t batch_check_layout(const uint8_t *seqs, const int64_t *offsets, const int32_t *set_offsets, int32_t n_sets) {
     if (!seqs || !offsets || !set_offsets) return fail(GIBBS_ERR_ARG, "null sequence buffer or set offsets (ArgumentNullException)");
     if (n_sets < 1) return fail(GIBBS_ERR_ARG, "n_sets must be >= 1");
     if (set_offsets[0] != 0) return fail(GIBBS_ERR_ARG, "set_offsets[0] must be 0 (it is %d)", set_offsets[0]);
     for (int32_t s = 0; s < n_sets; ++s)
         if (set_offsets[s + 1] <= set_offsets[s])
             return fail(GIBBS_ERR_ARG, "set %d is empty or set_offsets decrease (%d .. %d)", s, set_offsets[s], set_offsets[s + 1]);
+    return GIBBS_OK;
+}
+
+// gibbs_batch_create after batch_check_layout; the sets are sets set_base .. of set_total in the caller's numbering
+int32_t batch_create(const uint8_t *seqs, const int64_t *offsets, const int32_t *set_offsets, int32_t n_sets, int32_t device,
+                     int32_t set_base, int32_t set_total, gibbs_batch **out) {
     const int32_t n_seqs = set_offsets[n_sets];
     gibbs_batch *b = new (std::nothrow) gibbs_batch();
     if (!b) return fail(GIBBS_ERR_NOMEM, "host allocation failed");
@@ -2130,17 +2137,19 @@ int32_t gibbs_batch_create(const uint8_t *seqs, const int64_t *offsets, const in
     }
     b->n_sets = n_sets;
     b->n_seqs = n_seqs;
+    b->set_base = set_base;
+    b->set_total = set_total;
     // per-set symbol classes; a failure names the set and the sequence (gibbs_create would only name the symbol)
     for (int32_t s = 0; s < n_sets; ++s) {
         for (int32_t i = set_offsets[s]; i < set_offsets[s + 1]; ++i) {
             const int64_t l = offsets[i + 1] - offsets[i];
             if (l < 0) {
                 delete b;
-                return fail(GIBBS_ERR_ARG, "set %d, sequence %d: offsets must be non-decreasing", s, i - set_offsets[s]);
+                return fail(GIBBS_ERR_ARG, "set %d, sequence %d: offsets must be non-decreasing", set_base + s, i - set_offsets[s]);
             }
             if (l > GIBBS_MAX_LEN) {
                 delete b;
-                return fail(GIBBS_ERR_ARG, "set %d, sequence %d: longer than %d", s, i - set_offsets[s], GIBBS_MAX_LEN);
+                return fail(GIBBS_ERR_ARG, "set %d, sequence %d: longer than %d", set_base + s, i - set_offsets[s], GIBBS_MAX_LEN);
             }
             b->min_len[s] = std::min(b->min_len[s], (int32_t)l);
             b->max_len[s] = std::max(b->max_len[s], (int32_t)l);
@@ -2157,7 +2166,7 @@ int32_t gibbs_batch_create(const uint8_t *seqs, const int64_t *offsets, const in
                     delete b;
                     return fail(GIBBS_ERR_SYMBOL, "set %d, sequence %d: symbol '%c' (0x%02x) is outside '*'..'Z', the range of the "
                                                   "49-slot tables (IndexOutOfRangeException, fs:17-20)",
-                                s, i - set_offsets[s], c >= 32 && c < 127 ? (char)c : '?', c);
+                                set_base + s, i - set_offsets[s], c >= 32 && c < 127 ? (char)c : '?', c);
                 }
             }
         }
@@ -2177,6 +2186,17 @@ int32_t gibbs_batch_create(const uint8_t *seqs, const int64_t *offsets, const in
     }
     *out = b;
     return GIBBS_OK;
+}
+
+} // namespace
+
+int32_t gibbs_batch_create(const uint8_t *seqs, const int64_t *offsets, const int32_t *set_offsets, int32_t n_sets, int32_t device,
+                           gibbs_batch **out) {
+    if (!out) return fail(GIBBS_ERR_ARG, "null out pointer");
+    *out = nullptr;
+    const int32_t rc = batch_check_layout(seqs, offsets, set_offsets, n_sets);
+    if (rc) return rc;
+    return batch_create(seqs, offsets, set_offsets, n_sets, device, 0, n_sets, out);
 }
 
 int32_t gibbs_batch_destroy(gibbs_batch *b) {
@@ -2413,7 +2433,7 @@ int32_t gibbs_batch_fetch(gibbs_batch *b, int32_t *sites_out, double *scores_out
     rc = batch_queue_errors(b, err);
     if (rc) return rc;
     CUDA_TRY(cudaStreamSynchronize(h->stream));
-    rc = batch_check_errors(err);
+    rc = batch_check_errors(b, err);
     if (rc) return rc;
     if (stats_out) batch_stats(b, st, 0, stats_out);
     return GIBBS_OK;
@@ -2494,7 +2514,7 @@ int32_t gibbs_batch_fetch_best(gibbs_batch *b, int32_t repetitions, int32_t *sit
     rc = batch_queue_errors(b, err);
     if (rc) return rc;
     CUDA_TRY(cudaStreamSynchronize(h->stream));
-    rc = batch_check_errors(err);
+    rc = batch_check_errors(b, err);
     if (rc) return rc;
     b->best_valid = true;
     if (sites_out && M == 2)
@@ -2535,6 +2555,243 @@ int32_t gibbs_batch_fetch_best_positions(gibbs_batch *b, int32_t m, int32_t *pos
     if (rc) return rc;
     CUDA_TRY(cudaMemcpyAsync(positions_out, b->win_sites.p, (size_t)b->n_seqs * m * sizeof(int32_t), cudaMemcpyDeviceToHost, h->stream));
     CUDA_TRY(cudaStreamSynchronize(h->stream));
+    return GIBBS_OK;
+}
+
+/* ---- many sequence sets over several devices ----------------------------------------------------------------------- */
+// The sets are split once, at create time, into contiguous blocks, one per device slot; each slot holds an ordinary
+// gibbs_batch over its block (no set is replicated). Its set_base / set_total make its checks and messages those of one
+// batch over all the sets, and set s gives bit for bit what it gives in any batch, so the results are the one-device
+// batch's whatever the split.
+struct gibbs_multi_batch {
+    std::vector<gibbs_batch *> slot;   // nullptr: an empty slot (fewer sets than slots)
+    std::vector<int32_t> first, count; // slot i holds sets first[i] .. first[i] + count[i] - 1
+    std::vector<int32_t> set_off;      // [n_sets + 1] the caller's set_offsets
+    int32_t run_R = 0, run_k = 0;
+    bool run_done = false, best_valid = false;
+};
+
+namespace {
+
+// Contiguous blocks of sets, one per slot, whose largest cost is the least possible. The cost of a set is the sum of its
+// sequence lengths: up to k - 1 per sequence, the windows one sweep of one restart scores (k, the restart count and the
+// sampler are not known at create time). The least feasible bound is found by binary search over a greedy block count;
+// the blocks are then filled from the left up to it, keeping one set for each later slot while there are enough, so a
+// slot is left empty only when there are fewer sets than slots.
+void partition_sets(const std::vector<int64_t> &cost, int32_t slots, std::vector<int32_t> &first, std::vector<int32_t> &count) {
+    const int32_t S = (int32_t)cost.size();
+    int64_t lo = 0, hi = 0;
+    for (const int64_t c : cost) {
+        lo = std::max(lo, c);
+        hi += c;
+    }
+    while (lo < hi) { // least bound whose greedy blocks number at most `slots`
+        const int64_t mid = lo + (hi - lo) / 2;
+        int32_t blocks = 1;
+        int64_t sum = 0;
+        for (const int64_t c : cost) {
+            if (sum + c > mid) {
+                ++blocks;
+                sum = 0;
+            }
+            sum += c;
+        }
+        if (blocks <= slots) hi = mid;
+        else lo = mid + 1;
+    }
+    first.assign((size_t)slots, S);
+    count.assign((size_t)slots, 0);
+    int32_t next = 0;
+    for (int32_t i = 0; i < slots && next < S; ++i) {
+        first[i] = next;
+        int64_t sum = 0;
+        do {
+            sum += cost[next++];
+        } while (next < S && sum + cost[next] <= lo && S - next > slots - i - 1);
+        count[i] = next - first[i];
+    }
+}
+
+// the sum of the slots' statistics: counters and launches added, kernel_ms the slowest slot (the devices run concurrently),
+// the other fields those of the first slot
+void add_slot_stats(gibbs_run_stats &total, const gibbs_run_stats &st, bool first_slot) {
+    if (first_slot) total = st;
+    else {
+        total.site_updates += st.site_updates;
+        total.window_scores += st.window_scores;
+        total.sweeps += st.sweeps;
+        total.exact_rescans += st.exact_rescans;
+        total.capped_chains += st.capped_chains;
+        total.speculative_discards += st.speculative_discards;
+        total.kernel_launches += st.kernel_launches;
+        total.kernel_ms = std::max(total.kernel_ms, st.kernel_ms);
+    }
+}
+
+// checks the run on every slot first -- in set order, so a failure is the one a batch over all the sets reports -- then
+// queues each slot's run on its device without waiting for any of them
+int32_t multi_batch_run(gibbs_multi_batch *mb, const gibbs_params *p, const double *bg_per_set, int32_t R, int64_t chain_id_base,
+                        uint64_t seed, bool motif) {
+    if (!mb) return fail(GIBBS_ERR_ARG, "null multi-device batch");
+    mb->run_done = mb->best_valid = false;
+    for (size_t i = 0; i < mb->slot.size(); ++i) {
+        if (!mb->slot[i]) continue;
+        const int32_t rc = batch_check(mb->slot[i], p, bg_per_set ? bg_per_set + 4 * (size_t)mb->first[i] : nullptr, R, motif);
+        if (rc) return rc;
+    }
+    for (size_t i = 0; i < mb->slot.size(); ++i) {
+        if (!mb->slot[i]) continue;
+        const double *bg = bg_per_set ? bg_per_set + 4 * (size_t)mb->first[i] : nullptr;
+        const int32_t rc = motif ? gibbs_batch_run_motif_device(mb->slot[i], p, bg, R, chain_id_base, seed)
+                                 : gibbs_batch_run_device(mb->slot[i], p, bg, R, chain_id_base, seed);
+        if (rc) return rc;
+    }
+    mb->run_R = R;
+    mb->run_k = p->k;
+    mb->run_done = true;
+    return GIBBS_OK;
+}
+
+} // namespace
+
+int32_t gibbs_multi_batch_create(const uint8_t *seqs, const int64_t *offsets, const int32_t *set_offsets, int32_t n_sets,
+                                 const int32_t *devices, int32_t n_devices, gibbs_multi_batch **out) {
+    if (!out) return fail(GIBBS_ERR_ARG, "null out pointer");
+    *out = nullptr;
+    int32_t rc = batch_check_layout(seqs, offsets, set_offsets, n_sets);
+    if (rc) return rc;
+    if (n_devices < 0) return fail(GIBBS_ERR_ARG, "n_devices = %d must be >= 0", n_devices);
+    const int32_t visible = gibbs_device_count();
+    if (visible < 1) return fail(GIBBS_ERR_CUDA, "no CUDA device available; libgibbs_b200 has no CPU fallback");
+    if (n_devices == 0) n_devices = visible; // 0 = every visible device
+    // (an explicit device list may name a device twice: two slots then share it)
+    if (!devices && n_devices > visible) return fail(GIBBS_ERR_ARG, "n_devices = %d, %d visible", n_devices, visible);
+    gibbs_multi_batch *mb = new (std::nothrow) gibbs_multi_batch();
+    if (!mb) return fail(GIBBS_ERR_NOMEM, "host allocation failed");
+    std::vector<int32_t> so;
+    try {
+        std::vector<int64_t> cost((size_t)n_sets, 0);
+        for (int32_t s = 0; s < n_sets; ++s)
+            for (int32_t i = set_offsets[s]; i < set_offsets[s + 1]; ++i)
+                cost[s] += std::max<int64_t>(offsets[i + 1] - offsets[i], 0); // (bad offsets are reported by the slot's batch)
+        partition_sets(cost, n_devices, mb->first, mb->count);
+        mb->set_off.assign(set_offsets, set_offsets + n_sets + 1);
+        mb->slot.assign((size_t)n_devices, nullptr);
+    } catch (...) {
+        delete mb;
+        return fail(GIBBS_ERR_NOMEM, "host allocation failed");
+    }
+    for (int32_t i = 0; i < n_devices; ++i) {
+        const int32_t f = mb->first[i], c = mb->count[i];
+        if (c == 0) continue;
+        try {
+            so.resize((size_t)c + 1);
+        } catch (...) {
+            gibbs_multi_batch_destroy(mb);
+            return fail(GIBBS_ERR_NOMEM, "host allocation failed");
+        }
+        for (int32_t s = 0; s <= c; ++s) so[s] = set_offsets[f + s] - set_offsets[f];
+        rc = batch_create(seqs, offsets + set_offsets[f], so.data(), c, devices ? devices[i] : i, f, n_sets, &mb->slot[i]);
+        if (rc) {
+            gibbs_multi_batch_destroy(mb);
+            return rc;
+        }
+    }
+    *out = mb;
+    return GIBBS_OK;
+}
+
+int32_t gibbs_multi_batch_destroy(gibbs_multi_batch *mb) {
+    if (!mb) return GIBBS_OK;
+    for (gibbs_batch *b : mb->slot) gibbs_batch_destroy(b);
+    delete mb;
+    return GIBBS_OK;
+}
+
+int32_t gibbs_multi_batch_num_devices(const gibbs_multi_batch *mb) { return mb ? (int32_t)mb->slot.size() : 0; }
+
+int32_t gibbs_multi_batch_slot_sets(const gibbs_multi_batch *mb, int32_t slot, int32_t *first_set_out, int32_t *n_sets_out) {
+    if (!mb || !first_set_out || !n_sets_out) return fail(GIBBS_ERR_ARG, "null argument");
+    if (slot < 0 || slot >= (int32_t)mb->slot.size()) return fail(GIBBS_ERR_ARG, "slot %d outside 0..%d", slot, (int)mb->slot.size() - 1);
+    *first_set_out = mb->first[slot];
+    *n_sets_out = mb->count[slot];
+    return GIBBS_OK;
+}
+
+int32_t gibbs_multi_batch_run_device(gibbs_multi_batch *mb, const gibbs_params *p, const double *bg_per_set, int32_t restarts_per_set,
+                                     int64_t chain_id_base, uint64_t seed) {
+    return multi_batch_run(mb, p, bg_per_set, restarts_per_set, chain_id_base, seed, false);
+}
+
+int32_t gibbs_multi_batch_run_motif_device(gibbs_multi_batch *mb, const gibbs_params *p, const double *bg_per_set,
+                                           int32_t restarts_per_set, int64_t chain_id_base, uint64_t seed) {
+    return multi_batch_run(mb, p, bg_per_set, restarts_per_set, chain_id_base, seed, true);
+}
+
+int32_t gibbs_multi_batch_fetch(gibbs_multi_batch *mb, int32_t *sites_out, double *scores_out, double *sums_out,
+                                gibbs_run_stats *stats_out) {
+    if (!mb) return fail(GIBBS_ERR_ARG, "null multi-device batch");
+    if (!mb->run_done) return fail(GIBBS_ERR_ARG, "gibbs_multi_batch_fetch without a preceding run");
+    gibbs_run_stats total{};
+    bool first_slot = true;
+    for (size_t i = 0; i < mb->slot.size(); ++i) {
+        if (!mb->slot[i]) continue;
+        const size_t rows = (size_t)mb->run_R * mb->set_off[mb->first[i]], sums = (size_t)mb->run_R * mb->first[i];
+        gibbs_run_stats st{};
+        const int32_t rc = gibbs_batch_fetch(mb->slot[i], sites_out ? sites_out + rows : nullptr, scores_out ? scores_out + rows : nullptr,
+                                             sums_out ? sums_out + sums : nullptr, &st);
+        if (rc) return rc;
+        add_slot_stats(total, st, first_slot);
+        first_slot = false;
+    }
+    if (stats_out) *stats_out = total;
+    return GIBBS_OK;
+}
+
+int32_t gibbs_multi_batch_fetch_best(gibbs_multi_batch *mb, int32_t repetitions, int32_t *sites_out, double *scores_out, int32_t *n_out,
+                                     double *sum_out, int32_t *restart_out, int32_t *counts_out, gibbs_run_stats *stats_out) {
+    if (!mb) return fail(GIBBS_ERR_ARG, "null multi-device batch");
+    if (!mb->run_done) return fail(GIBBS_ERR_ARG, "gibbs_multi_batch_fetch_best without a preceding run");
+    mb->best_valid = false;
+    gibbs_run_stats total{};
+    bool first_slot = true;
+    for (size_t i = 0; i < mb->slot.size(); ++i) { // the slots in set order: a roulette failure names the lowest failing set
+        if (!mb->slot[i]) continue;
+        const size_t f = (size_t)mb->first[i], o = (size_t)mb->set_off[f];
+        gibbs_run_stats st{};
+        const int32_t rc = gibbs_batch_fetch_best(mb->slot[i], repetitions, sites_out ? sites_out + o : nullptr, scores_out ? scores_out + o : nullptr,
+                                                  n_out ? n_out + f : nullptr, sum_out ? sum_out + f : nullptr,
+                                                  restart_out ? restart_out + f : nullptr,
+                                                  counts_out ? counts_out + f * mb->run_k * 4 : nullptr, &st);
+        if (rc) return rc;
+        add_slot_stats(total, st, first_slot);
+        first_slot = false;
+    }
+    mb->best_valid = true;
+    if (stats_out) *stats_out = total;
+    return GIBBS_OK;
+}
+
+int32_t gibbs_multi_batch_fetch_positions(gibbs_multi_batch *mb, int32_t m, int32_t *positions_out) {
+    if (!mb || !positions_out) return fail(GIBBS_ERR_ARG, "null argument");
+    if (!mb->run_done) return fail(GIBBS_ERR_ARG, "gibbs_multi_batch_fetch_positions without a preceding run");
+    for (size_t i = 0; i < mb->slot.size(); ++i) {
+        if (!mb->slot[i]) continue;
+        const int32_t rc = gibbs_batch_fetch_positions(mb->slot[i], m, positions_out + (size_t)m * mb->run_R * mb->set_off[mb->first[i]]);
+        if (rc) return rc;
+    }
+    return GIBBS_OK;
+}
+
+int32_t gibbs_multi_batch_fetch_best_positions(gibbs_multi_batch *mb, int32_t m, int32_t *positions_out) {
+    if (!mb || !positions_out) return fail(GIBBS_ERR_ARG, "null argument");
+    if (!mb->run_done || !mb->best_valid)
+        return fail(GIBBS_ERR_ARG, "gibbs_multi_batch_fetch_best_positions without a preceding gibbs_multi_batch_fetch_best");
+    for (size_t i = 0; i < mb->slot.size(); ++i) {
+        if (!mb->slot[i]) continue;
+        const int32_t rc = gibbs_batch_fetch_best_positions(mb->slot[i], m, positions_out + (size_t)m * mb->set_off[mb->first[i]]);
+        if (rc) return rc;
+    }
     return GIBBS_OK;
 }
 

@@ -448,6 +448,8 @@ class BatchEngine:
     exactly what a GibbsEngine over sets[s] alone gives for the same parameters, seed and chain_id_base. run_device runs
     the SiteSampler, run_motif_device the MotifSampler; fetch / fetch_best serve the last run of either."""
 
+    _API = "gibbs_batch_"   # prefix of the C functions behind the methods
+
     def __init__(self, sets: Sequence[Sequence], device: int = 0):
         self._lib = _abi.load()
         self._b = C.c_void_p()
@@ -462,7 +464,7 @@ class BatchEngine:
 
     def close(self) -> None:
         if getattr(self, "_b", None) is not None and self._b.value:
-            self._lib.gibbs_batch_destroy(self._b)
+            getattr(self._lib, self._API + "destroy")(self._b)
             self._b = C.c_void_p()
 
     def __del__(self):
@@ -477,6 +479,9 @@ class BatchEngine:
     def __exit__(self, *exc):
         self.close()
 
+    def _call(self, name: str, *args) -> None:
+        _abi.check(getattr(self._lib, self._API + name)(self._b, *args))
+
     def _bg_per_set(self, bg_per_set):
         if bg_per_set is None:
             return None
@@ -489,8 +494,8 @@ class BatchEngine:
         """restarts_per_set restarts of every set; bg_per_set = [n_sets][4] backgrounds of the fixed-background family
         (None = params.bg for every set). Results stay in HBM until fetch() / fetch_best()."""
         bg = self._bg_per_set(bg_per_set)
-        _abi.check(self._lib.gibbs_batch_run_device(self._b, C.byref(params), _ptr(bg, C.c_double), C.c_int32(restarts_per_set),
-                                                    C.c_int64(chain_id_base), C.c_uint64(seed)))
+        self._call("run_device", C.byref(params), _ptr(bg, C.c_double), C.c_int32(restarts_per_set), C.c_int64(chain_id_base),
+                   C.c_uint64(seed))
         self._last = (int(restarts_per_set), int(params.k), 1)
 
     def run_motif_device(self, params: Params, restarts_per_set: int, *, bg_per_set=None, chain_id_base: int = 0,
@@ -499,8 +504,8 @@ class BatchEngine:
         run_device. fetch() then returns the newest position of every sequence (-1 = no site), fetch_positions(m) the
         Positions lists."""
         bg = self._bg_per_set(bg_per_set)
-        _abi.check(self._lib.gibbs_batch_run_motif_device(self._b, C.byref(params), _ptr(bg, C.c_double),
-                                                          C.c_int32(restarts_per_set), C.c_int64(chain_id_base), C.c_uint64(seed)))
+        self._call("run_motif_device", C.byref(params), _ptr(bg, C.c_double), C.c_int32(restarts_per_set),
+                   C.c_int64(chain_id_base), C.c_uint64(seed))
         self._last = (int(restarts_per_set), int(params.k), max(int(params.motif_amount), 1))
 
     def _need_run(self) -> tuple[int, int, int]:
@@ -515,8 +520,7 @@ class BatchEngine:
         scores = np.zeros(R * total, dtype=np.float64)
         sums = np.zeros((self.n_sets, R), dtype=np.float64)
         st = RunStats()
-        _abi.check(self._lib.gibbs_batch_fetch(self._b, _ptr(sites, C.c_int32), _ptr(scores, C.c_double), _ptr(sums, C.c_double),
-                                               C.byref(st)))
+        self._call("fetch", _ptr(sites, C.c_int32), _ptr(scores, C.c_double), _ptr(sums, C.c_double), C.byref(st))
         out_sites, out_scores = [], []
         for s in range(self.n_sets):
             a, n = R * int(self.set_offsets[s]), int(self.sizes[s])
@@ -536,9 +540,8 @@ class BatchEngine:
         restart = np.zeros(self.n_sets, dtype=np.int32)
         counts = np.zeros((self.n_sets, k, 4), dtype=np.int32) if want_counts else None
         st = RunStats()
-        _abi.check(self._lib.gibbs_batch_fetch_best(self._b, C.c_int32(repetitions), _ptr(sites, C.c_int32), _ptr(scores, C.c_double),
-                                                    _ptr(n_out, C.c_int32), _ptr(sums, C.c_double), _ptr(restart, C.c_int32),
-                                                    _ptr(counts, C.c_int32), C.byref(st)))
+        self._call("fetch_best", C.c_int32(repetitions), _ptr(sites, C.c_int32), _ptr(scores, C.c_double), _ptr(n_out, C.c_int32),
+                   _ptr(sums, C.c_double), _ptr(restart, C.c_int32), _ptr(counts, C.c_int32), C.byref(st))
         stats = {f: getattr(st, f) for f, _ in RunStats._fields_}
         out = []
         for s in range(self.n_sets):
@@ -553,7 +556,7 @@ class BatchEngine:
         R, _, _ = self._need_run()
         total = int(self.set_offsets[-1])
         pos = np.zeros(R * total * int(m), dtype=np.int32)
-        _abi.check(self._lib.gibbs_batch_fetch_positions(self._b, C.c_int32(m), _ptr(pos, C.c_int32)))
+        self._call("fetch_positions", C.c_int32(m), _ptr(pos, C.c_int32))
         return [pos[R * int(m) * int(self.set_offsets[s]): R * int(m) * int(self.set_offsets[s + 1])].reshape(R, int(self.sizes[s]), int(m))
                 for s in range(self.n_sets)]
 
@@ -563,9 +566,44 @@ class BatchEngine:
         self._need_run()
         total = int(self.set_offsets[-1])
         pos = np.zeros(total * int(m), dtype=np.int32)
-        _abi.check(self._lib.gibbs_batch_fetch_best_positions(self._b, C.c_int32(m), _ptr(pos, C.c_int32)))
+        self._call("fetch_best_positions", C.c_int32(m), _ptr(pos, C.c_int32))
         return [pos[int(m) * int(self.set_offsets[s]): int(m) * int(self.set_offsets[s + 1])].reshape(int(self.sizes[s]), int(m))
                 for s in range(self.n_sets)]
+
+
+class MultiBatchEngine(BatchEngine):
+    """A BatchEngine whose sets are split over several GPUs of the process (gibbs_multi_batch_*): contiguous blocks of sets,
+    one per device slot, chosen at create time so that the largest block holds the fewest bases. Every method returns
+    exactly what a one-device BatchEngine over the same sets returns; the slots run concurrently.
+    devices: the device of each slot (a device may be listed twice); None = devices 0 .. n_devices-1, n_devices = 0 = every
+    visible device."""
+
+    _API = "gibbs_multi_batch_"
+
+    def __init__(self, sets: Sequence[Sequence], n_devices: int = 0, devices: Optional[Sequence[int]] = None):
+        self._lib = _abi.load()
+        self._b = C.c_void_p()
+        buf, off, set_off = flatten_sets(sets)
+        self.n_sets = len(set_off) - 1
+        self.set_offsets = set_off.astype(np.int64)
+        self.sizes = np.diff(self.set_offsets)
+        dev = np.ascontiguousarray(devices, dtype=np.int32) if devices is not None else None
+        if dev is not None:
+            n_devices = len(dev)
+        _abi.check(self._lib.gibbs_multi_batch_create(_ptr(buf, C.c_uint8), _ptr(off, C.c_int64), _ptr(set_off, C.c_int32),
+                                                      C.c_int32(self.n_sets), _ptr(dev, C.c_int32), C.c_int32(n_devices),
+                                                      C.byref(self._b)))
+        self.n_devices = int(self._lib.gibbs_multi_batch_num_devices(self._b))
+        self._last = None
+
+    def slot_sets(self) -> list[tuple[int, int]]:
+        """(first set, number of sets) of every device slot, in slot order; (.., 0) for an empty slot."""
+        out = []
+        for i in range(self.n_devices):
+            first, n = C.c_int32(), C.c_int32()
+            _abi.check(self._lib.gibbs_multi_batch_slot_sets(self._b, C.c_int32(i), C.byref(first), C.byref(n)))
+            out.append((int(first.value), int(n.value)))
+        return out
 
 
 def device_count() -> int:

@@ -343,6 +343,42 @@ int32_t gibbs_batch_fetch_positions(gibbs_batch *b, int32_t m, int32_t *position
 /* the winners' Positions lists of the last gibbs_batch_fetch_best: int32 [sum_s N_s][m] (set s at m set_offsets[s]) */
 int32_t gibbs_batch_fetch_best_positions(gibbs_batch *b, int32_t m, int32_t *positions_out);
 
+/* ---- many independent sequence sets over several devices ------------------------------------------------------- */
+/*
+ * A batch whose sets are split over the devices of the process: at create time the sets are divided into contiguous
+ * blocks, one per device slot, that minimise the largest block cost (the cost of a set is the sum of its sequence
+ * lengths), and each slot holds a gibbs_batch over its block on its device. A slot is empty only when there are fewer
+ * sets than slots. The functions mirror the gibbs_batch_* calls with the same arguments and layouts, in the caller's
+ * set order; every output is bit for bit what one gibbs_batch over all the sets returns.
+ * devices = NULL: devices 0 .. n_devices-1; n_devices = 0: every visible device; a device may be listed twice (the slots
+ * then share it). Argument errors of gibbs_batch_create and n_devices < 0 are reported before any device is used.
+ * The run calls check the whole call as one batch over all the sets would (the same code and text, sets named by their
+ * index in the caller's list), then queue every slot's launches on its own device and stream and return without waiting;
+ * the devices run concurrently. The fetch calls copy each slot's block straight to its place in the caller's arrays.
+ * Stats: counters and kernel_launches summed over the slots, kernel_ms the slowest slot, the other fields the first slot's.
+ */
+typedef struct gibbs_multi_batch gibbs_multi_batch;
+int32_t gibbs_multi_batch_create(const uint8_t *seqs, const int64_t *offsets, const int32_t *set_offsets, int32_t n_sets,
+                                 const int32_t *devices, int32_t n_devices, gibbs_multi_batch **out);
+int32_t gibbs_multi_batch_destroy(gibbs_multi_batch *mb);
+int32_t gibbs_multi_batch_num_devices(const gibbs_multi_batch *mb);
+/* the contiguous block of sets that device slot i holds (n_sets_out = 0 for an empty slot) */
+int32_t gibbs_multi_batch_slot_sets(const gibbs_multi_batch *mb, int32_t slot, int32_t *first_set_out, int32_t *n_sets_out);
+/* arguments as gibbs_batch_run_device / gibbs_batch_run_motif_device */
+int32_t gibbs_multi_batch_run_device(gibbs_multi_batch *mb, const gibbs_params *p, const double *bg_per_set,
+                                     int32_t restarts_per_set, int64_t chain_id_base, uint64_t seed);
+int32_t gibbs_multi_batch_run_motif_device(gibbs_multi_batch *mb, const gibbs_params *p, const double *bg_per_set,
+                                           int32_t restarts_per_set, int64_t chain_id_base, uint64_t seed);
+/* layouts as gibbs_batch_fetch / _fetch_best / _fetch_positions / _fetch_best_positions; a roulette failure names the
+ * lowest failing set */
+int32_t gibbs_multi_batch_fetch(gibbs_multi_batch *mb, int32_t *sites_out, double *scores_out, double *sums_out,
+                                gibbs_run_stats *stats_out);
+int32_t gibbs_multi_batch_fetch_best(gibbs_multi_batch *mb, int32_t repetitions, int32_t *sites_out, double *scores_out,
+                                     int32_t *n_out, double *sum_out, int32_t *restart_out, int32_t *counts_out,
+                                     gibbs_run_stats *stats_out);
+int32_t gibbs_multi_batch_fetch_positions(gibbs_multi_batch *mb, int32_t m, int32_t *positions_out);
+int32_t gibbs_multi_batch_fetch_best_positions(gibbs_multi_batch *mb, int32_t m, int32_t *positions_out);
+
 /* ---- host buffers ------------------------------------------------------------------------------- */
 /* Page-locked host memory for the *_out arrays above (results of 1024 chains x 1000 sequences are
  * 12 MB; into pageable memory the copy is staged by the driver and pays first-touch page faults).
