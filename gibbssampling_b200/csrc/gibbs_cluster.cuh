@@ -118,7 +118,9 @@ static __global__ void __launch_bounds__(32 * CL_T, 1) chain_cluster_kernel(cons
     __syncthreads();
     cluster_barrier(); // every CTA of the cluster is running (remote shared memory may be written from here on)
 
-    unsigned long long st_updates = 0, st_windows = 0, st_slow = 0, st_spec = 0;
+    // site_updates and window_scores per sweep, as in chain_kernel; this warp's exact rescans and discarded updates of the
+    // current sweep (at most N each) are added at its end
+    unsigned st_slow = 0, st_spec = 0;
     int st_sweeps = 0, capped = 0;
     int phase, sweeps_in_phase;
     {
@@ -245,8 +247,6 @@ static __global__ void __launch_bounds__(32 * CL_T, 1) chain_cluster_kernel(cons
             changed |= any_moved;
             if (active) {
                 if (gw <= last_commit) {
-                    st_updates += 1;
-                    st_windows += (unsigned long long)Wn;
                     st_slow += (flag & 4) ? 1 : 0;
                     if ((flag & 1) && lane == 0) {
                         sites[n] = w;
@@ -297,6 +297,11 @@ static __global__ void __launch_bounds__(32 * CL_T, 1) chain_cluster_kernel(cons
         cp_async_wait_all(); // (a prefetch past the last round may still be in flight)
         __syncwarp();
         st_sweeps += 1;
+        if (lane == 0) {
+            if (st_slow) atomicAdd(a.stats + ST_EXACT_RESCANS, (unsigned long long)st_slow);
+            if (st_spec) atomicAdd(a.stats + ST_SPECULATED, (unsigned long long)st_spec);
+        }
+        st_slow = st_spec = 0;
         ++sweeps_in_phase;
         bool next = !changed; // positions(acc) = positions(bestMotif), fs:384
         if (!next && sweeps_in_phase >= a.max_sweeps) {
@@ -320,14 +325,15 @@ static __global__ void __launch_bounds__(32 * CL_T, 1) chain_cluster_kernel(cons
         }
     }
     cluster_barrier(); // nobody leaves while a neighbour may still write into its shared memory
-    if (lane == 0) {
-        atomicAdd(a.stats + ST_SITE_UPDATES, st_updates);
-        atomicAdd(a.stats + ST_WINDOW_SCORES, st_windows);
-        atomicAdd(a.stats + ST_EXACT_RESCANS, st_slow);
-        atomicAdd(a.stats + ST_SPECULATED, st_spec);
-    }
     if (crank != 0) return;
+    if (st_sweeps > 0) { // windows per sweep: the sum of len_n - k + 1 over the sequences, added per warp of rank 0
+        unsigned long long sum_w = 0;
+        for (int n = tid; n < N; n += THREADS) sum_w += (unsigned long long)(__ldg(a.s.len + n) - k + 1);
+        sum_w = warp_sum_u64(sum_w);
+        if (lane == 0) atomicAdd(a.stats + ST_WINDOW_SCORES, sum_w * (unsigned long long)st_sweeps);
+    }
     if (tid == 0) {
+        atomicAdd(a.stats + ST_SITE_UPDATES, (unsigned long long)N * (unsigned long long)st_sweeps);
         atomicAdd(a.stats + ST_SWEEPS, (unsigned long long)st_sweeps);
         if (!paused) atomicAdd(a.stats + ST_CAPPED, (unsigned long long)capped); // (a chain counts once, where it ends)
     }

@@ -713,30 +713,43 @@ __device__ __forceinline__ double lds_f64(uint32_t addr) {
 }
 // factor of column J: wcol[J][base J of the k-mer]; the address register is (base * 8) | table address (the table is
 // 32-byte aligned: one shift + one LOP3), the immediate selects the column (32 B each)
+template <int C>
+__device__ __forceinline__ double column_factor(uint32_t lo, uint32_t hi, uint32_t wcol_addr) {
+    const uint32_t word = C < 16 ? lo : hi;
+    constexpr int sh = 2 * (C & 15); // bit position of the base code inside its word
+    const uint32_t off = (sh >= 3 ? (word >> (sh - 3)) : (word << (3 - sh))) & 24u;
+    return lds_f64<C * 32>(off | wcol_addr);
+}
+// product of the factors of columns 0 .. J - 1, left to right: (w0 * w1) * w2 ... (fs:291-292; the fold's 1 * w0 is w0)
 template <int KP, int J>
 struct WindowProduct {
-    static __device__ __forceinline__ double upto(uint32_t lo, uint32_t hi, uint32_t wcol_addr, int k) {
-        const double prev = WindowProduct<KP, J - 1>::upto(lo, hi, wcol_addr, k);
-        constexpr int c = J - 1;                       // column of this factor
-        const uint32_t word = c < 16 ? lo : hi;
-        constexpr int sh = 2 * (c & 15);               // bit position of the base code inside its word
-        const uint32_t off = (sh >= 3 ? (word >> (sh - 3)) : (word << (3 - sh))) & 24u;
-        const double f = lds_f64<c * 32>(off | wcol_addr);
-        return c < k ? __dmul_rn(prev, f) : prev;      // ((1 * w0) * w1) * ... left to right (fs:291-292)
+    static __device__ __forceinline__ double upto(uint32_t lo, uint32_t hi, uint32_t wcol_addr) {
+        if constexpr (J == 1) {
+            return column_factor<0>(lo, hi, wcol_addr);
+        } else {
+            const double prev = WindowProduct<KP, J - 1>::upto(lo, hi, wcol_addr);
+            return __dmul_rn(prev, column_factor<J - 1>(lo, hi, wcol_addr));
+        }
     }
 };
-template <int KP>
-struct WindowProduct<KP, 0> {
-    static __device__ __forceinline__ double upto(uint32_t, uint32_t, uint32_t, int) { return 1.0; }
-};
 
+// Every window over all 2 KP columns of wcol: every table this reads holds 1.0 in the four entries of each column
+// k .. 2 KP - 1 (build_tables_impl, the MotifSampler's odds and background tables), and x * 1.0 == x exactly in float64
+// (device float64 keeps subnormals), so the product is the reference's k-factor fold bit for bit.
 template <int KP>
-__device__ __forceinline__ double exact_window(const uint32_t *row, int w, int k, const double *wcol) {
+__device__ __forceinline__ double exact_window(const uint32_t *row, int w, const double *wcol) {
     const uint64_t kmer = kmer_shared<KP>(row, w);
-    return WindowProduct<KP, 2 * KP>::upto((uint32_t)kmer, (uint32_t)(kmer >> 32), smem_u32(wcol), k);
+    return WindowProduct<KP, 2 * KP>::upto((uint32_t)kmer, (uint32_t)(kmer >> 32), smem_u32(wcol));
 }
 
 __device__ __forceinline__ bool better(double ohv, int ow, double hv, int w) { return ohv > hv || (ohv == hv && ow < w); }
+
+// sum over the warp; every lane ends with it
+__device__ __forceinline__ unsigned long long warp_sum_u64(unsigned long long v) {
+#pragma unroll
+    for (int o = 16; o; o >>= 1) v += __shfl_xor_sync(FULL, v, o);
+    return v;
+}
 
 // (max value, lowest index) over the warp; every lane ends with the result
 __device__ __forceinline__ void warp_argmax(double &hv, int &w) {
@@ -753,12 +766,12 @@ __device__ __forceinline__ void warp_argmax(double &hv, int &w) {
 
 // the reference loop itself (fs:302-314): every window in float64, first strict maximum from (0., 0)
 template <int KP>
-__device__ __forceinline__ void scan_exact_all(const uint32_t *row, int W, int k, const double *wcol, int lane,
+__device__ __forceinline__ void scan_exact_all(const uint32_t *row, int W, const double *wcol, int lane,
                                                double &hv_out, int &w_out) {
     double hv = 0.0;
     int hw = 0;
     for (int w = lane; w < W; w += 32) {
-        const double p = exact_window<KP>(row, w, k, wcol);
+        const double p = exact_window<KP>(row, w, wcol);
         if (p > hv) {
             hv = p;
             hw = w;
@@ -778,7 +791,7 @@ __device__ __noinline__ void scan_exact_masked(const uint32_t *row, const uint32
     int hw = 0;
     for (int w = lane; w < W; w += 32) {
         if (mask_kmer(mask, row_words, n, w, k) != 0) continue;
-        const double p = exact_window<KP>(row, w, k, wcol);
+        const double p = exact_window<KP>(row, w, wcol);
         if (p > hv) {
             hv = p;
             hw = w;
@@ -922,7 +935,7 @@ __device__ __forceinline__ bool pick_argmax_ch(const WarpTables &T, const uint32
         const int base0 = chunk_base<CH>(seg * G::CPS + src + 32 * (255 - (key & 255)), W);
         const int wi = base0 + lane;
         if (lane < CH && wi < W) {
-            const double pi = exact_window<KP>(row, wi, k, T.wcol);
+            const double pi = exact_window<KP>(row, wi, T.wcol);
             if (better(pi, wi, p, w)) {
                 p = pi;
                 w = wi;
@@ -957,7 +970,7 @@ __device__ __forceinline__ bool pick_argmax(const WarpTables &T, const uint32_t 
         else if (W > 128) slow = pick_argmax_ch<KP, 8>(T, row, W, k, lane, hv_out, w_out);
         else slow = pick_argmax_ch<KP, 4>(T, row, W, k, lane, hv_out, w_out);
     }
-    if (slow) scan_exact_all<KP>(row, W, k, T.wcol, lane, hv_out, w_out);
+    if (slow) scan_exact_all<KP>(row, W, T.wcol, lane, hv_out, w_out);
     return slow;
 }
 

@@ -704,7 +704,7 @@ static __global__ void __launch_bounds__(32) scan_kernel(const PrimArgs a, int m
     const int masked_n = row_masked(a.s, a.heldout) ? a.heldout : -1;
     if (mode == 0) {
         for (int w = lane; w < W; w += 32) {
-            double p = exact_window<KP>(row, w, a.k, WT.wcol);
+            double p = exact_window<KP>(row, w, WT.wcol);
             if (masked_n >= 0 && mask_kmer(a.s.mask, a.s.row_words, masked_n, w, a.k) != 0) p = 0.0; // PWM row of the symbol is 0
             if (a.raw_out) a.raw_out[w] = p;
             if (a.log2_out) a.log2_out[w] = log2_ref(p);

@@ -105,7 +105,7 @@ __device__ __forceinline__ int motif_gate(const WarpTables &T, const uint32_t *r
     int gated = 0;
     for (int w0 = 0; w0 < W; w0 += 32) {
         const int w = w0 + lane;
-        double s = w < W ? exact_window<KP>(row, w, k, T.wcol) : 0.0;
+        double s = w < W ? exact_window<KP>(row, w, T.wcol) : 0.0;
         if (MASKED && masked_n >= 0 && w < W && mask_kmer(sq->mask, sq->row_words, masked_n, w, k) != 0) s = 0.0;
         const bool g = w < W && s > raw_gate; // (raw_gate >= 0: a masked window never passes)
         const unsigned m = __ballot_sync(FULL, g);
@@ -370,7 +370,7 @@ __device__ __forceinline__ bool pick_unique_argmax_ch(const WarpTables &T, const
         const int seg = __shfl_sync(FULL, S1, src);
         const int wi = chunk_base<CH>(seg * G::CPS + src + 32 * (255 - (key & 255)), W) + lane;
         if (lane < CH && wi < W) {
-            const double pi = exact_window<KP>(row, wi, k, T.wcol);
+            const double pi = exact_window<KP>(row, wi, T.wcol);
             if (better(pi, wi, p, w)) {
                 p2 = fmax(p2, p);
                 p = pi;
