@@ -296,13 +296,14 @@ module SiteSampler =
         Native.bestOfRestartsOfSets numberOfRepetitions (seedOf None) motifLength pseudoCount alphabet sets (Some pcvs)
 
     // ---- data-derived background (fs:462-640, fs:697): background = 1, no pcv ---------------------------------
+    // Gap '-' is an alphabet member here when alphabet holds it (dnaBases): gap-padded alignments run with its PWM row.
     /// fs:697-701
     let doSiteSampling motifLength pseudoCount alphabet sources =
         (Native.runChainsWith None 15 1 (seedOf None) motifLength pseudoCount alphabet sources None None |> fst).[0]
-    /// fs:703-707
+    /// fs:703-707 (ppM has no Gap row: sets holding '-' with Gap in the alphabet raise NotSupportedException)
     let doSiteSamplingWithPPM motifLength pseudoCount alphabet sources (ppM:PositionMatrix.PositionProbabilityMatrix) =
         (Native.runChainsWith (Some ppM) 15 1 (seedOf None) motifLength pseudoCount alphabet sources None None |> fst).[0]
-    /// fs:644-661
+    /// fs:644-661 (as doSiteSamplingWithPPM for Gap)
     let getMotifsWithBestPWMSOfPPM motifLength pseudoCount alphabet sources (ppM:PositionMatrix.PositionProbabilityMatrix) =
         (Native.runChainsWith (Some ppM) 1 1 (seedOf None) motifLength pseudoCount alphabet sources None None |> fst).[0]
     /// fs:615-640 -- the script's live call (fsx:384)

@@ -137,16 +137,17 @@ struct gibbs_handle {
     DevBuf<uint8_t> ascii;
     DevBuf<int64_t> off;
     DevBuf<uint32_t> packed;
-    DevBuf<uint32_t> mask;     // same geometry as packed: 0b11 at symbols outside A,C,G,T
+    DevBuf<uint32_t> mask;     // same geometry as packed: 0b01 at Gap '-', 0b11 at the other symbols outside A,C,G,T
     DevBuf<int32_t> rowflag;   // [n] sequence holds such a symbol
     DevBuf<uint64_t> wide;     // gather copy of the packed rows (DeviceSeqs::wide), built on first use
     bool wide_valid = false;
     int32_t wide_words = 0;
     DevBuf<int32_t> len;
     DevBuf<int> flags;    // [1..3] wtab range
-    DevBuf<int> symflags; // pack_kernel: [0] 1 + byte outside '*'..'Z', [1] symbols outside A,C,G,T, [2] Gap seen
+    DevBuf<int> symflags; // pack_kernel: [0] 1 + byte outside '*'..'Z', [1] symbols outside A,C,G,T, [2] Gaps among them
     int64_t n_masked = 0;      // symbols outside A,C,G,T in the uploaded set
     bool has_gap = false;
+    int64_t n_gap = 0;         // Gaps '-' among them (the Gap slot of the set totals when Gap is in the alphabet)
 
     // PWM value table, keyed by the parameters it was built for
     DevBuf<WEnt> wtab;
@@ -222,6 +223,11 @@ int32_t set_device(const gibbs_handle *h) {
     return GIBBS_OK;
 }
 
+// Gap as an alphabet member has its PWM row for the SiteSampler with the data-derived background, where its background
+// probability comes from the counts like a base's. The fixed background would need pcv.[Gap], which gibbs_params (bg[4])
+// does not carry, and the MotifSampler has no Gap row in its tables.
+bool gap_row_built(const gibbs_params *p) { return p->sampler == GIBBS_SITE_SAMPLER && p->background == GIBBS_BG_DATA; }
+
 int32_t check_params(const gibbs_handle *h, const gibbs_params *p) {
     if (!h) return fail(GIBBS_ERR_ARG, "null handle");
     if (!p) return fail(GIBBS_ERR_ARG, "null params");
@@ -233,11 +239,12 @@ int32_t check_params(const gibbs_handle *h, const gibbs_params *p) {
     if (!(p->pseudocount >= 0.0)) return fail(GIBBS_ERR_ARG, "pseudocount must be >= 0");
     if (p->background != GIBBS_BG_FIXED && p->background != GIBBS_BG_DATA) return fail(GIBBS_ERR_ARG, "unknown background mode %d", p->background);
     // An alphabet of >= 5 symbols is taken to hold Gap like the script's dnaBases (fsx:368-369). Gap then has
-    // a PWM row of its own (quirk A.6-2), which the 4-row tables cannot hold; any other symbol outside A,C,G,T
-    // is not in the alphabet, has a PWM row of 0 (fs:283-287) and is handled by the mask plane.
-    if (h->has_gap && p->alphabet_size >= 5)
-        return fail(GIBBS_ERR_UNSUPPORTED, "sequences hold Gap '-' and alphabet_size = %d includes it: a fifth PWM row is not built "
-                                           "(pass alphabet_size = 4 to score Gap like any other non-alphabet symbol)", p->alphabet_size);
+    // a PWM row of its own (quirk A.6-2); any other symbol outside A,C,G,T is not in the alphabet, has a PWM row
+    // of 0 (fs:283-287) and is handled by the mask plane.
+    if (h->has_gap && p->alphabet_size >= 5 && !gap_row_built(p))
+        return fail(GIBBS_ERR_UNSUPPORTED, "sequences hold Gap '-' and alphabet_size = %d includes it: its PWM row is built for the "
+                                           "SiteSampler with the data-derived background only (pass alphabet_size = 4 to score Gap "
+                                           "like any other non-alphabet symbol)", p->alphabet_size);
     if (p->background == GIBBS_BG_FIXED)
         for (int b = 0; b < 4; ++b)
             if (!(p->bg[b] > 0.0)) return fail(GIBBS_ERR_ARG, "background probability bg[%d] must be > 0", b);
@@ -292,9 +299,10 @@ int fast_path_ok(const gibbs_handle *h, int k) { return fast_path_ok_range(h->wt
 // The ranking pass of the drifting background is valid when every odds ratio ppm / pcv, which lies in [pc / den, den / pc]
 // with den <= all bases of the set + one more sequence + |A| pc (or N - 1 + |A| pc), keeps every float64 product of k of
 // them in the normal range (|log2| < 1000), and pc >= 1e-30 keeps every float32 logarithm argument normal and finite.
-int drift_fast_path_ok(const int32_t gcnt[4], int32_t max_len, int32_t n, const gibbs_params *p) {
+// gaps = the set's Gaps when Gap is in the alphabet (they enter every denominator), else 0.
+int drift_fast_path_ok(const int32_t gcnt[4], int32_t gaps, int32_t max_len, int32_t n, const gibbs_params *p) {
     const double alpha_pc = (double)p->alphabet_size * p->pseudocount;
-    const double bases = (double)gcnt[0] + gcnt[1] + gcnt[2] + gcnt[3] + (double)max_len;
+    const double bases = (double)gcnt[0] + gcnt[1] + gcnt[2] + gcnt[3] + (double)gaps + (double)max_len;
     const double den = (bases > (double)n ? bases : (double)n) + alpha_pc;
     return (p->pseudocount >= 1e-30 && (double)p->k * log2(den / p->pseudocount) < 1000.0) ? 1 : 0;
 }
@@ -812,6 +820,7 @@ int32_t upload(gibbs_handle *h, const uint8_t *seqs, const int64_t *offsets, int
                     (bad - 1) >= 32 && (bad - 1) < 127 ? (char)(bad - 1) : '?', bad - 1);
     h->n_masked = sym[1];
     h->has_gap = sym[2] != 0;
+    h->n_gap = sym[2];
     try {
         h->len_host.resize((size_t)n_seqs);
     } catch (...) {
@@ -1179,6 +1188,9 @@ int32_t gibbs_run_device(gibbs_handle *h, const gibbs_params *p, int32_t n_chain
             return fail(GIBBS_ERR_ARG, "a start PPM is set (gibbs_set_start_ppm) but the run uses a fixed background: the reference "
                                        "has the ...OfPPM / ...WithPPM functions in the data-derived family only (fs:644, fs:1028)");
         if (h->start_ppm_k != p->k) return fail(GIBBS_ERR_ARG, "the start PPM has %d columns, the run k = %d", h->start_ppm_k, p->k);
+        if (h->has_gap && p->alphabet_size >= 5)
+            return fail(GIBBS_ERR_UNSUPPORTED, "a start PPM has rows A,C,G,T only, and the sequences hold Gap '-', which alphabet_size = %d "
+                                               "includes: its PPM row is missing", p->alphabet_size);
         a.ppm_given = h->start_ppm.p;
     }
     const bool drift = p->background == GIBBS_BG_DATA;
@@ -1189,10 +1201,14 @@ int32_t gibbs_run_device(gibbs_handle *h, const gibbs_params *p, int32_t n_chain
         a.ss = h->ss_valid ? h->ss.p : nullptr;
         a.ss_stride = h->max_len + 2;
         memcpy(a.gcnt, h->gcnt, sizeof a.gcnt);
+        if (p->alphabet_size >= 5 && gap_row_built(p)) { // Gap has a row of its own (else it is dead like N)
+            if (h->n_gap > INT32_MAX) return fail(GIBBS_ERR_ARG, "more than 2^31 Gaps: background counts overflow int32 (the reference counts in int32, fs:34)");
+            a.gap_total = (int32_t)h->n_gap;
+        }
         a.alpha_pc = (double)p->alphabet_size * p->pseudocount; // float alphabet.Length * pseudoCount, fs:117
         a.pc = p->pseudocount;
         // gibbs_set_option(GIBBS_OPT_EXACT_SCANS): every window in float64
-        a.drift_fast_ok = h->opt_exact_scans ? 0 : drift_fast_path_ok(h->gcnt, h->max_len, h->n, p);
+        a.drift_fast_ok = h->opt_exact_scans ? 0 : drift_fast_path_ok(h->gcnt, a.gap_total, h->max_len, h->n, p);
     }
     if (p->sampler == GIBBS_MOTIF_SAMPLER) {
         Stage stages[MAX_STAGES] = {};
@@ -1805,7 +1821,7 @@ struct gibbs_batch {
     std::vector<int32_t> seq_off;               // [n_sets + 1] first sequence of each set
     std::vector<int32_t> min_len, max_len;      // per set
     std::vector<int64_t> n_masked;              // symbols outside A,C,G,T per set
-    std::vector<uint8_t> has_gap;               // per set: holds Gap '-'
+    std::vector<int64_t> n_gap;                 // per set: Gaps '-'
     std::vector<int64_t> gcnt;                  // [n_sets][4] A,C,G,T counts (the data-derived background)
     DevBuf<int32_t> d_seq_off;
     // per-set tables, keyed by the parameters they were built for
@@ -1882,9 +1898,10 @@ int32_t batch_check(const gibbs_batch *b, const gibbs_params *p, const double *b
             return fail(GIBBS_ERR_SHORT_SEQ, "set %d, sequence %d: length %d is shorter than k=%d (Array.take, fs:152)", gs,
                         i - b->seq_off[s], b->h->len_host[i], p->k);
         }
-        if (b->has_gap[s] && p->alphabet_size >= 5)
-            return fail(GIBBS_ERR_UNSUPPORTED, "set %d holds Gap '-' and alphabet_size = %d includes it: a fifth PWM row is not built "
-                                               "(pass alphabet_size = 4 to score Gap like any other non-alphabet symbol)", gs, p->alphabet_size);
+        if (b->n_gap[s] > 0 && p->alphabet_size >= 5 && (motif || !gap_row_built(p)))
+            return fail(GIBBS_ERR_UNSUPPORTED, "set %d holds Gap '-' and alphabet_size = %d includes it: its PWM row is built for the "
+                                               "SiteSampler with the data-derived background only (pass alphabet_size = 4 to score Gap "
+                                               "like any other non-alphabet symbol)", gs, p->alphabet_size);
         if (motif && p->motif_amount == 2 && b->n_masked[s] > 0)
             return fail(GIBBS_ERR_UNSUPPORTED, "set %d holds symbols outside A,C,G,T: the MotifSampler builds them for motifAmount = 1 "
                                                "(motifAmount = 2 needs ACGT-only sequences)", gs);
@@ -1894,10 +1911,15 @@ int32_t batch_check(const gibbs_batch *b, const gibbs_params *p, const double *b
                 if (!(bg[x] > 0.0)) return fail(GIBBS_ERR_ARG, "set %d: background probability bg[%d] must be > 0", gs, x);
         if (p->background == GIBBS_BG_DATA)
             for (int x = 0; x < 4; ++x)
-                if (b->gcnt[4 * (size_t)s + x] > INT32_MAX)
+                if (b->gcnt[4 * (size_t)s + x] > INT32_MAX || b->n_gap[s] > INT32_MAX)
                     return fail(GIBBS_ERR_ARG, "set %d: more than 2^31 bases of one kind: background counts overflow int32 (fs:34)", gs);
     }
     return GIBBS_OK;
+}
+
+// the Gap slot of set s's totals when Gap has a row of its own (checked against int32 in batch_check), else 0
+int32_t batch_gap_total(const gibbs_batch *b, const gibbs_params *p, int32_t s) {
+    return p->alphabet_size >= 5 && gap_row_built(p) ? (int32_t)b->n_gap[s] : 0;
 }
 
 DeviceSeqs batch_seqs(const gibbs_batch *b, int32_t s) {
@@ -1979,7 +2001,7 @@ int32_t batch_tables(gibbs_batch *b, const gibbs_params *p, const double *bg_per
             CUDA_TRY(cudaGetLastError());
             int32_t g[4];
             for (int x = 0; x < 4; ++x) g[x] = (int32_t)b->gcnt[4 * (size_t)s + x];
-            b->fast[s] = drift_fast_path_ok(g, b->max_len[s], N, p);
+            b->fast[s] = drift_fast_path_ok(g, batch_gap_total(b, p, s), b->max_len[s], N, p);
         }
         *launches += b->n_sets;
     }
@@ -2030,6 +2052,7 @@ ChainArgs batch_set_args(const gibbs_batch *b, const gibbs_params *p, int32_t s,
         a.ss = h->ss_valid ? h->ss.p + (size_t)o * (size_t)(h->max_len + 2) * 4 : nullptr;
         a.ss_stride = h->max_len + 2;
         for (int x = 0; x < 4; ++x) a.gcnt[x] = (int32_t)b->gcnt[4 * (size_t)s + x];
+        a.gap_total = batch_gap_total(b, p, s);
         a.alpha_pc = (double)p->alphabet_size * p->pseudocount; // fs:117
         a.pc = p->pseudocount;
         a.drift_fast_ok = b->fast[s];
@@ -2129,7 +2152,7 @@ int32_t batch_create(const uint8_t *seqs, const int64_t *offsets, const int32_t 
         b->min_len.assign((size_t)n_sets, INT32_MAX);
         b->max_len.assign((size_t)n_sets, 0);
         b->n_masked.assign((size_t)n_sets, 0);
-        b->has_gap.assign((size_t)n_sets, 0);
+        b->n_gap.assign((size_t)n_sets, 0);
         b->gcnt.assign((size_t)n_sets * 4, 0);
     } catch (...) {
         delete b;
@@ -2161,7 +2184,7 @@ int32_t batch_create(const uint8_t *seqs, const int64_t *offsets, const int32_t 
                 else if (c == 'T') ++b->gcnt[4 * (size_t)s + 3];
                 else if (c >= 42 && c <= 90) {
                     ++b->n_masked[s];
-                    if (c == '-') b->has_gap[s] = 1;
+                    if (c == '-') ++b->n_gap[s];
                 } else {
                     delete b;
                     return fail(GIBBS_ERR_SYMBOL, "set %d, sequence %d: symbol '%c' (0x%02x) is outside '*'..'Z', the range of the "

@@ -45,8 +45,9 @@ struct DeviceSeqs {
     int32_t uniform_len;    // > 0: every sequence has this length (saves a dependent load per random draw)
     // Symbols outside A,C,G,T (IUPAC codes, Gap, Ter: any index the reference's 49-slot tables accept but
     // whose PWM row is 0 because it is not in `alphabet`, fs:283-287). Null when the set has none, so the
-    // pure-ACGT path pays one uniform branch. mask has the geometry of `packed` with 0b11 at such bases
-    // (their 2-bit code is 0); rowflag[i] != 0 iff sequence i holds at least one.
+    // pure-ACGT path pays one uniform branch. mask has the geometry of `packed` with 0b01 at Gap '-' and 0b11 at
+    // the other such symbols (their 2-bit code is 0): bit 0 marks every symbol outside A,C,G,T, bit 1 tells Gap
+    // from the rest (read only where Gap is a member of the alphabet); rowflag[i] != 0 iff sequence i holds one.
     const uint32_t *mask;
     const int32_t *rowflag;
     // Gather copy for the random starts of sets that do not fit shared memory: wide[i][m] = the 32 bases from base 8 m of
@@ -89,6 +90,10 @@ struct ChainArgs {
     int32_t gcnt[4];
     double alpha_pc, pc;
     int32_t drift_fast_ok;    // the float32 ranking pass may be used
+    // Gaps '-' of the set when Gap is a member of the alphabet (SiteSampler, data-derived background, alphabet_size >= 5),
+    // else 0: Gap is then a dead symbol like N. Read by the MASKED instantiations only; it fills the padding before `ss`,
+    // so the layout of ChainArgs (and the code of every other instantiation) is unchanged.
+    int32_t gap_total;
     const int32_t *ss;        // [n][ss_stride][4] prefix tables of every sequence (prefix_kernel), or null
     int32_t ss_stride;        // entries (int4) per sequence: max_len + 2
     // pause / resume at sweep boundaries: once few chains are still running they are continued by a
@@ -156,6 +161,11 @@ __device__ __forceinline__ TeamSmem carve_smem(unsigned char *base, int team_war
     s.row0 = reinterpret_cast<uint32_t *>(base + TEAM_FIXED_BYTES + team_warps * WARP_TABLE_BYTES);
     return s;
 }
+
+// The MASKED instantiations (1 or 4 warps: a ring of at most 8 barriers) keep the gap row of `total` -- Gaps per column
+// over the current sites, [32] -- in the upper half of the barrier array, which their rings leave unused.
+__device__ __forceinline__ int32_t *gap_row(const TeamSmem &s) { return reinterpret_cast<int32_t *>(s.bar + MAX_RING / 2); }
+static_assert(MAX_RING / 2 * 8 >= 32 * 4, "gap row");
 
 __device__ __forceinline__ WarpTables warp_tables(const TeamSmem &s, int warp) {
     unsigned char *b = s.warp_tables + warp * WARP_TABLE_BYTES;
@@ -367,6 +377,18 @@ static __device__ __noinline__ void hist_fix(const uint32_t *__restrict__ mask, 
     while (m) {
         const int j = (__ffsll((long long)m) - 1) >> 1;
         atomicAdd(&fix[j], 1);
+        m &= ~(3ull << (2 * j));
+    }
+}
+
+// hist_fix, and the Gaps among those columns counted into gap[] (the gap row of the counts)
+static __device__ __noinline__ void hist_fix_gap(const uint32_t *__restrict__ mask, int row_words, int i, int pos, int k, int32_t *fix,
+                                                 int32_t *gap) {
+    uint64_t m = mask_kmer(mask, row_words, i, pos, k);
+    while (m) {
+        const int j = (__ffsll((long long)m) - 1) >> 1;
+        atomicAdd(&fix[j], 1);
+        if (((m >> (2 * j)) & 3u) == 1u) atomicAdd(&gap[j], 1);
         m &= ~(3ull << (2 * j));
     }
 }
@@ -614,13 +636,14 @@ __device__ __forceinline__ typename KmerCounter<KP>::Word gather_kmer_wide(const
 
 // counts over the sites of all sequences except `exclude` (sites < 0 = no site), positions shifted
 // by `mode`: the fused PFM of fs:392-396 (exclude = held-out) or the all-sites total. All T warps
-// of the team take part; ends with a team sync.
-template <int KP, int T>
+// of the team take part; ends with a team sync. GAP and gap != null: also the gap row, Gaps per column, into gap[32].
+template <int KP, int T, bool GAP = false>
 __device__ __forceinline__ void site_counts(const DeviceSeqs &s, const int32_t *sites, int exclude, int k, int mode,
-                                            int32_t *total, const uint32_t *lut, int32_t *fix, int tid) {
+                                            int32_t *total, const uint32_t *lut, int32_t *fix, int tid, int32_t *gap = nullptr) {
     constexpr int THREADS = 32 * T;
     for (int e = tid; e < MAX_COLS * 4; e += THREADS) total[e] = 0;
     if (s.mask != nullptr && tid < MAX_COLS) fix[tid] = 0;
+    if (GAP && gap != nullptr && tid < MAX_COLS) gap[tid] = 0;
     team_sync<T>();
     Hist<KP> h;
     h.clear();
@@ -635,7 +658,10 @@ __device__ __forceinline__ void site_counts(const DeviceSeqs &s, const int32_t *
                 if (site >= 0) {
                     const int pos = shifted_site(site, __ldg(s.len + i), k, mode);
                     h.add(kmer_global<KP>(s.packed + (size_t)i * s.row_words, pos), lut);
-                    if (row_masked(s, i)) hist_fix(s.mask, s.row_words, i, pos, k, fix);
+                    if (row_masked(s, i)) {
+                        if (GAP && gap != nullptr) hist_fix_gap(s.mask, s.row_words, i, pos, k, fix, gap);
+                        else hist_fix(s.mask, s.row_words, i, pos, k, fix);
+                    }
                 }
             }
         }

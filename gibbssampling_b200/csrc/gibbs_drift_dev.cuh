@@ -9,9 +9,10 @@ namespace gibbs {
 __device__ __forceinline__ int base_at(const uint32_t *row, int pos) { return (row[pos >> 4] >> ((pos & 15) * 2)) & 3; }
 
 // getBestPWMSs (fs:462-479) for the staged row. ppm = smem [k][4] float64 PPM of the leave-one-out counts.
-// f0[b] = fused background counts of the others; cn[b] = base counts of this sequence.
+// f0[b] = fused background counts of the others; cn[b] = base counts of this sequence; f0g = f0[Gap] when Gap is a
+// member of the alphabet (else 0): a row without Gap still has it in every denominator (fs:116 sums every slot).
 __device__ __forceinline__ void scan_drifting(const uint32_t *row, int W, int k, const double *ppm, const int *f0,
-                                              const int *cn, double pc, double alpha_pc, int lane, double &hv_out,
+                                              const int *cn, int f0g, double pc, double alpha_pc, int lane, double &hv_out,
                                               int &w_out) {
     const int B = (W + 31) >> 5;
     const int w_begin = min(W, lane * B), w_end = min(W, w_begin + B);
@@ -51,7 +52,7 @@ __device__ __forceinline__ void scan_drifting(const uint32_t *row, int W, int k,
         uint32_t oc = 0;
         for (int j = 0; j < k; ++j) oc += 1u << (8 * base_at(row, w_begin + j));
         for (int w = w_begin; w < w_end; ++w) {
-            int F[4], sum = 0;
+            int F[4], sum = f0g;
 #pragma unroll
             for (int b = 0; b < 4; ++b) {
                 run[b] += (int)((oc >> (8 * b)) & 255u);
@@ -138,7 +139,7 @@ __device__ __forceinline__ double drift_exact_window(const uint32_t *row, int w,
 // Returns false when the exact scan has to run instead (a lane with two windows inside the margin).
 template <int KP>
 __device__ __forceinline__ bool scan_drifting_fast(const uint32_t *row, int W, int k, const double *ppm, const float *pt,
-                                                   const int *f0, const int *cn, double pc, double alpha_pc, int lane,
+                                                   const int *f0, const int *cn, int f0g, double pc, double alpha_pc, int lane,
                                                    double &hv_out, int &w_out) {
     const int B = (W + 31) >> 5;
     const int w_begin = min(W, lane * B), w_end = min(W, w_begin + B);
@@ -175,7 +176,7 @@ __device__ __forceinline__ bool scan_drifting_fast(const uint32_t *row, int W, i
         for (int j = 0; j < k; ++j) oc += 1u << (8 * base_at(row, w_begin + j));
         for (int w = w_begin; w < w_end; ++w) {
             float bg = 0.0f;
-            int sum = 0;
+            int sum = f0g;
 #pragma unroll
             for (int b = 0; b < 4; ++b) {
                 const int ob = (int)((oc >> (8 * b)) & 255u);
@@ -220,7 +221,7 @@ __device__ __forceinline__ bool scan_drifting_fast(const uint32_t *row, int W, i
         const int src = __ffs(cand) - 1;
         cand &= cand - 1;
         const int wc = __shfl_sync(FULL, w1, src);
-        int F[4], sum = 0;
+        int F[4], sum = f0g;
 #pragma unroll
         for (int b = 0; b < 4; ++b) {
             F[b] = f0[b] + (wc + 1) * cn[b] - __shfl_sync(FULL, run1[b], src);
@@ -253,7 +254,7 @@ __device__ __forceinline__ bool scan_drifting_fast(const uint32_t *row, int W, i
 // per window and eight live registers.
 template <int KP>
 __device__ __forceinline__ bool scan_drifting_tables(const uint32_t *row, const int4 *__restrict__ ss, int W, int k, const double *ppm,
-                                                     const float *pt, const int *f0, const int *cn, double pc, double alpha_pc,
+                                                     const float *pt, const int *f0, const int *cn, int f0g, double pc, double alpha_pc,
                                                      int lane, double &hv_out, int &w_out) {
     const float ninf = __int_as_float(0xff800000);
     const float pcf = (float)pc, apcf = (float)alpha_pc, kf = (float)k;
@@ -266,7 +267,7 @@ __device__ __forceinline__ bool scan_drifting_tables(const uint32_t *row, const 
                             (b1.w - b0.w) - (a1.w - a0.w)};
         const int run[4] = {b1.x - sk.x - a1.x, b1.y - sk.y - a1.y, b1.z - sk.z - a1.z, b1.w - sk.w - a1.w};
         float bg = 0.0f;
-        int sum = 0;
+        int sum = f0g;
 #pragma unroll
         for (int b = 0; b < 4; ++b) {
             const int F = f0[b] + (w + 1) * cn[b] - run[b];
@@ -301,7 +302,7 @@ __device__ __forceinline__ bool scan_drifting_tables(const uint32_t *row, const 
         const int wc = __shfl_sync(FULL, w1, src);
         const int4 a1 = __ldg(ss + wc + 1), b1 = __ldg(ss + wc + k + 1);
         const int run[4] = {b1.x - sk.x - a1.x, b1.y - sk.y - a1.y, b1.z - sk.z - a1.z, b1.w - sk.w - a1.w};
-        int F[4], sum = 0;
+        int F[4], sum = f0g;
 #pragma unroll
         for (int b = 0; b < 4; ++b) {
             F[b] = f0[b] + (wc + 1) * cn[b] - run[b];
@@ -335,6 +336,7 @@ __device__ __forceinline__ bool scan_drifting_tables(const uint32_t *row, const 
 // denominator of createNormalizedPCVOfFCV, which sums all 49 slots (fs:116). The other sequences' dead rows were
 // dropped by fuseFrequencyVectors (fs:67-69).
 __device__ __forceinline__ int mask_at(const uint32_t *__restrict__ mrow, int pos) { return (__ldg(mrow + (pos >> 4)) >> ((pos & 15) * 2)) & 1; }
+__device__ __forceinline__ int mask2_at(const uint32_t *__restrict__ mrow, int pos) { return (__ldg(mrow + (pos >> 4)) >> ((pos & 15) * 2)) & 3; }
 
 static __device__ __noinline__ void scan_drifting_masked(const uint32_t *row, const uint32_t *__restrict__ mrow, int W, int k, const double *ppm,
                                                   const int *f0, const int *cn, int Mn, double pc, double alpha_pc, int lane,
@@ -415,6 +417,137 @@ static __device__ __noinline__ void scan_drifting_masked(const uint32_t *row, co
     w_out = hw;
 }
 
+// The same scan when Gap '-' is a member of the alphabet (a.gap_total > 0): Gap is not dead, fuseFrequencyVectors keeps
+// its row, so it holds F_w[Gap] = f0g + (w + 1) g_n - sum_{m <= w} gapocc_m like a base (f0g = the others' Gaps outside
+// their sites, g_n = the Gaps of this sequence), and a window over a Gap multiplies in P[Gap, j] / q_w[Gap] (gcol[j] =
+// P[Gap, j]). Mn counts Gaps too; the dead symbols are Mn - g_n. (A function of its own: sets whose Gap is dead keep
+// the scan above as it was.)
+static __device__ __noinline__ void scan_drifting_gapped(const uint32_t *row, const uint32_t *__restrict__ mrow, int W, int k, const double *ppm,
+                                                  const int *f0, const int *cn, int Mn, double pc, double alpha_pc, int lane,
+                                                  double &hv_out, int &w_out, const double *gcol, int f0g, int gn) {
+    const int B = (W + 31) >> 5;
+    const int w_begin = min(W, lane * B), w_end = min(W, w_begin + B);
+    const int Md = Mn - gn; // dead symbols of the sequence
+    // byte-packed occurrences of A,C,G,T in the window (masked bases excluded) + the dead count + the Gap count
+    auto add = [&](uint32_t &occ, int &om, int &og, int pos, int sign) {
+        const int m = mask2_at(mrow, pos);
+        if (m == 0) occ += (uint32_t)sign << (8 * base_at(row, pos));
+        else if (m == 1) og += sign;
+        else om += sign;
+    };
+    int blocksum[6] = {0, 0, 0, 0, 0, 0};
+    if (w_begin < w_end) {
+        uint32_t occ = 0;
+        int om = 0, og = 0;
+        for (int j = 0; j < k; ++j) add(occ, om, og, w_begin + j, 1);
+        for (int w = w_begin; w < w_end; ++w) {
+#pragma unroll
+            for (int b = 0; b < 4; ++b) blocksum[b] += (int)((occ >> (8 * b)) & 255u);
+            blocksum[4] += om;
+            blocksum[5] += og;
+            if (w + 1 < w_end) {
+                add(occ, om, og, w, -1);
+                add(occ, om, og, w + k, 1);
+            }
+        }
+    }
+    int run[6];
+#pragma unroll
+    for (int b = 0; b < 6; ++b) {
+        int v = blocksum[b];
+#pragma unroll
+        for (int o = 1; o < 32; o <<= 1) {
+            const int t = __shfl_up_sync(FULL, v, o);
+            if (lane >= o) v += t;
+        }
+        run[b] = v - blocksum[b];
+    }
+    double hv = 0.0;
+    int hw = 0;
+    if (w_begin < w_end) {
+        uint32_t oc = 0;
+        int om = 0, og = 0;
+        for (int j = 0; j < k; ++j) add(oc, om, og, w_begin + j, 1);
+        for (int w = w_begin; w < w_end; ++w) {
+            int F[4], sum = 0;
+#pragma unroll
+            for (int b = 0; b < 4; ++b) {
+                run[b] += (int)((oc >> (8 * b)) & 255u);
+                F[b] = f0[b] + (w + 1) * cn[b] - run[b];
+                sum += F[b];
+            }
+            run[4] += om;
+            run[5] += og;
+            sum += (w + 1) * Md - run[4];                                         // the dead rows (fs:116 sums every slot)
+            const int Fg = f0g + (w + 1) * gn - run[5];                             // the Gap row
+            sum += Fg;
+            if (om == 0) {                                                          // else the window scores 0
+                const double den = __dadd_rn((double)sum, alpha_pc);
+                double pcv[4];
+#pragma unroll
+                for (int b = 0; b < 4; ++b) pcv[b] = __ddiv_rn(__dadd_rn((double)F[b], pc), den);
+                double v = 1.0;
+                if (og == 0) {
+                    for (int j = 0; j < k; ++j) {
+                        const int b = base_at(row, w + j);
+                        const double q = b == 0 ? pcv[0] : b == 1 ? pcv[1] : b == 2 ? pcv[2] : pcv[3];
+                        v = __dmul_rn(v, __ddiv_rn(ppm[j * 4 + b], q));
+                    }
+                } else { // a window over Gaps (no dead symbol here: a masked column is a Gap)
+                    const double qg = __ddiv_rn(__dadd_rn((double)Fg, pc), den); // fs:119 for the Gap slot
+                    for (int j = 0; j < k; ++j) {
+                        const int b = base_at(row, w + j);
+                        const double q = b == 0 ? pcv[0] : b == 1 ? pcv[1] : b == 2 ? pcv[2] : pcv[3];
+                        double r;
+                        if (mask_at(mrow, w + j)) r = __ddiv_rn(gcol[j], qg);
+                        else r = __ddiv_rn(ppm[j * 4 + b], q);
+                        v = __dmul_rn(v, r);
+                    }
+                }
+                if (v > hv) {
+                    hv = v;
+                    hw = w;
+                }
+            }
+            if (w + 1 < w_end) {
+                add(oc, om, og, w, -1);
+                add(oc, om, og, w + k, 1);
+            }
+        }
+    }
+    warp_argmax(hv, hw);
+    hv_out = hv;
+    w_out = hw;
+}
+
+// Gap as a member of the alphabet (gap_total > 0, MASKED instantiations only; rare path, out of line): the Gap column of
+// the PPM, P[Gap, j] = pvals[C[Gap, j]] (normalizePPM, fs:255-261, like the A,C,G,T rows), into gcol when the held-out
+// row holds symbols outside A,C,G,T (mrow != null; only its exact scan reads the column). Returns x = f0[Gap] = the set's
+// Gaps - this sequence's - the Gaps of the other sites (fs:565-568, fs:67-69), y = this sequence's Gaps (from its mask
+// row). gap = the gap row of the counts (site_counts / random_loo_counts_impl); own_mk = mask k-mer of the own site (0:
+// none). Scalars only: a ChainArgs reference would make the caller copy its kernel parameters to local memory.
+static __device__ __noinline__ int2 drift_gap_tables(const int32_t *gap, uint64_t own_mk, int k, const double *__restrict__ pvals,
+                                                     int gap_total, const uint32_t *__restrict__ mrow, int row_words, double *gcol,
+                                                     int lane) {
+    int s = 0;
+    if (lane < k) { // k <= 32
+        int c = gap[lane];
+        if (((own_mk >> (2 * lane)) & 3u) == 1u) c -= 1;
+        s = c;
+        if (mrow != nullptr) gcol[lane] = __ldg(pvals + c);
+    }
+    int g = 0;
+    if (mrow != nullptr)
+        for (int i = lane; i < row_words; i += 32) { // pairs 0b01: Gap (the row is zero past its end)
+            const uint32_t x = __ldg(mrow + i);
+            g += __popc(x & ~(x >> 1) & 0x55555555u);
+        }
+    const int gn = __reduce_add_sync(FULL, g);
+    const int f0g = gap_total - gn - __reduce_add_sync(FULL, s);
+    __syncwarp();
+    return make_int2(f0g, gn);
+}
+
 // ------------------------------------------------------------------------------------------------
 // one site update with the drifting background, the pieces chain_kernel<.., DRIFT = true> calls
 // ------------------------------------------------------------------------------------------------
@@ -446,23 +579,29 @@ __device__ __forceinline__ void drift_tables(const WarpTables &W, const int32_t 
 
 // getBestPWMSs (fs:462-479) for the staged row; returns true when every window was scored in float64.
 // masked_n >= 0: the held-out sequence holds symbols outside A,C,G,T (a.s.mask != null); seq = its index (prefix tables)
+// f0g, gn: f0[Gap] and the held-out sequence's Gaps (drift_gap_tables) when Gap is a member of the alphabet, else 0;
+// the Gap column of the PPM is in W.ptab (as float64) for a masked row, which builds no pair table.
 template <int KP>
 __device__ __forceinline__ bool drift_pick(const WarpTables &W, const uint32_t *row, int Wn, int k, const ChainArgs &a, bool fast,
                                            const int (&f0)[4], const int (&cn)[4], int lane, double &p, int &w, int masked_n = -1,
-                                           int seq = -1) {
+                                           int seq = -1, int f0g = 0, int gn = 0) {
     if (masked_n >= 0) {
-        scan_drifting_masked(row, a.s.mask + (size_t)masked_n * a.s.row_words, Wn, k, W.wcol, f0, cn, __ldg(a.maskcnt + masked_n), a.pc,
-                             a.alpha_pc, lane, p, w);
+        const uint32_t *mrow = a.s.mask + (size_t)masked_n * a.s.row_words;
+        if (a.gap_total > 0)
+            scan_drifting_gapped(row, mrow, Wn, k, W.wcol, f0, cn, __ldg(a.maskcnt + masked_n), a.pc, a.alpha_pc, lane, p, w,
+                                 reinterpret_cast<const double *>(W.ptab), f0g, gn);
+        else
+            scan_drifting_masked(row, mrow, Wn, k, W.wcol, f0, cn, __ldg(a.maskcnt + masked_n), a.pc, a.alpha_pc, lane, p, w);
         return true;
     }
     bool ranked = false;
     if (fast && a.ss != nullptr && seq >= 0)
         ranked = scan_drifting_tables<KP>(row, reinterpret_cast<const int4 *>(a.ss) + (size_t)seq * a.ss_stride, Wn, k, W.wcol,
-                                          reinterpret_cast<const float *>(W.ptab), f0, cn, a.pc, a.alpha_pc, lane, p, w);
+                                          reinterpret_cast<const float *>(W.ptab), f0, cn, f0g, a.pc, a.alpha_pc, lane, p, w);
     else if (fast)
-        ranked = scan_drifting_fast<KP>(row, Wn, k, W.wcol, reinterpret_cast<const float *>(W.ptab), f0, cn, a.pc, a.alpha_pc,
+        ranked = scan_drifting_fast<KP>(row, Wn, k, W.wcol, reinterpret_cast<const float *>(W.ptab), f0, cn, f0g, a.pc, a.alpha_pc,
                                         lane, p, w);
-    if (!ranked) scan_drifting(row, Wn, k, W.wcol, f0, cn, a.pc, a.alpha_pc, lane, p, w);
+    if (!ranked) scan_drifting(row, Wn, k, W.wcol, f0, cn, f0g, a.pc, a.alpha_pc, lane, p, w);
     return !ranked;
 }
 

@@ -19,8 +19,8 @@ __device__ __forceinline__ int next_phase(int from, int mask) {
 // ------------------------------------------------------------------------------------------------
 // ASCII -> 2-bit rows + mask plane. One thread per packed word.
 // flags[0] = 1 + a byte outside '*'..'Z' (the reference's 49-slot tables cannot index it: IndexOutOfRange, fs:17-20)
-// flags[1] = number of symbols inside that range but outside A,C,G,T (mask plane 0b11, code 0)
-// flags[2] = 1 if one of them is Gap '-' (a member of the script's alphabet, fsx:368-369)
+// flags[1] = number of symbols inside that range but outside A,C,G,T (mask plane 0b11, code 0; Gap '-': 0b01)
+// flags[2] = number of them that are Gap '-' (a member of the script's alphabet, fsx:368-369)
 static __global__ void pack_kernel(const uint8_t *__restrict__ ascii, const int64_t *__restrict__ off, int n, int row_words,
                             uint32_t *__restrict__ packed, uint32_t *__restrict__ mask, int32_t *__restrict__ rowflag,
                             int32_t *__restrict__ len_out, int *flags) {
@@ -31,7 +31,7 @@ static __global__ void pack_kernel(const uint8_t *__restrict__ ascii, const int6
     const int len = (int)(off[i + 1] - o);
     if (wd == 0) len_out[i] = len;
     uint32_t v = 0, m = 0;
-    int other = 0;
+    int other = 0, gaps = 0;
     const int b0 = wd * 16;
 #pragma unroll
     for (int x = 0; x < 16; ++x) {
@@ -44,9 +44,9 @@ static __global__ void pack_kernel(const uint8_t *__restrict__ ascii, const int6
             else if (c == 'G') code = 2;
             else if (c == 'T') code = 3;
             else if (c >= 42 && c <= 90) {
-                m |= 3u << (2 * x);
+                m |= (c == '-' ? 1u : 3u) << (2 * x);
                 ++other;
-                if (c == '-') atomicExch(flags + 2, 1);
+                gaps += c == '-';
             } else {
                 atomicExch(flags, 1 + (int)c);
             }
@@ -57,6 +57,7 @@ static __global__ void pack_kernel(const uint8_t *__restrict__ ascii, const int6
     mask[t] = m;
     if (other) {
         atomicAdd(flags + 1, other);
+        if (gaps) atomicAdd(flags + 2, gaps);
         rowflag[i] = 1;
     }
 }
@@ -139,7 +140,7 @@ static __global__ void wtab_kernel(int n, double pc, double den, double q0, doub
 // WIDE = gather from the 64-bit copy (DeviceSeqs::wide) instead of the packed rows in global memory.
 template <int KP, int NB, bool MASKED, bool SROWS, bool UNI, bool PHILOX, bool WIDE = false>
 __device__ __forceinline__ void random_draw_loop(const ChainArgs &a, uint64_t chain_uid, int chain_local, int n, int32_t *counts,
-                                                 int lane, int32_t *fix, const uint32_t *base_rows) {
+                                                 int lane, int32_t *fix, const uint32_t *base_rows, int32_t *gap) {
     using Word = typename KmerCounter<KP>::Word;
     const int N = a.s.n, k = a.k;
     const int row_words = a.s.row_words;
@@ -187,7 +188,10 @@ __device__ __forceinline__ void random_draw_loop(const ChainArgs &a, uint64_t ch
                     }
                     const Word km = WIDE ? gather_kmer_wide<KP>(a.s.wide, a.s.wide_words, i, pos) : gather_kmer<KP, SROWS>(base_rows, row_words, i, pos);
                     kmer[q][x] = ok ? km : (Word)0; // code 0 in every column: counted nowhere
-                    if (MASKED && ok && __ldg(a.s.rowflag + i) != 0) hist_fix(a.s.mask, row_words, i, pos, k, fix);
+                    if (MASKED && ok && __ldg(a.s.rowflag + i) != 0) {
+                        if (gap) hist_fix_gap(a.s.mask, row_words, i, pos, k, fix, gap);
+                        else hist_fix(a.s.mask, row_words, i, pos, k, fix);
+                    }
                 }
             }
 #pragma unroll
@@ -199,12 +203,14 @@ __device__ __forceinline__ void random_draw_loop(const ChainArgs &a, uint64_t ch
     KmerCounter<KP>::finish(counts, k, lane);
 }
 
+// gap (MASKED only, may be null): the gap row of the counts, Gaps per column of the drawn sites, into gap[32]
 template <int KP, int NB, bool MASKED, bool SROWS = false>
 __device__ __forceinline__ void random_loo_counts_impl(const ChainArgs &a, uint64_t chain_uid, int chain_local, int n,
                                                        int32_t *counts, int lane, int32_t *fix,
-                                                       const uint32_t *rows = nullptr) {
+                                                       const uint32_t *rows = nullptr, int32_t *gap = nullptr) {
     const int N = a.s.n, k = a.k;
     if (MASKED) fix[lane] = 0; // fix[] = the warp's lgcol, free until build_tables
+    if (MASKED && gap) gap[lane] = 0;
     if (N < 2) {
         for (int e = lane; e < 8 * KP; e += 32) counts[e] = 0;
         __syncwarp();
@@ -214,15 +220,15 @@ __device__ __forceinline__ void random_loo_counts_impl(const ChainArgs &a, uint6
     bool done = false;
     if constexpr (!SROWS && KP <= 13) { // the 64-bit gather copy holds every k-mer of k <= 25 in one aligned word
         if (a.rng_mode == 0 && a.s.wide != nullptr && k <= 25) {
-            if (a.s.uniform_len > 0) random_draw_loop<KP, NB, MASKED, false, true, true, true>(a, chain_uid, chain_local, n, counts, lane, fix, base_rows);
-            else random_draw_loop<KP, NB, MASKED, false, false, true, true>(a, chain_uid, chain_local, n, counts, lane, fix, base_rows);
+            if (a.s.uniform_len > 0) random_draw_loop<KP, NB, MASKED, false, true, true, true>(a, chain_uid, chain_local, n, counts, lane, fix, base_rows, MASKED ? gap : nullptr);
+            else random_draw_loop<KP, NB, MASKED, false, false, true, true>(a, chain_uid, chain_local, n, counts, lane, fix, base_rows, MASKED ? gap : nullptr);
             done = true;
         }
     }
     if (done) {
-    } else if (a.rng_mode != 0) random_draw_loop<KP, 1, MASKED, SROWS, false, false>(a, chain_uid, chain_local, n, counts, lane, fix, base_rows);
-    else if (a.s.uniform_len > 0) random_draw_loop<KP, NB, MASKED, SROWS, true, true>(a, chain_uid, chain_local, n, counts, lane, fix, base_rows);
-    else random_draw_loop<KP, NB, MASKED, SROWS, false, true>(a, chain_uid, chain_local, n, counts, lane, fix, base_rows);
+    } else if (a.rng_mode != 0) random_draw_loop<KP, 1, MASKED, SROWS, false, false>(a, chain_uid, chain_local, n, counts, lane, fix, base_rows, MASKED ? gap : nullptr);
+    else if (a.s.uniform_len > 0) random_draw_loop<KP, NB, MASKED, SROWS, true, true>(a, chain_uid, chain_local, n, counts, lane, fix, base_rows, MASKED ? gap : nullptr);
+    else random_draw_loop<KP, NB, MASKED, SROWS, false, true>(a, chain_uid, chain_local, n, counts, lane, fix, base_rows, MASKED ? gap : nullptr);
     if (MASKED) {
         if (lane < k) counts[lane * 4] -= fix[lane];
         __syncwarp();

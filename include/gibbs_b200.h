@@ -17,8 +17,11 @@
  *     fs:17-20) is accepted, anything else is GIBBS_ERR_SYMBOL. A, C, G, T are the alphabet the
  *     tables are built for; any other symbol is treated as NOT in `alphabet`: its PWM row is 0
  *     (fs:283-287), a window that holds it scores 0, a site base that is one is not counted.
- *     Gap '-' with alphabet_size >= 5 (the script's dnaBases, where Gap IS an alphabet member
- *     with a PWM row of its own) and any such symbol under the MotifSampler are
+ *     Gap '-' with alphabet_size >= 5 (the script's dnaBases) IS an alphabet member with a PWM
+ *     row of its own: built for the SiteSampler with the data-derived background (its background
+ *     probability comes from the counts like a base's). Under a fixed background (gibbs_params
+ *     carries bg[4], no pcv.[Gap]), under the MotifSampler, and with a start PPM
+ *     (gibbs_set_start_ppm: rows A,C,G,T only) a set holding Gap with alphabet_size >= 5 is
  *     GIBBS_ERR_UNSUPPORTED
  *   - base order of every 4-wide table: A, C, G, T
  *   - (float*int)[] results: parallel arrays double score[n] (log2, fs:303) and int32 site[n]
@@ -230,7 +233,8 @@ int32_t gibbs_run_device(gibbs_handle *h, const gibbs_params *p, int32_t n_chain
  *   scores_out double [n_chains][n_seqs]  log2 score / PWMS per sequence
  *   sums_out   double [n_chains]          Array.sum of the scores, left to right (fs:445)
  *   best_chain_out                        first chain with the largest sum (strict >, fs:450)
- *   counts_out int32 [k][4]               PWM counts (all N sites) of the best chain
+ *   counts_out int32 [k][4]               PWM counts (all N sites) of the best chain: rows A,C,G,T
+ *                                         only, also when Gap is an alphabet member
  */
 int32_t gibbs_fetch(gibbs_handle *h, int32_t *sites_out, double *scores_out, double *sums_out,
                     int32_t *best_chain_out, int32_t *counts_out, gibbs_run_stats *stats_out);
