@@ -1,7 +1,8 @@
 """Build recipe of libgibbs_b200.so (sm_100a only, in-tree so the .so travels with the repo).
 
 The library is several translation units compiled in parallel and linked by nvcc:
-  gibbs_api.cu        the extern "C" boundary, setup / primitive / init / MotifSampler kernels
+  gibbs_api.cu        the extern "C" boundary, setup / primitive / init / MotifSampler kernels and
+                      the winner-fetch kernels (gibbs_fetch.cuh, included by no other unit)
   gibbs_motif_tu.cu   the MotifSampler kernel, one team size per unit
   gibbs_motif2_tu.cu  the MotifSampler with motifAmount = 2
   gibbs_cluster_tu.cu one chain on a thread-block cluster of 4 / 8 CTAs (the last hand-over stages), one size per unit
@@ -35,7 +36,7 @@ DEPS = [API_SOURCE, CHAIN_SOURCE, INIT_SOURCE, CLUSTER_SOURCE, MOTIF_SOURCE, MOT
     os.path.join(CSRC, f) for f in (
         "gibbs_device.cuh", "gibbs_kernels.cuh", "gibbs_motif.cuh", "gibbs_drift.cuh", "gibbs_drift_dev.cuh", "gibbs_cluster.cuh",
         "gibbs_motif2.cuh", "gibbs_batch.cuh", "gibbs_motif_batch.cuh", "gibbs_chain_body.inc", "gibbs_restart_select_body.inc",
-        "gibbs_motif_body.inc", "gibbs_motif2_body.inc",
+        "gibbs_motif_body.inc", "gibbs_motif2_body.inc", "gibbs_fetch.cuh",
     )] + [os.path.join(ROOT, "include", "gibbs_b200.h"), os.path.abspath(__file__)]
 
 # (entry point declared in gibbs_api.cu, warps per chain, masked symbols, drifting background)

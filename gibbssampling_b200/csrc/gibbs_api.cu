@@ -11,6 +11,7 @@
 #include "gibbs_drift.cuh"
 #include "gibbs_batch.cuh"
 #include "gibbs_motif_batch.cuh"
+#include "gibbs_fetch.cuh"
 
 #include <algorithm>
 #include <cmath>
@@ -209,10 +210,11 @@ struct gibbs_handle {
     DevBuf<double> sc2;                // motifAmount = 2: window products of the current held-out sequence, per chain
     int32_t run_m = 1;                 // motifAmount of the last run
     int32_t start_m = 0;               // gibbs_set_start_motif_state staged Positions lists for this many sites (0 = none)
-    bool best_valid = false;           // win_sites holds the winner of a gibbs_fetch_best on the last run
+    bool best_valid = false;           // win_sites holds the winners of a fetch_best on the last run
     int32_t run_init_path = 0;         // where the random starts of the last run ran (GIBBS_INIT_*)
-    DevBuf<int32_t> win_sites;         // gibbs_fetch_best: the winner's rows + [n] restart index
-    DevBuf<double> win_scores;         // [n] scores + [n] sum
+    DevBuf<int32_t> win_sites;         // fetch_winners: the winners' sites + [S] restart indices (+ [2 n] pair elements)
+    DevBuf<double> win_scores;         // [n] winners' scores + [S] sums
+    DevBuf<int32_t> counts;            // fetch_winners: PWM counts [m][S][k][4] of the winners' sites
     size_t smem_optin = 0;             // largest dynamic shared memory a block may opt in to
 };
 
@@ -872,6 +874,120 @@ int32_t upload_if_changed(std::vector<T> &host, std::vector<T> &cache, DevBuf<T>
     return GIBBS_OK;
 }
 
+// Waits for the copies queued on h's stream, then reports a roulette pick of the last run that lay beyond the accumulated
+// mass (MotifSampler: one error flag per set, S of them). A batch names the first such set by its number in the caller's
+// list, set_base + s; a single-set handle passes set_base = -1 and names none.
+int32_t sync_roulette(const gibbs_handle *h, int32_t S, int32_t set_base) {
+    std::vector<int32_t> err;
+    if (h->run_sampler == GIBBS_MOTIF_SAMPLER) {
+        try {
+            err.assign((size_t)S, 0);
+        } catch (...) {
+            return fail(GIBBS_ERR_NOMEM, "host allocation failed");
+        }
+        CUDA_TRY(cudaMemcpyAsync(err.data(), h->err_flag.p, (size_t)S * sizeof(int32_t), cudaMemcpyDeviceToHost, h->stream));
+    }
+    CUDA_TRY(cudaStreamSynchronize(h->stream));
+    for (int32_t s = 0; s < (int32_t)err.size(); ++s) {
+        if (!err[s]) continue;
+        if (set_base < 0) return fail(GIBBS_ERR_ROULETTE, "a roulette pick lay beyond the accumulated mass (ArgumentException, fs:753)");
+        return fail(GIBBS_ERR_ROULETTE, "set %d: a roulette pick lay beyond the accumulated mass (ArgumentException, fs:753)", set_base + s);
+    }
+    return GIBBS_OK;
+}
+
+// The winner of the promote-or-restart loop (fs:435-459) of each of the S sets of h's last run -- set s holds sequences
+// seq_off[s] .. seq_off[s + 1] - 1 of the handle; a single-set handle is S = 1, seq_off {0, n} -- and what the fetch_best
+// calls return of it. select(sites, m, motif, best_out, win_sums) launches the restart selection over the run's site
+// entries into win_sites / win_scores; counts(sites, out) the PWM counts [S][k][4] of S site arrays. Everything is queued
+// before the one synchronisation. st receives the run's device counters and extra_launches the launches made here, for
+// the caller's statistics; set_base as in sync_roulette.
+template <typename Select, typename Counts>
+int32_t fetch_winners(gibbs_handle *h, int32_t S, const int32_t *seq_off, int32_t set_base, Select select, Counts counts,
+                      int32_t *sites_out, double *scores_out, int32_t *n_out, double *sum_out, int32_t *restart_out,
+                      int32_t *counts_out, unsigned long long *st, int *extra_launches) {
+    const int32_t NT = h->n, M = h->run_m, k = h->run_k;
+    const bool motif = h->run_sampler == GIBBS_MOTIF_SAMPLER;
+    const size_t NS = (size_t)M * NT, per = (size_t)S * k * 4; // NS site entries of the winners (Positions lists for m = 2)
+    std::vector<int32_t> best, pairs, counts2; // motifAmount = 2: the Positions lists and the counts of both their elements
+    try {
+        best.resize((size_t)S);
+        if (sites_out && M == 2) pairs.resize(NS);
+        if (counts_out && M == 2) counts2.resize(per * 2);
+    } catch (...) {
+        return fail(GIBBS_ERR_NOMEM, "host allocation failed");
+    }
+    CUDA_TRY(h->win_sites.reserve(NS + S + (M == 2 ? 2 * (size_t)NT : 0)));
+    CUDA_TRY(h->win_scores.reserve((size_t)NT + S));
+    int32_t rc = select(M == 2 ? h->pos2.p : h->sites.p, M, motif ? 1 : 0, h->win_sites.p + NS, h->win_scores.p + NT);
+    if (rc) return rc;
+    *extra_launches = 1;
+    CUDA_TRY(cudaMemcpyAsync(best.data(), h->win_sites.p + NS, (size_t)S * sizeof(int32_t), cudaMemcpyDeviceToHost, h->stream));
+    if (sum_out) CUDA_TRY(cudaMemcpyAsync(sum_out, h->win_scores.p + NT, (size_t)S * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
+    if (sites_out) // (motifAmount = 2: sites_out gets the newest position of each Positions list)
+        CUDA_TRY(cudaMemcpyAsync(M == 1 ? sites_out : pairs.data(), h->win_sites.p, NS * sizeof(int32_t), cudaMemcpyDeviceToHost, h->stream));
+    if (scores_out) CUDA_TRY(cudaMemcpyAsync(scores_out, h->win_scores.p, (size_t)NT * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
+    if (counts_out) { // PWM counts of every winner's sites (all zero where the initial value survived: its sites are -1)
+        CUDA_TRY(h->counts.reserve(per * M));
+        for (int which = 0; which < M; ++which) { // motifAmount = 2: both elements of every Positions pair
+            const int32_t *src = h->win_sites.p;
+            if (M == 2) {
+                int32_t *tmp = h->win_sites.p + NS + S + (size_t)which * NT;
+                pair_element_kernel<<<(NT + 255) / 256, 256, 0, h->stream>>>(h->win_sites.p, NT, which, tmp);
+                CUDA_TRY(cudaGetLastError());
+                ++*extra_launches;
+                src = tmp;
+            }
+            rc = counts(src, h->counts.p + per * which);
+            if (rc) return rc;
+            ++*extra_launches;
+        }
+        CUDA_TRY(cudaMemcpyAsync(M == 1 ? counts_out : counts2.data(), h->counts.p, per * M * sizeof(int32_t), cudaMemcpyDeviceToHost, h->stream));
+    }
+    CUDA_TRY(cudaMemcpyAsync(st, h->stats.p, ST_NSLOTS * sizeof(unsigned long long), cudaMemcpyDeviceToHost, h->stream));
+    rc = sync_roulette(h, S, set_base);
+    if (rc) return rc;
+    h->best_valid = true;
+    if (sites_out && M == 2)
+        for (int32_t i = 0; i < NT; ++i) sites_out[i] = pairs[(size_t)2 * i];
+    if (counts_out && M == 2)
+        for (size_t e = 0; e < per; ++e) counts_out[e] = counts2[e] + counts2[per + e];
+    for (int32_t s = 0; s < S; ++s) {
+        // loop 0 [||] [|(0., 0)|] returned its initial value (quirk A.6-8); the MotifSampler's is [|{PWMS 0; Positions []}|]
+        const bool initial = best[s] < 0;
+        if (initial && sites_out) sites_out[seq_off[s]] = motif ? -1 : 0;
+        if (initial && scores_out) scores_out[seq_off[s]] = 0.0;
+        if (n_out) n_out[s] = initial ? 1 : seq_off[s + 1] - seq_off[s];
+        if (restart_out) restart_out[s] = best[s];
+    }
+    return GIBBS_OK;
+}
+
+// MotifIndex.Positions of every restart of the last run (gibbs_fetch_positions, gibbs_batch_fetch_positions); missing is
+// the message when there is no run
+int32_t fetch_positions(gibbs_handle *h, int32_t m, int32_t *positions_out, const char *missing) {
+    if (!h->run_done) return fail(GIBBS_ERR_ARG, "%s", missing);
+    if (m != h->run_m) return fail(GIBBS_ERR_ARG, "the last run had motif_amount = %d", h->run_m);
+    int32_t rc = set_device(h);
+    if (rc) return rc;
+    const size_t cells = (size_t)h->run_chains * h->n;
+    CUDA_TRY(cudaMemcpyAsync(positions_out, m == 2 ? h->pos2.p : h->sites.p, cells * m * sizeof(int32_t), cudaMemcpyDeviceToHost, h->stream));
+    CUDA_TRY(cudaStreamSynchronize(h->stream));
+    return GIBBS_OK;
+}
+
+// the winners' Positions lists of the last fetch_best (gibbs_fetch_best_positions, gibbs_batch_fetch_best_positions);
+// missing is the message when there is none
+int32_t fetch_best_positions(gibbs_handle *h, int32_t m, int32_t *positions_out, const char *missing) {
+    if (!h->run_done || !h->best_valid) return fail(GIBBS_ERR_ARG, "%s", missing);
+    if (m != h->run_m) return fail(GIBBS_ERR_ARG, "the last run had motif_amount = %d", h->run_m);
+    int32_t rc = set_device(h);
+    if (rc) return rc;
+    CUDA_TRY(cudaMemcpyAsync(positions_out, h->win_sites.p, (size_t)h->n * m * sizeof(int32_t), cudaMemcpyDeviceToHost, h->stream));
+    CUDA_TRY(cudaStreamSynchronize(h->stream));
+    return GIBBS_OK;
+}
+
 } // namespace
 
 extern "C" {
@@ -1375,26 +1491,12 @@ int32_t gibbs_set_start_motif_state(gibbs_handle *h, int32_t n_chains, int32_t m
 
 int32_t gibbs_fetch_positions(gibbs_handle *h, int32_t m, int32_t *positions_out) {
     if (!h || !positions_out) return fail(GIBBS_ERR_ARG, "null argument");
-    if (!h->run_done) return fail(GIBBS_ERR_ARG, "gibbs_fetch_positions without a preceding gibbs_run_device");
-    if (m != h->run_m) return fail(GIBBS_ERR_ARG, "the last run had motif_amount = %d", h->run_m);
-    int32_t rc = set_device(h);
-    if (rc) return rc;
-    const size_t cells = (size_t)h->run_chains * h->n;
-    const int32_t *src = m == 2 ? h->pos2.p : h->sites.p;
-    CUDA_TRY(cudaMemcpyAsync(positions_out, src, cells * m * sizeof(int32_t), cudaMemcpyDeviceToHost, h->stream));
-    CUDA_TRY(cudaStreamSynchronize(h->stream));
-    return GIBBS_OK;
+    return fetch_positions(h, m, positions_out, "gibbs_fetch_positions without a preceding gibbs_run_device");
 }
 
 int32_t gibbs_fetch_best_positions(gibbs_handle *h, int32_t m, int32_t *positions_out) {
     if (!h || !positions_out) return fail(GIBBS_ERR_ARG, "null argument");
-    if (!h->run_done || !h->best_valid) return fail(GIBBS_ERR_ARG, "gibbs_fetch_best_positions without a preceding gibbs_fetch_best");
-    if (m != h->run_m) return fail(GIBBS_ERR_ARG, "the last run had motif_amount = %d", h->run_m);
-    int32_t rc = set_device(h);
-    if (rc) return rc;
-    CUDA_TRY(cudaMemcpyAsync(positions_out, h->win_sites.p, (size_t)h->n * m * sizeof(int32_t), cudaMemcpyDeviceToHost, h->stream));
-    CUDA_TRY(cudaStreamSynchronize(h->stream));
-    return GIBBS_OK;
+    return fetch_best_positions(h, m, positions_out, "gibbs_fetch_best_positions without a preceding gibbs_fetch_best");
 }
 
 int32_t gibbs_fetch(gibbs_handle *h, int32_t *sites_out, double *scores_out, double *sums_out, int32_t *best_chain_out,
@@ -1411,11 +1513,8 @@ int32_t gibbs_fetch(gibbs_handle *h, int32_t *sites_out, double *scores_out, dou
     if (sums_out) CUDA_TRY(cudaMemcpyAsync(sums_out, h->sums.p, (size_t)h->run_chains * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
     unsigned long long st[ST_NSLOTS];
     CUDA_TRY(cudaMemcpyAsync(st, h->stats.p, sizeof st, cudaMemcpyDeviceToHost, h->stream));
-    int32_t roulette_error = 0;
-    if (h->run_sampler == GIBBS_MOTIF_SAMPLER)
-        CUDA_TRY(cudaMemcpyAsync(&roulette_error, h->err_flag.p, sizeof(int32_t), cudaMemcpyDeviceToHost, h->stream));
-    CUDA_TRY(cudaStreamSynchronize(h->stream));
-    if (roulette_error) return fail(GIBBS_ERR_ROULETTE, "a roulette pick lay beyond the accumulated mass (ArgumentException, fs:753)");
+    rc = sync_roulette(h, 1, -1);
+    if (rc) return rc;
     int extra_launches = 0;
     if (counts_out) {
         rc = launch_all_counts(h, dev_seqs(h), h->sites.p + (size_t)best * h->n, h->run_k, h->best.p + 1);
@@ -1440,78 +1539,19 @@ int32_t gibbs_fetch_best(gibbs_handle *h, int32_t repetitions, int32_t *sites_ou
     if (repetitions < 0) repetitions = 0;
     int32_t rc = set_device(h);
     if (rc) return rc;
-    const int32_t N = h->n, M = h->run_m, NS = N * M; // NS site entries per restart (Positions lists for motifAmount = 2)
-    CUDA_TRY(h->win_sites.reserve((size_t)NS + 1 + 2 * (size_t)N));
-    CUDA_TRY(h->win_scores.reserve((size_t)N + 1));
-    restart_select_kernel<<<1, 32, 0, h->stream>>>(h->sums.p, M == 2 ? h->pos2.p : h->sites.p, h->scores.p, h->run_chains, N, NS,
-                                                  repetitions, h->run_sampler == GIBBS_MOTIF_SAMPLER ? 1 : 0, h->win_sites.p + NS,
-                                                  h->win_sites.p, h->win_scores.p, h->win_scores.p + N);
-    CUDA_TRY(cudaGetLastError());
-    int extra_launches = 1;
-    // the winner is at a fixed device address: everything is queued before the one synchronisation
-    int32_t best = -1;
-    double sum = 0.0;
-    std::vector<int32_t> pairs; // motifAmount = 2: the Positions lists; sites_out gets the newest position of each
-    CUDA_TRY(cudaMemcpyAsync(&best, h->win_sites.p + NS, sizeof(int32_t), cudaMemcpyDeviceToHost, h->stream));
-    CUDA_TRY(cudaMemcpyAsync(&sum, h->win_scores.p + N, sizeof(double), cudaMemcpyDeviceToHost, h->stream));
-    if (sites_out) {
-        if (M == 1) {
-            CUDA_TRY(cudaMemcpyAsync(sites_out, h->win_sites.p, (size_t)N * sizeof(int32_t), cudaMemcpyDeviceToHost, h->stream));
-        } else {
-            try {
-                pairs.resize((size_t)NS);
-            } catch (...) {
-                return fail(GIBBS_ERR_NOMEM, "host allocation failed");
-            }
-            CUDA_TRY(cudaMemcpyAsync(pairs.data(), h->win_sites.p, (size_t)NS * sizeof(int32_t), cudaMemcpyDeviceToHost, h->stream));
-        }
-    }
-    if (scores_out) CUDA_TRY(cudaMemcpyAsync(scores_out, h->win_scores.p, (size_t)N * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
-    std::vector<int32_t> counts2;
-    if (counts_out) { // PWM counts of the winner's sites (all zero when the initial value survived)
-        if (M == 1) {
-            rc = launch_all_counts(h, dev_seqs(h), h->win_sites.p, h->run_k, h->best.p + 1);
-            if (rc) return rc;
-            ++extra_launches;
-            CUDA_TRY(cudaMemcpyAsync(counts_out, h->best.p + 1, (size_t)h->run_k * 4 * sizeof(int32_t), cudaMemcpyDeviceToHost, h->stream));
-        } else { // both elements of every Positions pair
-            try {
-                counts2.assign((size_t)h->run_k * 4 * 2, 0);
-            } catch (...) {
-                return fail(GIBBS_ERR_NOMEM, "host allocation failed");
-            }
-            for (int which = 0; which < 2; ++which) {
-                int32_t *tmp = h->win_sites.p + NS + 1 + (size_t)which * N;
-                pair_element_kernel<<<(N + 255) / 256, 256, 0, h->stream>>>(h->win_sites.p, N, which, tmp);
-                CUDA_TRY(cudaGetLastError());
-                rc = launch_all_counts(h, dev_seqs(h), tmp, h->run_k, h->best.p + 1);
-                if (rc) return rc;
-                extra_launches += 2;
-                CUDA_TRY(cudaMemcpyAsync(counts2.data() + (size_t)which * h->run_k * 4, h->best.p + 1, (size_t)h->run_k * 4 * sizeof(int32_t),
-                                         cudaMemcpyDeviceToHost, h->stream));
-            }
-        }
-    }
+    auto select = [&](const int32_t *sites, int m, int motif, int32_t *best_out, double *win_sum) -> int32_t {
+        restart_select_kernel<<<1, 32, 0, h->stream>>>(h->sums.p, sites, h->scores.p, h->run_chains, h->n, m * h->n, repetitions, motif,
+                                                      best_out, h->win_sites.p, h->win_scores.p, win_sum);
+        CUDA_TRY(cudaGetLastError());
+        return GIBBS_OK;
+    };
+    auto counts = [&](const int32_t *sites, int32_t *out) { return launch_all_counts(h, dev_seqs(h), sites, h->run_k, out); };
+    const int32_t seq_off[2] = {0, h->n};
     unsigned long long st[ST_NSLOTS];
-    CUDA_TRY(cudaMemcpyAsync(st, h->stats.p, sizeof st, cudaMemcpyDeviceToHost, h->stream));
-    int32_t roulette_error = 0;
-    if (h->run_sampler == GIBBS_MOTIF_SAMPLER)
-        CUDA_TRY(cudaMemcpyAsync(&roulette_error, h->err_flag.p, sizeof(int32_t), cudaMemcpyDeviceToHost, h->stream));
-    CUDA_TRY(cudaStreamSynchronize(h->stream));
-    if (roulette_error) return fail(GIBBS_ERR_ROULETTE, "a roulette pick lay beyond the accumulated mass (ArgumentException, fs:753)");
-    h->best_valid = true;
-    if (sites_out && M == 2)
-        for (int32_t i = 0; i < N; ++i) sites_out[i] = pairs[(size_t)2 * i];
-    if (counts_out && M == 2)
-        for (int32_t e = 0; e < h->run_k * 4; ++e) counts_out[e] = counts2[(size_t)e] + counts2[(size_t)h->run_k * 4 + e];
-    if (best < 0) { // loop 0 [||] [|(0., 0)|] returned its initial value (quirk A.6-8)
-        if (sites_out) sites_out[0] = h->run_sampler == GIBBS_MOTIF_SAMPLER ? -1 : 0;
-        if (scores_out) scores_out[0] = 0.0;
-        if (counts_out) memset(counts_out, 0, (size_t)h->run_k * 4 * sizeof(int32_t));
-    }
-    if (n_out) *n_out = best < 0 ? 1 : N;
-    if (sum_out) *sum_out = sum;
-    if (restart_out) *restart_out = best;
+    int extra_launches = 0;
+    rc = fetch_winners(h, 1, seq_off, -1, select, counts, sites_out, scores_out, n_out, sum_out, restart_out, counts_out, st,
+                       &extra_launches);
+    if (rc) return rc;
     if (stats_out) {
         float ms = 0.f;
         CUDA_TRY(cudaEventElapsedTime(&ms, h->ev0, h->ev1));
@@ -1811,7 +1851,9 @@ int32_t gibbs_measure_smem_bandwidth(int32_t device, int32_t iters, double *gbps
 // The sets are uploaded as one concatenation into an internal handle (rows with a common row_words, lengths, mask plane,
 // stream, events); every set then gets its own ChainArgs that point into it (gibbs_batch.cuh), and for the MotifSampler its
 // own Motif2Args (gibbs_motif_batch.cuh). Per-set W / drift / background window tables are built with the single-set setup
-// kernels, one small launch per set, and kept while the parameters stay the same.
+// kernels, one small launch per set, and kept while the parameters stay the same. The run state, results and scratch are
+// the internal handle's, set-major (set s at R seq_off[s], restart-major within it) with one roulette flag per set in
+// err_flag; the handle's own table caches stay unset, since the batch keeps its tables per set.
 struct gibbs_batch {
     gibbs_handle *h = nullptr;
     int32_t n_sets = 0, n_seqs = 0;
@@ -1844,17 +1886,6 @@ struct gibbs_batch {
     DevBuf<ChainArgs> d_args;
     DevBuf<Motif2Args> d_margs;
     DevBuf<int32_t> d_groups;
-    // MotifSampler scratch (per-set slices), Positions lists of motifAmount = 2, roulette error flag per set
-    DevBuf<double> cand_l, gbuf, sc;
-    DevBuf<int32_t> cand_w, pos2, err;
-    // results
-    DevBuf<int32_t> sites, win_sites;           // win_sites: [m n_seqs] winners' sites + [n_sets] restart index (+ [2 n_seqs] pair elements)
-    DevBuf<double> hv, scores, sums, win_scores; // win_scores: [n_seqs] winners' scores + [n_sets] sums
-    DevBuf<int32_t> counts;
-    DevBuf<unsigned long long> stats;
-    int32_t run_R = 0, run_k = 0, run_launches = 0, run_team = 0, run_fast = 0;
-    int32_t run_sampler = GIBBS_SITE_SAMPLER, run_m = 1; // sampler and motifAmount of the last run
-    bool run_done = false, best_valid = false;
 };
 
 namespace {
@@ -2019,13 +2050,14 @@ int32_t batch_tables(gibbs_batch *b, const gibbs_params *p, const double *bg_per
 
 // the result buffers of a run of R restarts per set, the statistics cleared
 int32_t batch_results(gibbs_batch *b, int32_t R) {
+    gibbs_handle *h = b->h;
     const size_t cells = (size_t)R * b->n_seqs;
-    CUDA_TRY(b->sites.reserve(cells));
-    CUDA_TRY(b->hv.reserve(cells));
-    CUDA_TRY(b->scores.reserve(cells));
-    CUDA_TRY(b->sums.reserve((size_t)b->n_sets * R));
-    CUDA_TRY(b->stats.reserve(ST_NSLOTS));
-    CUDA_TRY(cudaMemsetAsync(b->stats.p, 0, ST_NSLOTS * sizeof(unsigned long long), b->h->stream));
+    CUDA_TRY(h->sites.reserve(cells));
+    CUDA_TRY(h->hv.reserve(cells));
+    CUDA_TRY(h->scores.reserve(cells));
+    CUDA_TRY(h->sums.reserve((size_t)b->n_sets * R));
+    CUDA_TRY(h->stats.reserve(ST_NSLOTS));
+    CUDA_TRY(cudaMemsetAsync(h->stats.p, 0, ST_NSLOTS * sizeof(unsigned long long), h->stream));
     return GIBBS_OK;
 }
 
@@ -2040,10 +2072,10 @@ ChainArgs batch_set_args(const gibbs_batch *b, const gibbs_params *p, int32_t s,
     a.k = p->k;
     a.sampler = GIBBS_SITE_SAMPLER;
     a.n_chains = R;
-    a.sites = b->sites.p + (size_t)R * o;
-    a.hv = b->hv.p + (size_t)R * o;
-    a.scores = b->scores.p + (size_t)R * o;
-    a.sums = b->sums.p + (size_t)R * s;
+    a.sites = h->sites.p + (size_t)R * o;
+    a.hv = h->hv.p + (size_t)R * o;
+    a.scores = h->scores.p + (size_t)R * o;
+    a.sums = h->sums.p + (size_t)R * s;
     a.fast_ok = b->fast[s];
     if (drift) {
         a.pvals = b->pvals.p + (size_t)m * o;
@@ -2093,7 +2125,7 @@ int32_t batch_launch_chains(gibbs_batch *b, const ChainArgs &run, bool drift, bo
         if (n == 0) continue;
         const bool masked = g >= 2;
         const int team = (g & 1) ? 1 : 4;
-        if (!b->run_team) b->run_team = team;
+        if (!h->run_team) h->run_team = team;
         BatchTable bt;
         bt.sets = b->d_args.p;
         bt.set_ids = b->d_groups.p + at[g];
@@ -2107,26 +2139,6 @@ int32_t batch_launch_chains(gibbs_batch *b, const ChainArgs &run, bool drift, bo
         CUDA_TRY(f(r, bt, n * R, team_smem_bytes(h->row_words, team), h->stream));
         ++*launches;
     }
-    return GIBBS_OK;
-}
-
-// copies the per-set roulette error flags of a MotifSampler run into err (queued; read after the stream synchronises)
-int32_t batch_queue_errors(const gibbs_batch *b, std::vector<int32_t> &err) {
-    if (b->run_sampler != GIBBS_MOTIF_SAMPLER) return GIBBS_OK;
-    try {
-        err.assign((size_t)b->n_sets, 0);
-    } catch (...) {
-        return fail(GIBBS_ERR_NOMEM, "host allocation failed");
-    }
-    CUDA_TRY(cudaMemcpyAsync(err.data(), b->err.p, (size_t)b->n_sets * sizeof(int32_t), cudaMemcpyDeviceToHost, b->h->stream));
-    return GIBBS_OK;
-}
-
-int32_t batch_check_errors(const gibbs_batch *b, const std::vector<int32_t> &err) {
-    for (size_t s = 0; s < err.size(); ++s)
-        if (err[s])
-            return fail(GIBBS_ERR_ROULETTE, "set %d: a roulette pick lay beyond the accumulated mass (ArgumentException, fs:753)",
-                        b->set_base + (int)s);
     return GIBBS_OK;
 }
 
@@ -2241,7 +2253,7 @@ int32_t gibbs_batch_run_device(gibbs_batch *b, const gibbs_params *p, const doub
     gibbs_handle *h = b->h;
     rc = set_device(h);
     if (rc) return rc;
-    b->run_done = false;
+    h->run_done = false;
     const int32_t R = restarts_per_set, S = b->n_sets;
     const bool drift = p->background == GIBBS_BG_DATA;
     int launches = 0;
@@ -2259,7 +2271,7 @@ int32_t gibbs_batch_run_device(gibbs_batch *b, const gibbs_params *p, const doub
     run.rng_mode = GIBBS_RNG_PHILOX;
     run.seed = seed;
     run.chain_id_base = chain_id_base;
-    run.stats = b->stats.p;
+    run.stats = h->stats.p;
 
     std::vector<ChainArgs> args((size_t)S);
     int fast_all = 1;
@@ -2273,21 +2285,22 @@ int32_t gibbs_batch_run_device(gibbs_batch *b, const gibbs_params *p, const doub
     if (rc) return rc;
     rc = upload_if_changed(args, b->args_host, b->d_args, h->stream);
     if (rc) return rc;
-    b->run_team = 0;
+    h->run_team = 0;
     CUDA_TRY(cudaEventRecord(h->ev0, h->stream));
     for (int init = 1; init >= 0; --init) { // every group's random starts, then every group's sweeps
         rc = batch_launch_chains(b, run, drift, init != 0, ids, g_at, R, &launches);
         if (rc) return rc;
     }
     CUDA_TRY(cudaEventRecord(h->ev1, h->stream));
-    b->run_R = R;
-    b->run_k = p->k;
-    b->run_fast = fast_all;
-    b->run_launches = launches;
-    b->run_sampler = GIBBS_SITE_SAMPLER;
-    b->run_m = 1;
-    b->best_valid = false;
-    b->run_done = true;
+    h->run_chains = R;
+    h->run_k = p->k;
+    h->run_fast = fast_all;
+    h->run_launches = launches;
+    h->run_init_path = GIBBS_INIT_CHAIN;
+    h->run_sampler = GIBBS_SITE_SAMPLER;
+    h->run_m = 1;
+    h->best_valid = false;
+    h->run_done = true;
     return GIBBS_OK;
 }
 
@@ -2298,7 +2311,7 @@ int32_t gibbs_batch_run_motif_device(gibbs_batch *b, const gibbs_params *p, cons
     gibbs_handle *h = b->h;
     rc = set_device(h);
     if (rc) return rc;
-    b->run_done = false;
+    h->run_done = false;
     const int32_t R = restarts_per_set, S = b->n_sets, M = p->motif_amount == 2 ? 2 : 1;
     const bool drift = p->background == GIBBS_BG_DATA;
     int launches = 0;
@@ -2317,15 +2330,15 @@ int32_t gibbs_batch_run_motif_device(gibbs_batch *b, const gibbs_params *p, cons
         scr[s + 1] = scr[s] + (size_t)R * (M == 2 ? 1 : batch_team(b, s)) * W;
     }
     const size_t cells = (size_t)R * b->n_seqs;
-    CUDA_TRY(b->cand_l.reserve(scr[S]));
-    CUDA_TRY(b->cand_w.reserve(scr[S]));
-    if (drift) CUDA_TRY(b->gbuf.reserve(scr[S]));
+    CUDA_TRY(h->cand_l.reserve(scr[S]));
+    CUDA_TRY(h->cand_w.reserve(scr[S]));
+    if (drift) CUDA_TRY(h->gbuf.reserve(scr[S]));
     if (M == 2) {
-        CUDA_TRY(b->sc.reserve(scr[S]));
-        CUDA_TRY(b->pos2.reserve(cells * 2));
+        CUDA_TRY(h->sc2.reserve(scr[S]));
+        CUDA_TRY(h->pos2.reserve(cells * 2));
     }
-    CUDA_TRY(b->err.reserve((size_t)S));
-    CUDA_TRY(cudaMemsetAsync(b->err.p, 0, (size_t)S * sizeof(int32_t), h->stream));
+    CUDA_TRY(h->err_flag.reserve((size_t)S));
+    CUDA_TRY(cudaMemsetAsync(h->err_flag.p, 0, (size_t)S * sizeof(int32_t), h->stream));
 
     // per-set arguments: the ChainArgs of the random starts and, around them, the MotifSampler's own
     std::vector<ChainArgs> args((size_t)S);
@@ -2350,9 +2363,9 @@ int32_t gibbs_batch_run_motif_device(gibbs_batch *b, const gibbs_params *p, cons
             m.bg.gmax_i = b->bg_max_i.p + o;
         }
         m.bg.wstride = wstride[s];
-        m.cand_l = b->cand_l.p + scr[s];
-        m.cand_w = b->cand_w.p + scr[s];
-        m.error = b->err.p + s;
+        m.cand_l = h->cand_l.p + scr[s];
+        m.cand_w = h->cand_w.p + scr[s];
+        m.error = h->err_flag.p + s;
         m.data_bg = drift ? 1 : 0;
         m.greedy_fast_ok = b->fast[s];
         if (drift) {
@@ -2361,14 +2374,14 @@ int32_t gibbs_batch_run_motif_device(gibbs_batch *b, const gibbs_params *p, cons
             memcpy(m.gcnt, a.gcnt, sizeof m.gcnt);
             m.alpha_pc = a.alpha_pc;
             m.pc = a.pc;
-            m.gbuf = b->gbuf.p + scr[s];
+            m.gbuf = h->gbuf.p + scr[s];
         }
         m.roulette_scan_ok = h->opt_exact_scans ? 0 : 1;
         m.ascii = h->ascii.p;
         m.off = h->off.p + o;
         if (M == 2) {
-            q.pos2 = b->pos2.p + 2 * (size_t)R * o;
-            q.sc = b->sc.p + scr[s];
+            q.pos2 = h->pos2.p + 2 * (size_t)R * o;
+            q.sc = h->sc2.p + scr[s];
         }
     }
     std::vector<int32_t> ids[BATCH_GROUPS + 1];
@@ -2389,13 +2402,13 @@ int32_t gibbs_batch_run_motif_device(gibbs_batch *b, const gibbs_params *p, cons
     run.rng_mode = GIBBS_RNG_PHILOX;
     run.seed = seed;
     run.chain_id_base = chain_id_base;
-    run.stats = b->stats.p;
+    run.stats = h->stats.p;
     MotifArgs mrun{};
     mrun.c = run;
     mrun.c.phase_mask = GIBBS_PHASE_STOCHASTIC | GIBBS_PHASE_MOTIF_GREEDY;
     mrun.c.cutoff = p->cutoff;
     mrun.init_done = 1;
-    b->run_team = 0;
+    h->run_team = 0;
     CUDA_TRY(cudaEventRecord(h->ev0, h->stream));
     rc = batch_launch_chains(b, run, drift, true, ids, g_at, R, &launches);
     if (rc) return rc;
@@ -2404,15 +2417,15 @@ int32_t gibbs_batch_run_motif_device(gibbs_batch *b, const gibbs_params *p, cons
         const MotifBatchTable bt{b->d_margs.p, b->d_groups.p + g_at[BATCH_GROUPS], b->d_groups.p + g_at[BATCH_GROUPS] + n, n};
         CUDA_TRY(launch_motif2_batch(mrun, bt, n * R, team_smem_bytes(h->row_words, 1), h->stream));
         ++launches;
-        b->run_team = 1;
+        h->run_team = 1;
     } else {
-        b->run_team = 0;
+        h->run_team = 0;
         for (int g = 0; g < BATCH_GROUPS; ++g) {
             const int n = (int)ids[g].size();
             if (n == 0) continue;
             const bool masked = g >= 2;
             const int team = (g & 1) ? 1 : 4;
-            if (!b->run_team) b->run_team = team;
+            if (!h->run_team) h->run_team = team;
             const MotifBatchTable bt{b->d_margs.p, b->d_groups.p + g_at[g], b->d_groups.p + g_at[g] + n, n};
             MotifBatchLaunch f;
             rc = find_unit(MOTIF_BATCH_UNITS, "MotifSampler batch", team, masked, false, false, &f);
@@ -2422,163 +2435,82 @@ int32_t gibbs_batch_run_motif_device(gibbs_batch *b, const gibbs_params *p, cons
         }
     }
     CUDA_TRY(cudaEventRecord(h->ev1, h->stream));
-    b->run_R = R;
-    b->run_k = p->k;
-    b->run_fast = fast_all;
-    b->run_launches = launches;
-    b->run_sampler = GIBBS_MOTIF_SAMPLER;
-    b->run_m = M;
-    b->best_valid = false;
-    b->run_done = true;
+    h->run_chains = R;
+    h->run_k = p->k;
+    h->run_fast = fast_all;
+    h->run_launches = launches;
+    h->run_init_path = GIBBS_INIT_CHAIN;
+    h->run_sampler = GIBBS_MOTIF_SAMPLER;
+    h->run_m = M;
+    h->best_valid = false;
+    h->run_done = true;
     return GIBBS_OK;
 }
 
-static void batch_stats(const gibbs_batch *b, const unsigned long long *st, int extra_launches, gibbs_run_stats *out) {
+static void batch_stats(const gibbs_handle *h, const unsigned long long *st, int extra_launches, gibbs_run_stats *out) {
     float ms = 0.f;
-    if (cudaEventElapsedTime(&ms, b->h->ev0, b->h->ev1) != cudaSuccess) cudaGetLastError();
-    fill_stats(out, st, b->run_launches + extra_launches, b->run_fast, b->run_team, GIBBS_INIT_CHAIN, ms);
+    if (cudaEventElapsedTime(&ms, h->ev0, h->ev1) != cudaSuccess) cudaGetLastError();
+    fill_stats(out, st, h->run_launches + extra_launches, h->run_fast, h->run_team, h->run_init_path, ms);
 }
 
 int32_t gibbs_batch_fetch(gibbs_batch *b, int32_t *sites_out, double *scores_out, double *sums_out, gibbs_run_stats *stats_out) {
     if (!b) return fail(GIBBS_ERR_ARG, "null batch");
-    if (!b->run_done) return fail(GIBBS_ERR_ARG, "gibbs_batch_fetch without a preceding gibbs_batch_run_device");
     gibbs_handle *h = b->h;
+    if (!h->run_done) return fail(GIBBS_ERR_ARG, "gibbs_batch_fetch without a preceding gibbs_batch_run_device");
     int32_t rc = set_device(h);
     if (rc) return rc;
-    const size_t cells = (size_t)b->run_R * b->n_seqs;
-    if (sites_out) CUDA_TRY(cudaMemcpyAsync(sites_out, b->sites.p, cells * sizeof(int32_t), cudaMemcpyDeviceToHost, h->stream));
-    if (scores_out) CUDA_TRY(cudaMemcpyAsync(scores_out, b->scores.p, cells * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
+    const size_t cells = (size_t)h->run_chains * b->n_seqs;
+    if (sites_out) CUDA_TRY(cudaMemcpyAsync(sites_out, h->sites.p, cells * sizeof(int32_t), cudaMemcpyDeviceToHost, h->stream));
+    if (scores_out) CUDA_TRY(cudaMemcpyAsync(scores_out, h->scores.p, cells * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
     if (sums_out)
-        CUDA_TRY(cudaMemcpyAsync(sums_out, b->sums.p, (size_t)b->run_R * b->n_sets * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
+        CUDA_TRY(cudaMemcpyAsync(sums_out, h->sums.p, (size_t)h->run_chains * b->n_sets * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
     unsigned long long st[ST_NSLOTS];
-    CUDA_TRY(cudaMemcpyAsync(st, b->stats.p, sizeof st, cudaMemcpyDeviceToHost, h->stream));
-    std::vector<int32_t> err;
-    rc = batch_queue_errors(b, err);
+    CUDA_TRY(cudaMemcpyAsync(st, h->stats.p, sizeof st, cudaMemcpyDeviceToHost, h->stream));
+    rc = sync_roulette(h, b->n_sets, b->set_base);
     if (rc) return rc;
-    CUDA_TRY(cudaStreamSynchronize(h->stream));
-    rc = batch_check_errors(b, err);
-    if (rc) return rc;
-    if (stats_out) batch_stats(b, st, 0, stats_out);
+    if (stats_out) batch_stats(h, st, 0, stats_out);
     return GIBBS_OK;
 }
 
 int32_t gibbs_batch_fetch_best(gibbs_batch *b, int32_t repetitions, int32_t *sites_out, double *scores_out, int32_t *n_out,
                                double *sum_out, int32_t *restart_out, int32_t *counts_out, gibbs_run_stats *stats_out) {
     if (!b) return fail(GIBBS_ERR_ARG, "null batch");
-    if (!b->run_done) return fail(GIBBS_ERR_ARG, "gibbs_batch_fetch_best without a preceding gibbs_batch_run_device");
-    if (repetitions < 0) repetitions = 0;
     gibbs_handle *h = b->h;
+    if (!h->run_done) return fail(GIBBS_ERR_ARG, "gibbs_batch_fetch_best without a preceding gibbs_batch_run_device");
+    if (repetitions < 0) repetitions = 0;
     int32_t rc = set_device(h);
     if (rc) return rc;
-    const int32_t S = b->n_sets, NT = b->n_seqs, k = b->run_k, M = b->run_m;
-    const bool motif = b->run_sampler == GIBBS_MOTIF_SAMPLER;
-    const size_t NS = (size_t)M * NT; // site entries of the winners (Positions lists for motifAmount = 2)
-    CUDA_TRY(b->win_sites.reserve(NS + S + (M == 2 ? 2 * (size_t)NT : 0)));
-    CUDA_TRY(b->win_scores.reserve((size_t)NT + S));
-    if (motif)
-        restart_select_motif_batch_kernel<<<S, 32, 0, h->stream>>>(b->sums.p, M == 2 ? b->pos2.p : b->sites.p, b->scores.p, b->d_seq_off.p,
-                                                                   b->run_R, repetitions, M, b->win_sites.p + NS, b->win_sites.p,
-                                                                   b->win_scores.p, b->win_scores.p + NT);
-    else
-        restart_select_batch_kernel<<<S, 32, 0, h->stream>>>(b->sums.p, b->sites.p, b->scores.p, b->d_seq_off.p, b->run_R, repetitions,
-                                                            b->win_sites.p + NT, b->win_sites.p, b->win_scores.p, b->win_scores.p + NT);
-    CUDA_TRY(cudaGetLastError());
-    int extra_launches = 1;
-    std::vector<int32_t> best((size_t)S), pairs, counts2;
-    CUDA_TRY(cudaMemcpyAsync(best.data(), b->win_sites.p + NS, (size_t)S * sizeof(int32_t), cudaMemcpyDeviceToHost, h->stream));
-    if (sum_out) CUDA_TRY(cudaMemcpyAsync(sum_out, b->win_scores.p + NT, (size_t)S * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
-    if (sites_out) {
-        if (M == 1) {
-            CUDA_TRY(cudaMemcpyAsync(sites_out, b->win_sites.p, (size_t)NT * sizeof(int32_t), cudaMemcpyDeviceToHost, h->stream));
-        } else { // sites_out gets the newest position of each Positions list
-            try {
-                pairs.resize(NS);
-            } catch (...) {
-                return fail(GIBBS_ERR_NOMEM, "host allocation failed");
-            }
-            CUDA_TRY(cudaMemcpyAsync(pairs.data(), b->win_sites.p, NS * sizeof(int32_t), cudaMemcpyDeviceToHost, h->stream));
-        }
-    }
-    if (scores_out) CUDA_TRY(cudaMemcpyAsync(scores_out, b->win_scores.p, (size_t)NT * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
-    if (counts_out) { // PWM counts of every winner's sites (all zero where the initial value survived: its sites are -1)
-        const size_t per = (size_t)S * k * 4;
-        CUDA_TRY(b->counts.reserve(per * M));
-        for (int which = 0; which < M; ++which) { // motifAmount = 2: both elements of every Positions pair
-            const int32_t *src = b->win_sites.p;
-            if (M == 2) {
-                int32_t *tmp = b->win_sites.p + NS + S + (size_t)which * NT;
-                pair_element_kernel<<<(NT + 255) / 256, 256, 0, h->stream>>>(b->win_sites.p, NT, which, tmp);
-                CUDA_TRY(cudaGetLastError());
-                ++extra_launches;
-                src = tmp;
-            }
-            rc = with_kp(k, [&](auto kp) -> int32_t {
-                all_counts_batch_kernel<kp()><<<S, 32, 0, h->stream>>>(b->d_args.p, b->d_seq_off.p, src, k, b->counts.p + per * which);
-                CUDA_TRY(cudaGetLastError());
-                return GIBBS_OK;
-            });
-            if (rc) return rc;
-            ++extra_launches;
-        }
-        if (M == 1) {
-            CUDA_TRY(cudaMemcpyAsync(counts_out, b->counts.p, per * sizeof(int32_t), cudaMemcpyDeviceToHost, h->stream));
-        } else {
-            try {
-                counts2.resize(per * 2);
-            } catch (...) {
-                return fail(GIBBS_ERR_NOMEM, "host allocation failed");
-            }
-            CUDA_TRY(cudaMemcpyAsync(counts2.data(), b->counts.p, per * 2 * sizeof(int32_t), cudaMemcpyDeviceToHost, h->stream));
-        }
-    }
+    const int32_t S = b->n_sets, k = h->run_k;
+    auto select = [&](const int32_t *sites, int m, int motif, int32_t *best_out, double *win_sums) -> int32_t {
+        restart_select_batch_kernel<<<S, 32, 0, h->stream>>>(h->sums.p, sites, h->scores.p, b->d_seq_off.p, h->run_chains, repetitions, m,
+                                                            motif, best_out, h->win_sites.p, h->win_scores.p, win_sums);
+        CUDA_TRY(cudaGetLastError());
+        return GIBBS_OK;
+    };
+    auto counts = [&](const int32_t *sites, int32_t *out) {
+        return with_kp(k, [&](auto kp) -> int32_t {
+            all_counts_batch_kernel<kp()><<<S, 32, 0, h->stream>>>(b->d_args.p, b->d_seq_off.p, sites, k, out);
+            CUDA_TRY(cudaGetLastError());
+            return GIBBS_OK;
+        });
+    };
     unsigned long long st[ST_NSLOTS];
-    CUDA_TRY(cudaMemcpyAsync(st, b->stats.p, sizeof st, cudaMemcpyDeviceToHost, h->stream));
-    std::vector<int32_t> err;
-    rc = batch_queue_errors(b, err);
+    int extra_launches = 0;
+    rc = fetch_winners(h, S, b->seq_off.data(), b->set_base, select, counts, sites_out, scores_out, n_out, sum_out, restart_out,
+                       counts_out, st, &extra_launches);
     if (rc) return rc;
-    CUDA_TRY(cudaStreamSynchronize(h->stream));
-    rc = batch_check_errors(b, err);
-    if (rc) return rc;
-    b->best_valid = true;
-    if (sites_out && M == 2)
-        for (int32_t i = 0; i < NT; ++i) sites_out[i] = pairs[(size_t)2 * i];
-    if (counts_out && M == 2)
-        for (size_t e = 0; e < (size_t)S * k * 4; ++e) counts_out[e] = counts2[e] + counts2[(size_t)S * k * 4 + e];
-    for (int32_t s = 0; s < S; ++s) {
-        // loop 0 [||] [|(0., 0)|] returned its initial value (quirk A.6-8); the MotifSampler's is [|{PWMS 0; Positions []}|]
-        const bool initial = best[s] < 0;
-        if (initial && sites_out) sites_out[b->seq_off[s]] = motif ? -1 : 0;
-        if (initial && scores_out) scores_out[b->seq_off[s]] = 0.0;
-        if (n_out) n_out[s] = initial ? 1 : b->seq_off[s + 1] - b->seq_off[s];
-        if (restart_out) restart_out[s] = best[s];
-    }
-    if (stats_out) batch_stats(b, st, extra_launches, stats_out);
+    if (stats_out) batch_stats(h, st, extra_launches, stats_out);
     return GIBBS_OK;
 }
 
 int32_t gibbs_batch_fetch_positions(gibbs_batch *b, int32_t m, int32_t *positions_out) {
     if (!b || !positions_out) return fail(GIBBS_ERR_ARG, "null argument");
-    if (!b->run_done) return fail(GIBBS_ERR_ARG, "gibbs_batch_fetch_positions without a preceding run");
-    if (m != b->run_m) return fail(GIBBS_ERR_ARG, "the last run had motif_amount = %d", b->run_m);
-    gibbs_handle *h = b->h;
-    int32_t rc = set_device(h);
-    if (rc) return rc;
-    const size_t cells = (size_t)b->run_R * b->n_seqs;
-    CUDA_TRY(cudaMemcpyAsync(positions_out, m == 2 ? b->pos2.p : b->sites.p, cells * m * sizeof(int32_t), cudaMemcpyDeviceToHost, h->stream));
-    CUDA_TRY(cudaStreamSynchronize(h->stream));
-    return GIBBS_OK;
+    return fetch_positions(b->h, m, positions_out, "gibbs_batch_fetch_positions without a preceding run");
 }
 
 int32_t gibbs_batch_fetch_best_positions(gibbs_batch *b, int32_t m, int32_t *positions_out) {
     if (!b || !positions_out) return fail(GIBBS_ERR_ARG, "null argument");
-    if (!b->run_done || !b->best_valid) return fail(GIBBS_ERR_ARG, "gibbs_batch_fetch_best_positions without a preceding gibbs_batch_fetch_best");
-    if (m != b->run_m) return fail(GIBBS_ERR_ARG, "the last run had motif_amount = %d", b->run_m);
-    gibbs_handle *h = b->h;
-    int32_t rc = set_device(h);
-    if (rc) return rc;
-    CUDA_TRY(cudaMemcpyAsync(positions_out, b->win_sites.p, (size_t)b->n_seqs * m * sizeof(int32_t), cudaMemcpyDeviceToHost, h->stream));
-    CUDA_TRY(cudaStreamSynchronize(h->stream));
-    return GIBBS_OK;
+    return fetch_best_positions(b->h, m, positions_out, "gibbs_batch_fetch_best_positions without a preceding gibbs_batch_fetch_best");
 }
 
 /* ---- many sequence sets over several devices ----------------------------------------------------------------------- */

@@ -66,35 +66,4 @@ static __global__ void __launch_bounds__(32 * T, GIBBS_BATCH_MIN_BLOCKS(T, DRIFT
 #include "gibbs_chain_body.inc"
 }
 
-// restart_select_kernel once per set (one warp each): sums [set][R], sites / scores [set][R][N_s] at R * seq_off[set]
-static __global__ void __launch_bounds__(32) restart_select_batch_kernel(const double *all_sums, const int32_t *all_sites,
-                                                                         const double *all_scores, const int32_t *seq_off, int n_chains,
-                                                                         int reps, int32_t *best_out, int32_t *all_win_sites,
-                                                                         double *all_win_scores, double *win_sums) {
-    const int set = blockIdx.x, lane = threadIdx.x;
-    const int o = seq_off[set], N = seq_off[set + 1] - o, NS = N, motif = 0;
-    const size_t cells = (size_t)n_chains * o;
-    const double *sums = all_sums + (size_t)set * n_chains;
-    const int32_t *sites = all_sites + cells;
-    const double *scores = all_scores + cells;
-    int32_t *out = best_out + set, *win_sites = all_win_sites + o;
-    double *win_scores = all_win_scores + o, *win_sum = win_sums + set;
-#include "gibbs_restart_select_body.inc"
-}
-
-// all_counts_kernel once per set: PWM counts [set][k][4] of the winners' sites (-1 = none: all zero)
-template <int KP>
-static __global__ void __launch_bounds__(32) all_counts_batch_kernel(const ChainArgs *sets, const int32_t *seq_off, const int32_t *sites,
-                                                                     int k, int32_t *counts_out) {
-    __shared__ int32_t total[MAX_COLS * 4];
-    __shared__ uint32_t lut[16];
-    __shared__ int32_t fix[MAX_COLS];
-    const int s = blockIdx.x, lane = threadIdx.x;
-    if (lane < 16) lut[lane] = hist_lut_entry(lane);
-    __syncwarp();
-    const DeviceSeqs ds = sets[s].s;
-    site_counts<KP, 1>(ds, sites + seq_off[s], -1, k, SHIFT_NONE, total, lut, fix, lane);
-    for (int e = lane; e < k * 4; e += 32) counts_out[(size_t)s * k * 4 + e] = total[e];
-}
-
 } // namespace gibbs

@@ -728,18 +728,6 @@ static __global__ void __launch_bounds__(32) scan_kernel(const PrimArgs a, int m
     }
 }
 
-// counts of all N sites of one chain (PWM counts reported with the best chain)
-template <int KP>
-static __global__ void __launch_bounds__(32) all_counts_kernel(DeviceSeqs s, const int32_t *sites, int k, int32_t *counts_out) {
-    extern __shared__ __align__(128) unsigned char smem_raw[];
-    const int lane = threadIdx.x;
-    const TeamSmem S = carve_smem(smem_raw, 1);
-    if (lane < 16) S.lut[lane] = hist_lut_entry(lane);
-    __syncwarp();
-    site_counts<KP, 1>(s, sites, -1, k, SHIFT_NONE, S.total, S.lut, S.fix, lane);
-    for (int e = lane; e < k * 4; e += 32) counts_out[e] = S.total[e];
-}
-
 // first chain with the largest sum (strict >), the restart selection of fs:450 / fs:156-170: what the sequential
 //   best = 0; for c = 1 ..: if sums[c] > sums[best] then best = c
 // returns (a NaN sum never wins a comparison; with sums[0] = NaN nothing beats it). One CTA.
@@ -774,33 +762,6 @@ static __global__ void __launch_bounds__(256) best_chain_kernel(const double *su
         // every sum NaN or -inf: nothing is > sums[0]
         *best_out = (s0 != s0 || s_i[0] == INT32_MAX || !(s_v[0] > s0)) ? 0 : s_i[0];
     }
-}
-
-// ------------------------------------------------------------------------------------------------
-// the promote-or-restart loop of fs:435-459 (= fs:616-640, fs:665-689, fs:857-881, fs:974-998; quirk A.6-8), decided on
-// the device over the restarts of one run (chain r = restart r)
-// ------------------------------------------------------------------------------------------------
-//   loop n acc best:  n > reps -> best | acc = best -> best | sum acc > sum best -> loop (n+1) [||] (acc unless empty)
-//                     | else -> loop (n+1) (next restart) best          starting from  loop 0 [||] [|(0., 0)|]
-// Every restart costs one iteration and every promotion one more, so restart r sits in `acc` at iteration
-// r + 1 + 2 * (promotions so far). One warp walks the sums 32 restarts at a time and stops only at EVENTS: the iteration
-// cap, a sum equal to the best one (acc = best needs the arrays compared, rare) or a larger sum (promotion). A promoted
-// restart with a negative sum ends the loop (0. > sum best then burns the remaining iterations without running anything).
-// out[0] = index of the returned restart, -1 = the initial value survived (the caller returns [|(0., 0)|]);
-// the winner's rows are copied to win_sites / win_scores so that one fixed-address copy brings them to the host.
-// motif = the MotifIndex flavour of the initial value: {PWMS 0.; Positions []} (site -1) instead of (0., 0).
-// NS = site entries per restart: N, or 2 N for Positions lists of up to two sites (motifAmount = 2).
-static __global__ void __launch_bounds__(32) restart_select_kernel(const double *sums, const int32_t *sites, const double *scores,
-                                                                   int n_chains, int N, int NS, int reps, int motif, int32_t *out,
-                                                                   int32_t *win_sites, double *win_scores, double *win_sum) {
-    const int lane = threadIdx.x;
-#include "gibbs_restart_select_body.inc" // (shared with restart_select_batch_kernel, gibbs_batch.cuh)
-}
-
-// element `which` of every Positions pair: the site arrays the one-site kernels take
-static __global__ void pair_element_kernel(const int32_t *pos2, int n, int which, int32_t *out) {
-    const int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i < n) out[i] = pos2[2 * i + which];
 }
 
 // ------------------------------------------------------------------------------------------------

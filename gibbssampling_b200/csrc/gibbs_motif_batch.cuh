@@ -117,23 +117,4 @@ static __global__ void __launch_bounds__(32) motif2_batch_kernel(const MotifArgs
 #include "gibbs_motif2_body.inc"
 }
 
-// restart_select_kernel of a MotifSampler run once per set (one warp each): sums [set][R], scores [set][R][N_s] at
-// R * seq_off[set], sites [set][R][N_s][m] at m R seq_off[set] (m = 2: the Positions lists). The SiteSampler's
-// restart_select_batch_kernel stays as it is: gibbs_batch.cuh is compiled into every chain_batch_kernel unit.
-static __global__ void __launch_bounds__(32) restart_select_motif_batch_kernel(const double *all_sums, const int32_t *all_sites,
-                                                                               const double *all_scores, const int32_t *seq_off,
-                                                                               int n_chains, int reps, int m, int32_t *best_out,
-                                                                               int32_t *all_win_sites, double *all_win_scores,
-                                                                               double *win_sums) {
-    const int set = blockIdx.x, lane = threadIdx.x;
-    const int o = seq_off[set], N = seq_off[set + 1] - o, NS = m * N, motif = 1;
-    const size_t cells = (size_t)n_chains * o;
-    const double *sums = all_sums + (size_t)set * n_chains;
-    const int32_t *sites = all_sites + cells * m;
-    const double *scores = all_scores + cells;
-    int32_t *out = best_out + set, *win_sites = all_win_sites + (size_t)m * o;
-    double *win_scores = all_win_scores + o, *win_sum = win_sums + set;
-#include "gibbs_restart_select_body.inc"
-}
-
 } // namespace gibbs

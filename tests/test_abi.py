@@ -21,6 +21,13 @@ def test_library_is_built_in_tree():
     assert os.path.dirname(_build.LIB_PATH).endswith("gibbssampling_b200")
 
 
+def test_every_source_file_is_a_build_dependency():
+    """build() without force rebuilds only when a file in DEPS is newer than the library: an edit to a source missing
+    from DEPS would leave the old library in place."""
+    sources = {os.path.join(_build.CSRC, f) for f in os.listdir(_build.CSRC) if f.endswith((".cu", ".cuh", ".inc"))}
+    assert sources - set(_build.DEPS) == set()
+
+
 def test_every_declared_symbol_is_exported():
     lib = _abi.load()
     declared = _declared_symbols()

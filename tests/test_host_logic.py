@@ -145,7 +145,7 @@ def test_unbuilt_reference_entry_points_say_so():
 
 
 # ---------------------------------------------------------------------------------------------
-# the event walk of restart_select_kernel (gibbs_kernels.cuh), modelled lane by lane
+# the event walk of restart_select_kernel (gibbs_fetch.cuh), modelled lane by lane
 # ---------------------------------------------------------------------------------------------
 def _event_walk(sums, scores, sites, reps, motif=False):
     """Python model of restart_select_kernel: 32 restarts per step, stopping only at events (iteration cap, a sum equal
